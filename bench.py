@@ -6,7 +6,7 @@ Workload (BASELINE.json configs[2], the configuration the metric is quoted on):
   -> 11 windows of 216 x (1656 | 1728 | 1656), GDG per window (bpgdg_decoder, max_iter=8, multi_thread tree).
 A "step" = one pass of the whole window pipeline over one batch of `--batch` synthetic shots per GPU.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl ours|reference] [--dump-outputs DIR]
 Under torchrun (N > 1) every rank decodes its own batch (weak scaling); the only collective is the
 all-reduce of the failure counters.  Prints ONE JSON line on rank 0.
 """
@@ -333,6 +333,28 @@ def gpu_sample(swd, shots, seed):
     return swd.sample_device(shots, seed=seed)
 
 
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(dirname, out):
+    """Writes what the timed path (SlidingWindowDecoder.decode_device) returned in its last step as DIR/<name>.npy:
+    counts (flagged, failed) and window_unconverged whole, as float64; the residual syndromes and observables it leaves in
+    det / obs as float32 rows of a fixed seeded sample of the batch's shots (their indices in sampled_shots.npy), as many as
+    keep the files within DUMP_BYTES.  Same arguments, same inputs: two builds can be compared file by file."""
+    det, obs = out["residual_det"], out["residual_obs"]
+    B = det.shape[0]
+    rows = min(B, (DUMP_BYTES - (1 << 20)) // (4 * (det.shape[1] + obs.shape[1]) + 8))
+    idx = np.sort(np.random.default_rng(0).choice(B, size=rows, replace=False))
+    arrays = {"counts": out["counts"].cpu().numpy().astype(np.float64),
+              "window_unconverged": out["window_unconverged"].cpu().numpy().astype(np.float64),
+              "sampled_shots": idx.astype(np.float64),
+              "residual_det": det.cpu().numpy()[idx].astype(np.float32),
+              "residual_obs": obs.cpu().numpy()[idx].astype(np.float32)}
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), a)
+
+
 def config_block(args):
     """The workload the metric is quoted on - the same dict in the product arm and in the reference arm."""
     return {"workload": WL["name"], "shots_per_step_per_gpu": args.batch, "decoder": WL["decoder_name"], "streams": args.streams,
@@ -370,9 +392,14 @@ def run_ours(args):
             dist.barrier()
             torch.cuda.synchronize()
 
+    last_step = {}
+
     def step_resident(i):
         det = det_all[i].clone(); obs = obs_all[i].clone()
-        return swd.decode_device(det, obs)["counts"]
+        out = swd.decode_device(det, obs)
+        if i == W + K - 1:              # the last timed step: what --dump-outputs writes
+            last_step.update(out, residual_det=det, residual_obs=obs)
+        return out["counts"]
 
     def step_single_stream(i):          # kernels launched back to back on one stream: clean per-kernel event times
         det = det_all[i].clone(); obs = obs_all[i].clone()
@@ -425,6 +452,9 @@ def run_ours(args):
 
     ms_res, counts_res = timed(step_resident, False)
     ctr_timed = read_counters()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last_step)
+    last_step.clear()
     ms_e2e, counts_e2e = timed(step_e2e, False)
     ms_e2ec, counts_e2ec = timed(step_e2e_corr, False)
     assert np.array_equal(counts_e2e, counts_res) and np.array_equal(counts_e2ec, counts_res), "e2e legs disagree with the resident leg"
@@ -684,7 +714,13 @@ def main():
     ap.add_argument("--total-shots", type=int, default=0, help="strong scaling: decode ONE job of this many shots (configs[2]: 10000000), sharded over the GPUs; "
                                                             "sampling inside the clock; prints wall seconds")
     ap.add_argument("--ref-seconds", type=float, default=90.0, help="--impl reference: CPU seconds spent on warm-up + timed steps together")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32 / float64, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.total_shots):
+        ap.error("--dump-outputs writes the outputs of the timed steps of --impl ours; it does not apply to --impl reference or --total-shots")
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(3, args.warmup) if args.impl == "ours" else args.warmup
     # the contract is ONE JSON line on stdout: libraries that write to fd 1 themselves (NCCL prints its version banner
     # there) are sent to stderr, the line itself goes to the saved descriptor

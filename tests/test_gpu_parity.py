@@ -857,15 +857,14 @@ def test_streamed_bp_equals_shared_memory_bp(name, force, monkeypatch):
     """The HBM-streamed full-window BP (swd_stream.cuh: one thread per shot, shot-interleaved messages; what graphs beyond
     one SM's shared memory run) forced on windows that also fit the shared-memory kernel: corrections, flags, path metrics,
     BP decisions, iteration counts and the posterior history must be bit-identical, and equal to the reference's goldens.
-    SWD_FORCE_BIG_OSD: the same for osd_kernel's large-window layout (sort keys alias T, reduced columns / scan array in HBM)."""
+    SWD_FORCE_BIG_OSD: the same for osd_kernel's large-window layout (sort keys alias T, reduced columns / scan array in HBM);
+    a GDG decoder has no OSD stage, so there the switch must leave every output unchanged."""
     from slidingwindowdecoder_b200 import bpgdg_decoder, osd_window
     g = load_golden(name)
     cls = osd_window if "osdw" in name else bpgdg_decoder
     a = cls(g["mat"], channel_probs=g["priors"], **g["kwargs"])
     ra = a.decode_batch(g["synd"], return_pm=True)
     oa = a.last_outputs() if cls is osd_window else None
-    if force == "SWD_FORCE_BIG_OSD" and "osdw" not in name:
-        pytest.skip("OSD layout only")
     monkeypatch.setenv(force, "1")
     b = cls(g["mat"], channel_probs=g["priors"], **g["kwargs"])
     rb = b.decode_batch(g["synd"], return_pm=True)
