@@ -133,6 +133,22 @@ int  swd_decode_batch_host_packed(swd_decoder *d, const uint64_t *synd_packed, i
                                   uint64_t *corr_packed, uint8_t *converge, double *min_pm);
 int  swd_decode_batch_device_packed(swd_decoder *d, const uint64_t *d_synd_packed, int64_t B,
                                     uint64_t *d_corr_packed, uint8_t *d_converge, double *d_min_pm, void *stream);
+/* Per-shot channel priors: the four entry points above with one more argument, channel_llr [B*n] row-major (host pointer for
+ * the _host variants, device pointer for the _device variants; B rows of n LLRs, column order of the decoder's pcm).  Row b
+ * decodes syndrome b exactly as a decoder created with channel_llr = row b would (corrections, converge, min_pm and the
+ * osd_window outputs of swd_osd_last_outputs).  Allowed values are those swd_create accepts: 0.0 (erasure, p = 1/2), +inf
+ * (p = 0), negative values (p > 1/2).  NaN is undefined behaviour (the branch-path kernels mark decided variable nodes with
+ * NaN messages).  channel_llr == NULL returns SWD_ERR_INVALID.  The _host variants copy the priors one workspace chunk at a
+ * time (8 bytes per prior over PCIe: device-resident priors are the intended use); the _device variants read them on
+ * `stream`, so calls on one decoder must be stream-ordered. */
+int  swd_decode_batch_host_llr(swd_decoder *d, const uint8_t *synd, int64_t B, uint8_t *corr, uint8_t *converge, double *min_pm,
+                               const double *channel_llr);
+int  swd_decode_batch_device_llr(swd_decoder *d, const uint8_t *d_synd, int64_t B, uint8_t *d_corr, uint8_t *d_converge,
+                                 double *d_min_pm, const double *d_channel_llr, void *stream);
+int  swd_decode_batch_host_packed_llr(swd_decoder *d, const uint64_t *synd_packed, int64_t B, uint64_t *corr_packed,
+                                      uint8_t *converge, double *min_pm, const double *channel_llr);
+int  swd_decode_batch_device_packed_llr(swd_decoder *d, const uint64_t *d_synd_packed, int64_t B, uint64_t *d_corr_packed,
+                                        uint8_t *d_converge, double *d_min_pm, const double *d_channel_llr, void *stream);
 /* the two conversions on their own (device pointers), for callers that keep shot data packed (window driver, samplers) */
 int  swd_pack_bits(int device, const uint8_t *d_bytes, int64_t B, int nbits, uint64_t *d_packed, void *stream);
 int  swd_unpack_bits(int device, const uint64_t *d_packed, int64_t B, int nbits, uint8_t *d_bytes, void *stream);

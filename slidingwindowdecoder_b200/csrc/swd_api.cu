@@ -49,10 +49,12 @@ static path_fn_t pick_path_kernel(int dmax, int T) {
 }
 
 typedef void (*pre_fn_t)(GraphDev, const u8 *, long long, int, double, u8 *, u8 *, Workspace, double *, int, PreSmem, int *, double *);
+struct PreFns { pre_fn_t f, f_llr; };     // a pre-BP instantiation and its per-shot-prior twin
 struct swd_decoder {
     swd_config cfg;
     path_fn_t path_fn = nullptr;
     pre_fn_t pre_fn = nullptr;
+    pre_fn_t pre_fn_llr = nullptr; int grid1_llr = 0;     // per-shot priors (the *_llr entry points)
     int m = 0, n = 0, nnz = 0, nn = 0, max_col_deg = 0, max_row_deg = 0, es_max = 0, rank = -1;
     bool osd_only = false;
     int device = 0, num_sm = 0;
@@ -67,6 +69,7 @@ struct swd_decoder {
     PreSmem PRE{};
     // graphs whose messages exceed one SM's shared memory: HBM-streamed full-window BP (swd_stream.cuh)
     bool stream_mode = false; int Ts = 256; size_t stream_smem = 0; StreamWs sw{}; void *sw_block = nullptr; long long sw_G = 0;
+    double *sw_llrT = nullptr; long long sw_llr_G = 0;     // per-shot priors of a tile, [n][G] (allocated by the first per-shot call)
     SortSmem SS{};
     OsdSmem OS{};
     GdgDev P{};
@@ -83,6 +86,7 @@ struct swd_decoder {
     u8 *d_synd = nullptr, *d_corr = nullptr, *d_conv = nullptr; double *d_pm = nullptr; u64 *d_psynd = nullptr, *d_pcorr = nullptr;
     u8 *h_pin = nullptr; size_t h_pin_bytes = 0;
     long long stage_cap = 0;
+    double *d_llr = nullptr; long long llr_cap = 0;       // one chunk of host per-shot priors (swd_decode_batch_host*_llr)
     cudaStream_t stream = nullptr;
     // accumulated counters
     swd_counters ctr{};
@@ -375,6 +379,8 @@ extern "C" void swd_destroy(swd_decoder *d) {
     if (d->ws_block) cudaFree(d->ws_block);
     if (d->hscratch) cudaFree(d->hscratch);
     if (d->sw_block) cudaFree(d->sw_block);
+    if (d->sw_llrT) cudaFree(d->sw_llrT);
+    if (d->d_llr) cudaFree(d->d_llr);
     if (d->d_synd) cudaFree(d->d_synd);
     if (d->d_corr) cudaFree(d->d_corr);
     if (d->d_conv) cudaFree(d->d_conv);
@@ -513,31 +519,40 @@ static int setup_kernels(swd_decoder *d) {
     }
     int occ = 0, st;
     if (!d->stream_mode) {
-#define SWD_PRE_PICK(D, MT, MB) (ps ? (staged ? pre_bp_kernel<D, MT, MB, true, true> : pre_bp_kernel<D, MT, MB, true, false>) \
-                                    : (staged ? pre_bp_kernel<D, MT, MB, false, true> : pre_bp_kernel<D, MT, MB, false, false>))
-    if (ps) d->pre_fn = d->max_col_deg <= 8 ? SWD_PRE_PICK(8, 256, 2) : SWD_PRE_PICK(16, 256, 2);
-    else d->pre_fn = d->max_col_deg <= 6 ? SWD_PRE_PICK(6, 256, SWD_PRE_MINB) : (d->max_col_deg <= 8 ? SWD_PRE_PICK(8, 256, SWD_PRE_MINB) : SWD_PRE_PICK(16, 256, 2));
-    st = occupancy(d->pre_fn, d->T1, S1.total, &occ);
+#define SWD_PRE_PICK(D, MT, MB, SH) (ps ? (staged ? pre_bp_kernel<D, MT, MB, true, true, SH> : pre_bp_kernel<D, MT, MB, true, false, SH>) \
+                                        : (staged ? pre_bp_kernel<D, MT, MB, false, true, SH> : pre_bp_kernel<D, MT, MB, false, false, SH>))
+#define SWD_PRE_BOTH(D, MT, MB) PreFns{SWD_PRE_PICK(D, MT, MB, false), SWD_PRE_PICK(D, MT, MB, true)}
+    PreFns pf;
+    if (ps) pf = d->max_col_deg <= 8 ? SWD_PRE_BOTH(8, 256, 2) : SWD_PRE_BOTH(16, 256, 2);
+    else pf = d->max_col_deg <= 6 ? SWD_PRE_BOTH(6, 256, SWD_PRE_MINB) : (d->max_col_deg <= 8 ? SWD_PRE_BOTH(8, 256, SWD_PRE_MINB) : SWD_PRE_BOTH(16, 256, 2));
+    st = occupancy(pf.f, d->T1, S1.total, &occ);
     if (st) return st;
     if (!ps && d->max_col_deg <= 8 && (int)(233472 / (S1.total + 1024)) > occ && !getenv("SWD_T1")) {
         // small windows: shared memory would allow more CTAs than the 3-per-SM register budget (85) of the default instantiation -
         // take the 64-register one when it raises the number of resident warps ([[72,12,6]] windows: 4 instead of 3 CTAs of 224 threads)
-        pre_fn_t f4 = d->max_col_deg <= 6 ? SWD_PRE_PICK(6, 256, 4) : SWD_PRE_PICK(8, 256, 4);
+        PreFns f4 = d->max_col_deg <= 6 ? SWD_PRE_BOTH(6, 256, 4) : SWD_PRE_BOTH(8, 256, 4);
         int occ4 = 0;
-        if ((st = occupancy(f4, d->T1, S1.total, &occ4))) return st;
-        if (occ4 > occ) { d->pre_fn = f4; occ = occ4; }
+        if ((st = occupancy(f4.f, d->T1, S1.total, &occ4))) return st;
+        if (occ4 > occ) { pf = f4; occ = occ4; }
     }
     if (occ * d->T1 < 512 && !getenv("SWD_T1")) {
         // shared memory allows fewer than 16 warps per SM with 256-thread CTAs: use one large CTA per SM instead
         const int want = std::min(1024, std::max(256, r32up(std::max((n + 3) / 4, m))));
-        pre_fn_t big = d->max_col_deg <= 6 && !ps ? SWD_PRE_PICK(6, 1024, 1) : (d->max_col_deg <= 8 ? SWD_PRE_PICK(8, 1024, 1) : SWD_PRE_PICK(16, 1024, 1));
+        PreFns big = d->max_col_deg <= 6 && !ps ? SWD_PRE_BOTH(6, 1024, 1) : (d->max_col_deg <= 8 ? SWD_PRE_BOTH(8, 1024, 1) : SWD_PRE_BOTH(16, 1024, 1));
         int occ_big = 0;
-        if ((st = occupancy(big, want, S1.total, &occ_big))) return st;
-        if (occ_big * want > occ * d->T1) { d->pre_fn = big; d->T1 = want; occ = occ_big; }
+        if ((st = occupancy(big.f, want, S1.total, &occ_big))) return st;
+        if (occ_big * want > occ * d->T1) { pf = big; d->T1 = want; occ = occ_big; }
     }
+#undef SWD_PRE_BOTH
 #undef SWD_PRE_PICK
     if (occ < 1) { set_err("pre_bp_kernel does not fit"); return SWD_ERR_UNSUPPORTED; }
+    d->pre_fn = pf.f; d->pre_fn_llr = pf.f_llr;
     d->grid1 = d->num_sm * occ;
+    // the per-shot twin: same CTA size and shared memory; its grid never exceeds grid1 (hscratch is sized for grid1 CTAs)
+    int occ_llr = 0;
+    if ((st = occupancy(pf.f_llr, d->T1, S1.total, &occ_llr))) return st;
+    if (occ_llr < 1) { set_err("pre_bp_kernel (per-shot priors) does not fit"); return SWD_ERR_UNSUPPORTED; }
+    d->grid1_llr = d->num_sm * std::min(occ, occ_llr);
     } else d->grid1 = d->num_sm;
     // ---- K2
     SortSmem &S2 = d->SS;
@@ -580,7 +595,12 @@ static int setup_kernels(swd_decoder *d) {
         if (S2.total <= 227 * 1024) S2.key_bytes = kb; else sort_layout(S2.key_bytes);
     }
     if (S2.total > 227 * 1024) { set_err("sort/reset kernel does not fit in shared memory"); return SWD_ERR_UNSUPPORTED; }
-    if ((st = occupancy(sort_reset_kernel, d->T2, S2.total, &occ))) return st;
+    {   // the per-shot twin runs on the same grid (persistent CTAs stride over the work list)
+        int occ_llr = 0;
+        if ((st = occupancy(sort_reset_kernel<true>, d->T2, S2.total, &occ_llr))) return st;
+        if (occ_llr < 1) { set_err("sort_reset_kernel (per-shot priors) does not fit"); return SWD_ERR_UNSUPPORTED; }
+    }
+    if ((st = occupancy(sort_reset_kernel<false>, d->T2, S2.total, &occ))) return st;
     if (occ < 1) { set_err("sort_reset_kernel does not fit"); return SWD_ERR_UNSUPPORTED; }
     d->grid2 = d->num_sm * occ;
     // ---- K3
@@ -717,7 +737,8 @@ static int alloc_workspace(swd_decoder *d, long long want, cudaStream_t s) {
     if (osd && d->OS.big && !d->ow.big_scratch) {
         if (cudaMalloc(&d->ow.big_scratch, (size_t)d->grid5 * d->OS.big_stride) != cudaSuccess) { set_err("OSD scratch cudaMalloc failed"); return SWD_ERR_NOMEM; }
     }
-    if (!d->hscratch && !d->stream_mode) CK(cudaMalloc(&d->hscratch, (size_t)d->grid1 * 4 * n * sizeof(double)));
+    // four posterior rows per CTA, and a fifth for the per-shot twin's slot-ordered priors
+    if (!d->hscratch && !d->stream_mode) CK(cudaMalloc(&d->hscratch, (size_t)d->grid1 * 5 * n * sizeof(double)));
     d->cap = cap;
     return SWD_OK;
 }
@@ -733,14 +754,16 @@ static int pull_stats(swd_decoder *d, cudaStream_t s) {
 }
 
 // HBM-streamed full-window BP (graphs beyond one SM's shared memory): tiles of G = grid * Ts shots, one thread per shot
-static int stream_pre_bp(swd_decoder *d, const u8 *d_synd, long long B, u8 *d_corr, u8 *d_conv, int full_hist, int *iter_out,
+static int stream_pre_bp(swd_decoder *d, const GraphDev &g, const u8 *d_synd, long long B, u8 *d_corr, u8 *d_conv, int full_hist, int *iter_out,
                          double *lpr_out, cudaStream_t s) {
     const int Ts = d->Ts, n = d->n;
     size_t budget = (size_t)48 << 30;
     if (const char *e = getenv("SWD_STREAM_BYTES")) budget = (size_t)atoll(e);
     const size_t per_shot = (size_t)8 * (d->nnz + 4 * (size_t)n) + 4 * (size_t)((n + 31) / 32) + 4 * (size_t)((d->m + 31) / 32) + 8;
     typedef void (*sfn_t)(GraphDev, const u8 *, long long, long long, int, double, StreamWs, int, u64 *);
-    sfn_t fn = d->max_col_deg <= 6 ? pre_bp_stream_kernel<6> : (d->max_col_deg <= 8 ? pre_bp_stream_kernel<8> : pre_bp_stream_kernel<16>);
+    const bool shot_llr = g.llr_shot != nullptr;
+    sfn_t fn = shot_llr ? (d->max_col_deg <= 6 ? pre_bp_stream_kernel<6, true> : (d->max_col_deg <= 8 ? pre_bp_stream_kernel<8, true> : pre_bp_stream_kernel<16, true>))
+                        : (d->max_col_deg <= 6 ? pre_bp_stream_kernel<6> : (d->max_col_deg <= 8 ? pre_bp_stream_kernel<8> : pre_bp_stream_kernel<16>));
     int socc = 0;
     { int st = occupancy(fn, Ts, d->stream_smem, &socc); if (st) return st; }
     if (socc < 1) { set_err("pre_bp_stream_kernel does not fit"); return SWD_ERR_UNSUPPORTED; }
@@ -764,11 +787,22 @@ static int stream_pre_bp(swd_decoder *d, const u8 *d_synd, long long B, u8 *d_co
         d->sw.itdone = (int *)(b + o_it); d->sw.conv = b + o_cv; d->sw.syndw = (u32 *)(b + o_sy);
         d->sw_G = want;
     }
+    if (shot_llr && d->sw_llr_G < d->sw_G) {
+        CK(cudaStreamSynchronize(s));
+        if (d->sw_llrT) { cudaFree(d->sw_llrT); d->sw_llrT = nullptr; d->sw_llr_G = 0; }
+        if (cudaMalloc(&d->sw_llrT, (size_t)8 * n * d->sw_G) != cudaSuccess) { set_err("streamed-BP prior buffer cudaMalloc failed"); return SWD_ERR_NOMEM; }
+        d->sw_llr_G = d->sw_G;
+    }
     for (long long t0 = 0; t0 < B; t0 += d->sw_G) {
         const long long nb = std::min<long long>(d->sw_G, B - t0);
         StreamWs sw = d->sw; sw.G = (nb + Ts - 1) / Ts * Ts;
-        fn<<<(unsigned)(sw.G / Ts), Ts, d->stream_smem, s>>>(d->g, d_synd, B, t0, d->cfg.max_iter, d->cfg.ms_scaling_factor, sw, full_hist, d->ws.stats);
-        pre_bp_stream_finish_kernel<<<(unsigned)std::min<long long>((nb + 7) / 8, 8 * (long long)d->num_sm), 256, 0, s>>>(d->g, B, t0, sw, d_corr, d_conv, d->ws,
+        if (shot_llr) {
+            sw.llrT = d->sw_llrT;
+            llr_transpose_kernel<<<dim3((unsigned)((n + 31) / 32), (unsigned)((nb + 31) / 32)), 256, 0, s>>>(g.llr_shot, B, t0, n, sw.G, d->sw_llrT);
+            d->ctr.kernel_launches++;
+        }
+        fn<<<(unsigned)(sw.G / Ts), Ts, d->stream_smem, s>>>(g, d_synd, B, t0, d->cfg.max_iter, d->cfg.ms_scaling_factor, sw, full_hist, d->ws.stats);
+        pre_bp_stream_finish_kernel<<<(unsigned)std::min<long long>((nb + 7) / 8, 8 * (long long)d->num_sm), 256, 0, s>>>(g, B, t0, sw, d_corr, d_conv, d->ws,
                                                                                                               iter_out, lpr_out);
         d->ctr.kernel_launches += 2;
     }
@@ -776,23 +810,25 @@ static int stream_pre_bp(swd_decoder *d, const u8 *d_synd, long long B, u8 *d_co
     return SWD_OK;
 }
 
-// one chunk (B <= cap), everything asynchronous on `s`
+// one chunk (B <= cap), everything asynchronous on `s`.  d_llr: the chunk's per-shot priors [B][n] (device) or nullptr
 static int launch_chunk(swd_decoder *d, const u8 *d_synd, long long B, u8 *d_corr, u8 *d_conv, double *d_pm, cudaStream_t s,
-                        long long chunk_base) {
+                        long long chunk_base, const double *d_llr) {
     const swd_config &c = d->cfg;
+    GraphDev g = d->g;
+    g.llr_shot = d_llr;
     CK(cudaMemsetAsync(d->ws.counters, 0, 64 * sizeof(int), s));
-    const int g1 = (int)std::min<long long>(B, d->grid1);
+    const int g1 = (int)std::min<long long>(B, d_llr ? d->grid1_llr : d->grid1);
     const int full_hist = (c.kind == SWD_KIND_OSD_WINDOW) ? 1 : 0;
     int *iter_out = (c.kind == SWD_KIND_OSD_WINDOW) ? d->ow.bp_iter + chunk_base : nullptr;
     double *lpr_out = (c.kind == SWD_KIND_OSD_WINDOW) ? d->ow.lpr + (size_t)chunk_base * d->n * 4 : nullptr;
     if (d->stream_mode) {
         KTimer kt(d, s, SWD_K_PRE_BP);
-        int st = stream_pre_bp(d, d_synd, B, d_corr, d_conv, full_hist, iter_out, lpr_out, s);
+        int st = stream_pre_bp(d, g, d_synd, B, d_corr, d_conv, full_hist, iter_out, lpr_out, s);
         if (st) return st;
     } else {
     KTimer kt(d, s, SWD_K_PRE_BP);
-    d->pre_fn<<<g1, d->T1, d->PRE.total, s>>>(d->g, d_synd, B, c.max_iter, c.ms_scaling_factor, d_corr, d_conv, d->ws,
-                                              d->hscratch, full_hist, d->PRE, iter_out, lpr_out);
+    (d_llr ? d->pre_fn_llr : d->pre_fn)<<<g1, d->T1, d->PRE.total, s>>>(g, d_synd, B, c.max_iter, c.ms_scaling_factor, d_corr, d_conv, d->ws,
+                                                                     d->hscratch, full_hist, d->PRE, iter_out, lpr_out);
     d->ctr.kernel_launches++;
     }
     if (d_pm) {
@@ -810,7 +846,8 @@ static int launch_chunk(swd_decoder *d, const u8 *d_synd, long long B, u8 *d_cor
     const SubLayout &LsA = one_tier ? d->LsB : d->LsA;
     const PathSmem &PSA = one_tier ? d->PSB : d->PS;
     { KTimer kt(d, s, SWD_K_SORT_RESET);
-      sort_reset_kernel<<<g2, d->T2, d->SS.total, s>>>(d->g, d_synd, d->ws, d->L, lat ? d->Plat : d->P, d->SS, d_corr, capA); }
+      if (d_llr) sort_reset_kernel<true><<<g2, d->T2, d->SS.total, s>>>(g, d_synd, d->ws, d->L, lat ? d->Plat : d->P, d->SS, d_corr, capA);
+      else sort_reset_kernel<false><<<g2, d->T2, d->SS.total, s>>>(g, d_synd, d->ws, d->L, lat ? d->Plat : d->P, d->SS, d_corr, capA); }
     d->ctr.kernel_launches++;
     const size_t smem3 = (size_t)LsA.blob_bytes + PSA.total;
     const size_t smem3B = (size_t)d->LsB.blob_bytes + d->PSB.total;
@@ -822,7 +859,7 @@ static int launch_chunk(swd_decoder *d, const u8 *d_synd, long long B, u8 *d_cor
     if (c.kind == SWD_KIND_OSD_WINDOW) {
         for (int stage = 0; stage < 2; stage++) {
             KTimer kt(d, s, stage == 0 ? SWD_K_POST_BP : SWD_K_OSD);
-            int st = osd_launch(d->g, d_synd, d->ws, d->L, LsA, d->LsB, PSA, d->PSB, capA, d->grid3B, smem3B, d->P, d->OS, d->ow, d->dmax, d->T3, g3, smem3, d->T5, d->grid5,
+            int st = osd_launch(g, d_synd, d->ws, d->L, LsA, d->LsB, PSA, d->PSB, capA, d->grid3B, smem3B, d->P, d->OS, d->ow, d->dmax, d->T3, g3, smem3, d->T5, d->grid5,
                                 c.osd_method, c.osd_order, d->rank, d_corr, d_conv, d_pm, B, chunk_base, s, &d->ctr.kernel_launches,
                                 d->ow.need_osd + d->cap, stage);
             if (st) { set_err("osd launch failed"); return st; }
@@ -854,18 +891,26 @@ static int launch_chunk(swd_decoder *d, const u8 *d_synd, long long B, u8 *d_cor
     return SWD_OK;
 }
 
-extern "C" int swd_decode_batch_device(swd_decoder *d, const uint8_t *d_synd, int64_t B, uint8_t *d_corr, uint8_t *d_conv,
-                                       double *d_pm, void *stream) {
-    if (!d || B < 0 || (B > 0 && (!d_synd || !d_corr || !d_conv))) { set_err("decode: null argument"); return SWD_ERR_INVALID; }
-    if (B == 0) return SWD_OK;
-    CK(cudaSetDevice(d->device));
-    cudaStream_t s = (cudaStream_t)stream;
+// llr: per-shot priors [B][n] or nullptr; llr_host: llr is a host array, copied one workspace chunk at a time into d->d_llr
+static int decode_device_impl(swd_decoder *d, const uint8_t *d_synd, int64_t B, uint8_t *d_corr, uint8_t *d_conv, double *d_pm,
+                              cudaStream_t s, const double *llr, bool llr_host) {
     int st = alloc_workspace(d, B, s);
     if (st) return st;
     if (d->cfg.kind == SWD_KIND_OSD_WINDOW) { st = osd_reserve_outputs(&d->ow, B, d->n, s); if (st) { set_err("osd output alloc failed"); return st; } }
+    if (llr_host && d->llr_cap < d->cap) {
+        CK(cudaStreamSynchronize(s));
+        if (d->d_llr) { cudaFree(d->d_llr); d->d_llr = nullptr; d->llr_cap = 0; }
+        if (cudaMalloc(&d->d_llr, (size_t)8 * d->n * d->cap) != cudaSuccess) { set_err("prior staging cudaMalloc failed"); return SWD_ERR_NOMEM; }
+        d->llr_cap = d->cap;
+    }
     for (long long b0 = 0; b0 < B; b0 += d->cap) {
         const long long nb = std::min<long long>(d->cap, B - b0);
-        st = launch_chunk(d, d_synd + b0 * d->m, nb, d_corr + b0 * d->n, d_conv + b0, d_pm ? d_pm + b0 : nullptr, s, b0);
+        const double *cl = llr ? llr + (size_t)b0 * d->n : nullptr;
+        if (llr_host) {     // the buffer is reused chunk after chunk: stream order puts each copy after the previous chunk's kernels
+            CK(cudaMemcpyAsync(d->d_llr, cl, (size_t)8 * nb * d->n, cudaMemcpyHostToDevice, s));
+            cl = d->d_llr;
+        }
+        st = launch_chunk(d, d_synd + b0 * d->m, nb, d_corr + b0 * d->n, d_conv + b0, d_pm ? d_pm + b0 : nullptr, s, b0, cl);
         if (st) return st;
         // fold the per-chunk GDG count into the running statistics (device side, no sync)
         accumulate_count_kernel<<<1, 1, 0, s>>>(d->ws.counters, d->ws.stats);
@@ -876,20 +921,49 @@ extern "C" int swd_decode_batch_device(swd_decoder *d, const uint8_t *d_synd, in
     return SWD_OK;
 }
 
-extern "C" int swd_decode_batch_host(swd_decoder *d, const uint8_t *synd, int64_t B, uint8_t *corr, uint8_t *conv, double *pm) {
-    if (!d || B < 0 || (B > 0 && (!synd || !corr || !conv))) { set_err("decode: null argument"); return SWD_ERR_INVALID; }
+extern "C" int swd_decode_batch_device(swd_decoder *d, const uint8_t *d_synd, int64_t B, uint8_t *d_corr, uint8_t *d_conv,
+                                       double *d_pm, void *stream) {
+    if (!d || B < 0 || (B > 0 && (!d_synd || !d_corr || !d_conv))) { set_err("decode: null argument"); return SWD_ERR_INVALID; }
     if (B == 0) return SWD_OK;
+    CK(cudaSetDevice(d->device));
+    return decode_device_impl(d, d_synd, B, d_corr, d_conv, d_pm, (cudaStream_t)stream, nullptr, false);
+}
+
+extern "C" int swd_decode_batch_device_llr(swd_decoder *d, const uint8_t *d_synd, int64_t B, uint8_t *d_corr, uint8_t *d_conv,
+                                           double *d_pm, const double *d_channel_llr, void *stream) {
+    if (!d || B < 0 || !d_channel_llr || (B > 0 && (!d_synd || !d_corr || !d_conv))) { set_err("decode: null argument"); return SWD_ERR_INVALID; }
+    if (d->osd_only) { set_err("decode: not a window decoder"); return SWD_ERR_INVALID; }
+    if (B == 0) return SWD_OK;
+    CK(cudaSetDevice(d->device));
+    return decode_device_impl(d, d_synd, B, d_corr, d_conv, d_pm, (cudaStream_t)stream, d_channel_llr, false);
+}
+
+static int decode_host_impl(swd_decoder *d, const uint8_t *synd, int64_t B, uint8_t *corr, uint8_t *conv, double *pm, const double *llr) {
     CK(cudaSetDevice(d->device));
     { int st0 = ensure_stage(d, B); if (st0) return st0; }
     cudaStream_t s = d->stream;
     CK(cudaMemcpyAsync(d->d_synd, synd, (size_t)B * d->m, cudaMemcpyHostToDevice, s));
-    int st = swd_decode_batch_device(d, d->d_synd, B, d->d_corr, d->d_conv, d->d_pm, s);
+    int st = decode_device_impl(d, d->d_synd, B, d->d_corr, d->d_conv, d->d_pm, s, llr, llr != nullptr);
     if (st) return st;
     CK(cudaMemcpyAsync(corr, d->d_corr, (size_t)B * d->n, cudaMemcpyDeviceToHost, s));
     CK(cudaMemcpyAsync(conv, d->d_conv, (size_t)B, cudaMemcpyDeviceToHost, s));
     if (pm) CK(cudaMemcpyAsync(pm, d->d_pm, (size_t)B * 8, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
     return SWD_OK;
+}
+
+extern "C" int swd_decode_batch_host(swd_decoder *d, const uint8_t *synd, int64_t B, uint8_t *corr, uint8_t *conv, double *pm) {
+    if (!d || B < 0 || (B > 0 && (!synd || !corr || !conv))) { set_err("decode: null argument"); return SWD_ERR_INVALID; }
+    if (B == 0) return SWD_OK;
+    return decode_host_impl(d, synd, B, corr, conv, pm, nullptr);
+}
+
+extern "C" int swd_decode_batch_host_llr(swd_decoder *d, const uint8_t *synd, int64_t B, uint8_t *corr, uint8_t *conv, double *pm,
+                                         const double *channel_llr) {
+    if (!d || B < 0 || !channel_llr || (B > 0 && (!synd || !corr || !conv))) { set_err("decode: null argument"); return SWD_ERR_INVALID; }
+    if (d->osd_only) { set_err("decode: not a window decoder"); return SWD_ERR_INVALID; }
+    if (B == 0) return SWD_OK;
+    return decode_host_impl(d, synd, B, corr, conv, pm, channel_llr);
 }
 
 // ---- bit-packed shot I/O ------------------------------------------------------------------------------------------
@@ -931,37 +1005,58 @@ static int ensure_stage(swd_decoder *d, long long B) {
 }
 
 // packed device pointers; the byte images live in the decoder's staging buffers (calls on one decoder must be stream-ordered)
+static int decode_device_packed_impl(swd_decoder *d, const uint64_t *d_synd_packed, int64_t B, uint64_t *d_corr_packed, uint8_t *d_conv,
+                                     double *d_pm, cudaStream_t s, const double *llr, bool llr_host) {
+    CK(cudaSetDevice(d->device));
+    int st = ensure_stage(d, B);
+    if (st) return st;
+    if ((st = launch_unpack((const u64 *)d_synd_packed, B, d->m, d->d_synd, s))) return st;
+    if ((st = decode_device_impl(d, d->d_synd, B, d->d_corr, d_conv, d_pm, s, llr, llr_host))) return st;
+    d->ctr.kernel_launches += 2;
+    return launch_pack(d->d_corr, B, d->n, (u64 *)d_corr_packed, s);
+}
 extern "C" int swd_decode_batch_device_packed(swd_decoder *d, const uint64_t *d_synd_packed, int64_t B, uint64_t *d_corr_packed,
                                               uint8_t *d_conv, double *d_pm, void *stream) {
     if (!d || B < 0 || (B > 0 && (!d_synd_packed || !d_corr_packed || !d_conv))) { set_err("decode: null argument"); return SWD_ERR_INVALID; }
     if (B == 0) return SWD_OK;
-    CK(cudaSetDevice(d->device));
-    cudaStream_t s = (cudaStream_t)stream;
-    int st = ensure_stage(d, B);
-    if (st) return st;
-    if ((st = launch_unpack((const u64 *)d_synd_packed, B, d->m, d->d_synd, s))) return st;
-    if ((st = swd_decode_batch_device(d, d->d_synd, B, d->d_corr, d_conv, d_pm, s))) return st;
-    d->ctr.kernel_launches += 2;
-    return launch_pack(d->d_corr, B, d->n, (u64 *)d_corr_packed, s);
+    return decode_device_packed_impl(d, d_synd_packed, B, d_corr_packed, d_conv, d_pm, (cudaStream_t)stream, nullptr, false);
+}
+extern "C" int swd_decode_batch_device_packed_llr(swd_decoder *d, const uint64_t *d_synd_packed, int64_t B, uint64_t *d_corr_packed,
+                                                  uint8_t *d_conv, double *d_pm, const double *d_channel_llr, void *stream) {
+    if (!d || B < 0 || !d_channel_llr || (B > 0 && (!d_synd_packed || !d_corr_packed || !d_conv))) { set_err("decode: null argument"); return SWD_ERR_INVALID; }
+    if (d->osd_only) { set_err("decode: not a window decoder"); return SWD_ERR_INVALID; }
+    if (B == 0) return SWD_OK;
+    return decode_device_packed_impl(d, d_synd_packed, B, d_corr_packed, d_conv, d_pm, (cudaStream_t)stream, d_channel_llr, false);
 }
 
 // packed host pointers: 8x fewer bytes over PCIe in both directions
-extern "C" int swd_decode_batch_host_packed(swd_decoder *d, const uint64_t *synd_packed, int64_t B, uint64_t *corr_packed, uint8_t *conv,
-                                            double *pm) {
-    if (!d || B < 0 || (B > 0 && (!synd_packed || !corr_packed || !conv))) { set_err("decode: null argument"); return SWD_ERR_INVALID; }
-    if (B == 0) return SWD_OK;
+static int decode_host_packed_impl(swd_decoder *d, const uint64_t *synd_packed, int64_t B, uint64_t *corr_packed, uint8_t *conv,
+                                   double *pm, const double *llr) {
     CK(cudaSetDevice(d->device));
     int st = ensure_stage(d, B);
     if (st) return st;
     cudaStream_t s = d->stream;
     const size_t ws = (size_t)((d->m + 63) / 64) * 8, wc = (size_t)((d->n + 63) / 64) * 8;
     CK(cudaMemcpyAsync(d->d_psynd, synd_packed, (size_t)B * ws, cudaMemcpyHostToDevice, s));
-    if ((st = swd_decode_batch_device_packed(d, (const uint64_t *)d->d_psynd, B, (uint64_t *)d->d_pcorr, d->d_conv, d->d_pm, s))) return st;
+    if ((st = decode_device_packed_impl(d, (const uint64_t *)d->d_psynd, B, (uint64_t *)d->d_pcorr, d->d_conv, d->d_pm, s, llr, llr != nullptr))) return st;
     CK(cudaMemcpyAsync(corr_packed, d->d_pcorr, (size_t)B * wc, cudaMemcpyDeviceToHost, s));
     CK(cudaMemcpyAsync(conv, d->d_conv, (size_t)B, cudaMemcpyDeviceToHost, s));
     if (pm) CK(cudaMemcpyAsync(pm, d->d_pm, (size_t)B * 8, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
     return SWD_OK;
+}
+extern "C" int swd_decode_batch_host_packed(swd_decoder *d, const uint64_t *synd_packed, int64_t B, uint64_t *corr_packed, uint8_t *conv,
+                                            double *pm) {
+    if (!d || B < 0 || (B > 0 && (!synd_packed || !corr_packed || !conv))) { set_err("decode: null argument"); return SWD_ERR_INVALID; }
+    if (B == 0) return SWD_OK;
+    return decode_host_packed_impl(d, synd_packed, B, corr_packed, conv, pm, nullptr);
+}
+extern "C" int swd_decode_batch_host_packed_llr(swd_decoder *d, const uint64_t *synd_packed, int64_t B, uint64_t *corr_packed, uint8_t *conv,
+                                                double *pm, const double *channel_llr) {
+    if (!d || B < 0 || !channel_llr || (B > 0 && (!synd_packed || !corr_packed || !conv))) { set_err("decode: null argument"); return SWD_ERR_INVALID; }
+    if (d->osd_only) { set_err("decode: not a window decoder"); return SWD_ERR_INVALID; }
+    if (B == 0) return SWD_OK;
+    return decode_host_packed_impl(d, synd_packed, B, corr_packed, conv, pm, channel_llr);
 }
 
 extern "C" int swd_is_streamed(swd_decoder *d) { return d ? (d->stream_mode ? 1 : 0) : -1; }
@@ -1247,7 +1342,7 @@ static int bp4_osd_pass(swd_decoder *d, const u8 *d_synd, const double *d_keys, 
         const long long nb = std::min<long long>(d->cap, B - b0);
         CK(cudaMemsetAsync(d->ws.counters, 0, 64 * sizeof(int), s));
         bp4_osd_setup_kernel<<<(unsigned)std::min<long long>((nb * d->n + 255) / 256, 4096), 256, 0, s>>>(d->ws, d->ow.need_osd, d_keys + b0 * d->n, d_conv + b0, nb, d->n);
-        osd_kernel<<<d->grid5, d->T5, d->OS.total, s>>>(d->g, d_synd + b0 * d->m, d->ws, d->L, d->P, d->OS, d->ow, d->cfg.osd_method, d->cfg.osd_order,
+        osd_kernel<false><<<d->grid5, d->T5, d->OS.total, s>>>(d->g, d_synd + b0 * d->m, d->ws, d->L, d->P, d->OS, d->ow, d->cfg.osd_method, d->cfg.osd_order,
                                                         d->rank, d_tmp + b0 * d->n, nullptr, b0);
         d->ctr.kernel_launches += 2;
     }

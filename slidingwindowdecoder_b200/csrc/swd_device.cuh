@@ -86,6 +86,9 @@ struct GraphDev {               // static window graph (device pointers)
     const u16 *cpj;             // [nnz]  jagged-diagonal map: cpj[jb[k] + sl] = physical slot of the k-th edge of the column at
                                 //        ownership slot sl (sl < number of columns of degree > k): lane-contiguous 16-bit loads
     int jb[17];
+    // per-shot priors of the current chunk: row b = channel LLRs of chunk shot b (row-major [B][n], column order of the graph).
+    // nullptr: every shot uses `llr`.  Set per launch by the *_llr entry points; read by the SHOT instantiations only.
+    const double *llr_shot;
 };
 
 struct GdgDev {                 // parameters of the decimation tree

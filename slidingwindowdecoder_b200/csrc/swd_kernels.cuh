@@ -84,7 +84,10 @@ __device__ __forceinline__ double pre_vn_uniform_apply(double *msg, u32 *upar, c
 // STAGED = true: the per-slot records (first edge, degree) and the CSC->CSR map live in shared memory (copied once per
 // persistent CTA): the variable pass then chases vrec -> cpos -> msg through shared memory instead of
 // vord -> cp -> cpos through L1 (ncu r1g: long_scoreboard was the second largest stall of this kernel).
-template <int DMAX, int MAXT, int MINB, bool PS, bool STAGED>
+// SHOT = true: per-shot priors (g.llr_shot, row `shot`).  Iteration 1 computes its check pass instead of reading the static
+// table c2b1 (which was built to be bit-identical to that pass), and the shot's priors are gathered once into slot order
+// in a fifth row of the CTA's hscratch (stride 5 n instead of 4 n): the variable pass reads them as coalesced as llr_s.
+template <int DMAX, int MAXT, int MINB, bool PS, bool STAGED, bool SHOT = false>
 __global__ void __launch_bounds__(MAXT, MINB)
 pre_bp_kernel(GraphDev g, const u8 *__restrict__ synd, long long B, int max_iter, double alpha,
               u8 *__restrict__ dec_out, u8 *__restrict__ conv_out, Workspace ws, double *hscratch,
@@ -97,7 +100,8 @@ pre_bp_kernel(GraphDev g, const u8 *__restrict__ synd, long long B, int max_iter
     int *misc = (int *)(smem + S.off_misc);
     const int T = blockDim.x, tid = threadIdx.x;
     const int m = g.m, n = g.n;
-    double *hs = hscratch + (size_t)blockIdx.x * 4 * n;           // last four posteriors, ownership-slot order (coalesced)
+    double *hs = hscratch + (size_t)blockIdx.x * (SHOT ? 5 : 4) * n;   // last four posteriors, ownership-slot order (coalesced)
+    double *hl = hs + (size_t)4 * n;                               // SHOT: the shot's priors in ownership-slot order
     const double fpos = alpha;
     u64 edge_iters = 0;
     const u32 *vrec = g.vrec; const u16 *cpj = g.cpj; const u32 *prow = g.prow;
@@ -113,7 +117,7 @@ pre_bp_kernel(GraphDev g, const u8 *__restrict__ synd, long long B, int max_iter
 
     for (long long shot = blockIdx.x; shot < B; shot += gridDim.x) {
         for (int r = tid; r < m; r += T) s_synd[r] = synd[shot * m + r];
-        const bool table1 = !PS && g.c2b1 != nullptr;        // iteration 1's check pass comes from the static table
+        const bool table1 = !PS && !SHOT && g.c2b1 != nullptr;        // iteration 1's check pass comes from the static table
         if (table1) {
             __syncthreads();
             for (int r = tid; r < m; r += T) upar[r] = 0;
@@ -124,7 +128,9 @@ pre_bp_kernel(GraphDev g, const u8 *__restrict__ synd, long long B, int max_iter
         for (int sl = tid; sl < n; sl += T) {                  // pyx:55-60
             const u32 vr = vrec[sl];
             const int d = (int)(vr >> 16);
-            const double l = g.llr_s[sl];
+            double l;
+            if (SHOT) { l = g.llr_shot[(size_t)shot * n + g.vord[sl]]; hl[sl] = l; }      // read back by this thread only
+            else l = g.llr_s[sl];
 #pragma unroll 1
             for (int k = 0; k < d; k++) msg[cpj[g.jb[k] + sl]] = l;
             s_dec[sl] = 0;
@@ -224,7 +230,7 @@ pre_bp_kernel(GraphDev g, const u8 *__restrict__ synd, long long B, int max_iter
                 const bool uni = SWD_PRE_UNIFORM && dw >= 1 && dw <= 6 && __all_sync(FULLMASK, d == dw);     // implies sl < n in every lane
                 if (uni) {
                     double t;
-                    const double pr = g.llr_s[sl];
+                    const double pr = SHOT ? hl[sl] : g.llr_s[sl];
                     switch (dw) {
                         case 1: t = pre_vn_uniform_apply<1>(msg, upar, cpj + sl, g.jb, g.cr, pr, e0, s_dec + sl); break;
                         case 2: t = pre_vn_uniform_apply<2>(msg, upar, cpj + sl, g.jb, g.cr, pr, e0, s_dec + sl); break;
@@ -236,7 +242,7 @@ pre_bp_kernel(GraphDev g, const u8 *__restrict__ synd, long long B, int max_iter
                     if (keep) hs_it[sl] = t;
                 } else
                 if (sl < n) {
-                    const double t = pre_vn_update<DMAX>(msg, upar, cpj + sl, g.jb, g.cr, g.llr_s[sl], e0, d, dw, s_dec + sl);
+                    const double t = pre_vn_update<DMAX>(msg, upar, cpj + sl, g.jb, g.cr, SHOT ? hl[sl] : g.llr_s[sl], e0, d, dw, s_dec + sl);
                     if (keep) hs_it[sl] = t;
                 }
             }
@@ -291,6 +297,8 @@ struct SortSmem { int off_key, off_idx, off_posof, off_blob, off_u32a, off_u32b,
                   int big;            // n beyond the register sort: block_select_sort_big only (key / idx hold cap_sel entries)
                   int key_bytes; };
 
+// SHOT = true: the kept columns' priors come from the shot's row of g.llr_shot
+template <bool SHOT = false>
 __global__ void __launch_bounds__(1024, 1)
 sort_reset_kernel(GraphDev g, const u8 *__restrict__ synd, Workspace ws, SubLayout L, GdgDev P, SortSmem S,
                   u8 *__restrict__ dec_out, int capA) {
@@ -349,7 +357,7 @@ sort_reset_kernel(GraphDev g, const u8 *__restrict__ synd, Workspace ws, SubLayo
         for (int j = tid; j < (partial ? nn : n); j += T) posof[idx[j]] = (u16)j;
         for (int j = tid; j < nn; j += T) {
             const int c = idx[j];
-            col[j] = (u16)c; prior[j] = g.llr[c];
+            col[j] = (u16)c; prior[j] = SHOT ? g.llr_shot[(size_t)shot * n + c] : g.llr[c];
             ua[j] = (u32)(g.cp[c + 1] - g.cp[c]);
             vn_mask[j] = -1; s_error[j] = 0;
         }

@@ -190,6 +190,8 @@ post_bp_kernel(Workspace ws, SubLayout LG, SubLayout L, PathSmem S, GdgDev P, in
 // ----------------------------------------------------------------------------------------------
 // OSD: one CTA per shot that needs it
 // ----------------------------------------------------------------------------------------------
+// SHOT = true: path metrics from the shot's row of g.llr_shot
+template <bool SHOT = false>
 __global__ void __launch_bounds__(1024, 1)
 osd_kernel(GraphDev g, const u8 *__restrict__ synd, Workspace ws, SubLayout L, GdgDev P, OsdSmem S, OsdWork ow,
            int method, int order_w, int rank, u8 *__restrict__ dec_out, double *__restrict__ pm_out, long long chunk_base) {
@@ -416,7 +418,7 @@ osd_kernel(GraphDev g, const u8 *__restrict__ synd, Workspace ws, SubLayout L, G
                     if (emask) { u32 e2 = emask; while (e2) { const int t = __ffs(e2) - 1; e2 &= e2 - 1; y ^= vt[t * W64 + w]; } }
                     on = (y >> (info & 63)) & 1ull;
                 }
-                if (on) pm += g.llr[cI];
+                if (on) pm += SHOT ? g.llr_shot[(size_t)shot * n + cI] : g.llr[cI];
             }
             if (cand == 0) pm0 = pm;
             else if (pm < best) { best = pm; besti = (int)cand; }       // candidates visited in ascending id per thread
@@ -486,7 +488,8 @@ __global__ void osd_finish_kernel(Workspace ws, SubLayout L, GdgDev P, OsdWork o
 }
 
 // min_pm of BP-converged shots: ordered fp64 sum over ascending column (osd_window.pyx:168-170,190-191);
-// also mirrors bp_decoding for shots that never left the BP stages.  One warp per shot.
+// also mirrors bp_decoding for shots that never left the BP stages.  One warp per shot.  SHOT = true: llr is [B][n], row b.
+template <bool SHOT = false>
 __global__ void osd_pm_kernel(const double *__restrict__ llr, int n, const u8 *__restrict__ dec, const u8 *__restrict__ conv,
                               long long B, double *__restrict__ pm_out, OsdWork ow, long long chunk_base, const u8 *__restrict__ in_list) {
     const int lane = threadIdx.x & 31, wpb = blockDim.x >> 5;
@@ -499,7 +502,8 @@ __global__ void osd_pm_kernel(const double *__restrict__ llr, int n, const u8 *_
             const u8 bit = (v < n) ? row[v] : 0;
             if (!in_list[b] && v < n) ow.bp_dec[(size_t)(chunk_base + b) * n + v] = bit;
             u32 bm = __ballot_sync(FULLMASK, bit != 0);
-            if (cv) while (bm) { const int kk = __ffs(bm) - 1; bm &= bm - 1; pm += llr[base + kk]; }
+            if (SHOT) { if (cv) while (bm) { const int kk = __ffs(bm) - 1; bm &= bm - 1; pm += llr[(size_t)b * n + base + kk]; } }
+            else if (cv) while (bm) { const int kk = __ffs(bm) - 1; bm &= bm - 1; pm += llr[base + kk]; }
         }
         if (cv && lane == 0 && pm_out) pm_out[b] = pm;
     }
@@ -566,9 +570,12 @@ static inline int osd_setup(int m, int n, int nn, int rank, int method, int orde
     int t = ((m + 1 + 31) / 32) * 32; if (t < 128) t = 128; if (t > 1024) t = 1024;
     if (np2 / 8 >= t && np2 / 8 <= 1024) t = np2 / 8;     // 8 sort keys per thread in registers; more warps for the block scan
     *T5 = t;
-    if (cudaFuncSetAttribute(osd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess) return -3;
-    int occ = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, osd_kernel, t, S->total) != cudaSuccess || occ < 1) return -2;
+    if (cudaFuncSetAttribute(osd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess) return -3;
+    if (cudaFuncSetAttribute(osd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess) return -3;
+    int occ = 0, occ_shot = 0;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, osd_kernel<false>, t, S->total) != cudaSuccess || occ < 1) return -2;
+    // the per-shot twin runs on the same grid (the CTAs draw shots from a ticket counter, any grid size is correct)
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_shot, osd_kernel<true>, t, S->total) != cudaSuccess || occ_shot < 1) return -2;
     *grid5 = num_sm * occ;
     return 0;
 }
@@ -602,11 +609,16 @@ static inline int osd_launch(const GraphDev &g, const u8 *d_synd, const Workspac
         if (capA < L.es_max) { post<<<grid3B, T3, smem3B, s>>>(ws, L, LsB, PSB, P, g.n, ow, chunk_base, 1, capA, d_corr); *launches += 1; }
         return cudaGetLastError() == cudaSuccess ? 0 : -3;
     }
-    if (order_w >= 0) osd_kernel<<<grid5, T5, OS.total, s>>>(g, d_synd, ws, L, P, OS, ow, method, order_w, rank, d_corr, d_pm, chunk_base);
+    if (order_w >= 0) {
+        if (g.llr_shot) osd_kernel<true><<<grid5, T5, OS.total, s>>>(g, d_synd, ws, L, P, OS, ow, method, order_w, rank, d_corr, d_pm, chunk_base);
+        else osd_kernel<false><<<grid5, T5, OS.total, s>>>(g, d_synd, ws, L, P, OS, ow, method, order_w, rank, d_corr, d_pm, chunk_base);
+    }
     osd_finish_kernel<<<grid5, 128, 0, s>>>(ws, L, P, ow, g.n, d_corr, d_conv, chunk_base, order_w < 0 ? 1 : 0);
     cudaMemsetAsync(in_list, 0, (size_t)B, s);
     osd_mark_list_kernel<<<64, 256, 0, s>>>(ws, in_list);
-    osd_pm_kernel<<<(unsigned)((B + 7) / 8 < 1 ? 1 : ((B + 7) / 8 > 65535 ? 65535 : (B + 7) / 8)), 256, 0, s>>>(g.llr, g.n, d_corr, d_conv, B, d_pm, ow, chunk_base, in_list);
+    const unsigned gpm = (unsigned)((B + 7) / 8 < 1 ? 1 : ((B + 7) / 8 > 65535 ? 65535 : (B + 7) / 8));
+    if (g.llr_shot) osd_pm_kernel<true><<<gpm, 256, 0, s>>>(g.llr_shot, g.n, d_corr, d_conv, B, d_pm, ow, chunk_base, in_list);
+    else osd_pm_kernel<false><<<gpm, 256, 0, s>>>(g.llr, g.n, d_corr, d_conv, B, d_pm, ow, chunk_base, in_list);
     *launches += 4;
     return cudaGetLastError() == cudaSuccess ? 0 : -3;
 }

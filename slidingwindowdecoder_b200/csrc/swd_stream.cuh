@@ -21,6 +21,7 @@ struct StreamWs {
     int *itdone;        // [G] iterations executed
     u8 *conv;           // [G]
     long long G;        // shots per tile = threads of the launch
+    const double *llrT; // [n][G] per-shot priors of the tile, transposed like hs (per-shot calls only)
 };
 
 // Memory-level parallelism is what this kernel lives on.  Both passes read the messages in a sequence that is known in
@@ -42,7 +43,9 @@ __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commi
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
-template <int DM>
+// SHOT = true: priors from sw.llrT (the tile's rows of g.llr_shot, transposed by llr_transpose_kernel): one coalesced line
+// per warp, as the messages, where a row-major read would cost one sector per lane.
+template <int DM, bool SHOT = false>
 __global__ void __launch_bounds__(256, SWD_STREAM_MINB)
 pre_bp_stream_kernel(GraphDev g, const u8 *__restrict__ synd, long long B, long long tile_base, int max_iter, double alpha,
                      StreamWs sw, int full_hist, u64 *stats) {
@@ -88,7 +91,7 @@ pre_bp_stream_kernel(GraphDev g, const u8 *__restrict__ synd, long long B, long 
 #pragma unroll 4
             for (int p = p0; p < p1; p++) {
                 double b;
-                if (it == 0) b = __ldg(g.llr + __ldg(g.rc + p));
+                if (it == 0) b = SHOT ? sw.llrT[(size_t)__ldg(g.rc + p) * G + gid] : __ldg(g.llr + __ldg(g.rc + p));
                 else {
                     cp_async_wait<K - 1>();
                     b = ring[(p & (K - 1)) * T];
@@ -111,7 +114,8 @@ pre_bp_stream_kernel(GraphDev g, const u8 *__restrict__ synd, long long B, long 
             for (int p = p0; p < p1; p++) {
                 u32 ng;
                 if (p - p0 < 64) ng = (u32)((neg >> (p - p0)) & 1ull);
-                else ng = (u32)(((it == 0) ? __ldg(g.llr + __ldg(g.rc + p)) : msg[(size_t)p * G]) <= 0.0);   // rows longer than 64: re-read (not yet overwritten)
+                else ng = (u32)(((it == 0) ? (SHOT ? sw.llrT[(size_t)__ldg(g.rc + p) * G + gid] : __ldg(g.llr + __ldg(g.rc + p)))
+                                           : msg[(size_t)p * G]) <= 0.0);   // rows longer than 64: re-read (not yet overwritten)
                 msg[(size_t)p * G] = flip_sign((p == arg) ? q2 : q1, par ^ ng);
             }
         }
@@ -126,7 +130,7 @@ pre_bp_stream_kernel(GraphDev g, const u8 *__restrict__ synd, long long B, long 
         for (int v = 0; v < n; v++) {
             const int e0 = __ldg(g.cp + v), d = __ldg(g.cp + v + 1) - e0;
             double cc[DM], pre[DM]; int pp[DM];
-            double t = __ldg(g.llr + v);
+            double t = SHOT ? sw.llrT[(size_t)v * G + gid] : __ldg(g.llr + v);
 #pragma unroll
             for (int k = 0; k < DM; k++) {
                 if (k < d) {
@@ -201,5 +205,24 @@ __global__ void pre_bp_stream_finish_kernel(GraphDev g, long long B, long long t
                 }
             }
         }
+    }
+}
+
+// Per-shot priors of one tile, [nb][n] row-major (rows tile_base.. of g.llr_shot) -> llrT [n][G]: 32 x 32 blocks through
+// shared memory, coalesced on both sides.  Rows past the batch are left unwritten (their lanes never read them).
+__global__ void __launch_bounds__(256)
+llr_transpose_kernel(const double *__restrict__ llr_shot, long long B, long long tile_base, int n, long long G, double *__restrict__ llrT) {
+    __shared__ double t[32][33];
+    const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;          // 8 rows of 32
+    const long long s0 = tile_base + (long long)blockIdx.y * 32;     // first shot of the block
+    const int v0 = blockIdx.x * 32;
+    for (int i = ty; i < 32; i += 8) {
+        const long long shot = s0 + i; const int v = v0 + tx;
+        if (shot < B && v < n) t[i][tx] = llr_shot[(size_t)shot * n + v];
+    }
+    __syncthreads();
+    for (int i = ty; i < 32; i += 8) {
+        const int v = v0 + i; const long long shot = s0 + tx;
+        if (shot < B && v < n) llrT[(size_t)v * G + (shot - tile_base)] = t[tx][i];
     }
 }

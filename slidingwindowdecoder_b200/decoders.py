@@ -112,28 +112,66 @@ class _window_decoder_base:
         return self._converge
 
     # ------------------------------------------------------------------ batched entry points
-    def decode_batch(self, syndromes, return_pm=False):
+    def _host_llr(self, channel_llr, B):
+        """numpy float64 [B, n] per-shot priors for a host call (checked, C-contiguous)."""
+        if _is_torch_cuda(channel_llr) or not isinstance(channel_llr, np.ndarray):
+            raise ValueError("channel_llr must be a numpy float64 array when the syndromes are numpy arrays "
+                             f"(got {type(channel_llr).__name__})")
+        if channel_llr.dtype != np.float64:
+            raise ValueError(f"channel_llr must be float64, got {channel_llr.dtype}")
+        if channel_llr.shape != (B, self.n):
+            raise ValueError(f"channel_llr must have shape [B, n] = [{B}, {self.n}], got {channel_llr.shape}")
+        if np.isnan(channel_llr).any():
+            raise ValueError("channel_llr contains NaN (allowed: finite values, +-inf; 0.0 marks an erasure)")
+        return np.ascontiguousarray(channel_llr)
+
+    def _device_llr(self, channel_llr, B, device):
+        """torch CUDA float64 [B, n] per-shot priors for a device call (checked, contiguous).  NaN is not checked here
+        (that would synchronise the stream): it is undefined behaviour, as at the C-ABI."""
+        if not _is_torch_cuda(channel_llr):
+            raise ValueError("channel_llr must be a torch CUDA float64 tensor when the syndromes are torch CUDA tensors "
+                             f"(got {type(channel_llr).__name__})")
+        import torch
+        if channel_llr.dtype != torch.float64:
+            raise ValueError(f"channel_llr must be float64, got {channel_llr.dtype}")
+        if tuple(channel_llr.shape) != (B, self.n):
+            raise ValueError(f"channel_llr must have shape [B, n] = [{B}, {self.n}], got {tuple(channel_llr.shape)}")
+        if channel_llr.device != device:
+            raise ValueError(f"channel_llr lives on {channel_llr.device}, syndromes on {device}")
+        return channel_llr.contiguous()
+
+    def decode_batch(self, syndromes, return_pm=False, channel_llr=None):
         """syndromes: [B, m] of 0/1.  numpy in -> numpy out (host copies inside the call);
         torch CUDA uint8 tensor in -> torch CUDA tensors out (asynchronous on the current stream).
+        channel_llr: optional per-shot priors [B, n] float64 (numpy with numpy syndromes, a torch CUDA tensor on the
+        decoder's device with torch syndromes): row b decodes syndrome b as a decoder built with channel_llr = row b would.
+        0.0 marks an erasure (p = 1/2); +inf and negative values are allowed, NaN is not.
         Returns (corrections [B, n] uint8, converge [B] uint8[, min_pm [B] float64])."""
         if _is_torch_cuda(syndromes):
-            return self._decode_batch_torch(syndromes, return_pm)
+            return self._decode_batch_torch(syndromes, return_pm, channel_llr)
         s = np.ascontiguousarray(np.asarray(syndromes), dtype=np.uint8)
         if s.ndim != 2 or s.shape[1] != self.m:
             raise ValueError(f"decode_batch expects syndromes of shape [B, {self.m}], got {s.shape}")
         B = s.shape[0]
+        llr = None if channel_llr is None else self._host_llr(channel_llr, B)
         corr = np.empty((B, self.n), dtype=np.uint8)
         conv = np.empty(B, dtype=np.uint8)
         pm = np.empty(B, dtype=np.float64)
-        st = self._lib.swd_decode_batch_host(self._handle, s.ctypes.data, B, corr.ctypes.data, conv.ctypes.data, pm.ctypes.data)
-        _lib.check(st, "swd_decode_batch_host")
+        if llr is None:
+            st = self._lib.swd_decode_batch_host(self._handle, s.ctypes.data, B, corr.ctypes.data, conv.ctypes.data, pm.ctypes.data)
+            _lib.check(st, "swd_decode_batch_host")
+        else:
+            st = self._lib.swd_decode_batch_host_llr(self._handle, s.ctypes.data, B, corr.ctypes.data, conv.ctypes.data, pm.ctypes.data,
+                                                     llr.ctypes.data)
+            _lib.check(st, "swd_decode_batch_host_llr")
         self._last_B = B
         return (corr, conv, pm) if return_pm else (corr, conv)
 
-    def decode_batch_packed(self, synd_packed, return_pm=False):
+    def decode_batch_packed(self, synd_packed, return_pm=False, channel_llr=None):
         """Bit-packed twin of decode_batch (swd_decode_batch_host_packed / _device_packed): synd_packed [B, ceil(m/64)] uint64
         (see pack_bits) -> (corrections [B, ceil(n/64)] uint64, converge [B] uint8[, min_pm]).  numpy in -> numpy out with the
-        copies inside the call; torch CUDA int64/uint64 tensor in -> torch CUDA tensors out on the current stream."""
+        copies inside the call; torch CUDA int64/uint64 tensor in -> torch CUDA tensors out on the current stream.
+        channel_llr: optional per-shot priors [B, n] float64, as for decode_batch."""
         wm, wn = (self.m + 63) // 64, (self.n + 63) // 64
         if _is_torch_cuda(synd_packed):
             import torch
@@ -143,25 +181,38 @@ class _window_decoder_base:
             if s.device.index != self._device:
                 raise ValueError(f"syndromes live on cuda:{s.device.index}, decoder on cuda:{self._device}")
             B = s.shape[0]
+            llr = None if channel_llr is None else self._device_llr(channel_llr, B, s.device)
             corr = torch.empty((B, wn), dtype=torch.int64, device=s.device)
             conv = torch.empty(B, dtype=torch.uint8, device=s.device)
             pm = torch.empty(B, dtype=torch.float64, device=s.device)
             stream = torch.cuda.current_stream(s.device).cuda_stream
-            st = self._lib.swd_decode_batch_device_packed(self._handle, s.data_ptr(), B, corr.data_ptr(), conv.data_ptr(), pm.data_ptr(),
-                                                          C.c_void_p(stream))
-            _lib.check(st, "swd_decode_batch_device_packed")
+            if llr is None:
+                st = self._lib.swd_decode_batch_device_packed(self._handle, s.data_ptr(), B, corr.data_ptr(), conv.data_ptr(), pm.data_ptr(),
+                                                              C.c_void_p(stream))
+                _lib.check(st, "swd_decode_batch_device_packed")
+                self._keepalive = s
+            else:
+                st = self._lib.swd_decode_batch_device_packed_llr(self._handle, s.data_ptr(), B, corr.data_ptr(), conv.data_ptr(),
+                                                                  pm.data_ptr(), llr.data_ptr(), C.c_void_p(stream))
+                _lib.check(st, "swd_decode_batch_device_packed_llr")
+                self._keepalive = (s, llr)
             self._last_B = B
-            self._keepalive = s
             return (corr, conv, pm) if return_pm else (corr, conv)
         s = np.ascontiguousarray(synd_packed, dtype=np.uint64)
         if s.ndim != 2 or s.shape[1] != wm:
             raise ValueError(f"decode_batch_packed expects uint64 words of shape [B, {wm}], got {s.shape}")
         B = s.shape[0]
+        llr = None if channel_llr is None else self._host_llr(channel_llr, B)
         corr = np.empty((B, wn), dtype=np.uint64)
         conv = np.empty(B, dtype=np.uint8)
         pm = np.empty(B, dtype=np.float64)
-        st = self._lib.swd_decode_batch_host_packed(self._handle, s.ctypes.data, B, corr.ctypes.data, conv.ctypes.data, pm.ctypes.data)
-        _lib.check(st, "swd_decode_batch_host_packed")
+        if llr is None:
+            st = self._lib.swd_decode_batch_host_packed(self._handle, s.ctypes.data, B, corr.ctypes.data, conv.ctypes.data, pm.ctypes.data)
+            _lib.check(st, "swd_decode_batch_host_packed")
+        else:
+            st = self._lib.swd_decode_batch_host_packed_llr(self._handle, s.ctypes.data, B, corr.ctypes.data, conv.ctypes.data,
+                                                            pm.ctypes.data, llr.ctypes.data)
+            _lib.check(st, "swd_decode_batch_host_packed_llr")
         self._last_B = B
         return (corr, conv, pm) if return_pm else (corr, conv)
 
@@ -170,7 +221,7 @@ class _window_decoder_base:
         """True if the full-window BP streams its messages from HBM (the window graph exceeds one SM's shared memory)."""
         return bool(self._lib.swd_is_streamed(self._handle) == 1)
 
-    def _decode_batch_torch(self, syndromes, return_pm):
+    def _decode_batch_torch(self, syndromes, return_pm, channel_llr=None):
         import torch
         s = syndromes
         if s.dtype != torch.uint8:
@@ -181,15 +232,22 @@ class _window_decoder_base:
         if s.device.index != self._device:
             raise ValueError(f"syndromes live on cuda:{s.device.index}, decoder on cuda:{self._device}")
         B = s.shape[0]
+        llr = None if channel_llr is None else self._device_llr(channel_llr, B, s.device)
         corr = torch.empty((B, self.n), dtype=torch.uint8, device=s.device)
         conv = torch.empty(B, dtype=torch.uint8, device=s.device)
         pm = torch.empty(B, dtype=torch.float64, device=s.device)
         stream = torch.cuda.current_stream(s.device).cuda_stream
-        st = self._lib.swd_decode_batch_device(self._handle, s.data_ptr(), B, corr.data_ptr(), conv.data_ptr(), pm.data_ptr(),
-                                               C.c_void_p(stream))
-        _lib.check(st, "swd_decode_batch_device")
+        if llr is None:
+            st = self._lib.swd_decode_batch_device(self._handle, s.data_ptr(), B, corr.data_ptr(), conv.data_ptr(), pm.data_ptr(),
+                                                   C.c_void_p(stream))
+            _lib.check(st, "swd_decode_batch_device")
+            self._keepalive = s
+        else:
+            st = self._lib.swd_decode_batch_device_llr(self._handle, s.data_ptr(), B, corr.data_ptr(), conv.data_ptr(), pm.data_ptr(),
+                                                       llr.data_ptr(), C.c_void_p(stream))
+            _lib.check(st, "swd_decode_batch_device_llr")
+            self._keepalive = (s, llr)
         self._last_B = B
-        self._keepalive = s
         return (corr, conv, pm) if return_pm else (corr, conv)
 
     def _decode_one(self, input_vector):

@@ -74,6 +74,7 @@ class SlidingWindowDecoder:
             self.decoder_sets.append(decs)
         self.decoders = self.decoder_sets[0]
         self._side_streams = None
+        self._llr_cache = {}                   # per-shot priors: plan column order, static noisy-column LLRs per window decoder
         # guessing.py:149-158,229-236: the GDG driver decodes the LAST window a second time with BP + OSD-CS
         # (ldpc.BpOsdDecoder there, this repository's BpOsdDecoder facade here) and reports a second set of counts.
         # last_window_osd = True or a dict of BpOsdDecoder kwargs (defaults: the reference's max_iter=200, OSD_CS 10).
@@ -138,8 +139,42 @@ class SlidingWindowDecoder:
             cache[id(dec)] = (h, cp, ri)
         return cache[id(dec)][0]
 
-    def _run_windows(self, det, obs, decs, total, window_events, osd_dec=None, residuals=False):
-        """The window loop for one (sub-)batch on the current stream; det / obs are updated in place."""
+    def _plan_llr(self, channel_llr, det):
+        """Per-shot priors [B, num_col] in the column order of the DEM given to build_windows (torch CUDA float64 on det's
+        device) -> the same rows in the plan's column order."""
+        torch = self.torch
+        if not (torch.is_tensor(channel_llr) and channel_llr.is_cuda):
+            raise ValueError(f"channel_llr must be a torch CUDA float64 tensor here, got {type(channel_llr).__name__}")
+        if channel_llr.dtype != torch.float64:
+            raise ValueError(f"channel_llr must be float64, got {channel_llr.dtype}")
+        if tuple(channel_llr.shape) != (det.shape[0], self.num_col):
+            raise ValueError(f"channel_llr must have shape [B, num_col] = [{det.shape[0]}, {self.num_col}], got {tuple(channel_llr.shape)}")
+        if channel_llr.device != det.device:
+            raise ValueError(f"channel_llr lives on {channel_llr.device}, shot data on {det.device}")
+        order = self.plan.col_order
+        if order is None:
+            return channel_llr.contiguous()
+        key = ("order", det.device)
+        if key not in self._llr_cache:
+            self._llr_cache[key] = torch.as_tensor(np.asarray(order, dtype=np.int64), device=det.device)
+        return channel_llr.index_select(1, self._llr_cache[key])
+
+    def _window_llr(self, w, dec, llr):
+        """Rows of window w: its DEM columns [col0, col0 + ncols_dem) of the plan-ordered priors, then the decoder's static LLRs
+        of the noisy-syndrome identity columns (method 1: the plan's fixed noisy_prior, the same for every shot)."""
+        torch = self.torch
+        body = llr[:, w.col0:w.col0 + w.ncols_dem]
+        if dec.n == w.ncols_dem:
+            return body.contiguous()
+        key = (id(dec), w.ncols_dem, llr.device)
+        if key not in self._llr_cache:
+            self._llr_cache[key] = torch.as_tensor(np.ascontiguousarray(dec.channel_llr[w.ncols_dem:]), device=llr.device)
+        tail = self._llr_cache[key]
+        return torch.cat([body, tail.unsqueeze(0).expand(llr.shape[0], -1)], dim=1)
+
+    def _run_windows(self, det, obs, decs, total, window_events, osd_dec=None, residuals=False, llr=None):
+        """The window loop for one (sub-)batch on the current stream; det / obs are updated in place.  llr: per-shot priors
+        [B, num_col] in the plan's column order, or None."""
         torch = self.torch
         B = det.shape[0]
         stream = C.c_void_p(torch.cuda.current_stream(det.device).cuda_stream)
@@ -153,7 +188,7 @@ class SlidingWindowDecoder:
             if w.last and osd_dec is not None:
                 # second decode of the last window with BP + OSD on the same residual syndrome (guessing.py:229-236)
                 det2, obs2 = det.clone(), obs.clone()
-                corr2, _ = osd_dec.decode_batch(synd)
+                corr2, _ = osd_dec.decode_batch(synd, channel_llr=None if llr is None else self._window_llr(w, osd_dec, llr))
                 _lib.check(self.lib.swd_window_commit(self._win, corr2.data_ptr(), B, corr2.shape[1], w.col0, w.ncommit, det2.data_ptr(),
                                                       obs2.data_ptr() if self.num_obs else None, stream), "commit")
                 counts_osd = torch.zeros(2, dtype=torch.int64, device=det.device)
@@ -161,7 +196,7 @@ class SlidingWindowDecoder:
                                                               counts_osd.data_ptr(), stream), "count")
             if window_events is not None:
                 window_events[w.index][0].record()
-            corr, conv = dec.decode_batch(synd)
+            corr, conv = dec.decode_batch(synd, channel_llr=None if llr is None else self._window_llr(w, dec, llr))
             if window_events is not None:
                 window_events[w.index][1].record()
             n_win = corr.shape[1]
@@ -182,20 +217,25 @@ class SlidingWindowDecoder:
                                                       counts.data_ptr(), stream), "count")
         return counts, torch.stack(unconv), counts_osd, (torch.stack(flagged) if residuals else None)
 
-    def decode_device(self, det, obs, return_corrections=False, window_events=None, streams=None, window_residuals=False):
+    def decode_device(self, det, obs, return_corrections=False, window_events=None, streams=None, window_residuals=False,
+                      channel_llr=None):
         """det [B, num_det], obs [B, num_obs]: torch CUDA uint8 tensors, MODIFIED IN PLACE into the residual
         syndrome / residual observables.  Returns dict with device tensors:
           counts uint64[2] = (flagged shots, failed shots), window_unconverged int64[num_win].
-        streams: use fewer concurrent sub-batches than the decoder was built with (1 = plain sequential launches)."""
+        streams: use fewer concurrent sub-batches than the decoder was built with (1 = plain sequential launches).
+        channel_llr: optional per-shot priors, torch CUDA float64 [B, num_col] in the column order of the DEM given to
+        build_windows (log((1-p)/p); 0.0 = erased).  Every window (and the last-window BP + OSD re-decode) decodes shot b with
+        row b's LLRs of its DEM columns; the noisy-syndrome columns of method 1 keep their static prior."""
         torch = self.torch
         B = det.shape[0]
+        llr = None if channel_llr is None else self._plan_llr(channel_llr, det)
         total = torch.zeros((B, self.num_col), dtype=torch.uint8, device=det.device) if return_corrections else None
         ns = self.nstreams if streams is None else max(1, min(int(streams), self.nstreams))
         if window_events is not None or B < 2 * ns:
             ns = 1
         if ns == 1:
             counts, unconv, counts_osd, wflag = self._run_windows(det, obs, self.decoders, total, window_events,
-                                                                  self.last_osd[0] if self.last_osd else None, window_residuals)
+                                                                  self.last_osd[0] if self.last_osd else None, window_residuals, llr)
         else:
             if self._side_streams is None:
                 self._side_streams = [torch.cuda.Stream(device=det.device) for _ in range(self.nstreams)]
@@ -209,8 +249,9 @@ class SlidingWindowDecoder:
                 with torch.cuda.stream(st):
                     parts.append(self._run_windows(det[lo:hi], obs[lo:hi], self.decoder_sets[i],
                                                    None if total is None else total[lo:hi], None,
-                                                   self.last_osd[i] if self.last_osd else None, window_residuals))
-                for t in (det, obs, total):
+                                                   self.last_osd[i] if self.last_osd else None, window_residuals,
+                                                   None if llr is None else llr[lo:hi]))
+                for t in (det, obs, total, llr):
                     if t is not None:
                         t.record_stream(st)
             for st in self._side_streams[:ns]:
@@ -228,12 +269,28 @@ class SlidingWindowDecoder:
             out["total_e_hat"] = total
         return out
 
-    def decode_packed(self, det_packed, obs_packed, return_corrections=True, pinned_out=None):
+    def _host_llr_to_device(self, channel_llr, B, dev):
+        """numpy (or torch CPU) float64 [B, num_col] per-shot priors -> torch CUDA tensor; NaN is rejected here."""
+        torch = self.torch
+        if torch.is_tensor(channel_llr):
+            if channel_llr.is_cuda:
+                raise ValueError("channel_llr is a CUDA tensor but the shot data are host arrays (use decode_device)")
+            channel_llr = channel_llr.numpy()
+        if not isinstance(channel_llr, np.ndarray) or channel_llr.dtype != np.float64:
+            raise ValueError(f"channel_llr must be a float64 array, got {getattr(channel_llr, 'dtype', type(channel_llr).__name__)}")
+        if channel_llr.shape != (B, self.num_col):
+            raise ValueError(f"channel_llr must have shape [B, num_col] = [{B}, {self.num_col}], got {channel_llr.shape}")
+        if np.isnan(channel_llr).any():
+            raise ValueError("channel_llr contains NaN (allowed: finite values, +-inf; 0.0 marks an erasure)")
+        return torch.from_numpy(np.ascontiguousarray(channel_llr)).to(dev)
+
+    def decode_packed(self, det_packed, obs_packed, return_corrections=True, pinned_out=None, channel_llr=None):
         """Host entry point with bit-packed shot data (decoders.pack_bits layout): det_packed [B, ceil(num_det/64)] and
         obs_packed [B, ceil(num_obs/64)] uint64 (numpy or pinned torch CPU tensors) -> dict(flagged, failed,
         window_unconverged, total_e_hat_packed [B, ceil(num_col/64)] uint64).  8x fewer bytes cross PCIe than with one byte
         per bit (configs[2]: 82 MB instead of 658 MB of corrections per 32768 shots).  pinned_out: optional pinned torch
-        int64 CPU tensor [B, ceil(num_col/64)] that receives the packed corrections."""
+        int64 CPU tensor [B, ceil(num_col/64)] that receives the packed corrections.  channel_llr: optional per-shot priors,
+        numpy float64 [B, num_col] (see decode_device)."""
         torch = self.torch
         dev = torch.device("cuda", self.device)
 
@@ -245,10 +302,11 @@ class SlidingWindowDecoder:
         stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
         det = torch.empty((B, self.num_det), dtype=torch.uint8, device=dev)
         obs = torch.empty((B, self.num_obs), dtype=torch.uint8, device=dev)
+        llr = None if channel_llr is None else self._host_llr_to_device(channel_llr, B, dev)
         _lib.check(self.lib.swd_unpack_bits(self.device, dp.data_ptr(), B, self.num_det, det.data_ptr(), stream), "unpack det")
         if self.num_obs:
             _lib.check(self.lib.swd_unpack_bits(self.device, op.data_ptr(), B, self.num_obs, obs.data_ptr(), stream), "unpack obs")
-        out = self.decode_device(det, obs, return_corrections)
+        out = self.decode_device(det, obs, return_corrections, channel_llr=llr)
         res = {}
         if return_corrections:
             wn = (self.num_col + 63) // 64
@@ -267,9 +325,10 @@ class SlidingWindowDecoder:
             res["total_e_hat_packed"] = res["total_e_hat_packed"].numpy().view(np.uint64)
         return res
 
-    def decode(self, det_data, obs_data, return_corrections=False):
+    def decode(self, det_data, obs_data, return_corrections=False, channel_llr=None):
         """Host entry point (numpy uint8 - or torch CPU tensors, e.g. pinned - in, python ints out): H2D copy, all windows,
-        D2H of the counters (and of the corrections, one byte per bit, if asked for; decode_packed moves 8x less)."""
+        D2H of the counters (and of the corrections, one byte per bit, if asked for; decode_packed moves 8x less).
+        channel_llr: optional per-shot priors, numpy float64 [B, num_col] (see decode_device)."""
         torch = self.torch
         dev = torch.device("cuda", self.device)
 
@@ -277,7 +336,8 @@ class SlidingWindowDecoder:
             t = x if torch.is_tensor(x) else torch.from_numpy(np.ascontiguousarray(x, dtype=np.uint8))
             return t.to(dev, non_blocking=True)
         det, obs = to_dev(det_data), to_dev(obs_data)
-        out = self.decode_device(det, obs, return_corrections)
+        llr = None if channel_llr is None else self._host_llr_to_device(channel_llr, det.shape[0], dev)
+        out = self.decode_device(det, obs, return_corrections, channel_llr=llr)
         counts = out["counts"].cpu().numpy()
         res = dict(shots=int(det.shape[0]), flagged=int(counts[0]), failed=int(counts[1]),
                    window_unconverged=out["window_unconverged"].cpu().numpy().tolist())

@@ -38,11 +38,17 @@ class WindowPlan:
     W: int
     F: int
     noisy_prior: np.ndarray = None
+    col_order: np.ndarray = None   # column j of chk / obs / priors is column col_order[j] of the DEM given to build_windows
 
 
 def reshuffle_by_round(chk, obs, priors, n=None, h=None):
     """guessing.py:49-84 (h = n/2 detectors per round) / SHYPS.ipynb cell 1 (h = r(2^r-1)): regroup the columns by
     (first, last) detector round; compute anchors."""
+    return _reshuffle(chk, obs, priors, n, h)[:4]
+
+
+def _reshuffle(chk, obs, priors, n=None, h=None):
+    """reshuffle_by_round plus the column order it applied (-> chk, obs, priors, anchors, order)."""
     chk = csc_matrix(chk)
     obs = csc_matrix(obs)
     num_row, num_col = chk.shape
@@ -77,7 +83,7 @@ def reshuffle_by_round(chk, obs, priors, n=None, h=None):
             anchors.append((j, c))
             j += h
     anchors.append((num_row, num_col))
-    return chk, obs, priors, anchors
+    return chk, obs, priors, anchors, order
 
 
 def build_windows(chk, obs, priors, n=None, W=3, F=1, method=1, noisy_prior=None, h=None, keep_cols=None):
@@ -89,7 +95,7 @@ def build_windows(chk, obs, priors, n=None, W=3, F=1, method=1, noisy_prior=None
         h = n // 2
     if keep_cols is None:
         keep_cols = 3 * h
-    chk, obs, priors, anchors = reshuffle_by_round(chk, obs, priors, h=h)
+    chk, obs, priors, anchors, order = _reshuffle(chk, obs, priors, h=h)
     if noisy_prior is None and method != 0:
         b = anchors[W]
         c = anchors[W - 1]
@@ -122,4 +128,4 @@ def build_windows(chk, obs, priors, n=None, W=3, F=1, method=1, noisy_prior=None
         commit_end = b[1] if last else anchors[top_left + F][1]
         windows.append(Window(i, mat, prior, a[0], b[0], a[1], commit_end - a[1], ncols_dem, last))
         top_left += F
-    return WindowPlan(chk, obs, priors, anchors, windows, h, W, F, None if method == 0 else np.asarray(noisy_prior))
+    return WindowPlan(chk, obs, priors, anchors, windows, h, W, F, None if method == 0 else np.asarray(noisy_prior), order)
