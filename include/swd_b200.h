@@ -235,6 +235,27 @@ int  swd_bp4_decode_batch_device(swd_bp4 *b, const uint8_t *d_synd_x, const uint
 int  swd_bp4_camel_decode_batch_device(swd_bp4 *b, const uint8_t *d_synd_x, const uint8_t *d_synd_z, int64_t B, uint8_t *d_dec,
                                        uint8_t *d_converge, double *d_min_pm, double *d_log_prob_ratios, int32_t *d_bp_iteration,
                                        void *stream);
+/* Per-shot channel priors: the four bp4 calls above with one more argument, channel_llr = five planes [5][B][n] of float64,
+ * row-major (a host pointer for the _host variants, a device pointer on `stream` for the _device variants).  Plane k, row b
+ * is the k-th LLR array of swd_bp4_create for shot b, in the order llr_x, llr_y, llr_z, prior_llr_x, prior_llr_z.  Row b
+ * decodes syndrome b exactly as a swd_bp4 created with those five rows would, in every output (dec, converge, bp_dec, osd0,
+ * log_prob_ratios, bp_iteration, min_pm).  The camel variants read planes 0-2 only; they take the same layout so that both
+ * calls can share one array.  Allowed values are finite doubles of either sign; an erased qubit (a uniformly random Pauli,
+ * px = py = pz = 1/4) is 0.0 in all five planes.  +-inf and NaN are undefined behaviour.  channel_llr == NULL returns
+ * SWD_ERR_INVALID.  The _host variants stage the priors in a device buffer of 5*B*n doubles, allocated on the first such
+ * call; the static calls never allocate it. */
+int  swd_bp4_decode_batch_host_llr(swd_bp4 *b, const uint8_t *synd_x, const uint8_t *synd_z, int64_t B, uint8_t *dec,
+                                   uint8_t *converge, uint8_t *bp_dec, uint8_t *osd0, double *log_prob_ratios,
+                                   int32_t *bp_iteration, const double *channel_llr);
+int  swd_bp4_decode_batch_device_llr(swd_bp4 *b, const uint8_t *d_synd_x, const uint8_t *d_synd_z, int64_t B, uint8_t *d_dec,
+                                     uint8_t *d_converge, uint8_t *d_bp_dec, uint8_t *d_osd0, double *d_log_prob_ratios,
+                                     int32_t *d_bp_iteration, const double *d_channel_llr, void *stream);
+int  swd_bp4_camel_decode_batch_host_llr(swd_bp4 *b, const uint8_t *synd_x, const uint8_t *synd_z, int64_t B, uint8_t *dec,
+                                         uint8_t *converge, double *min_pm, double *log_prob_ratios, int32_t *bp_iteration,
+                                         const double *channel_llr);
+int  swd_bp4_camel_decode_batch_device_llr(swd_bp4 *b, const uint8_t *d_synd_x, const uint8_t *d_synd_z, int64_t B,
+                                           uint8_t *d_dec, uint8_t *d_converge, double *d_min_pm, double *d_log_prob_ratios,
+                                           int32_t *d_bp_iteration, const double *d_channel_llr, void *stream);
 
 const char *swd_strerror(int status);
 const char *swd_last_error(void);

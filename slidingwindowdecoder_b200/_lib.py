@@ -37,7 +37,9 @@ EXPORTS = ["swd_create", "swd_destroy", "swd_decode_batch_host", "swd_decode_bat
            "swd_decode_batch_device_packed", "swd_decode_batch_host_llr", "swd_decode_batch_device_llr",
            "swd_decode_batch_host_packed_llr", "swd_decode_batch_device_packed_llr", "swd_pack_bits", "swd_unpack_bits", "swd_is_streamed", "swd_pre_bp_layout", "swd_osd_last_outputs",
            "swd_set_profiling", "swd_get_kernel_times", "swd_get_counters", "swd_reset_counters", "swd_rank", "swd_new_n", "swd_window_create", "swd_window_destroy",
-           "swd_window_extract", "swd_window_commit", "swd_window_count_failures", "swd_window_set_priors", "swd_window_sample", "swd_bp4_create", "swd_bp4_destroy", "swd_bp4_rank", "swd_bp4_decode_batch_host", "swd_bp4_camel_decode_batch_host", "swd_bp4_decode_batch_device", "swd_bp4_camel_decode_batch_device", "swd_strerror", "swd_last_error",
+           "swd_window_extract", "swd_window_commit", "swd_window_count_failures", "swd_window_set_priors", "swd_window_sample", "swd_bp4_create", "swd_bp4_destroy", "swd_bp4_rank", "swd_bp4_decode_batch_host", "swd_bp4_camel_decode_batch_host", "swd_bp4_decode_batch_device", "swd_bp4_camel_decode_batch_device",
+           "swd_bp4_decode_batch_host_llr", "swd_bp4_decode_batch_device_llr", "swd_bp4_camel_decode_batch_host_llr",
+           "swd_bp4_camel_decode_batch_device_llr", "swd_strerror", "swd_last_error",
            "swd_version"]
 
 _lib = None
@@ -124,6 +126,14 @@ def load():
     lib.swd_bp4_decode_batch_device.restype = C.c_int
     lib.swd_bp4_camel_decode_batch_device.argtypes = [vp, vp, vp, C.c_int64, vp, vp, vp, vp, vp, vp]
     lib.swd_bp4_camel_decode_batch_device.restype = C.c_int
+    lib.swd_bp4_decode_batch_host_llr.argtypes = [vp, u8p, u8p, C.c_int64, u8p, u8p, u8p, u8p, dp, vp, dp]
+    lib.swd_bp4_decode_batch_host_llr.restype = C.c_int
+    lib.swd_bp4_camel_decode_batch_host_llr.argtypes = [vp, u8p, u8p, C.c_int64, u8p, u8p, dp, dp, vp, dp]
+    lib.swd_bp4_camel_decode_batch_host_llr.restype = C.c_int
+    lib.swd_bp4_decode_batch_device_llr.argtypes = [vp, vp, vp, C.c_int64, vp, vp, vp, vp, vp, vp, dp, vp]
+    lib.swd_bp4_decode_batch_device_llr.restype = C.c_int
+    lib.swd_bp4_camel_decode_batch_device_llr.argtypes = [vp, vp, vp, C.c_int64, vp, vp, vp, vp, vp, dp, vp]
+    lib.swd_bp4_camel_decode_batch_device_llr.restype = C.c_int
     lib.swd_strerror.argtypes = [C.c_int]
     lib.swd_strerror.restype = C.c_char_p
     lib.swd_last_error.restype = C.c_char_p

@@ -1256,6 +1256,8 @@ struct swd_bp4 {
     double *llr = nullptr;                         // device: llr_x | llr_y | llr_z, n each
     Bp4Smem S{};
     int grid = 0;
+    int grid_llr[2] = {0, 0};                      // per-shot priors: bp4_kernel<false, true>, <true, true> (camel)
+    double *d_llr5 = nullptr; long long llr5_cap = 0;     // host per-shot priors staged on the device, [5][B][n]; first _llr call
     // per-batch device buffers
     long long cap = 0;
     u8 *synd_x = nullptr, *synd_z = nullptr, *bp_dec = nullptr, *conv = nullptr, *dec = nullptr, *osd0 = nullptr, *tmp = nullptr;
@@ -1289,6 +1291,7 @@ extern "C" void swd_bp4_destroy(swd_bp4 *b) {
     bp4_free_buffers(b);
     bp4_free_camel(b);
     if (b->llr) cudaFree(b->llr);
+    if (b->d_llr5) cudaFree(b->d_llr5);
     if (b->dx) swd_destroy(b->dx);
     if (b->dz) swd_destroy(b->dz);
     if (b->stream) cudaStreamDestroy(b->stream);
@@ -1326,6 +1329,16 @@ extern "C" int swd_bp4_create(int device, int mx, int mz, int n, const int32_t *
     if ((st = occupancy(bp4_kernel<true>, 256, b->S.total, &occ)) != SWD_OK || occ < 1 ||
         (st = occupancy(bp4_kernel<false>, 256, b->S.total, &occ)) != SWD_OK || occ < 1) { swd_bp4_destroy(b); if (!st) { set_err("bp4_kernel does not fit"); st = SWD_ERR_UNSUPPORTED; } return st; }
     b->grid = b->num_sm * occ;
+    // the per-shot twins get their own grids: their occupancy need not match the static instantiations'
+    int occ_llr = 0;
+    if ((st = occupancy(bp4_kernel<false, true>, 256, b->S.total, &occ_llr)) != SWD_OK || occ_llr < 1) {
+        swd_bp4_destroy(b); if (!st) { set_err("bp4_kernel (per-shot priors) does not fit"); st = SWD_ERR_UNSUPPORTED; } return st;
+    }
+    b->grid_llr[0] = b->num_sm * occ_llr;
+    if ((st = occupancy(bp4_kernel<true, true>, 256, b->S.total, &occ_llr)) != SWD_OK || occ_llr < 1) {
+        swd_bp4_destroy(b); if (!st) { set_err("bp4_kernel (camel, per-shot priors) does not fit"); st = SWD_ERR_UNSUPPORTED; } return st;
+    }
+    b->grid_llr[1] = b->num_sm * occ_llr;
     if (cudaStreamCreateWithFlags(&b->stream, cudaStreamNonBlocking) != cudaSuccess) { swd_bp4_destroy(b); set_err("stream create failed"); return SWD_ERR_CUDA; }
     *out = b;
     return SWD_OK;
@@ -1333,8 +1346,10 @@ extern "C" int swd_bp4_create(int device, int mx, int mz, int n, const int32_t *
 
 extern "C" int swd_bp4_rank(swd_bp4 *b, int which) { return !b ? -1 : (which == 0 ? b->dx->rank : b->dz->rank); }
 
-// OSD-only pass of an osd_window-kind decoder: ranking keys are supplied, converged shots are skipped
-static int bp4_osd_pass(swd_decoder *d, const u8 *d_synd, const double *d_keys, const u8 *d_conv, long long B, u8 *d_tmp, cudaStream_t s) {
+// OSD-only pass of an osd_window-kind decoder: ranking keys are supplied, converged shots are skipped.
+// d_prior: per-shot basis priors [B][n] (plane 3 or 4 of the five) or nullptr for the decoder's static priors
+static int bp4_osd_pass(swd_decoder *d, const u8 *d_synd, const double *d_keys, const u8 *d_conv, long long B, u8 *d_tmp, cudaStream_t s,
+                        const double *d_prior) {
     int st = alloc_workspace(d, B, s);
     if (st) return st;
     if ((st = osd_reserve_outputs(&d->ow, B, d->n, s))) { set_err("osd output alloc failed"); return SWD_ERR_NOMEM; }
@@ -1342,8 +1357,14 @@ static int bp4_osd_pass(swd_decoder *d, const u8 *d_synd, const double *d_keys, 
         const long long nb = std::min<long long>(d->cap, B - b0);
         CK(cudaMemsetAsync(d->ws.counters, 0, 64 * sizeof(int), s));
         bp4_osd_setup_kernel<<<(unsigned)std::min<long long>((nb * d->n + 255) / 256, 4096), 256, 0, s>>>(d->ws, d->ow.need_osd, d_keys + b0 * d->n, d_conv + b0, nb, d->n);
-        osd_kernel<false><<<d->grid5, d->T5, d->OS.total, s>>>(d->g, d_synd + b0 * d->m, d->ws, d->L, d->P, d->OS, d->ow, d->cfg.osd_method, d->cfg.osd_order,
-                                                        d->rank, d_tmp + b0 * d->n, nullptr, b0);
+        if (d_prior) {                                                         // chunk-local rows, as the window decoders
+            GraphDev g = d->g; g.llr_shot = d_prior + b0 * d->n;
+            osd_kernel<true><<<d->grid5, d->T5, d->OS.total, s>>>(g, d_synd + b0 * d->m, d->ws, d->L, d->P, d->OS, d->ow, d->cfg.osd_method, d->cfg.osd_order,
+                                                                  d->rank, d_tmp + b0 * d->n, nullptr, b0);
+        } else {
+            osd_kernel<false><<<d->grid5, d->T5, d->OS.total, s>>>(d->g, d_synd + b0 * d->m, d->ws, d->L, d->P, d->OS, d->ow, d->cfg.osd_method, d->cfg.osd_order,
+                                                                   d->rank, d_tmp + b0 * d->n, nullptr, b0);
+        }
         d->ctr.kernel_launches += 2;
     }
     CK(cudaGetLastError());
@@ -1363,24 +1384,41 @@ static int bp4_reserve(swd_bp4 *b, int64_t B) {
     return SWD_OK;
 }
 
-// BP4 + OSD per basis on device-resident syndromes; results are left in the decoder's own buffers (dec, conv, bp_dec, osd0, lpr, iters)
-static int bp4_run(swd_bp4 *b, const u8 *d_sx, const u8 *d_sz, int64_t B, cudaStream_t s) {
+// host per-shot priors [5][B][n] -> b->d_llr5 on `s` (allocated on the first call that needs it, grown with B)
+static int bp4_stage_llr(swd_bp4 *b, const double *llr5, int64_t B, cudaStream_t s) {
+    if (B > b->llr5_cap) {
+        if (b->d_llr5) { cudaFree(b->d_llr5); b->d_llr5 = nullptr; b->llr5_cap = 0; }
+        if (cudaMalloc(&b->d_llr5, (size_t)40 * B * b->n) != cudaSuccess) { set_err("bp4 prior staging cudaMalloc failed"); return SWD_ERR_NOMEM; }
+        b->llr5_cap = B;
+    }
+    CK(cudaMemcpyAsync(b->d_llr5, llr5, (size_t)40 * B * b->n, cudaMemcpyHostToDevice, s));
+    return SWD_OK;
+}
+
+// BP4 + OSD per basis on device-resident syndromes; results are left in the decoder's own buffers (dec, conv, bp_dec, osd0, lpr, iters).
+// d_llr5: per-shot priors, five planes [5][B][n] on the device (llr_x, llr_y, llr_z, prior_llr_x, prior_llr_z), or nullptr
+static int bp4_run(swd_bp4 *b, const u8 *d_sx, const u8 *d_sz, int64_t B, cudaStream_t s, const double *d_llr5) {
     const size_t n = b->n;
-    bp4_kernel<false><<<(int)std::min<long long>(B, b->grid), 256, b->S.total, s>>>(b->dx->g, b->dz->g, b->llr, b->llr + n, b->llr + 2 * n, d_sx, d_sz, B,
-                                                                                    b->max_iter, b->alpha, b->bp_dec, b->conv, b->iters, b->lpr, b->key_x, b->key_z, b->S, nullptr);
+    const size_t P = (size_t)B * n;                                            // plane stride
+    if (d_llr5)
+        bp4_kernel<false, true><<<(int)std::min<long long>(B, b->grid_llr[0]), 256, b->S.total, s>>>(b->dx->g, b->dz->g, d_llr5, d_llr5 + P, d_llr5 + 2 * P,
+            d_sx, d_sz, B, b->max_iter, b->alpha, b->bp_dec, b->conv, b->iters, b->lpr, b->key_x, b->key_z, b->S, nullptr);
+    else
+        bp4_kernel<false><<<(int)std::min<long long>(B, b->grid), 256, b->S.total, s>>>(b->dx->g, b->dz->g, b->llr, b->llr + n, b->llr + 2 * n, d_sx, d_sz, B,
+                                                                                        b->max_iter, b->alpha, b->bp_dec, b->conv, b->iters, b->lpr, b->key_x, b->key_z, b->S, nullptr);
     CK(cudaGetLastError());
     int st;
-    if ((st = bp4_osd_pass(b->dx, d_sx, b->key_x, b->conv, B, b->tmp, s))) return st;      // osd('x') -> z part
-    if ((st = bp4_osd_pass(b->dz, d_sz, b->key_z, b->conv, B, b->tmp, s))) return st;      // osd('z') -> x part
+    if ((st = bp4_osd_pass(b->dx, d_sx, b->key_x, b->conv, B, b->tmp, s, d_llr5 ? d_llr5 + 3 * P : nullptr))) return st;      // osd('x') -> z part
+    if ((st = bp4_osd_pass(b->dz, d_sz, b->key_z, b->conv, B, b->tmp, s, d_llr5 ? d_llr5 + 4 * P : nullptr))) return st;      // osd('z') -> x part
     bp4_finish_kernel<<<(unsigned)std::min<long long>((B * 2 * (long long)n + 255) / 256, 8192), 256, 0, s>>>(
         b->bp_dec, b->conv, b->dx->ow.osdw, b->dx->ow.osd0, b->dz->ow.osdw, b->dz->ow.osd0, B, (int)n, b->dec, b->osd0);
     CK(cudaGetLastError());
     return SWD_OK;
 }
 
-extern "C" int swd_bp4_decode_batch_host(swd_bp4 *b, const uint8_t *synd_x, const uint8_t *synd_z, int64_t B, uint8_t *dec, uint8_t *conv,
-                                         uint8_t *bp_dec, uint8_t *osd0, double *lpr, int32_t *bp_iteration) {
-    if (!b || B < 0 || (B > 0 && (!synd_x || !synd_z || !dec || !conv))) { set_err("swd_bp4_decode_batch_host: null argument"); return SWD_ERR_INVALID; }
+// host syndromes / outputs; llr5: host per-shot priors [5][B][n] or nullptr (static priors)
+static int bp4_decode_host_impl(swd_bp4 *b, const uint8_t *synd_x, const uint8_t *synd_z, int64_t B, uint8_t *dec, uint8_t *conv,
+                                uint8_t *bp_dec, uint8_t *osd0, double *lpr, int32_t *bp_iteration, const double *llr5) {
     if (B == 0) return SWD_OK;
     CK(cudaSetDevice(b->device));
     const size_t n = b->n;
@@ -1389,7 +1427,8 @@ extern "C" int swd_bp4_decode_batch_host(swd_bp4 *b, const uint8_t *synd_x, cons
     cudaStream_t s = b->stream;
     CK(cudaMemcpyAsync(b->synd_x, synd_x, (size_t)B * b->mx, cudaMemcpyHostToDevice, s));
     CK(cudaMemcpyAsync(b->synd_z, synd_z, (size_t)B * b->mz, cudaMemcpyHostToDevice, s));
-    if ((st = bp4_run(b, b->synd_x, b->synd_z, B, s))) return st;
+    if (llr5 && (st = bp4_stage_llr(b, llr5, B, s))) return st;
+    if ((st = bp4_run(b, b->synd_x, b->synd_z, B, s, llr5 ? b->d_llr5 : nullptr))) return st;
     CK(cudaMemcpyAsync(dec, b->dec, (size_t)B * 2 * n, cudaMemcpyDeviceToHost, s));
     CK(cudaMemcpyAsync(conv, b->conv, (size_t)B, cudaMemcpyDeviceToHost, s));
     if (bp_dec) CK(cudaMemcpyAsync(bp_dec, b->bp_dec, (size_t)B * 2 * n, cudaMemcpyDeviceToHost, s));
@@ -1400,18 +1439,29 @@ extern "C" int swd_bp4_decode_batch_host(swd_bp4 *b, const uint8_t *synd_x, cons
     return SWD_OK;
 }
 
-// the same with device pointers (e.g. torch tensors) on the caller's stream, no host synchronisation
-extern "C" int swd_bp4_decode_batch_device(swd_bp4 *b, const uint8_t *d_synd_x, const uint8_t *d_synd_z, int64_t B, uint8_t *d_dec,
-                                           uint8_t *d_conv, uint8_t *d_bp_dec, uint8_t *d_osd0, double *d_lpr, int32_t *d_bp_iteration,
-                                           void *stream) {
-    if (!b || B < 0 || (B > 0 && (!d_synd_x || !d_synd_z || !d_dec || !d_conv))) { set_err("swd_bp4_decode_batch_device: null argument"); return SWD_ERR_INVALID; }
+extern "C" int swd_bp4_decode_batch_host(swd_bp4 *b, const uint8_t *synd_x, const uint8_t *synd_z, int64_t B, uint8_t *dec, uint8_t *conv,
+                                         uint8_t *bp_dec, uint8_t *osd0, double *lpr, int32_t *bp_iteration) {
+    if (!b || B < 0 || (B > 0 && (!synd_x || !synd_z || !dec || !conv))) { set_err("swd_bp4_decode_batch_host: null argument"); return SWD_ERR_INVALID; }
+    return bp4_decode_host_impl(b, synd_x, synd_z, B, dec, conv, bp_dec, osd0, lpr, bp_iteration, nullptr);
+}
+
+extern "C" int swd_bp4_decode_batch_host_llr(swd_bp4 *b, const uint8_t *synd_x, const uint8_t *synd_z, int64_t B, uint8_t *dec, uint8_t *conv,
+                                             uint8_t *bp_dec, uint8_t *osd0, double *lpr, int32_t *bp_iteration, const double *channel_llr) {
+    if (!b || B < 0 || !channel_llr || (B > 0 && (!synd_x || !synd_z || !dec || !conv))) { set_err("swd_bp4_decode_batch_host_llr: null argument"); return SWD_ERR_INVALID; }
+    return bp4_decode_host_impl(b, synd_x, synd_z, B, dec, conv, bp_dec, osd0, lpr, bp_iteration, channel_llr);
+}
+
+// device syndromes / outputs on the caller's stream, no host synchronisation; d_llr5: device per-shot priors [5][B][n] or nullptr
+static int bp4_decode_device_impl(swd_bp4 *b, const uint8_t *d_synd_x, const uint8_t *d_synd_z, int64_t B, uint8_t *d_dec,
+                                  uint8_t *d_conv, uint8_t *d_bp_dec, uint8_t *d_osd0, double *d_lpr, int32_t *d_bp_iteration,
+                                  void *stream, const double *d_llr5) {
     if (B == 0) return SWD_OK;
     CK(cudaSetDevice(b->device));
     const size_t n = b->n;
     int st;
     if ((st = bp4_reserve(b, B))) return st;
     cudaStream_t s = (cudaStream_t)stream;
-    if ((st = bp4_run(b, d_synd_x, d_synd_z, B, s))) return st;
+    if ((st = bp4_run(b, d_synd_x, d_synd_z, B, s, d_llr5))) return st;
     CK(cudaMemcpyAsync(d_dec, b->dec, (size_t)B * 2 * n, cudaMemcpyDeviceToDevice, s));
     CK(cudaMemcpyAsync(d_conv, b->conv, (size_t)B, cudaMemcpyDeviceToDevice, s));
     if (d_bp_dec) CK(cudaMemcpyAsync(d_bp_dec, b->bp_dec, (size_t)B * 2 * n, cudaMemcpyDeviceToDevice, s));
@@ -1419,6 +1469,21 @@ extern "C" int swd_bp4_decode_batch_device(swd_bp4 *b, const uint8_t *d_synd_x, 
     if (d_lpr) CK(cudaMemcpyAsync(d_lpr, b->lpr, (size_t)B * n * 24, cudaMemcpyDeviceToDevice, s));
     if (d_bp_iteration) CK(cudaMemcpyAsync(d_bp_iteration, b->iters, (size_t)B * 4, cudaMemcpyDeviceToDevice, s));
     return SWD_OK;
+}
+
+// the same with device pointers (e.g. torch tensors) on the caller's stream, no host synchronisation
+extern "C" int swd_bp4_decode_batch_device(swd_bp4 *b, const uint8_t *d_synd_x, const uint8_t *d_synd_z, int64_t B, uint8_t *d_dec,
+                                           uint8_t *d_conv, uint8_t *d_bp_dec, uint8_t *d_osd0, double *d_lpr, int32_t *d_bp_iteration,
+                                           void *stream) {
+    if (!b || B < 0 || (B > 0 && (!d_synd_x || !d_synd_z || !d_dec || !d_conv))) { set_err("swd_bp4_decode_batch_device: null argument"); return SWD_ERR_INVALID; }
+    return bp4_decode_device_impl(b, d_synd_x, d_synd_z, B, d_dec, d_conv, d_bp_dec, d_osd0, d_lpr, d_bp_iteration, stream, nullptr);
+}
+
+extern "C" int swd_bp4_decode_batch_device_llr(swd_bp4 *b, const uint8_t *d_synd_x, const uint8_t *d_synd_z, int64_t B, uint8_t *d_dec,
+                                               uint8_t *d_conv, uint8_t *d_bp_dec, uint8_t *d_osd0, double *d_lpr, int32_t *d_bp_iteration,
+                                               const double *d_channel_llr, void *stream) {
+    if (!b || B < 0 || !d_channel_llr || (B > 0 && (!d_synd_x || !d_synd_z || !d_dec || !d_conv))) { set_err("swd_bp4_decode_batch_device_llr: null argument"); return SWD_ERR_INVALID; }
+    return bp4_decode_device_impl(b, d_synd_x, d_synd_z, B, d_dec, d_conv, d_bp_dec, d_osd0, d_lpr, d_bp_iteration, stream, d_channel_llr);
 }
 
 // bp4_osd.camel_decode (src/bp4_osd.pyx:223-248) for a batch: four BP runs per shot with the last qubit pinned to I / X / Z / Y,
@@ -1437,10 +1502,16 @@ static int bp4_camel_reserve(swd_bp4 *b, int64_t B) {
     return SWD_OK;
 }
 
-static int bp4_camel_run(swd_bp4 *b, const u8 *d_sx, const u8 *d_sz, int64_t B, cudaStream_t s) {
+// d_llr5: per-shot priors [5][B][n] on the device (planes 0-2 are read) or nullptr
+static int bp4_camel_run(swd_bp4 *b, const u8 *d_sx, const u8 *d_sz, int64_t B, cudaStream_t s, const double *d_llr5) {
     const size_t n = b->n;
-    bp4_kernel<true><<<(int)std::min<long long>(4 * B, b->grid), 256, b->S.total, s>>>(b->dx->g, b->dz->g, b->llr, b->llr + n, b->llr + 2 * n, d_sx, d_sz, B,
-                                                                                       b->max_iter, b->alpha, b->c_bp_dec, b->c_conv4, b->c_it4, b->c_lpr, nullptr, nullptr, b->S, b->c_pm4);
+    const size_t P = (size_t)B * n;
+    if (d_llr5)
+        bp4_kernel<true, true><<<(int)std::min<long long>(4 * B, b->grid_llr[1]), 256, b->S.total, s>>>(b->dx->g, b->dz->g, d_llr5, d_llr5 + P, d_llr5 + 2 * P,
+            d_sx, d_sz, B, b->max_iter, b->alpha, b->c_bp_dec, b->c_conv4, b->c_it4, b->c_lpr, nullptr, nullptr, b->S, b->c_pm4);
+    else
+        bp4_kernel<true><<<(int)std::min<long long>(4 * B, b->grid), 256, b->S.total, s>>>(b->dx->g, b->dz->g, b->llr, b->llr + n, b->llr + 2 * n, d_sx, d_sz, B,
+                                                                                           b->max_iter, b->alpha, b->c_bp_dec, b->c_conv4, b->c_it4, b->c_lpr, nullptr, nullptr, b->S, b->c_pm4);
     CK(cudaGetLastError());
     bp4_camel_finish_kernel<<<(unsigned)std::min<long long>((B + 7) / 8, 4096), 256, 0, s>>>(b->c_bp_dec, b->c_conv4, b->c_pm4, b->c_it4, B, (int)n,
                                                                                              b->c_dec, b->c_conv, b->c_pm, b->c_it);
@@ -1448,9 +1519,8 @@ static int bp4_camel_run(swd_bp4 *b, const u8 *d_sx, const u8 *d_sz, int64_t B, 
     return SWD_OK;
 }
 
-extern "C" int swd_bp4_camel_decode_batch_host(swd_bp4 *b, const uint8_t *synd_x, const uint8_t *synd_z, int64_t B, uint8_t *dec, uint8_t *conv,
-                                               double *min_pm, double *lpr, int32_t *bp_iteration) {
-    if (!b || B < 0 || (B > 0 && (!synd_x || !synd_z || !dec || !conv))) { set_err("swd_bp4_camel_decode_batch_host: null argument"); return SWD_ERR_INVALID; }
+static int bp4_camel_host_impl(swd_bp4 *b, const uint8_t *synd_x, const uint8_t *synd_z, int64_t B, uint8_t *dec, uint8_t *conv,
+                               double *min_pm, double *lpr, int32_t *bp_iteration, const double *llr5) {
     if (B == 0) return SWD_OK;
     CK(cudaSetDevice(b->device));
     const size_t n = b->n;
@@ -1459,7 +1529,8 @@ extern "C" int swd_bp4_camel_decode_batch_host(swd_bp4 *b, const uint8_t *synd_x
     cudaStream_t s = b->stream;
     CK(cudaMemcpyAsync(b->c_synd_x, synd_x, (size_t)B * b->mx, cudaMemcpyHostToDevice, s));
     CK(cudaMemcpyAsync(b->c_synd_z, synd_z, (size_t)B * b->mz, cudaMemcpyHostToDevice, s));
-    if ((st = bp4_camel_run(b, b->c_synd_x, b->c_synd_z, B, s))) return st;
+    if (llr5 && (st = bp4_stage_llr(b, llr5, B, s))) return st;
+    if ((st = bp4_camel_run(b, b->c_synd_x, b->c_synd_z, B, s, llr5 ? b->d_llr5 : nullptr))) return st;
     CK(cudaMemcpyAsync(dec, b->c_dec, (size_t)B * 2 * n, cudaMemcpyDeviceToHost, s));
     CK(cudaMemcpyAsync(conv, b->c_conv, (size_t)B, cudaMemcpyDeviceToHost, s));
     if (min_pm) CK(cudaMemcpyAsync(min_pm, b->c_pm, (size_t)B * 8, cudaMemcpyDeviceToHost, s));
@@ -1469,20 +1540,44 @@ extern "C" int swd_bp4_camel_decode_batch_host(swd_bp4 *b, const uint8_t *synd_x
     return SWD_OK;
 }
 
-extern "C" int swd_bp4_camel_decode_batch_device(swd_bp4 *b, const uint8_t *d_synd_x, const uint8_t *d_synd_z, int64_t B, uint8_t *d_dec,
-                                                 uint8_t *d_conv, double *d_min_pm, double *d_lpr, int32_t *d_bp_iteration, void *stream) {
-    if (!b || B < 0 || (B > 0 && (!d_synd_x || !d_synd_z || !d_dec || !d_conv))) { set_err("swd_bp4_camel_decode_batch_device: null argument"); return SWD_ERR_INVALID; }
+extern "C" int swd_bp4_camel_decode_batch_host(swd_bp4 *b, const uint8_t *synd_x, const uint8_t *synd_z, int64_t B, uint8_t *dec, uint8_t *conv,
+                                               double *min_pm, double *lpr, int32_t *bp_iteration) {
+    if (!b || B < 0 || (B > 0 && (!synd_x || !synd_z || !dec || !conv))) { set_err("swd_bp4_camel_decode_batch_host: null argument"); return SWD_ERR_INVALID; }
+    return bp4_camel_host_impl(b, synd_x, synd_z, B, dec, conv, min_pm, lpr, bp_iteration, nullptr);
+}
+
+extern "C" int swd_bp4_camel_decode_batch_host_llr(swd_bp4 *b, const uint8_t *synd_x, const uint8_t *synd_z, int64_t B, uint8_t *dec, uint8_t *conv,
+                                                   double *min_pm, double *lpr, int32_t *bp_iteration, const double *channel_llr) {
+    if (!b || B < 0 || !channel_llr || (B > 0 && (!synd_x || !synd_z || !dec || !conv))) { set_err("swd_bp4_camel_decode_batch_host_llr: null argument"); return SWD_ERR_INVALID; }
+    return bp4_camel_host_impl(b, synd_x, synd_z, B, dec, conv, min_pm, lpr, bp_iteration, channel_llr);
+}
+
+static int bp4_camel_device_impl(swd_bp4 *b, const uint8_t *d_synd_x, const uint8_t *d_synd_z, int64_t B, uint8_t *d_dec,
+                                 uint8_t *d_conv, double *d_min_pm, double *d_lpr, int32_t *d_bp_iteration, void *stream, const double *d_llr5) {
     if (B == 0) return SWD_OK;
     CK(cudaSetDevice(b->device));
     const size_t n = b->n;
     int st;
     if ((st = bp4_camel_reserve(b, B))) return st;
     cudaStream_t s = (cudaStream_t)stream;
-    if ((st = bp4_camel_run(b, d_synd_x, d_synd_z, B, s))) return st;
+    if ((st = bp4_camel_run(b, d_synd_x, d_synd_z, B, s, d_llr5))) return st;
     CK(cudaMemcpyAsync(d_dec, b->c_dec, (size_t)B * 2 * n, cudaMemcpyDeviceToDevice, s));
     CK(cudaMemcpyAsync(d_conv, b->c_conv, (size_t)B, cudaMemcpyDeviceToDevice, s));
     if (d_min_pm) CK(cudaMemcpyAsync(d_min_pm, b->c_pm, (size_t)B * 8, cudaMemcpyDeviceToDevice, s));
     if (d_lpr) CK(cudaMemcpyAsync(d_lpr, b->c_lpr, (size_t)B * n * 24, cudaMemcpyDeviceToDevice, s));
     if (d_bp_iteration) CK(cudaMemcpyAsync(d_bp_iteration, b->c_it, (size_t)B * 4, cudaMemcpyDeviceToDevice, s));
     return SWD_OK;
+}
+
+extern "C" int swd_bp4_camel_decode_batch_device(swd_bp4 *b, const uint8_t *d_synd_x, const uint8_t *d_synd_z, int64_t B, uint8_t *d_dec,
+                                                 uint8_t *d_conv, double *d_min_pm, double *d_lpr, int32_t *d_bp_iteration, void *stream) {
+    if (!b || B < 0 || (B > 0 && (!d_synd_x || !d_synd_z || !d_dec || !d_conv))) { set_err("swd_bp4_camel_decode_batch_device: null argument"); return SWD_ERR_INVALID; }
+    return bp4_camel_device_impl(b, d_synd_x, d_synd_z, B, d_dec, d_conv, d_min_pm, d_lpr, d_bp_iteration, stream, nullptr);
+}
+
+extern "C" int swd_bp4_camel_decode_batch_device_llr(swd_bp4 *b, const uint8_t *d_synd_x, const uint8_t *d_synd_z, int64_t B, uint8_t *d_dec,
+                                                     uint8_t *d_conv, double *d_min_pm, double *d_lpr, int32_t *d_bp_iteration,
+                                                     const double *d_channel_llr, void *stream) {
+    if (!b || B < 0 || !d_channel_llr || (B > 0 && (!d_synd_x || !d_synd_z || !d_dec || !d_conv))) { set_err("swd_bp4_camel_decode_batch_device_llr: null argument"); return SWD_ERR_INVALID; }
+    return bp4_camel_device_impl(b, d_synd_x, d_synd_z, B, d_dec, d_conv, d_min_pm, d_lpr, d_bp_iteration, stream, d_channel_llr);
 }

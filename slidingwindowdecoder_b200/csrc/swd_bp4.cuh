@@ -46,7 +46,9 @@ __device__ __forceinline__ void b4_row_update(double *msg, int p0, int p1, u32 p
 // initial value, and its contribution to the checks is folded into the syndrome (seed of the check pass = current_cn;
 // H.dec == s  <=>  H_rest.dec_rest == s ^ H_fix.dec_fix).  Per item: converge flag, iteration count, hard decision and the
 // path metric cal_pm (pyx:250-259, ordered sum); the posteriors of the last run (value 3) go to lpr.
-template <bool CAMEL>
+// SHOT = true: per-shot priors.  llrx / llry / llrz are then planes of [B][n] and the shot reads its own rows
+// (plane + shot * n) in bp_init, the variable pass and cal_pm; CAMEL's pinned-qubit messages are computed per item.
+template <bool CAMEL, bool SHOT = false>
 __global__ void __launch_bounds__(256)
 bp4_kernel(GraphDev gx, GraphDev gz, const double *__restrict__ llrx, const double *__restrict__ llry, const double *__restrict__ llrz,
            const u8 *__restrict__ synd_x, const u8 *__restrict__ synd_z, long long B, int max_iter, double alpha,
@@ -61,7 +63,7 @@ bp4_kernel(GraphDev gx, GraphDev gz, const double *__restrict__ llrx, const doub
     const long long items = CAMEL ? 4 * B : B;
     const int fix = CAMEL ? n - 1 : -1;
     double fix_mx = 0.0, fix_mz = 0.0;
-    if (CAMEL) {
+    if (CAMEL && !SHOT) {
         const double lx = llrx[fix], ly = llry[fix], lz = llrz[fix];
         fix_mx = b4_log1pexp(-1. * lx) - b4_logaddexp(-1. * ly, -1. * lz);
         fix_mz = b4_log1pexp(-1. * lz) - b4_logaddexp(-1. * ly, -1. * lz);
@@ -69,6 +71,13 @@ bp4_kernel(GraphDev gx, GraphDev gz, const double *__restrict__ llrx, const doub
     for (long long item = blockIdx.x; item < items; item += gridDim.x) {
         const long long shot = CAMEL ? (item >> 2) : item;
         const int value = CAMEL ? (int)(item & 3) : 0;
+        const double *Lx = SHOT ? llrx + (size_t)shot * n : llrx, *Ly = SHOT ? llry + (size_t)shot * n : llry;
+        const double *Lz = SHOT ? llrz + (size_t)shot * n : llrz;
+        if (CAMEL && SHOT) {
+            const double lx = Lx[fix], ly = Ly[fix], lz = Lz[fix];
+            fix_mx = b4_log1pexp(-1. * lx) - b4_logaddexp(-1. * ly, -1. * lz);
+            fix_mz = b4_log1pexp(-1. * lz) - b4_logaddexp(-1. * ly, -1. * lz);
+        }
         for (int r = tid; r < nmx; r += T) sx[r] = synd_x[shot * nmx + r];
         for (int r = tid; r < nmz; r += T) sz[r] = synd_z[shot * nmz + r];
         if (CAMEL) {
@@ -77,7 +86,7 @@ bp4_kernel(GraphDev gx, GraphDev gz, const double *__restrict__ llrx, const doub
             if (value & 1) for (int e = gz.cp[fix] + tid; e < gz.cp[fix + 1]; e += T) sz[gz.cr[e]] ^= 1;      // x part toggles the Hz checks
         }
         for (int v = tid; v < n; v += T) {                                     // bp_init, pyx:425-442
-            const double lx = llrx[v], ly = llry[v], lz = llrz[v];
+            const double lx = Lx[v], ly = Ly[v], lz = Lz[v];
             const double msg_x = b4_log1pexp(-1. * lx) - b4_logaddexp(-1. * ly, -1. * lz);
             const double msg_z = b4_log1pexp(-1. * lz) - b4_logaddexp(-1. * ly, -1. * lz);     // sic (pyx:438)
             for (int e = gx.cp[v]; e < gx.cp[v + 1]; e++) mx[gx.cpos[e]] = msg_x;
@@ -105,9 +114,9 @@ bp4_kernel(GraphDev gx, GraphDev gz, const double *__restrict__ llrx, const doub
                 double llrx_hx = 0.0, llrz_hz = 0.0;
                 for (int e = z0; e < z1; e++) llrx_hx += mz[gz.cpos[e]];
                 for (int e = x0; e < x1; e++) llrz_hz += mx[gx.cpos[e]];
-                const double llry_all = llrx_hx + llrz_hz + llry[v];
-                llrx_hx = llrx_hx + llrx[v];
-                llrz_hz = llrz_hz + llrz[v];
+                const double llry_all = llrx_hx + llrz_hz + Ly[v];
+                llrx_hx = llrx_hx + Lx[v];
+                llrz_hz = llrz_hz + Lz[v];
                 if (write_lp) { lp[3 * v] = llrx_hx; lp[3 * v + 1] = llry_all; lp[3 * v + 2] = llrz_hz; }
                 int idx;
                 if (0 < llrx_hx && 0 < llry_all && 0 < llrz_hz) idx = 0;
@@ -146,9 +155,9 @@ bp4_kernel(GraphDev gx, GraphDev gz, const double *__restrict__ llrx, const doub
                 double pm = 0.0;
                 for (int v = 0; v < n; v++) {
                     const int ex = bx[v], ez = bz[v];
-                    if (ex && ez) pm += llry[v];
-                    else if (ex) pm += llrx[v];
-                    else if (ez) pm += llrz[v];
+                    if (ex && ez) pm += Ly[v];
+                    else if (ex) pm += Lx[v];
+                    else if (ez) pm += Lz[v];
                 }
                 pm_out[item] = pm;
             }

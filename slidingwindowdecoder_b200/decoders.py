@@ -425,7 +425,9 @@ class bp4_osd:
     (0.0, as in the reference whose decode never updates it), `.bp_decoding_x/z`, `.osd0_decoding_x/z`,
     `.osdw_decoding_x/z`, `.log_prob_ratios` [n, 3], and `camel_decode(synd_x, synd_z)` (pyx:223-248: four BP runs with the last
     qubit pinned to I / X / Z / Y, best converged path metric; sets `.converge`, `.min_pm`).
-    Added: `decode_batch(synd_x[B, mx], synd_z[B, mz])`, `camel_decode_batch(...)`."""
+    Added: `decode_batch(synd_x[B, mx], synd_z[B, mz], channel_llr=None)`, `camel_decode_batch(...)`, and `.channel_llr`
+    [5, n]: the static priors llr_x, llr_y, llr_z, prior_llr_x, prior_llr_z.  Per-shot priors are a [5, B, n] float64 array
+    of the same five rows per shot (an erased qubit, px = py = pz = 1/4, is 0.0 in all five)."""
 
     def __init__(self, Hx, Hz, **kwargs):
         if not (isinstance(Hx, np.ndarray) or isinstance(Hx, spmatrix)):
@@ -455,6 +457,7 @@ class bp4_osd:
             den = float(px[v]) + float(py[v]); llr[3, v] = math.log((1.0 - den) / den)
             den = float(pz[v]) + float(py[v]); llr[4, v] = math.log((1.0 - den) / den)
         self._llr = np.ascontiguousarray(llr)
+        self.channel_llr = self._llr.copy()
         A, Bz = csc_matrix(Hx), csc_matrix(Hz)
         for M in (A, Bz):
             M.eliminate_zeros(); M.sort_indices()
@@ -485,20 +488,57 @@ class bp4_osd:
             self._lib.swd_bp4_destroy(h)
             self._handle = C.c_void_p()
 
-    def decode_batch(self, synd_x, synd_z):
+    def _host_llr(self, channel_llr, B):
+        """numpy float64 [5, B, n] per-shot priors for a host call (checked, C-contiguous)."""
+        if _is_torch_cuda(channel_llr) or not isinstance(channel_llr, np.ndarray):
+            raise ValueError("channel_llr must be a numpy float64 array when the syndromes are numpy arrays "
+                             f"(got {type(channel_llr).__name__})")
+        if channel_llr.dtype != np.float64:
+            raise ValueError(f"channel_llr must be float64, got {channel_llr.dtype}")
+        if channel_llr.shape != (5, B, self.n):
+            raise ValueError(f"channel_llr must have shape [5, B, n] = [5, {B}, {self.n}], got {channel_llr.shape}")
+        if not np.isfinite(channel_llr).all():
+            raise ValueError("channel_llr contains inf or NaN (allowed: finite values; 0.0 in all five planes marks an erasure)")
+        return np.ascontiguousarray(channel_llr)
+
+    def _device_llr(self, channel_llr, B, device):
+        """torch CUDA float64 [5, B, n] per-shot priors for a device call (checked, contiguous).  inf and NaN are not checked
+        here (that would synchronise the stream): they are undefined behaviour, as at the C-ABI."""
+        if not _is_torch_cuda(channel_llr):
+            raise ValueError("channel_llr must be a torch CUDA float64 tensor when the syndromes are torch CUDA tensors "
+                             f"(got {type(channel_llr).__name__})")
+        import torch
+        if channel_llr.dtype != torch.float64:
+            raise ValueError(f"channel_llr must be float64, got {channel_llr.dtype}")
+        if tuple(channel_llr.shape) != (5, B, self.n):
+            raise ValueError(f"channel_llr must have shape [5, B, n] = [5, {B}, {self.n}], got {tuple(channel_llr.shape)}")
+        if channel_llr.device != device:
+            raise ValueError(f"channel_llr lives on {channel_llr.device}, syndromes on {device}")
+        return channel_llr.contiguous()
+
+    def decode_batch(self, synd_x, synd_z, channel_llr=None):
         """-> dict(dec [B, 2, n] uint8, converge [B], bp_decoding [B, 2, n], osd0 [B, 2, n], log_prob_ratios [B, n, 3],
-        bp_iteration [B])"""
+        bp_iteration [B]).  channel_llr: optional per-shot priors [5, B, n] float64 (numpy with numpy syndromes, a torch CUDA
+        tensor on the decoder's device with torch syndromes): row b of the five planes decodes shot b as a bp4_osd built
+        with those priors would.  Finite values only; 0.0 in all five planes marks an erased qubit."""
         if _is_torch_cuda(synd_x) and _is_torch_cuda(synd_z):
-            return self._batch_torch(synd_x, synd_z, camel=False)
+            return self._batch_torch(synd_x, synd_z, camel=False, channel_llr=channel_llr)
         sx = np.ascontiguousarray(np.asarray(synd_x), dtype=np.uint8); sz = np.ascontiguousarray(np.asarray(synd_z), dtype=np.uint8)
         if sx.ndim != 2 or sz.ndim != 2 or sx.shape[1] != self.mx or sz.shape[1] != self.mz or sx.shape[0] != sz.shape[0]:
             raise ValueError(f"decode_batch expects syndromes of shape [B, {self.mx}] and [B, {self.mz}]")
         B, n = sx.shape[0], self.n
+        llr = None if channel_llr is None else self._host_llr(channel_llr, B)
         dec = np.empty((B, 2, n), dtype=np.uint8); bp = np.empty_like(dec); o0 = np.empty_like(dec)
         conv = np.empty(B, dtype=np.uint8); lpr = np.empty((B, n, 3)); it = np.empty(B, dtype=np.int32)
-        st = self._lib.swd_bp4_decode_batch_host(self._handle, sx.ctypes.data, sz.ctypes.data, B, dec.ctypes.data, conv.ctypes.data,
-                                                 bp.ctypes.data, o0.ctypes.data, lpr.ctypes.data, it.ctypes.data)
-        _lib.check(st, "swd_bp4_decode_batch_host")
+        if llr is None:
+            st = self._lib.swd_bp4_decode_batch_host(self._handle, sx.ctypes.data, sz.ctypes.data, B, dec.ctypes.data, conv.ctypes.data,
+                                                     bp.ctypes.data, o0.ctypes.data, lpr.ctypes.data, it.ctypes.data)
+            _lib.check(st, "swd_bp4_decode_batch_host")
+        else:
+            st = self._lib.swd_bp4_decode_batch_host_llr(self._handle, sx.ctypes.data, sz.ctypes.data, B, dec.ctypes.data,
+                                                         conv.ctypes.data, bp.ctypes.data, o0.ctypes.data, lpr.ctypes.data,
+                                                         it.ctypes.data, llr.ctypes.data)
+            _lib.check(st, "swd_bp4_decode_batch_host_llr")
         return dict(dec=dec, converge=conv, bp_decoding=bp, osd0=o0, log_prob_ratios=lpr, bp_iteration=it)
 
     def decode(self, input_vector_x, input_vector_z):
@@ -509,7 +549,7 @@ class bp4_osd:
         self.converge = int(self._last["converge"]); self.bp_iteration = int(self._last["bp_iteration"])
         return self._last["dec"].astype(np.int64)
 
-    def _batch_torch(self, synd_x, synd_z, camel):
+    def _batch_torch(self, synd_x, synd_z, camel, channel_llr=None):
         """torch CUDA uint8 tensors in -> dict of torch CUDA tensors out, asynchronous on the current stream (device-pointer
         entry points of the C-ABI; calls on one decoder must be stream-ordered)."""
         import torch
@@ -520,37 +560,58 @@ class bp4_osd:
         if sx.device.index != dev_index or sz.device.index != dev_index:
             raise ValueError(f"syndromes live on cuda:{sx.device.index} / cuda:{sz.device.index}, decoder on cuda:{dev_index}")
         B, n, dev = sx.shape[0], self.n, sx.device
+        llr = None if channel_llr is None else self._device_llr(channel_llr, B, dev)
         dec = torch.empty((B, 2, n), dtype=torch.uint8, device=dev); conv = torch.empty(B, dtype=torch.uint8, device=dev)
         lpr = torch.empty((B, n, 3), dtype=torch.float64, device=dev); it = torch.empty(B, dtype=torch.int32, device=dev)
         stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
         if camel:
             pm = torch.empty(B, dtype=torch.float64, device=dev)
-            st = self._lib.swd_bp4_camel_decode_batch_device(self._handle, sx.data_ptr(), sz.data_ptr(), B, dec.data_ptr(), conv.data_ptr(),
-                                                             pm.data_ptr(), lpr.data_ptr(), it.data_ptr(), stream)
-            _lib.check(st, "swd_bp4_camel_decode_batch_device")
+            if llr is None:
+                st = self._lib.swd_bp4_camel_decode_batch_device(self._handle, sx.data_ptr(), sz.data_ptr(), B, dec.data_ptr(), conv.data_ptr(),
+                                                                 pm.data_ptr(), lpr.data_ptr(), it.data_ptr(), stream)
+                _lib.check(st, "swd_bp4_camel_decode_batch_device")
+            else:
+                st = self._lib.swd_bp4_camel_decode_batch_device_llr(self._handle, sx.data_ptr(), sz.data_ptr(), B, dec.data_ptr(),
+                                                                     conv.data_ptr(), pm.data_ptr(), lpr.data_ptr(), it.data_ptr(),
+                                                                     llr.data_ptr(), stream)
+                _lib.check(st, "swd_bp4_camel_decode_batch_device_llr")
             out = dict(dec=dec, converge=conv, min_pm=pm, log_prob_ratios=lpr, bp_iteration=it)
         else:
             bp = torch.empty_like(dec); o0 = torch.empty_like(dec)
-            st = self._lib.swd_bp4_decode_batch_device(self._handle, sx.data_ptr(), sz.data_ptr(), B, dec.data_ptr(), conv.data_ptr(),
-                                                       bp.data_ptr(), o0.data_ptr(), lpr.data_ptr(), it.data_ptr(), stream)
-            _lib.check(st, "swd_bp4_decode_batch_device")
+            if llr is None:
+                st = self._lib.swd_bp4_decode_batch_device(self._handle, sx.data_ptr(), sz.data_ptr(), B, dec.data_ptr(), conv.data_ptr(),
+                                                           bp.data_ptr(), o0.data_ptr(), lpr.data_ptr(), it.data_ptr(), stream)
+                _lib.check(st, "swd_bp4_decode_batch_device")
+            else:
+                st = self._lib.swd_bp4_decode_batch_device_llr(self._handle, sx.data_ptr(), sz.data_ptr(), B, dec.data_ptr(),
+                                                               conv.data_ptr(), bp.data_ptr(), o0.data_ptr(), lpr.data_ptr(),
+                                                               it.data_ptr(), llr.data_ptr(), stream)
+                _lib.check(st, "swd_bp4_decode_batch_device_llr")
             out = dict(dec=dec, converge=conv, bp_decoding=bp, osd0=o0, log_prob_ratios=lpr, bp_iteration=it)
-        self._keepalive = (sx, sz)
+        self._keepalive = (sx, sz) if llr is None else (sx, sz, llr)
         return out
 
-    def camel_decode_batch(self, synd_x, synd_z):
-        """-> dict(dec [B, 2, n] uint8, converge [B], min_pm [B], log_prob_ratios [B, n, 3] and bp_iteration [B] of the last run)"""
+    def camel_decode_batch(self, synd_x, synd_z, channel_llr=None):
+        """-> dict(dec [B, 2, n] uint8, converge [B], min_pm [B], log_prob_ratios [B, n, 3] and bp_iteration [B] of the last run).
+        channel_llr: optional per-shot priors [5, B, n], as for decode_batch (planes 0-2 are used)."""
         if _is_torch_cuda(synd_x) and _is_torch_cuda(synd_z):
-            return self._batch_torch(synd_x, synd_z, camel=True)
+            return self._batch_torch(synd_x, synd_z, camel=True, channel_llr=channel_llr)
         sx = np.ascontiguousarray(np.asarray(synd_x), dtype=np.uint8); sz = np.ascontiguousarray(np.asarray(synd_z), dtype=np.uint8)
         if sx.ndim != 2 or sz.ndim != 2 or sx.shape[1] != self.mx or sz.shape[1] != self.mz or sx.shape[0] != sz.shape[0]:
             raise ValueError(f"camel_decode_batch expects syndromes of shape [B, {self.mx}] and [B, {self.mz}]")
         B, n = sx.shape[0], self.n
+        llr = None if channel_llr is None else self._host_llr(channel_llr, B)
         dec = np.empty((B, 2, n), dtype=np.uint8); conv = np.empty(B, dtype=np.uint8); pm = np.empty(B)
         lpr = np.empty((B, n, 3)); it = np.empty(B, dtype=np.int32)
-        st = self._lib.swd_bp4_camel_decode_batch_host(self._handle, sx.ctypes.data, sz.ctypes.data, B, dec.ctypes.data, conv.ctypes.data,
-                                                       pm.ctypes.data_as(C.POINTER(C.c_double)), lpr.ctypes.data_as(C.POINTER(C.c_double)), it.ctypes.data)
-        _lib.check(st, "swd_bp4_camel_decode_batch_host")
+        if llr is None:
+            st = self._lib.swd_bp4_camel_decode_batch_host(self._handle, sx.ctypes.data, sz.ctypes.data, B, dec.ctypes.data, conv.ctypes.data,
+                                                           pm.ctypes.data_as(C.POINTER(C.c_double)), lpr.ctypes.data_as(C.POINTER(C.c_double)), it.ctypes.data)
+            _lib.check(st, "swd_bp4_camel_decode_batch_host")
+        else:
+            st = self._lib.swd_bp4_camel_decode_batch_host_llr(self._handle, sx.ctypes.data, sz.ctypes.data, B, dec.ctypes.data,
+                                                               conv.ctypes.data, pm.ctypes.data, lpr.ctypes.data, it.ctypes.data,
+                                                               llr.ctypes.data)
+            _lib.check(st, "swd_bp4_camel_decode_batch_host_llr")
         return dict(dec=dec, converge=conv, min_pm=pm, log_prob_ratios=lpr, bp_iteration=it)
 
     def camel_decode(self, input_vector_x, input_vector_z):
