@@ -205,6 +205,28 @@ int  swd_window_set_priors(swd_window *w, const double *priors /* host, [num_col
 int  swd_window_sample(swd_window *w, uint64_t seed, int64_t shot_offset, int64_t B, uint8_t *d_det, uint8_t *d_obs,
                        uint8_t *d_err, void *stream);
 
+/* Code-capacity sampling on the device: depolarizing noise with heralded erasures on the n data qubits of a CSS code.  The plan
+ * has num_col = 2n columns: column v is the X part of qubit v, column n + v its Z part (the [B][2][n] layout of bp4 `dec`).  For
+ * a CSS pair build chk = [[0, Hx], [Hz, 0]], so det = [synd_x | synd_z] with synd_x = Hx . e_z and synd_z = Hz . e_x (the
+ * convention of swd_bp4_*), and obs = [[lz, 0], [0, lx]]: the X part is tested against the Z logicals and the Z part against
+ * the X logicals.  Nothing else is CSS-specific: the sampler XORs the chk / obs columns of the bits it sets.
+ * swd_window_set_pauli_priors: per-qubit px, py, pz (host, [n] each; non-negative, px + py + pz <= 1), erasure_rate in
+ * [0, 1], optional llr5 (host, [5][n]: the static rows of swd_bp4_create, llr_x, llr_y, llr_z, prior_llr_x, prior_llr_z).
+ * Thresholds are those of swd_window_set_priors, floor(x * 2^32) clamped to 0xffffffff, of px, px + py and (px + py) + pz
+ * and erasure_rate, computed in double on the host.  SWD_ERR_INVALID if num_col != 2n or a value is out of range.
+ * swd_window_sample_pauli draws, for shot s = shot_offset + b, one Philox4x32-10 call per qubit pair k keyed by `seed` with
+ * counter (k, 1, s & 0xffffffff, s >> 32); words 2j and 2j + 1 are the erasure draw w_e and the Pauli draw w_p of qubit 2k + j.
+ * The qubit is erased iff w_e < thr(erasure_rate); an erased qubit's Pauli is w_p >> 30 (0 I, 1 X, 2 Y, 3 Z), any other qubit
+ * is X if w_p < thr(px), else Y if w_p < thr(px + py), else Z if w_p < thr(px + py + pz), else I.  e_x = X or Y, e_z = Y or Z.
+ * Outputs (device, one byte per bit): d_det [B][num_det] and d_obs [B][num_obs] required; optional (NULL allowed) d_err
+ * [B][2n], d_erased [B][n], d_channel_llr [5][B][n] doubles (plane q row b = llr5[q] with 0.0 at the erased qubits of shot b;
+ * needs llr5).  Asynchronous on `stream`; B == 0 is a no-op.  Score decoded shots with swd_window_commit(w, d_dec, B, 2n, 0,
+ * 2n, d_det, d_obs, stream) and swd_window_count_failures. */
+int  swd_window_set_pauli_priors(swd_window *w, int n, const double *px, const double *py, const double *pz,
+                                 double erasure_rate, const double *llr5 /* [5*n] host, may be NULL */);
+int  swd_window_sample_pauli(swd_window *w, uint64_t seed, int64_t shot_offset, int64_t B, uint8_t *d_det, uint8_t *d_obs,
+                             uint8_t *d_err, uint8_t *d_erased, double *d_channel_llr, void *stream);
+
 /* ---- bp4_osd (src/bp4_osd.pyx:6-684): quaternary min-sum BP over the pair (Hx, Hz) of a CSS code under depolarizing
  * noise, then one OSD per basis for shots whose BP did not converge.  Replaces bp4_osd.__cinit__ / decode (pyx:8-221);
  * swd_bp4_camel_decode_batch_host replaces camel_decode (pyx:223-248).  The two graphs have no column- / row-weight limit

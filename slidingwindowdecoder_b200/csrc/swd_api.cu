@@ -1151,6 +1151,10 @@ struct swd_window {
     int device, num_det, num_col, num_obs;
     int *chk_cp = nullptr, *chk_ri = nullptr, *obs_cp = nullptr, *obs_ri = nullptr;
     u32 *thr = nullptr;          // floor(prior * 2^32) per DEM column (set by swd_window_set_priors)
+    u32 *pauli_thr = nullptr;    // code capacity (swd_window_set_pauli_priors): thr(px) | thr(px + py) | thr(px + py + pz), n each
+    u32 pauli_t_erase = 0;       // thr(erasure_rate)
+    int pauli_n = 0;             // 0 until swd_window_set_pauli_priors
+    double *pauli_llr5 = nullptr; // static LLR rows [5][n] copied into the per-shot planes, or nullptr
 };
 
 extern "C" int swd_window_create(int device, int num_det, int num_col, const int32_t *chk_cp, const int32_t *chk_ri, int num_obs,
@@ -1179,6 +1183,8 @@ extern "C" void swd_window_destroy(swd_window *w) {
     if (w->obs_cp) cudaFree(w->obs_cp);
     if (w->obs_ri) cudaFree(w->obs_ri);
     if (w->thr) cudaFree(w->thr);
+    if (w->pauli_thr) cudaFree(w->pauli_thr);
+    if (w->pauli_llr5) cudaFree(w->pauli_llr5);
     delete w;
 }
 extern "C" int swd_window_set_priors(swd_window *w, const double *priors) {
@@ -1193,6 +1199,49 @@ extern "C" int swd_window_set_priors(swd_window *w, const double *priors) {
     CK(cudaSetDevice(w->device));
     if (w->thr) { cudaFree(w->thr); w->thr = nullptr; }
     return upload(t, (void **)&w->thr);
+}
+static u32 prob_threshold(double p) {          // the rule of swd_window_set_priors: floor(p * 2^32), clamped to 0xffffffff
+    const double x = p * 4294967296.0;
+    return x >= 4294967295.0 ? 0xffffffffu : (u32)x;
+}
+extern "C" int swd_window_set_pauli_priors(swd_window *w, int n, const double *px, const double *py, const double *pz,
+                                           double erasure_rate, const double *llr5) {
+    if (!w || !px || !py || !pz || n <= 0 || w->num_col != 2 * n) { set_err("swd_window_set_pauli_priors: bad argument (num_col must be 2n)"); return SWD_ERR_INVALID; }
+    if (!(erasure_rate >= 0.0 && erasure_rate <= 1.0)) { set_err("swd_window_set_pauli_priors: erasure_rate outside [0, 1]"); return SWD_ERR_INVALID; }
+    std::vector<u32> t(3 * (size_t)n);
+    for (int v = 0; v < n; v++) {
+        if (!(px[v] >= 0.0 && py[v] >= 0.0 && pz[v] >= 0.0)) { set_err("swd_window_set_pauli_priors: negative or NaN probability"); return SWD_ERR_INVALID; }
+        const double xy = px[v] + py[v], xyz = xy + pz[v];
+        if (xyz > 1.0) { set_err("swd_window_set_pauli_priors: px + py + pz > 1"); return SWD_ERR_INVALID; }
+        t[v] = prob_threshold(px[v]); t[n + v] = prob_threshold(xy); t[2 * n + v] = prob_threshold(xyz);
+    }
+    CK(cudaSetDevice(w->device));
+    if (w->pauli_thr) { cudaFree(w->pauli_thr); w->pauli_thr = nullptr; }
+    if (w->pauli_llr5) { cudaFree(w->pauli_llr5); w->pauli_llr5 = nullptr; }
+    w->pauli_n = 0;
+    int st;
+    if ((st = upload(t, (void **)&w->pauli_thr))) return st;
+    if (llr5 && (st = upload(std::vector<double>(llr5, llr5 + 5 * (size_t)n), (void **)&w->pauli_llr5))) return st;
+    w->pauli_t_erase = prob_threshold(erasure_rate);
+    w->pauli_n = n;
+    return SWD_OK;
+}
+extern "C" int swd_window_sample_pauli(swd_window *w, uint64_t seed, int64_t shot_offset, int64_t B, uint8_t *d_det, uint8_t *d_obs,
+                                       uint8_t *d_err, uint8_t *d_erased, double *d_channel_llr, void *stream) {
+    if (!w || !d_det || B < 0 || shot_offset < 0 || (w->num_obs > 0 && !d_obs)) { set_err("swd_window_sample_pauli: bad argument"); return SWD_ERR_INVALID; }
+    if (!w->pauli_n) { set_err("swd_window_sample_pauli: call swd_window_set_pauli_priors first"); return SWD_ERR_INVALID; }
+    if (d_channel_llr && !w->pauli_llr5) { set_err("swd_window_sample_pauli: channel_llr needs the llr5 rows of swd_window_set_pauli_priors"); return SWD_ERR_INVALID; }
+    if (B == 0) return SWD_OK;
+    CK(cudaSetDevice(w->device));
+    const int wpb = 8;
+    const size_t smem = (size_t)wpb * (((w->num_det + 31) >> 5) + ((w->num_obs + 31) >> 5)) * sizeof(u32);
+    if (smem > 200 * 1024) { set_err("swd_window_sample_pauli: too many detectors for the shared-memory parity words"); return SWD_ERR_UNSUPPORTED; }
+    if (smem > 48 * 1024) CK(cudaFuncSetAttribute(window_sample_pauli_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    window_sample_pauli_kernel<<<(unsigned)std::min<long long>((B + wpb - 1) / wpb, 148 * 16), wpb * 32, smem, (cudaStream_t)stream>>>(
+        w->pauli_thr, w->pauli_t_erase, w->pauli_n, w->pauli_llr5, w->chk_cp, w->chk_ri, w->num_det, w->obs_cp, w->obs_ri,
+        w->num_obs, (unsigned long long)seed, (long long)shot_offset, (long long)B, d_det, d_obs, d_err, d_erased, d_channel_llr);
+    CK(cudaGetLastError());
+    return SWD_OK;
 }
 extern "C" int swd_window_sample(swd_window *w, uint64_t seed, int64_t shot_offset, int64_t B, uint8_t *d_det, uint8_t *d_obs,
                                  uint8_t *d_err, void *stream) {

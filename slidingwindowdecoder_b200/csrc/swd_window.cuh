@@ -1,6 +1,6 @@
 // swd_window.cuh — sliding-window bookkeeping kernels (guessing.py:204-227, osd.py:170-179):
 // window syndrome extraction, commit of the first F rounds with the sparse syndrome update
-// new_det = det + e_hat @ chk.T (the reference does a dense float GEMM), failure counters.
+// new_det = det + e_hat @ chk.T (the reference does a dense float GEMM), failure counters, DEM and code-capacity samplers.
 #pragma once
 #include "swd_device.cuh"
 
@@ -95,6 +95,60 @@ __global__ void window_sample_kernel(const u32 *__restrict__ thr, int num_col, c
                     for (int e = chk_cp[c]; e < chk_cp[c + 1]; e++) { const int row = chk_ri[e]; atomicXor(&dbits[row >> 5], 1u << (row & 31)); }
                     if (num_obs > 0) for (int e = obs_cp[c]; e < obs_cp[c + 1]; e++) { const int row = obs_ri[e]; atomicXor(&obits[row >> 5], 1u << (row & 31)); }
                 }
+            }
+        }
+        __syncwarp();
+        for (int i = lane; i < num_det; i += 32) det[b * num_det + i] = (u8)((dbits[i >> 5] >> (i & 31)) & 1u);
+        if (obs) for (int i = lane; i < num_obs; i += 32) obs[b * num_obs + i] = (u8)((obits[i >> 5] >> (i & 31)) & 1u);
+        __syncwarp();
+    }
+}
+
+// ----------------------------------------------------------------------------------------------
+// Code-capacity Pauli sampling: depolarizing noise with heralded erasures on n data qubits, as a plan over 2n columns
+// (column v = X part of qubit v, column n + v = its Z part).  One Philox call per qubit pair k with counter (k, 1, shot) -
+// the 1 keeps this stream apart from window_sample_kernel's - whose words 2j / 2j+1 are the erasure / Pauli draws of qubit
+// 2k + j, both always drawn.  Erased (w_e < t_erase): Pauli = w_p >> 30 (0 I, 1 X, 2 Y, 3 Z: exactly uniform); otherwise X,
+// Y, Z below the cumulative thresholds thr3[v], thr3[n + v], thr3[2n + v], else I.  e_x = X or Y, e_z = Y or Z; the chk / obs
+// columns of the set bits are XORed into shared-memory parity words as in window_sample_kernel.  channel_llr [5][B][n]
+// copies the host-computed rows llr5[5][n] with 0.0 at erased qubits (no log on the device).
+// ----------------------------------------------------------------------------------------------
+__device__ __forceinline__ void xor_column(int c, const int *__restrict__ cp, const int *__restrict__ ri, u32 *bits) {
+    for (int e = cp[c]; e < cp[c + 1]; e++) { const int row = ri[e]; atomicXor(&bits[row >> 5], 1u << (row & 31)); }
+}
+
+__global__ void window_sample_pauli_kernel(const u32 *__restrict__ thr3, u32 t_erase, int n, const double *__restrict__ llr5,
+                                           const int *__restrict__ chk_cp, const int *__restrict__ chk_ri, int num_det,
+                                           const int *__restrict__ obs_cp, const int *__restrict__ obs_ri, int num_obs,
+                                           unsigned long long seed, long long shot0, long long B, u8 *__restrict__ det,
+                                           u8 *__restrict__ obs, u8 *__restrict__ err, u8 *__restrict__ erased,
+                                           double *__restrict__ channel_llr) {
+    extern __shared__ u32 s_bits[];                           // per warp: ceil(num_det/32) + ceil(num_obs/32) words
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, wpb = blockDim.x >> 5;
+    const int wd = (num_det + 31) >> 5, wo = (num_obs + 31) >> 5;
+    u32 *dbits = s_bits + (size_t)wid * (wd + wo), *obits = dbits + wd;
+    const int npair = (n + 1) >> 1;
+    for (long long b = (long long)blockIdx.x * wpb + wid; b < B; b += (long long)gridDim.x * wpb) {
+        for (int i = lane; i < wd + wo; i += 32) dbits[i] = 0;
+        __syncwarp();
+        const unsigned long long shot = (unsigned long long)(shot0 + b);
+        for (int k = lane; k < npair; k += 32) {
+            u32 r[4];
+            philox4x32_10((u32)k, 1u, (u32)shot, (u32)(shot >> 32), (u32)seed, (u32)(seed >> 32), r);
+#pragma unroll
+            for (int j = 0; j < 2; j++) {
+                const int v = 2 * k + j;
+                if (v >= n) break;
+                const u32 we = r[2 * j], wp = r[2 * j + 1];
+                const bool er = we < t_erase;
+                const u32 pauli = er ? (wp >> 30) : wp < thr3[v] ? 1u : wp < thr3[n + v] ? 2u : wp < thr3[2 * n + v] ? 3u : 0u;
+                const bool ex = pauli == 1u || pauli == 2u, ez = pauli >= 2u;
+                if (err) { err[b * 2 * n + v] = (u8)ex; err[b * 2 * n + n + v] = (u8)ez; }
+                if (erased) erased[b * n + v] = (u8)er;
+                if (channel_llr)
+                    for (int q = 0; q < 5; q++) channel_llr[((long long)q * B + b) * n + v] = er ? 0.0 : llr5[q * n + v];
+                if (ex) { xor_column(v, chk_cp, chk_ri, dbits); if (num_obs > 0) xor_column(v, obs_cp, obs_ri, obits); }
+                if (ez) { xor_column(n + v, chk_cp, chk_ri, dbits); if (num_obs > 0) xor_column(n + v, obs_cp, obs_ri, obits); }
             }
         }
         __syncwarp();
