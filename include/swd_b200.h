@@ -227,6 +227,29 @@ int  swd_window_set_pauli_priors(swd_window *w, int n, const double *px, const d
 int  swd_window_sample_pauli(swd_window *w, uint64_t seed, int64_t shot_offset, int64_t B, uint8_t *d_det, uint8_t *d_obs,
                              uint8_t *d_err, uint8_t *d_erased, double *d_channel_llr, void *stream);
 
+/* Circuit-level sampling with heralded erasures on the device.  The window's columns are the DEM columns of a circuit; a
+ * noise location l (one DEPOLARIZE2 instruction, or one target of X_ERROR / Z_ERROR / DEPOLARIZE1: dem.noise_locations) has
+ * n_l = mech_ptr[l + 1] - mech_ptr[l] (1 .. 15) independent mechanisms k, each with a probability mech_prob[k] in [0, 1/2]
+ * and the DEM column of its symptom mech_col[k] (-1: empty symptom).  Location l is erased with probability
+ * erasure_rate[l] in [0, 1]; an erased location's mechanisms fire with probability exactly 1/2 (a uniformly random Pauli).
+ * swd_window_set_circuit_noise copies the tables (host arrays) and col_llr (host, [num_col], the static LLR row; NULL if no
+ * LLR rows will be asked for).  Thresholds thr(x) = floor(x * 2^32) clamped to 0xffffffff, computed in double on the host.
+ * SWD_ERR_INVALID for a NULL table, num_loc <= 0, mech_ptr[0] != 0, a count outside 1 .. 15, a column outside [-1, num_col),
+ * a probability outside [0, 1/2] or a rate outside [0, 1] (NaN included).
+ * swd_window_sample_circuit: for shot s = shot_offset + b, location l uses draws t = 0 .. n_l; draw t is word t & 3 of
+ * Philox4x32-10 keyed by `seed` with counter (l, 2 + (t >> 2), s & 0xffffffff, s >> 32).  Draw 0 is the erasure draw
+ * (erased iff w < thr(erasure_rate[l])); draw 1 + k is mechanism k, which fires iff w < (erased ? 0x80000000 : thr(p_k)).
+ * Every draw is made.  Outputs (device, one byte per bit): d_det [B][num_det] and d_obs [B][num_obs] required; optional
+ * (NULL allowed) d_err [B][num_col] (parity of the fired mechanisms per column: det = chk . err, obs = obs_mat . err),
+ * d_erased [B][num_loc], d_channel_llr [B][num_col] doubles (col_llr with 0.0 at every column of an erased location's
+ * mechanisms; needs col_llr).  Asynchronous on `stream`; B == 0 is a no-op; SWD_ERR_UNSUPPORTED if one warp's parity and
+ * column words do not fit in shared memory. */
+int  swd_window_set_circuit_noise(swd_window *w, int num_loc, const int32_t *mech_ptr, const int32_t *mech_col,
+                                  const double *mech_prob, const double *erasure_rate /* [num_loc] */,
+                                  const double *col_llr /* [num_col] host, may be NULL */);
+int  swd_window_sample_circuit(swd_window *w, uint64_t seed, int64_t shot_offset, int64_t B, uint8_t *d_det, uint8_t *d_obs,
+                               uint8_t *d_err, uint8_t *d_erased, double *d_channel_llr, void *stream);
+
 /* ---- bp4_osd (src/bp4_osd.pyx:6-684): quaternary min-sum BP over the pair (Hx, Hz) of a CSS code under depolarizing
  * noise, then one OSD per basis for shots whose BP did not converge.  Replaces bp4_osd.__cinit__ / decode (pyx:8-221);
  * swd_bp4_camel_decode_batch_host replaces camel_decode (pyx:223-248).  The two graphs have no column- / row-weight limit

@@ -1155,6 +1155,10 @@ struct swd_window {
     u32 pauli_t_erase = 0;       // thr(erasure_rate)
     int pauli_n = 0;             // 0 until swd_window_set_pauli_priors
     double *pauli_llr5 = nullptr; // static LLR rows [5][n] copied into the per-shot planes, or nullptr
+    uint4 *circ_work = nullptr;  // circuit noise (swd_window_set_circuit_noise): (l, m0, n_l, thr(e_l)) sorted by n_l
+    uint2 *circ_mech = nullptr;  // (DEM column or -1, thr(p)) per mechanism
+    double *circ_llr = nullptr;  // static LLR row [num_col], or nullptr
+    int circ_num_loc = 0;        // 0 until swd_window_set_circuit_noise
 };
 
 extern "C" int swd_window_create(int device, int num_det, int num_col, const int32_t *chk_cp, const int32_t *chk_ri, int num_obs,
@@ -1185,6 +1189,9 @@ extern "C" void swd_window_destroy(swd_window *w) {
     if (w->thr) cudaFree(w->thr);
     if (w->pauli_thr) cudaFree(w->pauli_thr);
     if (w->pauli_llr5) cudaFree(w->pauli_llr5);
+    if (w->circ_work) cudaFree(w->circ_work);
+    if (w->circ_mech) cudaFree(w->circ_mech);
+    if (w->circ_llr) cudaFree(w->circ_llr);
     delete w;
 }
 extern "C" int swd_window_set_priors(swd_window *w, const double *priors) {
@@ -1239,6 +1246,59 @@ extern "C" int swd_window_sample_pauli(swd_window *w, uint64_t seed, int64_t sho
     if (smem > 48 * 1024) CK(cudaFuncSetAttribute(window_sample_pauli_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     window_sample_pauli_kernel<<<(unsigned)std::min<long long>((B + wpb - 1) / wpb, 148 * 16), wpb * 32, smem, (cudaStream_t)stream>>>(
         w->pauli_thr, w->pauli_t_erase, w->pauli_n, w->pauli_llr5, w->chk_cp, w->chk_ri, w->num_det, w->obs_cp, w->obs_ri,
+        w->num_obs, (unsigned long long)seed, (long long)shot_offset, (long long)B, d_det, d_obs, d_err, d_erased, d_channel_llr);
+    CK(cudaGetLastError());
+    return SWD_OK;
+}
+extern "C" int swd_window_set_circuit_noise(swd_window *w, int num_loc, const int32_t *mech_ptr, const int32_t *mech_col,
+                                            const double *mech_prob, const double *erasure_rate, const double *col_llr) {
+    if (!w || num_loc <= 0 || !mech_ptr || !mech_col || !mech_prob || !erasure_rate) { set_err("swd_window_set_circuit_noise: bad argument"); return SWD_ERR_INVALID; }
+    if (mech_ptr[0] != 0) { set_err("swd_window_set_circuit_noise: mech_ptr[0] must be 0"); return SWD_ERR_INVALID; }
+    std::vector<uint4> work(num_loc);
+    for (int l = 0; l < num_loc; l++) {
+        const int n = mech_ptr[l + 1] - mech_ptr[l];
+        if (n < 1 || n > 15) { set_err("swd_window_set_circuit_noise: a location needs 1 to 15 mechanisms"); return SWD_ERR_INVALID; }
+        const double e = erasure_rate[l];
+        if (!(e >= 0.0 && e <= 1.0)) { set_err("swd_window_set_circuit_noise: erasure_rate outside [0, 1]"); return SWD_ERR_INVALID; }
+        work[l] = make_uint4((u32)l, (u32)mech_ptr[l], (u32)n, prob_threshold(e));
+    }
+    const int M = mech_ptr[num_loc];
+    std::vector<uint2> mech(M);
+    for (int k = 0; k < M; k++) {
+        const double p = mech_prob[k];
+        if (mech_col[k] < -1 || mech_col[k] >= w->num_col) { set_err("swd_window_set_circuit_noise: mech_col outside [-1, num_col)"); return SWD_ERR_INVALID; }
+        if (!(p >= 0.0 && p <= 0.5)) { set_err("swd_window_set_circuit_noise: mech_prob outside [0, 1/2]"); return SWD_ERR_INVALID; }
+        mech[k] = make_uint2((u32)mech_col[k], prob_threshold(p));
+    }
+    // lanes of a warp take consecutive work items: equal mechanism counts give them equal numbers of Philox calls
+    std::stable_sort(work.begin(), work.end(), [](const uint4 &a, const uint4 &b) { return a.z > b.z; });
+    CK(cudaSetDevice(w->device));
+    if (w->circ_work) { cudaFree(w->circ_work); w->circ_work = nullptr; }
+    if (w->circ_mech) { cudaFree(w->circ_mech); w->circ_mech = nullptr; }
+    if (w->circ_llr) { cudaFree(w->circ_llr); w->circ_llr = nullptr; }
+    w->circ_num_loc = 0;
+    int st;
+    if ((st = upload(work, (void **)&w->circ_work)) || (st = upload(mech, (void **)&w->circ_mech))) return st;
+    if (col_llr && (st = upload(std::vector<double>(col_llr, col_llr + w->num_col), (void **)&w->circ_llr))) return st;
+    w->circ_num_loc = num_loc;
+    return SWD_OK;
+}
+extern "C" int swd_window_sample_circuit(swd_window *w, uint64_t seed, int64_t shot_offset, int64_t B, uint8_t *d_det, uint8_t *d_obs,
+                                         uint8_t *d_err, uint8_t *d_erased, double *d_channel_llr, void *stream) {
+    if (!w || !d_det || B < 0 || shot_offset < 0 || (w->num_obs > 0 && !d_obs)) { set_err("swd_window_sample_circuit: bad argument"); return SWD_ERR_INVALID; }
+    if (!w->circ_num_loc) { set_err("swd_window_sample_circuit: call swd_window_set_circuit_noise first"); return SWD_ERR_INVALID; }
+    if (d_channel_llr && !w->circ_llr) { set_err("swd_window_sample_circuit: channel_llr needs the col_llr row of swd_window_set_circuit_noise"); return SWD_ERR_INVALID; }
+    if (B == 0) return SWD_OK;
+    CK(cudaSetDevice(w->device));
+    const int wc = (w->num_col + 31) >> 5;
+    const size_t warp_bytes = (size_t)(((w->num_det + 31) >> 5) + ((w->num_obs + 31) >> 5) + (d_err ? wc : 0) + (d_channel_llr ? wc : 0)) * sizeof(u32);
+    const size_t limit = 200 * 1024;
+    if (warp_bytes > limit) { set_err("swd_window_sample_circuit: one warp's parity and column words exceed the shared-memory limit"); return SWD_ERR_UNSUPPORTED; }
+    const int wpb = (int)std::min<size_t>(8, limit / warp_bytes);
+    const size_t smem = (size_t)wpb * warp_bytes;
+    if (smem > 48 * 1024) CK(cudaFuncSetAttribute(window_sample_circuit_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    window_sample_circuit_kernel<<<(unsigned)std::min<long long>((B + wpb - 1) / wpb, 148 * 16), wpb * 32, smem, (cudaStream_t)stream>>>(
+        w->circ_work, w->circ_num_loc, w->circ_mech, w->circ_llr, w->num_col, w->chk_cp, w->chk_ri, w->num_det, w->obs_cp, w->obs_ri,
         w->num_obs, (unsigned long long)seed, (long long)shot_offset, (long long)B, d_det, d_obs, d_err, d_erased, d_channel_llr);
     CK(cudaGetLastError());
     return SWD_OK;

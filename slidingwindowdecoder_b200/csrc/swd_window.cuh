@@ -1,6 +1,6 @@
 // swd_window.cuh — sliding-window bookkeeping kernels (guessing.py:204-227, osd.py:170-179):
 // window syndrome extraction, commit of the first F rounds with the sparse syndrome update
-// new_det = det + e_hat @ chk.T (the reference does a dense float GEMM), failure counters, DEM and code-capacity samplers.
+// new_det = det + e_hat @ chk.T (the reference does a dense float GEMM), failure counters, DEM, code-capacity and circuit-level samplers.
 #pragma once
 #include "swd_device.cuh"
 
@@ -154,6 +154,69 @@ __global__ void window_sample_pauli_kernel(const u32 *__restrict__ thr3, u32 t_e
         __syncwarp();
         for (int i = lane; i < num_det; i += 32) det[b * num_det + i] = (u8)((dbits[i >> 5] >> (i & 31)) & 1u);
         if (obs) for (int i = lane; i < num_obs; i += 32) obs[b * num_obs + i] = (u8)((obits[i >> 5] >> (i & 31)) & 1u);
+        __syncwarp();
+    }
+}
+
+// ----------------------------------------------------------------------------------------------
+// Circuit-level noise with heralded erasures, sampled per noise location (dem.noise_locations: one per DEPOLARIZE2, one per
+// target of X_ERROR / Z_ERROR / DEPOLARIZE1) rather than per merged DEM column.  Location l has n_l <= 15 mechanisms
+// mech[m0 .. m0 + n_l - 1] = (DEM column or -1, thr(p)) and uses draws t = 0 .. n_l: draw t is word t & 3 of the Philox call
+// with counter (l, 2 + (t >> 2), shot) - tags 0 and 1 belong to window_sample_kernel and window_sample_pauli_kernel.  Draw 0
+// is the erasure draw (erased iff w < thr(e_l)); draw 1 + k is mechanism k, which fires iff w < (erased ? 2^31 : thr(p_k)).
+// Every draw is made.  Lanes take locations from a work list sorted by n_l, work[i] = (l, m0, n_l, thr(e_l)), so that the
+// lanes of a warp make the same number of calls; the result depends on l only.  One warp per shot; a fired mechanism with a
+// column XORs that column of chk / obs into the shared-memory parity words (and its bit into the err words when err is
+// requested); an erased location ORs its columns into the erased-column words when channel_llr is requested.
+// channel_llr [B][num_col] = col_llr with 0.0 at the erased columns (no log on the device).
+// ----------------------------------------------------------------------------------------------
+__global__ void window_sample_circuit_kernel(const uint4 *__restrict__ work, int num_loc, const uint2 *__restrict__ mech,
+                                             const double *__restrict__ col_llr, int num_col,
+                                             const int *__restrict__ chk_cp, const int *__restrict__ chk_ri, int num_det,
+                                             const int *__restrict__ obs_cp, const int *__restrict__ obs_ri, int num_obs,
+                                             unsigned long long seed, long long shot0, long long B, u8 *__restrict__ det,
+                                             u8 *__restrict__ obs, u8 *__restrict__ err, u8 *__restrict__ erased,
+                                             double *__restrict__ channel_llr) {
+    extern __shared__ u32 s_bits[];        // per warp: det, obs, [err], [erased columns] words
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, wpb = blockDim.x >> 5;
+    const int wd = (num_det + 31) >> 5, wo = (num_obs + 31) >> 5, wc = (num_col + 31) >> 5;
+    const int we = err ? wc : 0, wx = channel_llr ? wc : 0, words = wd + wo + we + wx;
+    u32 *dbits = s_bits + (size_t)wid * words, *obits = dbits + wd, *ebits = obits + wo, *xbits = ebits + we;
+    for (long long b = (long long)blockIdx.x * wpb + wid; b < B; b += (long long)gridDim.x * wpb) {
+        for (int i = lane; i < words; i += 32) dbits[i] = 0;
+        __syncwarp();
+        const unsigned long long shot = (unsigned long long)(shot0 + b);
+        for (int i = lane; i < num_loc; i += 32) {
+            const uint4 wk = work[i];                   // (l, m0, n_l, thr(e_l))
+            const int n = (int)wk.z;
+            bool er = false;
+            for (int call = 0; 4 * call <= n; call++) {
+                u32 r[4];
+                philox4x32_10(wk.x, 2u + (u32)call, (u32)shot, (u32)(shot >> 32), (u32)seed, (u32)(seed >> 32), r);
+#pragma unroll
+                for (int q = 0; q < 4; q++) {
+                    const int t = 4 * call + q;
+                    if (t > n) break;
+                    if (t == 0) { er = r[0] < wk.w; continue; }
+                    const uint2 m = mech[wk.y + t - 1];
+                    const int c = (int)m.x;
+                    if (c < 0) continue;
+                    if (r[q] < (er ? 0x80000000u : m.y)) {
+                        xor_column(c, chk_cp, chk_ri, dbits);
+                        if (num_obs > 0) xor_column(c, obs_cp, obs_ri, obits);
+                        if (err) atomicXor(&ebits[c >> 5], 1u << (c & 31));
+                    }
+                    if (er && channel_llr) atomicOr(&xbits[c >> 5], 1u << (c & 31));
+                }
+            }
+            if (erased) erased[b * num_loc + wk.x] = (u8)er;
+        }
+        __syncwarp();
+        for (int i = lane; i < num_det; i += 32) det[b * num_det + i] = (u8)((dbits[i >> 5] >> (i & 31)) & 1u);
+        if (obs) for (int i = lane; i < num_obs; i += 32) obs[b * num_obs + i] = (u8)((obits[i >> 5] >> (i & 31)) & 1u);
+        if (err) for (int i = lane; i < num_col; i += 32) err[b * num_col + i] = (u8)((ebits[i >> 5] >> (i & 31)) & 1u);
+        if (channel_llr)
+            for (int i = lane; i < num_col; i += 32) channel_llr[b * num_col + i] = ((xbits[i >> 5] >> (i & 31)) & 1u) ? 0.0 : col_llr[i];
         __syncwarp();
     }
 }

@@ -17,6 +17,7 @@ Symptom sets are Python ints used as bit masks: bit d = detector d, bit num_dete
 observable o.
 """
 import math
+from dataclasses import dataclass
 
 import numpy as np
 from scipy.sparse import csc_matrix
@@ -279,13 +280,11 @@ def shyps_memory_circuit(r, p, num_repeat, z_basis=True):
     return c
 
 
-def detector_error_model(circ):
-    """-> (symptoms list[int], probs list[float], num_detectors, num_observables).
-
-    One entry per distinct non-empty symptom set; identical symptoms are merged with
-    p <- p1 (1-p2) + p2 (1-p1).  Entries are sorted lexicographically by their (detectors...,
-    observables...) target lists, detectors before observables.
-    """
+def _backward_pass(circ, record=None):
+    """Backward Pauli-sensitivity propagation over `circ` -> {symptom: merged probability} (mechanisms with an empty symptom
+    or p <= 0 are dropped; identical symptoms merge with p <- p1 (1-p2) + p2 (1-p1) in the order the pass meets them).
+    record: optional list; one entry (op index, target position, kind, [symptom per mechanism], [probability per mechanism])
+    is appended per noise location, in the pass's (backward) order, with the mechanisms in the order they are merged."""
     ND = circ.num_detectors
     # measurement index -> symptom mask
     meas_mask = {}
@@ -305,8 +304,15 @@ def detector_error_model(circ):
         q = merged.get(sym)
         merged[sym] = p if q is None else q * (1.0 - p) + p * (1.0 - q)
 
+    def location(oi, pos, name, syms, p):
+        for s in syms:
+            add(s, p)
+        if record is not None:
+            record.append((oi, pos, name, syms, p))
+
     mi = circ.num_measurements
-    for name, t, arg in reversed(circ.ops):
+    for oi in range(len(circ.ops) - 1, -1, -1):
+        name, t, arg = circ.ops[oi]
         if name == "CNOT":
             c_, t_ = t
             xs[c_] = xs.get(c_, 0) ^ xs.get(t_, 0)      # X on control spreads to target
@@ -334,36 +340,94 @@ def detector_error_model(circ):
             for q in t:
                 xs[q] = 0; zs[q] = 0
         elif name == "X_ERROR":
-            for q in t:
-                add(xs.get(q, 0), arg)
+            for k, q in enumerate(t):
+                location(oi, k, name, (xs.get(q, 0),), arg)
         elif name == "Z_ERROR":
-            for q in t:
-                add(zs.get(q, 0), arg)
+            for k, q in enumerate(t):
+                location(oi, k, name, (zs.get(q, 0),), arg)
         elif name == "DEPOLARIZE1":
             pc = 0.5 - 0.5 * math.sqrt(1.0 - 4.0 * arg / 3.0)
-            for q in t:
+            for k, q in enumerate(t):
                 x, z = xs.get(q, 0), zs.get(q, 0)
-                add(x, pc); add(z, pc); add(x ^ z, pc)
+                location(oi, k, name, (x, z, x ^ z), pc)
         elif name == "DEPOLARIZE2":
             pc = 0.5 - 0.5 * (1.0 - 16.0 * arg / 15.0) ** 0.125
             a, b = t
             pa = (0, xs.get(a, 0), zs.get(a, 0), xs.get(a, 0) ^ zs.get(a, 0))
             pb = (0, xs.get(b, 0), zs.get(b, 0), xs.get(b, 0) ^ zs.get(b, 0))
-            for i in range(4):
-                for j in range(4):
-                    if i or j:
-                        add(pa[i] ^ pb[j], pc)
+            location(oi, 0, name, tuple(pa[i] ^ pb[j] for i in range(4) for j in range(4) if i or j), pc)
         elif name in ("DETECTOR", "OBSERVABLE_INCLUDE", "TICK"):
             pass
         else:
             raise NotImplementedError(name)
     assert mi == 0
+    return merged
 
+
+def _sorted_dem(merged, circ):
     def targets(sym):
         return tuple(i for i in range(sym.bit_length()) if (sym >> i) & 1)
 
     items = sorted(merged.items(), key=lambda kv: targets(kv[0]))
-    return [k for k, _ in items], [v for _, v in items], ND, circ.num_observables
+    return [k for k, _ in items], [v for _, v in items], circ.num_detectors, circ.num_observables
+
+
+def detector_error_model(circ):
+    """-> (symptoms list[int], probs list[float], num_detectors, num_observables).
+
+    One entry per distinct non-empty symptom set; identical symptoms are merged with
+    p <- p1 (1-p2) + p2 (1-p1).  Entries are sorted lexicographically by their (detectors...,
+    observables...) target lists, detectors before observables.
+    """
+    return _sorted_dem(_backward_pass(circ), circ)
+
+
+NOISE_KINDS = ("X_ERROR", "Z_ERROR", "DEPOLARIZE1", "DEPOLARIZE2")
+
+
+@dataclass
+class NoiseLocations:
+    """The noise locations of a circuit and their independent mechanisms (see `noise_locations`)."""
+    kind: np.ndarray          # [L] str: the instruction of location l (one of NOISE_KINDS)
+    op: np.ndarray            # [L] int32: index of that instruction in circ.ops
+    mech_ptr: np.ndarray      # [L + 1] int32: the mechanisms of location l are mech_ptr[l] .. mech_ptr[l + 1] - 1
+    mech_col: np.ndarray      # [M] int32: DEM column of the mechanism's symptom, -1 if it has none
+    mech_prob: np.ndarray     # [M] float64: the mechanism's probability
+    mech_unmapped: np.ndarray  # [M] bool: non-empty symptom that is no DEM column (only when every mechanism with it has p = 0)
+
+    @property
+    def num_locations(self):
+        return len(self.kind)
+
+
+def _noise_locations(circ):
+    """-> (NoiseLocations, detector_error_model(circ)) from one backward pass."""
+    rec = []
+    dem = _sorted_dem(_backward_pass(circ, rec), circ)
+    rec.sort(key=lambda r: (r[0], r[1]))                 # program order
+    col = {s: j for j, s in enumerate(dem[0])}
+    counts = [len(r[3]) for r in rec]
+    mech_ptr = np.zeros(len(rec) + 1, dtype=np.int32)
+    mech_ptr[1:] = np.cumsum(counts)
+    syms = [s for r in rec for s in r[3]]
+    locs = NoiseLocations(kind=np.array([r[2] for r in rec], dtype=object),
+                          op=np.array([r[0] for r in rec], dtype=np.int32),
+                          mech_ptr=mech_ptr,
+                          mech_col=np.array([col.get(s, -1) for s in syms], dtype=np.int32),
+                          mech_prob=np.repeat(np.array([r[4] for r in rec], dtype=np.float64), counts),
+                          mech_unmapped=np.array([s != 0 and s not in col for s in syms], dtype=bool))
+    return locs, dem
+
+
+def noise_locations(circ):
+    """The noise locations of `circ` in program order: one per DEPOLARIZE2 instruction, one per target of an X_ERROR,
+    Z_ERROR or DEPOLARIZE1 instruction.  Each carries the independent mechanisms `detector_error_model` adds for it, in
+    the same order: X_ERROR / Z_ERROR one (probability p), DEPOLARIZE1 three (x, z, x^z; pc = 1/2 - 1/2 sqrt(1 - 4p/3)),
+    DEPOLARIZE2 fifteen ((i, j) != (0, 0) of the products of (I, X, Z, Y) on the two targets in row-major order;
+    pc = 1/2 - 1/2 (1 - 16p/15)^(1/8)).  mech_col refers to the column order of
+    dem_to_check_matrices(detector_error_model(circ)): XOR-combining mech_prob per column, locations last to first
+    (the targets of one instruction first to last), reproduces its priors bit for bit.  -> NoiseLocations."""
+    return _noise_locations(circ)[0]
 
 
 def dem_to_check_matrices(dem):

@@ -7,6 +7,10 @@
 `depolarizing_noise_decoding(code, p, num_shots, erasure_rate)` is the `bp4_osd` counterpart under depolarizing noise with
 heralded erasures: `CodeCapacitySampler` draws the errors, erasures and per-shot LLR planes on the device, and the commit /
 count kernels of the window driver score the corrections, so no shot data crosses PCIe.
+
+`CircuitNoiseSampler(circ, erasure_rate)` is the circuit-level counterpart: it samples the noise locations of an `Ops` circuit
+(dem.noise_locations), with heralded erasures, on the device and returns shots in the DEM's column order together with the
+per-shot LLR rows that `SlidingWindowDecoder.decode_device(channel_llr=...)` takes.
 """
 import ctypes as C
 import time
@@ -207,3 +211,93 @@ def depolarizing_noise_decoding(code, p, num_shots=1000, erasure_rate=0.0, batch
     if verbose:
         print("Elapsed time:", elapsed)
     return results
+
+
+class CircuitNoiseSampler:
+    """Circuit-level noise with heralded erasures, sampled per noise location on the device (`swd_window_sample_circuit`).
+
+    The locations are those of `dem.noise_locations(circ)`: one per DEPOLARIZE2 instruction, one per target of X_ERROR,
+    Z_ERROR or DEPOLARIZE1.  An erased location carries a uniformly random Pauli (each of its independent mechanisms fires
+    with probability 1/2); any other location keeps its Pauli channel, so at erasure rate 0 the shots have the law of the
+    DEM sampler.  `erasure_rate`: a scalar applies to every DEPOLARIZE2 location (gate erasure conversion), an array gives
+    one rate per location.  `.chk, .obs, .priors` are dem_to_check_matrices(detector_error_model(circ)) and
+    `.channel_llr` [num_col] their static LLRs log((1-p)/p); a shot's LLR row is 0.0 at the columns of its erased locations.
+    Shot s of a call depends only on (seed, shot_offset + s)."""
+
+    def __init__(self, circ, erasure_rate=0.0, device=0):
+        from .decoders import _libm_llr
+        from .dem import _noise_locations, dem_to_check_matrices
+        locs, dem = _noise_locations(circ)
+        L = locs.num_locations
+        if L == 0:
+            raise ValueError("the circuit has no noise locations")
+        if np.ndim(erasure_rate) == 0:
+            e = float(erasure_rate)
+            if not 0.0 <= e <= 1.0:
+                raise ValueError(f"erasure_rate must lie in [0, 1], got {e}")
+            rate = np.where(locs.kind == "DEPOLARIZE2", e, 0.0)
+        else:
+            rate = np.ascontiguousarray(erasure_rate, dtype=np.float64)
+            if rate.shape != (L,):
+                raise ValueError(f"erasure_rate must be a scalar or have shape ({L},) (one rate per noise location), got {rate.shape}")
+            if not ((rate >= 0.0) & (rate <= 1.0)).all():
+                raise ValueError("erasure_rate must lie in [0, 1] (and not be NaN) at every location")
+        lost = np.add.reduceat(locs.mech_unmapped.astype(np.int64), locs.mech_ptr[:-1]) > 0
+        if (lost & (rate > 0)).any():
+            raise ValueError(f"location {int(np.flatnonzero(lost & (rate > 0))[0])} has a non-zero erasure rate but a mechanism "
+                             "whose symptom is no DEM column (its probability is 0): its erasure cannot be represented")
+        chk, obs, priors = dem_to_check_matrices(dem)
+        chk.sort_indices(); obs.sort_indices()
+        import torch
+        self.torch = torch
+        self.device = int(device)
+        self.chk, self.obs, self.priors = chk, obs, priors
+        self.num_det, self.num_col = chk.shape
+        self.num_obs = obs.shape[0]
+        self.locations, self.num_locations = locs, L
+        self.erasure_rate = rate
+        self.channel_llr = _libm_llr(priors, self.num_col)
+        self._cp = (np.ascontiguousarray(chk.indptr, dtype=np.int32), np.ascontiguousarray(chk.indices, dtype=np.int32),
+                    np.ascontiguousarray(obs.indptr, dtype=np.int32), np.ascontiguousarray(obs.indices, dtype=np.int32))
+        self.lib = _lib.load()
+        i32p, dp = C.POINTER(C.c_int32), C.POINTER(C.c_double)
+        self._win = C.c_void_p()
+        _lib.check(self.lib.swd_window_create(self.device, self.num_det, self.num_col, *(a.ctypes.data_as(i32p) for a in self._cp[:2]),
+                                              self.num_obs, *(a.ctypes.data_as(i32p) for a in self._cp[2:]), C.byref(self._win)),
+                   "swd_window_create")
+        _lib.check(self.lib.swd_window_set_circuit_noise(self._win, L, locs.mech_ptr.ctypes.data_as(i32p), locs.mech_col.ctypes.data_as(i32p),
+                                                         locs.mech_prob.ctypes.data_as(dp), rate.ctypes.data_as(dp),
+                                                         self.channel_llr.ctypes.data_as(dp)),
+                   "swd_window_set_circuit_noise")
+
+    def __del__(self):
+        w = getattr(self, "_win", None)
+        if w is not None and w.value:
+            self.lib.swd_window_destroy(w)
+            self._win = C.c_void_p()
+
+    def sample(self, B, seed=0, shot_offset=0, return_errors=False, return_erasures=False, return_llr=False):
+        """-> (det [B, num_det], obs [B, num_obs][, err [B, num_col]][, erased [B, num_locations]] uint8
+        [, channel_llr [B, num_col] float64]) as torch CUDA tensors written on the current stream.  Columns are in the DEM's
+        order (what build_windows and decode_device(channel_llr=...) take); err is the parity of the fired mechanisms per
+        column, so det = chk . err and obs = obs . err."""
+        B, seed, shot_offset = int(B), int(seed), int(shot_offset)
+        if B < 0 or shot_offset < 0 or not 0 <= seed < 1 << 64:
+            raise ValueError(f"need B >= 0, shot_offset >= 0 and 0 <= seed < 2**64 (got {B}, {shot_offset}, {seed})")
+        torch = self.torch
+        dev = torch.device("cuda", self.device)
+        u8 = dict(dtype=torch.uint8, device=dev)
+        out = dict(det=torch.empty((B, self.num_det), **u8), obs=torch.empty((B, self.num_obs), **u8))
+        if return_errors:
+            out["err"] = torch.empty((B, self.num_col), **u8)
+        if return_erasures:
+            out["erased"] = torch.empty((B, self.num_locations), **u8)
+        if return_llr:
+            out["channel_llr"] = torch.empty((B, self.num_col), dtype=torch.float64, device=dev)
+        if B:
+            ptr = lambda k: out[k].data_ptr() if k in out and out[k].numel() else None    # noqa: E731
+            stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+            _lib.check(self.lib.swd_window_sample_circuit(self._win, seed, shot_offset, B, ptr("det"), ptr("obs"), ptr("err"),
+                                                          ptr("erased"), ptr("channel_llr"), stream),
+                       "swd_window_sample_circuit")
+        return tuple(out[k] for k in ("det", "obs", "err", "erased", "channel_llr") if k in out)
