@@ -250,6 +250,34 @@ int  swd_window_set_circuit_noise(swd_window *w, int num_loc, const int32_t *mec
 int  swd_window_sample_circuit(swd_window *w, uint64_t seed, int64_t shot_offset, int64_t B, uint8_t *d_det, uint8_t *d_obs,
                                uint8_t *d_err, uint8_t *d_erased, double *d_channel_llr, void *stream);
 
+/* Soft measurement readout on top of the circuit noise above.  A readout location is an X_ERROR (Z_ERROR) target whose next
+ * instruction on that qubit is M / MR (MX / MRX): dem.readout_locations.  readout_loc [num_readout] lists them (indices into
+ * the locations of swd_window_set_circuit_noise, each with exactly one mechanism, no two with the same DEM column).  The K =
+ * num_classes (1 .. 256) reliability classes are shared by all of them: a readout location draws class k with probability
+ * class_weight[k] (>= 0, summing to 1 within 1e-9) and then flips with probability flip_prob[k] in [0, 1/2] (its own
+ * probability in mech_prob is not used).  class_llr [num_readout * K] (host, row r = readout r; NULL if no LLR rows will be
+ * asked for) is the LLR of readout r's DEM column when r is in class k; rows of readouts without a column are not read.
+ * swd_window_set_circuit_readout copies the tables; SWD_ERR_INVALID for a NULL table, num_readout <= 0, a call before
+ * swd_window_set_circuit_noise, a location out of range or listed twice, a location with n_l != 1, K outside 1 .. 256, a
+ * negative or NaN weight, weights summing to more than 1e-9 away from 1, a flip_prob outside [0, 1/2] (NaN included), or
+ * two readout locations whose mechanisms share a DEM column.  A later swd_window_set_circuit_noise clears it, and
+ * swd_window_sample_circuit ignores it.
+ * swd_window_sample_circuit_readout: every location draws as in swd_window_sample_circuit except readout locations, which
+ * use words 0, 1, 2 of their one Philox call (counter (l, 2, s & 0xffffffff, s >> 32)): word 0 is the erasure draw, word 2
+ * the class (the number of k in 1 .. K-1 with w >= thr(class_weight[0] + .. + class_weight[k-1]), sums left to right in
+ * double) and word 1 the flip, which fires iff w < (erased ? 0x80000000 : thr(flip_prob[class])).  With K = 1 and flip_prob
+ * = {p} it reproduces swd_window_sample_circuit.  Outputs as swd_window_sample_circuit, plus optional d_readout
+ * [B][num_readout] (the classes, in readout_loc order); d_channel_llr [B][num_col] is col_llr with class_llr[r][class_r] at
+ * readout r's column and 0.0 at every column of an erased location (needs col_llr and class_llr).  SWD_ERR_INVALID before
+ * swd_window_set_circuit_readout and for the pointer / size errors of swd_window_sample_circuit; SWD_ERR_UNSUPPORTED if one
+ * warp's words and class bytes do not fit in shared memory. */
+int  swd_window_set_circuit_readout(swd_window *w, int num_readout, const int32_t *readout_loc, int num_classes,
+                                    const double *class_weight /* [K] */, const double *flip_prob /* [K] */,
+                                    const double *class_llr /* [num_readout * K] host, may be NULL */);
+int  swd_window_sample_circuit_readout(swd_window *w, uint64_t seed, int64_t shot_offset, int64_t B, uint8_t *d_det,
+                                       uint8_t *d_obs, uint8_t *d_err, uint8_t *d_erased, uint8_t *d_readout,
+                                       double *d_channel_llr, void *stream);
+
 /* ---- bp4_osd (src/bp4_osd.pyx:6-684): quaternary min-sum BP over the pair (Hx, Hz) of a CSS code under depolarizing
  * noise, then one OSD per basis for shots whose BP did not converge.  Replaces bp4_osd.__cinit__ / decode (pyx:8-221);
  * swd_bp4_camel_decode_batch_host replaces camel_decode (pyx:223-248).  The two graphs have no column- / row-weight limit

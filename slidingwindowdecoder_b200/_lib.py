@@ -39,6 +39,7 @@ EXPORTS = ["swd_create", "swd_destroy", "swd_decode_batch_host", "swd_decode_bat
            "swd_set_profiling", "swd_get_kernel_times", "swd_get_counters", "swd_reset_counters", "swd_rank", "swd_new_n", "swd_window_create", "swd_window_destroy",
            "swd_window_extract", "swd_window_commit", "swd_window_count_failures", "swd_window_set_priors", "swd_window_sample",
            "swd_window_set_pauli_priors", "swd_window_sample_pauli", "swd_window_set_circuit_noise", "swd_window_sample_circuit",
+           "swd_window_set_circuit_readout", "swd_window_sample_circuit_readout",
            "swd_bp4_create", "swd_bp4_destroy", "swd_bp4_rank", "swd_bp4_decode_batch_host", "swd_bp4_camel_decode_batch_host", "swd_bp4_decode_batch_device", "swd_bp4_camel_decode_batch_device",
            "swd_bp4_decode_batch_host_llr", "swd_bp4_decode_batch_device_llr", "swd_bp4_camel_decode_batch_host_llr",
            "swd_bp4_camel_decode_batch_device_llr", "swd_strerror", "swd_last_error",
@@ -121,6 +122,10 @@ def load():
     lib.swd_window_set_circuit_noise.restype = C.c_int
     lib.swd_window_sample_circuit.argtypes = [vp, C.c_uint64, C.c_int64, C.c_int64, u8p, u8p, u8p, u8p, dp, vp]
     lib.swd_window_sample_circuit.restype = C.c_int
+    lib.swd_window_set_circuit_readout.argtypes = [vp, C.c_int, i32p, C.c_int] + [C.POINTER(C.c_double)] * 3
+    lib.swd_window_set_circuit_readout.restype = C.c_int
+    lib.swd_window_sample_circuit_readout.argtypes = [vp, C.c_uint64, C.c_int64, C.c_int64, u8p, u8p, u8p, u8p, u8p, dp, vp]
+    lib.swd_window_sample_circuit_readout.restype = C.c_int
     lib.swd_bp4_create.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, i32p, i32p, i32p, i32p] + [C.POINTER(C.c_double)] * 5 + \
                                   [C.c_int, C.c_double, C.c_int, C.c_int, C.POINTER(vp)]
     lib.swd_bp4_create.restype = C.c_int

@@ -1159,7 +1159,22 @@ struct swd_window {
     uint2 *circ_mech = nullptr;  // (DEM column or -1, thr(p)) per mechanism
     double *circ_llr = nullptr;  // static LLR row [num_col], or nullptr
     int circ_num_loc = 0;        // 0 until swd_window_set_circuit_noise
+    std::vector<uint4> circ_work_h;   // host copies of circ_work and of the mechanisms' columns (readout set-up reads them)
+    std::vector<int> circ_col_h;
+    uint4 *ro_work = nullptr;    // soft readout (swd_window_set_circuit_readout): circ_work with z = 1 | (r + 1) << 4 at readout r
+    u32 *ro_thr = nullptr;       // thr(w_0 + .. + w_{k-1}) for k = 1 .. K-1, then thr(q_k) for k = 0 .. K-1
+    int *ro_col = nullptr;       // [num_col] readout location whose mechanism is in column c, or -1
+    double *ro_llr = nullptr;    // class_llr [num_readout][K], or nullptr
+    int ro_num = 0, ro_K = 0;    // 0 until swd_window_set_circuit_readout
 };
+
+static void clear_circuit_readout(swd_window *w) {
+    if (w->ro_work) { cudaFree(w->ro_work); w->ro_work = nullptr; }
+    if (w->ro_thr) { cudaFree(w->ro_thr); w->ro_thr = nullptr; }
+    if (w->ro_col) { cudaFree(w->ro_col); w->ro_col = nullptr; }
+    if (w->ro_llr) { cudaFree(w->ro_llr); w->ro_llr = nullptr; }
+    w->ro_num = w->ro_K = 0;
+}
 
 extern "C" int swd_window_create(int device, int num_det, int num_col, const int32_t *chk_cp, const int32_t *chk_ri, int num_obs,
                                  const int32_t *obs_cp, const int32_t *obs_ri, swd_window **out) {
@@ -1192,6 +1207,7 @@ extern "C" void swd_window_destroy(swd_window *w) {
     if (w->circ_work) cudaFree(w->circ_work);
     if (w->circ_mech) cudaFree(w->circ_mech);
     if (w->circ_llr) cudaFree(w->circ_llr);
+    clear_circuit_readout(w);
     delete w;
 }
 extern "C" int swd_window_set_priors(swd_window *w, const double *priors) {
@@ -1276,11 +1292,84 @@ extern "C" int swd_window_set_circuit_noise(swd_window *w, int num_loc, const in
     if (w->circ_work) { cudaFree(w->circ_work); w->circ_work = nullptr; }
     if (w->circ_mech) { cudaFree(w->circ_mech); w->circ_mech = nullptr; }
     if (w->circ_llr) { cudaFree(w->circ_llr); w->circ_llr = nullptr; }
+    clear_circuit_readout(w);
     w->circ_num_loc = 0;
     int st;
     if ((st = upload(work, (void **)&w->circ_work)) || (st = upload(mech, (void **)&w->circ_mech))) return st;
     if (col_llr && (st = upload(std::vector<double>(col_llr, col_llr + w->num_col), (void **)&w->circ_llr))) return st;
+    w->circ_work_h = work;
+    w->circ_col_h.assign(mech_col, mech_col + M);
     w->circ_num_loc = num_loc;
+    return SWD_OK;
+}
+extern "C" int swd_window_set_circuit_readout(swd_window *w, int num_readout, const int32_t *readout_loc, int num_classes,
+                                              const double *class_weight, const double *flip_prob, const double *class_llr) {
+    if (!w || num_readout <= 0 || !readout_loc || !class_weight || !flip_prob) { set_err("swd_window_set_circuit_readout: bad argument"); return SWD_ERR_INVALID; }
+    if (!w->circ_num_loc) { set_err("swd_window_set_circuit_readout: call swd_window_set_circuit_noise first"); return SWD_ERR_INVALID; }
+    const int K = num_classes, L = w->circ_num_loc;
+    if (K < 1 || K > 256) { set_err("swd_window_set_circuit_readout: num_classes outside 1 .. 256"); return SWD_ERR_INVALID; }
+    std::vector<u32> thr(2 * K - 1);
+    double sum = 0.0;
+    for (int k = 0; k < K; k++) {
+        const double x = class_weight[k], q = flip_prob[k];
+        if (!(x >= 0.0)) { set_err("swd_window_set_circuit_readout: a class weight is negative or NaN"); return SWD_ERR_INVALID; }
+        if (!(q >= 0.0 && q <= 0.5)) { set_err("swd_window_set_circuit_readout: flip_prob outside [0, 1/2]"); return SWD_ERR_INVALID; }
+        if (k > 0) thr[k - 1] = prob_threshold(sum);
+        sum += x;
+        thr[K - 1 + k] = prob_threshold(q);
+    }
+    if (!(std::fabs(sum - 1.0) <= 1e-9)) { set_err("swd_window_set_circuit_readout: class weights do not sum to 1"); return SWD_ERR_INVALID; }
+    std::vector<int> slot(L, -1), col_ro(w->num_col, -1);       // slot[l]: position of location l in circ_work
+    for (int i = 0; i < L; i++) slot[w->circ_work_h[i].x] = i;
+    std::vector<uint4> work = w->circ_work_h;
+    for (int r = 0; r < num_readout; r++) {
+        const int l = readout_loc[r];
+        if (l < 0 || l >= L) { set_err("swd_window_set_circuit_readout: readout_loc outside [0, num_loc)"); return SWD_ERR_INVALID; }
+        uint4 &wk = work[slot[l]];
+        if (wk.z >> 4) { set_err("swd_window_set_circuit_readout: a location is listed twice"); return SWD_ERR_INVALID; }
+        if (wk.z != 1) { set_err("swd_window_set_circuit_readout: a readout location needs exactly one mechanism"); return SWD_ERR_INVALID; }
+        const int c = w->circ_col_h[wk.y];
+        if (c >= 0) {
+            if (col_ro[c] >= 0) { set_err("swd_window_set_circuit_readout: two readout locations share a DEM column"); return SWD_ERR_INVALID; }
+            col_ro[c] = r;
+        }
+        wk.z = 1u | (u32)(r + 1) << 4;
+    }
+    // readout items last among the single-mechanism locations, so that fewer warps mix the two paths
+    std::stable_sort(work.begin(), work.end(), [](const uint4 &a, const uint4 &b) {
+        return (a.z & 15u) != (b.z & 15u) ? (a.z & 15u) > (b.z & 15u) : (a.z >> 4 == 0) && (b.z >> 4 != 0);
+    });
+    CK(cudaSetDevice(w->device));
+    clear_circuit_readout(w);
+    int st;
+    if ((st = upload(work, (void **)&w->ro_work)) || (st = upload(thr, (void **)&w->ro_thr)) || (st = upload(col_ro, (void **)&w->ro_col))) {
+        clear_circuit_readout(w); return st;
+    }
+    if (class_llr && (st = upload(std::vector<double>(class_llr, class_llr + (size_t)num_readout * K), (void **)&w->ro_llr))) {
+        clear_circuit_readout(w); return st;
+    }
+    w->ro_num = num_readout;
+    w->ro_K = K;
+    return SWD_OK;
+}
+// one warp per shot, up to 8 warps per block; the per-warp words (and readout class bytes) live in dynamic shared memory
+template <bool READOUT>
+static int launch_sample_circuit(swd_window *w, const uint4 *work, const CircuitReadout &ro, uint64_t seed, int64_t shot_offset,
+                                 int64_t B, uint8_t *d_det, uint8_t *d_obs, uint8_t *d_err, uint8_t *d_erased, double *d_channel_llr,
+                                 void *stream, const char *who) {
+    CK(cudaSetDevice(w->device));
+    const int wc = (w->num_col + 31) >> 5;
+    const size_t warp_bytes = (size_t)(((w->num_det + 31) >> 5) + ((w->num_obs + 31) >> 5) + (d_err ? wc : 0) + (d_channel_llr ? wc : 0) +
+                                       (READOUT && d_channel_llr ? (ro.num_readout + 3) >> 2 : 0)) * sizeof(u32);
+    const size_t limit = 200 * 1024;
+    if (warp_bytes > limit) { set_err(std::string(who) + ": one warp's parity and column words exceed the shared-memory limit"); return SWD_ERR_UNSUPPORTED; }
+    const int wpb = (int)std::min<size_t>(8, limit / warp_bytes);
+    const size_t smem = (size_t)wpb * warp_bytes;
+    if (smem > 48 * 1024) CK(cudaFuncSetAttribute(window_sample_circuit_kernel<READOUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    window_sample_circuit_kernel<READOUT><<<(unsigned)std::min<long long>((B + wpb - 1) / wpb, 148 * 16), wpb * 32, smem, (cudaStream_t)stream>>>(
+        work, w->circ_num_loc, w->circ_mech, w->circ_llr, w->num_col, w->chk_cp, w->chk_ri, w->num_det, w->obs_cp, w->obs_ri,
+        w->num_obs, (unsigned long long)seed, (long long)shot_offset, (long long)B, d_det, d_obs, d_err, d_erased, d_channel_llr, ro);
+    CK(cudaGetLastError());
     return SWD_OK;
 }
 extern "C" int swd_window_sample_circuit(swd_window *w, uint64_t seed, int64_t shot_offset, int64_t B, uint8_t *d_det, uint8_t *d_obs,
@@ -1289,19 +1378,21 @@ extern "C" int swd_window_sample_circuit(swd_window *w, uint64_t seed, int64_t s
     if (!w->circ_num_loc) { set_err("swd_window_sample_circuit: call swd_window_set_circuit_noise first"); return SWD_ERR_INVALID; }
     if (d_channel_llr && !w->circ_llr) { set_err("swd_window_sample_circuit: channel_llr needs the col_llr row of swd_window_set_circuit_noise"); return SWD_ERR_INVALID; }
     if (B == 0) return SWD_OK;
-    CK(cudaSetDevice(w->device));
-    const int wc = (w->num_col + 31) >> 5;
-    const size_t warp_bytes = (size_t)(((w->num_det + 31) >> 5) + ((w->num_obs + 31) >> 5) + (d_err ? wc : 0) + (d_channel_llr ? wc : 0)) * sizeof(u32);
-    const size_t limit = 200 * 1024;
-    if (warp_bytes > limit) { set_err("swd_window_sample_circuit: one warp's parity and column words exceed the shared-memory limit"); return SWD_ERR_UNSUPPORTED; }
-    const int wpb = (int)std::min<size_t>(8, limit / warp_bytes);
-    const size_t smem = (size_t)wpb * warp_bytes;
-    if (smem > 48 * 1024) CK(cudaFuncSetAttribute(window_sample_circuit_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    window_sample_circuit_kernel<<<(unsigned)std::min<long long>((B + wpb - 1) / wpb, 148 * 16), wpb * 32, smem, (cudaStream_t)stream>>>(
-        w->circ_work, w->circ_num_loc, w->circ_mech, w->circ_llr, w->num_col, w->chk_cp, w->chk_ri, w->num_det, w->obs_cp, w->obs_ri,
-        w->num_obs, (unsigned long long)seed, (long long)shot_offset, (long long)B, d_det, d_obs, d_err, d_erased, d_channel_llr);
-    CK(cudaGetLastError());
-    return SWD_OK;
+    return launch_sample_circuit<false>(w, w->circ_work, CircuitReadout{}, seed, shot_offset, B, d_det, d_obs, d_err, d_erased,
+                                        d_channel_llr, stream, "swd_window_sample_circuit");
+}
+extern "C" int swd_window_sample_circuit_readout(swd_window *w, uint64_t seed, int64_t shot_offset, int64_t B, uint8_t *d_det,
+                                                 uint8_t *d_obs, uint8_t *d_err, uint8_t *d_erased, uint8_t *d_readout,
+                                                 double *d_channel_llr, void *stream) {
+    if (!w || !d_det || B < 0 || shot_offset < 0 || (w->num_obs > 0 && !d_obs)) { set_err("swd_window_sample_circuit_readout: bad argument"); return SWD_ERR_INVALID; }
+    if (!w->ro_num) { set_err("swd_window_sample_circuit_readout: call swd_window_set_circuit_readout first"); return SWD_ERR_INVALID; }
+    if (d_channel_llr && (!w->circ_llr || !w->ro_llr)) {
+        set_err("swd_window_sample_circuit_readout: channel_llr needs the col_llr row and the class_llr table"); return SWD_ERR_INVALID;
+    }
+    if (B == 0) return SWD_OK;
+    const CircuitReadout ro{w->ro_thr, w->ro_thr + (w->ro_K - 1), w->ro_col, w->ro_llr, d_readout, w->ro_K, w->ro_num};
+    return launch_sample_circuit<true>(w, w->ro_work, ro, seed, shot_offset, B, d_det, d_obs, d_err, d_erased, d_channel_llr, stream,
+                                       "swd_window_sample_circuit_readout");
 }
 extern "C" int swd_window_sample(swd_window *w, uint64_t seed, int64_t shot_offset, int64_t B, uint8_t *d_det, uint8_t *d_obs,
                                  uint8_t *d_err, void *stream) {

@@ -169,26 +169,74 @@ __global__ void window_sample_pauli_kernel(const u32 *__restrict__ thr3, u32 t_e
 // column XORs that column of chk / obs into the shared-memory parity words (and its bit into the err words when err is
 // requested); an erased location ORs its columns into the erased-column words when channel_llr is requested.
 // channel_llr [B][num_col] = col_llr with 0.0 at the erased columns (no log on the device).
+//
+// READOUT (soft measurement readout, swd_window_sample_circuit_readout): readout location r (an X_ERROR / Z_ERROR target
+// measured next in its basis, n_l = 1) is marked in its work item, work[i].z = 1 | (r + 1) << 4.  It makes the same single
+// Philox call; word 0 is the erasure draw, word 2 the class draw (class = number of k in 1 .. K-1 with w >= ro.cthr[k - 1],
+// a non-decreasing table) and word 1 the flip, which fires iff w < (erased ? 2^31 : ro.qthr[class]).  The class goes to
+// ro.cls [B][num_readout] when requested and, when channel_llr is requested, to a per-warp byte array in shared memory after
+// the erased-column words; the rows then take ro.llr[r][class] at the column of readout r (ro.col_ro[c] = r, or -1) unless
+// that column is erased.  Every other location draws exactly as without READOUT.
 // ----------------------------------------------------------------------------------------------
+struct CircuitReadout {
+    const u32 *cthr;        // [K - 1] thr(w_0 + .. + w_{k-1}), k = 1 .. K-1
+    const u32 *qthr;        // [K] thr(q_k)
+    const int *col_ro;      // [num_col] the readout location whose mechanism is in column c, or -1
+    const double *llr;      // [num_readout][K] per-class LLR of the readout's column (rows only)
+    u8 *cls;                // [B][num_readout] classes out, or nullptr
+    int K, num_readout;
+};
+
+template <bool READOUT>
 __global__ void window_sample_circuit_kernel(const uint4 *__restrict__ work, int num_loc, const uint2 *__restrict__ mech,
                                              const double *__restrict__ col_llr, int num_col,
                                              const int *__restrict__ chk_cp, const int *__restrict__ chk_ri, int num_det,
                                              const int *__restrict__ obs_cp, const int *__restrict__ obs_ri, int num_obs,
                                              unsigned long long seed, long long shot0, long long B, u8 *__restrict__ det,
                                              u8 *__restrict__ obs, u8 *__restrict__ err, u8 *__restrict__ erased,
-                                             double *__restrict__ channel_llr) {
-    extern __shared__ u32 s_bits[];        // per warp: det, obs, [err], [erased columns] words
+                                             double *__restrict__ channel_llr, const CircuitReadout ro) {
+    extern __shared__ u32 s_bits[];        // per warp: det, obs, [err], [erased columns] words, [readout class bytes]
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, wpb = blockDim.x >> 5;
     const int wd = (num_det + 31) >> 5, wo = (num_obs + 31) >> 5, wc = (num_col + 31) >> 5;
-    const int we = err ? wc : 0, wx = channel_llr ? wc : 0, words = wd + wo + we + wx;
+    const int we = err ? wc : 0, wx = channel_llr ? wc : 0;
+    const int words = wd + wo + we + wx + (READOUT && channel_llr ? (ro.num_readout + 3) >> 2 : 0);
     u32 *dbits = s_bits + (size_t)wid * words, *obits = dbits + wd, *ebits = obits + wo, *xbits = ebits + we;
+    u8 *cbytes = (u8 *)(xbits + wx);
     for (long long b = (long long)blockIdx.x * wpb + wid; b < B; b += (long long)gridDim.x * wpb) {
         for (int i = lane; i < words; i += 32) dbits[i] = 0;
         __syncwarp();
         const unsigned long long shot = (unsigned long long)(shot0 + b);
         for (int i = lane; i < num_loc; i += 32) {
             const uint4 wk = work[i];                   // (l, m0, n_l, thr(e_l))
-            const int n = (int)wk.z;
+            if constexpr (READOUT) {
+                if (wk.z >> 4) {                        // readout location r: erasure, flip and class from one call
+                    const int r = (int)(wk.z >> 4) - 1;
+                    u32 w[4];
+                    philox4x32_10(wk.x, 2u, (u32)shot, (u32)(shot >> 32), (u32)seed, (u32)(seed >> 32), w);
+                    const bool er = w[0] < wk.w;
+                    int lo = 0, hi = ro.K - 1;          // upper bound of w[2] in cthr
+                    while (lo < hi) {
+                        const int mid = (lo + hi) >> 1;
+                        if (w[2] >= ro.cthr[mid]) lo = mid + 1; else hi = mid;
+                    }
+                    const int c = (int)mech[wk.y].x;
+                    if (c >= 0) {
+                        if (w[1] < (er ? 0x80000000u : ro.qthr[lo])) {
+                            xor_column(c, chk_cp, chk_ri, dbits);
+                            if (num_obs > 0) xor_column(c, obs_cp, obs_ri, obits);
+                            if (err) atomicXor(&ebits[c >> 5], 1u << (c & 31));
+                        }
+                        if (channel_llr) {
+                            if (er) atomicOr(&xbits[c >> 5], 1u << (c & 31));
+                            cbytes[r] = (u8)lo;
+                        }
+                    }
+                    if (ro.cls) ro.cls[b * ro.num_readout + r] = (u8)lo;
+                    if (erased) erased[b * num_loc + wk.x] = (u8)er;
+                    continue;
+                }
+            }
+            const int n = READOUT ? (int)(wk.z & 15u) : (int)wk.z;
             bool er = false;
             for (int call = 0; 4 * call <= n; call++) {
                 u32 r[4];
@@ -215,7 +263,17 @@ __global__ void window_sample_circuit_kernel(const uint4 *__restrict__ work, int
         for (int i = lane; i < num_det; i += 32) det[b * num_det + i] = (u8)((dbits[i >> 5] >> (i & 31)) & 1u);
         if (obs) for (int i = lane; i < num_obs; i += 32) obs[b * num_obs + i] = (u8)((obits[i >> 5] >> (i & 31)) & 1u);
         if (err) for (int i = lane; i < num_col; i += 32) err[b * num_col + i] = (u8)((ebits[i >> 5] >> (i & 31)) & 1u);
-        if (channel_llr)
+        if constexpr (READOUT) {
+            if (channel_llr)
+                for (int i = lane; i < num_col; i += 32) {
+                    double v = 0.0;
+                    if (!((xbits[i >> 5] >> (i & 31)) & 1u)) {
+                        const int r = ro.col_ro[i];
+                        v = r >= 0 ? ro.llr[(size_t)r * ro.K + cbytes[r]] : col_llr[i];
+                    }
+                    channel_llr[b * num_col + i] = v;
+                }
+        } else if (channel_llr)
             for (int i = lane; i < num_col; i += 32) channel_llr[b * num_col + i] = ((xbits[i >> 5] >> (i & 31)) & 1u) ? 0.0 : col_llr[i];
         __syncwarp();
     }

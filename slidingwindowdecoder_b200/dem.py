@@ -11,7 +11,9 @@ turns `circuit.detector_error_model()` into (chk, obs, priors) with dem_to_check
   * `detector_error_model`: backward Pauli-sensitivity propagation (which detectors/observables
     would an X or Z fault at this point flip), independent-mechanism probabilities for the
     depolarising channels, and merging of mechanisms with identical symptoms,
-  * `dem_to_check_matrices`: same return values as the reference function.
+  * `dem_to_check_matrices`: same return values as the reference function,
+  * `readout_locations`, `with_readout_error`, `gaussian_readout` / `ReadoutModel`: the measurement flips of a circuit and
+    the soft-readout model that CircuitNoiseSampler samples them with.
 
 Symptom sets are Python ints used as bit masks: bit d = detector d, bit num_detectors + o =
 observable o.
@@ -445,3 +447,111 @@ def dem_to_check_matrices(dem):
     chk = csc_matrix((np.ones(len(rows), dtype=np.uint8), (rows, cols)), shape=(ND, nf))
     obs = csc_matrix((np.ones(len(orow), dtype=np.uint8), (orow, ocol)), shape=(NO, nf))
     return chk, obs, np.array(probs, dtype=np.float64)
+
+
+_READOUT_BASIS = {"X_ERROR": ("M", "MR"), "Z_ERROR": ("MX", "MRX")}
+
+
+def _readout_flips(circ):
+    """-> (readout location indices, {op index: number of its targets that are readout flips}) in one forward scan.  The
+    location index of an X_ERROR / Z_ERROR target is its position in noise_locations' program order."""
+    pending = {}                # qubit -> (location, flip kind, op index) of the last X_ERROR / Z_ERROR on it
+    out, per_op, loc = [], {}, 0
+    for oi, (name, t, _) in enumerate(circ.ops):
+        if name in ("DETECTOR", "OBSERVABLE_INCLUDE", "TICK"):
+            continue
+        for q in t:
+            prev = pending.pop(q, None)
+            if prev is not None and name in _READOUT_BASIS[prev[1]]:
+                out.append(prev[0])
+                per_op[prev[2]] = per_op.get(prev[2], 0) + 1
+        if name in _READOUT_BASIS:
+            for k, q in enumerate(t):
+                pending[q] = (loc + k, name, oi)
+        if name in ("X_ERROR", "Z_ERROR", "DEPOLARIZE1"):
+            loc += len(t)
+        elif name == "DEPOLARIZE2":
+            loc += 1
+    return np.array(sorted(out), dtype=np.int32), per_op
+
+
+def readout_locations(circ):
+    """The measurement flips of `circ`: every X_ERROR (Z_ERROR) target whose next instruction on that qubit is M or MR (MX
+    or MRX), DETECTOR, OBSERVABLE_INCLUDE and TICK skipped.  -> int32 array of indices into noise_locations(circ),
+    increasing.  Each is a single-mechanism location, so soft readout information about it changes one DEM column."""
+    return _readout_flips(circ)[0]
+
+
+def with_readout_error(circ, p_meas):
+    """A copy of `circ` with the probability of every measurement flip (readout_locations) set to p_meas in [0, 1/2], so that
+    readout noise can be set apart from gate noise.  ValueError for an X_ERROR / Z_ERROR instruction whose targets are only
+    partly measurement flips (none of the package's circuits has one)."""
+    p_meas = float(p_meas)
+    if not 0.0 <= p_meas <= 0.5:
+        raise ValueError(f"p_meas must lie in [0, 1/2], got {p_meas}")
+    _, per_op = _readout_flips(circ)
+    out = Ops()
+    out.num_measurements, out.num_detectors, out.num_observables = circ.num_measurements, circ.num_detectors, circ.num_observables
+    out.ops = list(circ.ops)
+    for oi, n in per_op.items():
+        name, t, _ = circ.ops[oi]
+        if n != len(t):
+            raise ValueError(f"instruction {oi} ({name}) has {n} measurement-flip targets out of {len(t)}; split it first")
+        out.ops[oi] = (name, t, p_meas)
+    return out
+
+
+@dataclass
+class ReadoutModel:
+    """Soft measurement readout shared by all readout locations: a location draws reliability class k with probability
+    weights[k] and then flips with probability flip_prob[k].  1 <= K <= 256 classes; weights >= 0 summing to 1 (within
+    1e-9), flip_prob in [0, 1/2].  Its marginal flip probability sum_k weights[k] flip_prob[k] must equal the readout
+    locations' probability in the circuit, so that the DEM and its priors do not change."""
+    weights: np.ndarray
+    flip_prob: np.ndarray
+
+    def __post_init__(self):
+        self.weights = np.array(self.weights, dtype=np.float64).reshape(-1)
+        self.flip_prob = np.array(self.flip_prob, dtype=np.float64).reshape(-1)
+        K = len(self.weights)
+        if not 1 <= K <= 256 or self.flip_prob.shape != (K,):
+            raise ValueError(f"need 1 to 256 classes with one weight and one flip probability each, got {K} and {len(self.flip_prob)}")
+        if not (self.weights >= 0.0).all() or not abs(math.fsum(self.weights) - 1.0) <= 1e-9:
+            raise ValueError("class weights must be non-negative and sum to 1")
+        if not ((self.flip_prob >= 0.0) & (self.flip_prob <= 0.5)).all():
+            raise ValueError("flip probabilities must lie in [0, 1/2]")
+
+    @property
+    def num_classes(self):
+        return len(self.weights)
+
+    @property
+    def marginal(self):
+        """sum_k weights[k] flip_prob[k]: the flip probability of a readout location."""
+        return float(np.dot(self.weights, self.flip_prob))
+
+
+def gaussian_readout(p_meas, num_classes):
+    """ReadoutModel of a symmetric Gaussian readout: the signal is x = +-1 + sigma z with Phi(-1/sigma) = p_meas in (0, 1/2),
+    binned into num_classes equiprobable bins of |x| (class 0 the least reliable), q[k] = P(wrong sign | |x| in bin k).
+    sum w q = p_meas up to rounding; num_classes = 1 gives q = [p_meas]."""
+    from scipy.optimize import brentq
+    from scipy.stats import norm
+    p_meas, K = float(p_meas), int(num_classes)
+    if not 0.0 < p_meas < 0.5:
+        raise ValueError(f"p_meas must lie in (0, 1/2), got {p_meas}")
+    if not 1 <= K <= 256:
+        raise ValueError(f"num_classes must lie in 1 .. 256, got {num_classes}")
+    if K == 1:
+        return ReadoutModel([1.0], [p_meas])
+    sigma = -1.0 / norm.ppf(p_meas)
+
+    def mass(a):                            # P(|x| <= a)
+        return norm.cdf((a - 1.0) / sigma) - norm.cdf((-a - 1.0) / sigma)
+
+    hi = 1.0 + 40.0 * sigma
+    edges = [0.0] + [brentq(lambda a, k=k: mass(a) - k / K, 0.0, hi, xtol=1e-15, rtol=4 * np.finfo(float).eps) for k in range(1, K)]
+    wrong_below = np.array([norm.cdf((-a - 1.0) / sigma) for a in edges] + [0.0])   # P(x < -a) for x = +1 + sigma z
+    w = np.full(K, 1.0 / K)
+    q = np.minimum((wrong_below[:-1] - wrong_below[1:]) * K, 0.5)
+    return ReadoutModel(w, q)

@@ -4,6 +4,8 @@
   sliding_window_osd_decoder  <- osd.py:15-199       (BP+OSD per window; shorten=True uses osd_window)
   circuit_erasure_decoding    the window decoder under circuit noise with heralded gate erasures, with and without the
                               per-shot erasure information (no reference counterpart)
+  circuit_soft_readout_decoding  the same under Gaussian soft measurement readout, with and without the per-shot readout
+                              reliability (no reference counterpart)
 
 Same arguments, same printed statistics (per-window flagged counts, overall flagged / logical errors, logical error
 per round); the per-shot Python loops are replaced by one batched call per window with the shot data resident on the
@@ -128,6 +130,61 @@ def circuit_erasure_decoding(N, p, erasure_rate, num_repeat=12, num_shots=10000,
     import torch
     from .simulation import CircuitNoiseSampler
     p, num_shots, batch = float(p), int(num_shots), int(batch)
+    code, A_list, B_list = _check_circuit_args(N, p, num_shots, batch, shot_offset, decoder)
+    sampler = CircuitNoiseSampler(bb_memory_circuit(code, A_list, B_list, p, num_repeat, z_basis=z_basis), erasure_rate=erasure_rate,
+                                  device=device)
+    erased = torch.zeros((), dtype=torch.int64, device=torch.device("cuda", int(device)))
+
+    def sample(B, off):
+        det, obs, er, L = sampler.sample(B, seed=seed, shot_offset=off, return_erasures=True, return_llr=True)
+        erased.add_(er.sum(dtype=torch.int64))
+        return det, obs, L
+
+    res = _two_leg_decoding(sampler, code.N, sample, ("static", "erasure_aware"), num_shots, batch, shot_offset, num_repeat, W, F,
+                            decoder, device, streams, decoder_kwargs)
+    res["erased_fraction"] = int(erased.item()) / max(1, num_shots * sampler.num_locations)
+    return res
+
+
+def circuit_soft_readout_decoding(N, p, p_meas=None, num_classes=16, num_repeat=12, num_shots=10000, W=3, F=1, z_basis=True,
+                                  decoder="gdg", batch=32768, seed=0, shot_offset=0, device=0, streams=2, **decoder_kwargs):
+    """Logical error rate of the sliding-window decoder on the BB-code memory experiment `bb_memory_circuit` (gate noise p,
+    `num_repeat` rounds) whose measurement flips have probability p_meas (default p; dem.with_readout_error) and come from a
+    symmetric Gaussian readout binned into `num_classes` reliability classes (dem.gaussian_readout).  Shots
+    [shot_offset, shot_offset + num_shots) of the seed's stream are sampled on the device (CircuitNoiseSampler with the
+    readout model) in batches of `batch`, and each batch is decoded twice by one SlidingWindowDecoder (method 1 windows, W,
+    F; decoder "gdg" or "osd" as circuit_erasure_decoding):
+      static      with the DEM's priors: hard measurement outcomes only;
+      soft_aware  with the sampled per-shot LLR rows (the class LLR at the DEM column of every measurement flip).
+    The noisy-syndrome identity columns of method-1 windows keep their static prior.  Counts do not depend on `batch` or
+    `streams`, and `distributed.shard_range` splits a job by shot_offset.  -> dict with per leg num_flagged, num_logical,
+    p_l, p_l_per_round, window_unconverged (list per window), plus class_histogram (list of K counts over all readout
+    locations of all shots) and elapsed (seconds)."""
+    import torch
+    from .dem import gaussian_readout, with_readout_error
+    from .simulation import CircuitNoiseSampler
+    p, num_shots, batch = float(p), int(num_shots), int(batch)
+    p_meas = p if p_meas is None else float(p_meas)
+    code, A_list, B_list = _check_circuit_args(N, p, num_shots, batch, shot_offset, decoder)
+    model = gaussian_readout(p_meas, num_classes)
+    circ = bb_memory_circuit(code, A_list, B_list, p, num_repeat, z_basis=z_basis)
+    sampler = CircuitNoiseSampler(with_readout_error(circ, p_meas), readout=model, device=device)
+    K = model.num_classes
+    hist = torch.zeros(K, dtype=torch.int64, device=torch.device("cuda", int(device)))
+
+    def sample(B, off):
+        det, obs, cls, L = sampler.sample(B, seed=seed, shot_offset=off, return_readout=True, return_llr=True)
+        hist.add_(torch.bincount(cls.reshape(-1).long(), minlength=K))
+        return det, obs, L
+
+    res = _two_leg_decoding(sampler, code.N, sample, ("static", "soft_aware"), num_shots, batch, shot_offset, num_repeat, W, F,
+                            decoder, device, streams, decoder_kwargs)
+    res["class_histogram"] = [int(k) for k in hist.cpu().tolist()]
+    return res
+
+
+def _check_circuit_args(N, p, num_shots, batch, shot_offset, decoder):
+    """The argument checks of the circuit-noise drivers -> bb_code(N)."""
     if not 0.0 < p < 0.5:
         raise ValueError(f"p must lie in (0, 0.5), got {p}")
     if num_shots < 0 or batch <= 0 or int(shot_offset) < 0:
@@ -135,25 +192,27 @@ def circuit_erasure_decoding(N, p, erasure_rate, num_repeat=12, num_shots=10000,
     if decoder not in ("gdg", "osd"):
         raise ValueError(f"decoder must be 'gdg' or 'osd', got {decoder!r}")
     try:
-        code, A_list, B_list = bb_code(N)
+        return bb_code(N)
     except KeyError:
         raise ValueError(f"unsupported N = {N}") from None
+
+
+def _two_leg_decoding(sampler, n, sample, legs, num_shots, batch, shot_offset, num_repeat, W, F, decoder, device, streams,
+                      decoder_kwargs):
+    """Decode shots [shot_offset, shot_offset + num_shots) of `sample(B, offset) -> (det, obs, rows)` twice per batch: leg 0
+    with the DEM priors, leg 1 with the rows.  -> dict with the per-leg counts and elapsed."""
+    import torch
     kw = dict(_GDG_DEFAULTS if decoder == "gdg" else _OSD_DEFAULTS)
     kw.update(decoder_kwargs)
-    sampler = CircuitNoiseSampler(bb_memory_circuit(code, A_list, B_list, p, num_repeat, z_basis=z_basis), erasure_rate=erasure_rate,
-                                  device=device)
-    plan = build_windows(sampler.chk, sampler.obs, sampler.priors, code.N, W=W, F=F, method=1)
+    plan = build_windows(sampler.chk, sampler.obs, sampler.priors, n, W=W, F=F, method=1)
     swd = SlidingWindowDecoder(plan, decoder=decoder, device=device, streams=streams, **kw)
-    legs = ("static", "erasure_aware")
     dev = torch.device("cuda", int(device))
     counts = torch.zeros((2, 2), dtype=torch.int64, device=dev)
     unconv = torch.zeros((2, len(plan.windows)), dtype=torch.int64, device=dev)
-    erased = torch.zeros((), dtype=torch.int64, device=dev)
     t0 = time.perf_counter()
     for start in range(0, num_shots, batch):
         B = min(batch, num_shots - start)
-        det, obs, er, L = sampler.sample(B, seed=seed, shot_offset=int(shot_offset) + start, return_erasures=True, return_llr=True)
-        erased += er.sum(dtype=torch.int64)
+        det, obs, L = sample(B, int(shot_offset) + start)
         out = swd.decode_device(det.clone(), obs.clone())
         counts[0] += out["counts"]
         unconv[0] += out["window_unconverged"]
@@ -161,8 +220,7 @@ def circuit_erasure_decoding(N, p, erasure_rate, num_repeat=12, num_shots=10000,
         counts[1] += out["counts"]
         unconv[1] += out["window_unconverged"]
     c, u = counts.cpu().tolist(), unconv.cpu().tolist()
-    n_erased = int(erased.item())
-    res = dict(erased_fraction=n_erased / max(1, num_shots * sampler.num_locations), elapsed=time.perf_counter() - t0)
+    res = dict(elapsed=time.perf_counter() - t0)
     for i, leg in enumerate(legs):
         p_l = c[i][1] / max(1, num_shots)
         res[leg] = dict(num_flagged=int(c[i][0]), num_logical=int(c[i][1]), p_l=p_l, p_l_per_round=1 - (1 - p_l) ** (1 / num_repeat),

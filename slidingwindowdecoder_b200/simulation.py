@@ -10,7 +10,8 @@ count kernels of the window driver score the corrections, so no shot data crosse
 
 `CircuitNoiseSampler(circ, erasure_rate)` is the circuit-level counterpart: it samples the noise locations of an `Ops` circuit
 (dem.noise_locations), with heralded erasures, on the device and returns shots in the DEM's column order together with the
-per-shot LLR rows that `SlidingWindowDecoder.decode_device(channel_llr=...)` takes.
+per-shot LLR rows that `SlidingWindowDecoder.decode_device(channel_llr=...)` takes.  With `readout=` a dem.ReadoutModel
+it also draws a reliability class per measurement flip (soft readout) and writes the matching rows.
 """
 import ctypes as C
 import time
@@ -222,11 +223,21 @@ class CircuitNoiseSampler:
     DEM sampler.  `erasure_rate`: a scalar applies to every DEPOLARIZE2 location (gate erasure conversion), an array gives
     one rate per location.  `.chk, .obs, .priors` are dem_to_check_matrices(detector_error_model(circ)) and
     `.channel_llr` [num_col] their static LLRs log((1-p)/p); a shot's LLR row is 0.0 at the columns of its erased locations.
-    Shot s of a call depends only on (seed, shot_offset + s)."""
+    Shot s of a call depends only on (seed, shot_offset + s).
 
-    def __init__(self, circ, erasure_rate=0.0, device=0):
+    `readout`: None, or a dem.ReadoutModel for soft measurement readout (`swd_window_sample_circuit_readout`).  Each
+    measurement flip (`.readout_locations` = dem.readout_locations(circ)) draws a reliability class k with probability
+    weights[k] and flips with probability flip_prob[k]; every flip's probability in the circuit must equal the model's
+    marginal (within 1e-9 relative), so the DEM is unchanged.  `.class_llr` [num_readout, K] is the LLR of readout r's DEM
+    column when r is in class k (the column's prior XOR-folded as in noise_locations with r's probability replaced by
+    flip_prob[k]; 0.0 for a readout without a column), and a shot's LLR row takes class_llr[r, class_r] at that column,
+    0.0 at the columns of erased locations overriding it."""
+
+    def __init__(self, circ, erasure_rate=0.0, readout=None, device=0):
         from .decoders import _libm_llr
-        from .dem import _noise_locations, dem_to_check_matrices
+        from .dem import ReadoutModel, _noise_locations, dem_to_check_matrices, readout_locations
+        if readout is not None and not isinstance(readout, ReadoutModel):
+            raise ValueError(f"readout must be None or a dem.ReadoutModel, got {type(readout).__name__}")
         locs, dem = _noise_locations(circ)
         L = locs.num_locations
         if L == 0:
@@ -248,6 +259,23 @@ class CircuitNoiseSampler:
                              "whose symptom is no DEM column (its probability is 0): its erasure cannot be represented")
         chk, obs, priors = dem_to_check_matrices(dem)
         chk.sort_indices(); obs.sort_indices()
+        self.readout = readout
+        if readout is not None:
+            ro = readout_locations(circ)
+            if len(ro) == 0:
+                raise ValueError("the circuit has no readout locations (X_ERROR / Z_ERROR right before a measurement in its basis)")
+            p_ro, m = locs.mech_prob[locs.mech_ptr[ro]], readout.marginal
+            bad = np.flatnonzero(np.abs(p_ro - m) > 1e-9 * np.maximum(np.abs(p_ro), abs(m)))
+            if len(bad):
+                raise ValueError(f"readout location {int(ro[bad[0]])} has probability {p_ro[bad[0]]!r}, but the readout model's "
+                                 f"marginal sum(w q) is {m!r} (dem.with_readout_error sets it)")
+            cols = locs.mech_col[locs.mech_ptr[ro]]
+            u, n = np.unique(cols[cols >= 0], return_counts=True)
+            if (n > 1).any():
+                raise ValueError(f"two readout locations share DEM column {int(u[n > 1][0])}: their soft information cannot be "
+                                 "given per column")
+            self.readout_locations = ro
+            self.class_llr = _readout_class_llr(locs, ro, readout.flip_prob, len(priors))
         import torch
         self.torch = torch
         self.device = int(device)
@@ -269,6 +297,12 @@ class CircuitNoiseSampler:
                                                          locs.mech_prob.ctypes.data_as(dp), rate.ctypes.data_as(dp),
                                                          self.channel_llr.ctypes.data_as(dp)),
                    "swd_window_set_circuit_noise")
+        if readout is not None:
+            _lib.check(self.lib.swd_window_set_circuit_readout(self._win, len(self.readout_locations),
+                                                               self.readout_locations.ctypes.data_as(i32p), readout.num_classes,
+                                                               readout.weights.ctypes.data_as(dp), readout.flip_prob.ctypes.data_as(dp),
+                                                               self.class_llr.ctypes.data_as(dp)),
+                       "swd_window_set_circuit_readout")
 
     def __del__(self):
         w = getattr(self, "_win", None)
@@ -276,14 +310,17 @@ class CircuitNoiseSampler:
             self.lib.swd_window_destroy(w)
             self._win = C.c_void_p()
 
-    def sample(self, B, seed=0, shot_offset=0, return_errors=False, return_erasures=False, return_llr=False):
-        """-> (det [B, num_det], obs [B, num_obs][, err [B, num_col]][, erased [B, num_locations]] uint8
-        [, channel_llr [B, num_col] float64]) as torch CUDA tensors written on the current stream.  Columns are in the DEM's
-        order (what build_windows and decode_device(channel_llr=...) take); err is the parity of the fired mechanisms per
-        column, so det = chk . err and obs = obs . err."""
+    def sample(self, B, seed=0, shot_offset=0, return_errors=False, return_erasures=False, return_llr=False, return_readout=False):
+        """-> (det [B, num_det], obs [B, num_obs][, err [B, num_col]][, erased [B, num_locations]][, readout [B, num_readout]]
+        uint8 [, channel_llr [B, num_col] float64]) as torch CUDA tensors written on the current stream.  Columns are in the
+        DEM's order (what build_windows and decode_device(channel_llr=...) take); err is the parity of the fired mechanisms
+        per column, so det = chk . err and obs = obs . err; readout holds the classes in readout_locations order (needs a
+        readout model)."""
         B, seed, shot_offset = int(B), int(seed), int(shot_offset)
         if B < 0 or shot_offset < 0 or not 0 <= seed < 1 << 64:
             raise ValueError(f"need B >= 0, shot_offset >= 0 and 0 <= seed < 2**64 (got {B}, {shot_offset}, {seed})")
+        if return_readout and self.readout is None:
+            raise ValueError("return_readout needs a sampler built with a readout model")
         torch = self.torch
         dev = torch.device("cuda", self.device)
         u8 = dict(dtype=torch.uint8, device=dev)
@@ -292,12 +329,54 @@ class CircuitNoiseSampler:
             out["err"] = torch.empty((B, self.num_col), **u8)
         if return_erasures:
             out["erased"] = torch.empty((B, self.num_locations), **u8)
+        if return_readout:
+            out["readout"] = torch.empty((B, len(self.readout_locations)), **u8)
         if return_llr:
             out["channel_llr"] = torch.empty((B, self.num_col), dtype=torch.float64, device=dev)
         if B:
             ptr = lambda k: out[k].data_ptr() if k in out and out[k].numel() else None    # noqa: E731
             stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-            _lib.check(self.lib.swd_window_sample_circuit(self._win, seed, shot_offset, B, ptr("det"), ptr("obs"), ptr("err"),
-                                                          ptr("erased"), ptr("channel_llr"), stream),
-                       "swd_window_sample_circuit")
-        return tuple(out[k] for k in ("det", "obs", "err", "erased", "channel_llr") if k in out)
+            if self.readout is None:
+                _lib.check(self.lib.swd_window_sample_circuit(self._win, seed, shot_offset, B, ptr("det"), ptr("obs"), ptr("err"),
+                                                              ptr("erased"), ptr("channel_llr"), stream),
+                           "swd_window_sample_circuit")
+            else:
+                _lib.check(self.lib.swd_window_sample_circuit_readout(self._win, seed, shot_offset, B, ptr("det"), ptr("obs"),
+                                                                      ptr("err"), ptr("erased"), ptr("readout"), ptr("channel_llr"),
+                                                                      stream),
+                           "swd_window_sample_circuit_readout")
+        return tuple(out[k] for k in ("det", "obs", "err", "erased", "readout", "channel_llr") if k in out)
+
+
+def _readout_class_llr(locs, readout, flip_prob, num_col):
+    """class_llr [R, K] of CircuitNoiseSampler: for readout r with DEM column c, the mechanisms of c are XOR-folded in
+    detector_error_model's order (locations last to first, the targets of one instruction first to last, mechanisms in
+    order; p <= 0 skipped, p <- q (1 - p) + p (1 - q)) with r's probability replaced by flip_prob[k], and the result goes
+    through log((1 - p) / p) as decoders._libm_llr.  With flip_prob = [p_r] this is the static LLR of c bit for bit."""
+    from .decoders import _libm_llr
+    q = np.asarray(flip_prob, dtype=np.float64)
+    R, K, L = len(readout), len(q), locs.num_locations
+    out = np.zeros((R, K), dtype=np.float64)
+    ro_mech = locs.mech_ptr[readout]
+    ro_col = locs.mech_col[ro_mech]
+    want = np.zeros(num_col, dtype=bool)
+    want[ro_col[ro_col >= 0]] = True
+    order = np.lexsort((np.arange(L), -locs.op.astype(np.int64)))
+    mechs = np.concatenate([np.arange(locs.mech_ptr[l], locs.mech_ptr[l + 1]) for l in order])
+    col = locs.mech_col[mechs]
+    mechs = mechs[(col >= 0) & want[np.maximum(col, 0)]]
+    mechs = mechs[np.argsort(locs.mech_col[mechs], kind="stable")]          # grouped by column, fold order kept
+    bounds = np.searchsorted(locs.mech_col[mechs], np.arange(num_col + 1))
+    for r in range(R):
+        c = int(ro_col[r])
+        if c < 0:
+            continue
+        acc, seen = np.zeros(K), np.zeros(K, dtype=bool)
+        for m in mechs[bounds[c]:bounds[c + 1]]:
+            p = q if m == ro_mech[r] else np.full(K, locs.mech_prob[m])
+            use = p > 0.0
+            acc = np.where(use & seen, acc * (1.0 - p) + p * (1.0 - acc), np.where(use, p, acc))
+            seen |= use
+        # a column with no mechanism of positive probability has prior 0 (LLR +inf, as _libm_llr)
+        out[r] = _libm_llr(np.where(seen, acc, 0.0), K)
+    return out
