@@ -5,6 +5,8 @@ There is no CPU fallback: if the CUDA library is missing or no GPU is visible th
 import ctypes as C
 import os
 
+import numpy as np
+
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("SWD_LIB", os.path.join(_HERE, "libswd_b200.so"))
 
@@ -33,17 +35,62 @@ KIND_BPGDG, KIND_BPGD, KIND_OSD_WINDOW = 0, 1, 2
 KERNEL_CLASSES = ["pre_bp", "sort_reset", "path_main", "path_side", "select", "osd", "path_trunk", "post_bp"]
 OK, ERR_INVALID, ERR_UNSUPPORTED, ERR_CUDA, ERR_NOMEM = 0, -1, -2, -3, -4
 
-EXPORTS = ["swd_create", "swd_destroy", "swd_decode_batch_host", "swd_decode_batch_device", "swd_decode_batch_host_packed",
-           "swd_decode_batch_device_packed", "swd_decode_batch_host_llr", "swd_decode_batch_device_llr",
-           "swd_decode_batch_host_packed_llr", "swd_decode_batch_device_packed_llr", "swd_pack_bits", "swd_unpack_bits", "swd_is_streamed", "swd_pre_bp_layout", "swd_osd_last_outputs",
-           "swd_set_profiling", "swd_get_kernel_times", "swd_get_counters", "swd_reset_counters", "swd_rank", "swd_new_n", "swd_window_create", "swd_window_destroy",
-           "swd_window_extract", "swd_window_commit", "swd_window_count_failures", "swd_window_set_priors", "swd_window_sample",
-           "swd_window_set_pauli_priors", "swd_window_sample_pauli", "swd_window_set_circuit_noise", "swd_window_sample_circuit",
-           "swd_window_set_circuit_readout", "swd_window_sample_circuit_readout",
-           "swd_bp4_create", "swd_bp4_destroy", "swd_bp4_rank", "swd_bp4_decode_batch_host", "swd_bp4_camel_decode_batch_host", "swd_bp4_decode_batch_device", "swd_bp4_camel_decode_batch_device",
-           "swd_bp4_decode_batch_host_llr", "swd_bp4_decode_batch_device_llr", "swd_bp4_camel_decode_batch_host_llr",
-           "swd_bp4_camel_decode_batch_device_llr", "swd_strerror", "swd_last_error",
-           "swd_version"]
+_vp, _i32p, _u8p, _dp, _f64p = C.c_void_p, C.POINTER(C.c_int32), C.c_void_p, C.c_void_p, C.POINTER(C.c_double)
+_vpp = C.POINTER(_vp)
+_i = C.c_int
+
+# name -> (restype, argtypes) of every exported symbol (argtypes None: left unset)
+_SIGNATURES = {
+    "swd_create": (_i, [C.POINTER(SwdConfig), _i, _i, _i32p, _i32p, _f64p, _vpp]),
+    "swd_destroy": (None, [_vp]),
+    "swd_decode_batch_host": (_i, [_vp, _u8p, C.c_int64, _u8p, _u8p, _dp]),
+    "swd_decode_batch_device": (_i, [_vp, _u8p, C.c_int64, _u8p, _u8p, _dp, _vp]),
+    "swd_decode_batch_host_packed": (_i, [_vp, _vp, C.c_int64, _vp, _u8p, _dp]),
+    "swd_decode_batch_device_packed": (_i, [_vp, _vp, C.c_int64, _vp, _u8p, _dp, _vp]),
+    "swd_decode_batch_host_llr": (_i, [_vp, _u8p, C.c_int64, _u8p, _u8p, _dp, _dp]),
+    "swd_decode_batch_device_llr": (_i, [_vp, _u8p, C.c_int64, _u8p, _u8p, _dp, _dp, _vp]),
+    "swd_decode_batch_host_packed_llr": (_i, [_vp, _vp, C.c_int64, _vp, _u8p, _dp, _dp]),
+    "swd_decode_batch_device_packed_llr": (_i, [_vp, _vp, C.c_int64, _vp, _u8p, _dp, _dp, _vp]),
+    "swd_pack_bits": (_i, [_i, _vp, C.c_int64, _i, _vp, _vp]),
+    "swd_unpack_bits": (_i, [_i, _vp, C.c_int64, _i, _vp, _vp]),
+    "swd_is_streamed": (_i, [_vp]),
+    "swd_pre_bp_layout": (_i, [_i, _i, _i32p, _i32p, _i, _vp, _vp, _vp]),
+    "swd_osd_last_outputs": (_i, [_vp, C.c_int64, _u8p, _u8p, _u8p, _dp, _vp]),
+    "swd_set_profiling": (_i, [_vp, _i]),
+    "swd_get_kernel_times": (_i, [_vp, _f64p, C.POINTER(C.c_uint64)]),
+    "swd_get_counters": (_i, [_vp, C.POINTER(SwdCounters)]),
+    "swd_reset_counters": (_i, [_vp]),
+    "swd_rank": (_i, [_vp]),
+    "swd_new_n": (_i, [_vp]),
+    "swd_window_create": (_i, [_i, _i, _i, _i32p, _i32p, _i, _i32p, _i32p, _vpp]),
+    "swd_window_destroy": (None, [_vp]),
+    "swd_window_extract": (_i, [_vp, _u8p, C.c_int64, _i, _i, _u8p, _vp]),
+    "swd_window_commit": (_i, [_vp, _u8p, C.c_int64, _i, _i, _i, _u8p, _u8p, _vp]),
+    "swd_window_count_failures": (_i, [_vp, _u8p, _u8p, C.c_int64, _vp, _vp]),
+    "swd_window_set_priors": (_i, [_vp, _f64p]),
+    "swd_window_sample": (_i, [_vp, C.c_uint64, C.c_int64, C.c_int64, _u8p, _u8p, _u8p, _vp]),
+    "swd_window_set_pauli_priors": (_i, [_vp, _i] + [_f64p] * 3 + [C.c_double, _f64p]),
+    "swd_window_sample_pauli": (_i, [_vp, C.c_uint64, C.c_int64, C.c_int64, _u8p, _u8p, _u8p, _u8p, _dp, _vp]),
+    "swd_window_set_circuit_noise": (_i, [_vp, _i, _i32p, _i32p] + [_f64p] * 3),
+    "swd_window_sample_circuit": (_i, [_vp, C.c_uint64, C.c_int64, C.c_int64, _u8p, _u8p, _u8p, _u8p, _dp, _vp]),
+    "swd_window_set_circuit_readout": (_i, [_vp, _i, _i32p, _i] + [_f64p] * 3),
+    "swd_window_sample_circuit_readout": (_i, [_vp, C.c_uint64, C.c_int64, C.c_int64, _u8p, _u8p, _u8p, _u8p, _u8p, _dp, _vp]),
+    "swd_bp4_create": (_i, [_i, _i, _i, _i, _i32p, _i32p, _i32p, _i32p] + [_f64p] * 5 + [_i, C.c_double, _i, _i, _vpp]),
+    "swd_bp4_destroy": (None, [_vp]),
+    "swd_bp4_rank": (_i, [_vp, _i]),
+    "swd_bp4_decode_batch_host": (_i, [_vp, _u8p, _u8p, C.c_int64, _u8p, _u8p, _u8p, _u8p, _dp, _vp]),
+    "swd_bp4_camel_decode_batch_host": (_i, [_vp, _u8p, _u8p, C.c_int64, _u8p, _u8p, _dp, _dp, _vp]),
+    "swd_bp4_decode_batch_device": (_i, [_vp, _vp, _vp, C.c_int64, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "swd_bp4_camel_decode_batch_device": (_i, [_vp, _vp, _vp, C.c_int64, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "swd_bp4_decode_batch_host_llr": (_i, [_vp, _u8p, _u8p, C.c_int64, _u8p, _u8p, _u8p, _u8p, _dp, _vp, _dp]),
+    "swd_bp4_decode_batch_device_llr": (_i, [_vp, _vp, _vp, C.c_int64, _vp, _vp, _vp, _vp, _vp, _vp, _dp, _vp]),
+    "swd_bp4_camel_decode_batch_host_llr": (_i, [_vp, _u8p, _u8p, C.c_int64, _u8p, _u8p, _dp, _dp, _vp, _dp]),
+    "swd_bp4_camel_decode_batch_device_llr": (_i, [_vp, _vp, _vp, C.c_int64, _vp, _vp, _vp, _vp, _vp, _dp, _vp]),
+    "swd_strerror": (C.c_char_p, [_i]),
+    "swd_last_error": (C.c_char_p, None),
+    "swd_version": (C.c_char_p, None),
+}
+EXPORTS = list(_SIGNATURES)
 
 _lib = None
 
@@ -57,104 +104,48 @@ def load():
         raise RuntimeError(f"{LIB_PATH} not found: build it with `python -c 'import __graft_entry__ as g; g.build()'` "
                            "(make -C slidingwindowdecoder_b200/csrc). There is no CPU fallback.")
     lib = C.CDLL(LIB_PATH)
-    vp, i32p, u8p, dp = C.c_void_p, C.POINTER(C.c_int32), C.c_void_p, C.c_void_p
-    lib.swd_create.argtypes = [C.POINTER(SwdConfig), C.c_int, C.c_int, i32p, i32p, C.POINTER(C.c_double), C.POINTER(vp)]
-    lib.swd_create.restype = C.c_int
-    lib.swd_destroy.argtypes = [vp]
-    lib.swd_destroy.restype = None
-    lib.swd_decode_batch_host.argtypes = [vp, u8p, C.c_int64, u8p, u8p, dp]
-    lib.swd_decode_batch_host.restype = C.c_int
-    lib.swd_decode_batch_device.argtypes = [vp, u8p, C.c_int64, u8p, u8p, dp, vp]
-    lib.swd_decode_batch_device.restype = C.c_int
-    lib.swd_decode_batch_host_packed.argtypes = [vp, vp, C.c_int64, vp, u8p, dp]
-    lib.swd_decode_batch_host_packed.restype = C.c_int
-    lib.swd_decode_batch_device_packed.argtypes = [vp, vp, C.c_int64, vp, u8p, dp, vp]
-    lib.swd_decode_batch_device_packed.restype = C.c_int
-    lib.swd_decode_batch_host_llr.argtypes = [vp, u8p, C.c_int64, u8p, u8p, dp, dp]
-    lib.swd_decode_batch_host_llr.restype = C.c_int
-    lib.swd_decode_batch_device_llr.argtypes = [vp, u8p, C.c_int64, u8p, u8p, dp, dp, vp]
-    lib.swd_decode_batch_device_llr.restype = C.c_int
-    lib.swd_decode_batch_host_packed_llr.argtypes = [vp, vp, C.c_int64, vp, u8p, dp, dp]
-    lib.swd_decode_batch_host_packed_llr.restype = C.c_int
-    lib.swd_decode_batch_device_packed_llr.argtypes = [vp, vp, C.c_int64, vp, u8p, dp, dp, vp]
-    lib.swd_decode_batch_device_packed_llr.restype = C.c_int
-    lib.swd_pack_bits.argtypes = [C.c_int, vp, C.c_int64, C.c_int, vp, vp]
-    lib.swd_pack_bits.restype = C.c_int
-    lib.swd_unpack_bits.argtypes = [C.c_int, vp, C.c_int64, C.c_int, vp, vp]
-    lib.swd_unpack_bits.restype = C.c_int
-    lib.swd_is_streamed.argtypes = [vp]
-    lib.swd_is_streamed.restype = C.c_int
-    lib.swd_pre_bp_layout.argtypes = [C.c_int, C.c_int, i32p, i32p, C.c_int, vp, vp, vp]
-    lib.swd_pre_bp_layout.restype = C.c_int
-    lib.swd_osd_last_outputs.argtypes = [vp, C.c_int64, u8p, u8p, u8p, dp, vp]
-    lib.swd_osd_last_outputs.restype = C.c_int
-    lib.swd_get_counters.argtypes = [vp, C.POINTER(SwdCounters)]
-    lib.swd_get_counters.restype = C.c_int
-    lib.swd_set_profiling.argtypes = [vp, C.c_int]
-    lib.swd_set_profiling.restype = C.c_int
-    lib.swd_get_kernel_times.argtypes = [vp, C.POINTER(C.c_double), C.POINTER(C.c_uint64)]
-    lib.swd_get_kernel_times.restype = C.c_int
-    lib.swd_reset_counters.argtypes = [vp]
-    lib.swd_reset_counters.restype = C.c_int
-    lib.swd_rank.argtypes = [vp]
-    lib.swd_rank.restype = C.c_int
-    lib.swd_new_n.argtypes = [vp]
-    lib.swd_new_n.restype = C.c_int
-    lib.swd_window_create.argtypes = [C.c_int, C.c_int, C.c_int, i32p, i32p, C.c_int, i32p, i32p, C.POINTER(vp)]
-    lib.swd_window_create.restype = C.c_int
-    lib.swd_window_destroy.argtypes = [vp]
-    lib.swd_window_destroy.restype = None
-    lib.swd_window_extract.argtypes = [vp, u8p, C.c_int64, C.c_int, C.c_int, u8p, vp]
-    lib.swd_window_extract.restype = C.c_int
-    lib.swd_window_commit.argtypes = [vp, u8p, C.c_int64, C.c_int, C.c_int, C.c_int, u8p, u8p, vp]
-    lib.swd_window_commit.restype = C.c_int
-    lib.swd_window_count_failures.argtypes = [vp, u8p, u8p, C.c_int64, vp, vp]
-    lib.swd_window_count_failures.restype = C.c_int
-    lib.swd_window_set_priors.argtypes = [vp, C.POINTER(C.c_double)]
-    lib.swd_window_set_priors.restype = C.c_int
-    lib.swd_window_sample.argtypes = [vp, C.c_uint64, C.c_int64, C.c_int64, u8p, u8p, u8p, vp]
-    lib.swd_window_sample.restype = C.c_int
-    lib.swd_window_set_pauli_priors.argtypes = [vp, C.c_int] + [C.POINTER(C.c_double)] * 3 + [C.c_double, C.POINTER(C.c_double)]
-    lib.swd_window_set_pauli_priors.restype = C.c_int
-    lib.swd_window_sample_pauli.argtypes = [vp, C.c_uint64, C.c_int64, C.c_int64, u8p, u8p, u8p, u8p, dp, vp]
-    lib.swd_window_sample_pauli.restype = C.c_int
-    lib.swd_window_set_circuit_noise.argtypes = [vp, C.c_int, i32p, i32p] + [C.POINTER(C.c_double)] * 3
-    lib.swd_window_set_circuit_noise.restype = C.c_int
-    lib.swd_window_sample_circuit.argtypes = [vp, C.c_uint64, C.c_int64, C.c_int64, u8p, u8p, u8p, u8p, dp, vp]
-    lib.swd_window_sample_circuit.restype = C.c_int
-    lib.swd_window_set_circuit_readout.argtypes = [vp, C.c_int, i32p, C.c_int] + [C.POINTER(C.c_double)] * 3
-    lib.swd_window_set_circuit_readout.restype = C.c_int
-    lib.swd_window_sample_circuit_readout.argtypes = [vp, C.c_uint64, C.c_int64, C.c_int64, u8p, u8p, u8p, u8p, u8p, dp, vp]
-    lib.swd_window_sample_circuit_readout.restype = C.c_int
-    lib.swd_bp4_create.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, i32p, i32p, i32p, i32p] + [C.POINTER(C.c_double)] * 5 + \
-                                  [C.c_int, C.c_double, C.c_int, C.c_int, C.POINTER(vp)]
-    lib.swd_bp4_create.restype = C.c_int
-    lib.swd_bp4_destroy.argtypes = [vp]
-    lib.swd_bp4_destroy.restype = None
-    lib.swd_bp4_rank.argtypes = [vp, C.c_int]
-    lib.swd_bp4_rank.restype = C.c_int
-    lib.swd_bp4_decode_batch_host.argtypes = [vp, u8p, u8p, C.c_int64, u8p, u8p, u8p, u8p, dp, vp]
-    lib.swd_bp4_decode_batch_host.restype = C.c_int
-    lib.swd_bp4_camel_decode_batch_host.argtypes = [vp, u8p, u8p, C.c_int64, u8p, u8p, dp, dp, vp]
-    lib.swd_bp4_camel_decode_batch_host.restype = C.c_int
-    lib.swd_bp4_decode_batch_device.argtypes = [vp, vp, vp, C.c_int64, vp, vp, vp, vp, vp, vp, vp]
-    lib.swd_bp4_decode_batch_device.restype = C.c_int
-    lib.swd_bp4_camel_decode_batch_device.argtypes = [vp, vp, vp, C.c_int64, vp, vp, vp, vp, vp, vp]
-    lib.swd_bp4_camel_decode_batch_device.restype = C.c_int
-    lib.swd_bp4_decode_batch_host_llr.argtypes = [vp, u8p, u8p, C.c_int64, u8p, u8p, u8p, u8p, dp, vp, dp]
-    lib.swd_bp4_decode_batch_host_llr.restype = C.c_int
-    lib.swd_bp4_camel_decode_batch_host_llr.argtypes = [vp, u8p, u8p, C.c_int64, u8p, u8p, dp, dp, vp, dp]
-    lib.swd_bp4_camel_decode_batch_host_llr.restype = C.c_int
-    lib.swd_bp4_decode_batch_device_llr.argtypes = [vp, vp, vp, C.c_int64, vp, vp, vp, vp, vp, vp, dp, vp]
-    lib.swd_bp4_decode_batch_device_llr.restype = C.c_int
-    lib.swd_bp4_camel_decode_batch_device_llr.argtypes = [vp, vp, vp, C.c_int64, vp, vp, vp, vp, vp, dp, vp]
-    lib.swd_bp4_camel_decode_batch_device_llr.restype = C.c_int
-    lib.swd_strerror.argtypes = [C.c_int]
-    lib.swd_strerror.restype = C.c_char_p
-    lib.swd_last_error.restype = C.c_char_p
-    lib.swd_version.restype = C.c_char_p
+    for name, (restype, argtypes) in _SIGNATURES.items():
+        fn = getattr(lib, name)
+        fn.restype, fn.argtypes = restype, argtypes
     _lib = lib
     return lib
+
+
+def call(name, args, llr=None, stream=None):
+    """Calls entry point `name` with args, or its per-shot-prior twin name + "_llr" with the priors pointer llr appended;
+    device entry points take `stream` last.  Raises on an error status."""
+    if llr is not None:
+        name, args = name + "_llr", (*args, llr)
+    if stream is not None:
+        args = (*args, stream)
+    check(getattr(load(), name)(*args), name)
+
+
+def current_stream(device):
+    """The current torch CUDA stream of `device` as the `void *stream` argument of the C-ABI."""
+    import torch
+    return C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
+
+
+class Window:
+    """Owns one swd_window handle over `chk` (and `obs`, or no observables if None): CSC matrices with sorted indices.  The
+    object is passed to the C-ABI as the handle (ctypes reads `_as_parameter_`) and destroys it when collected."""
+
+    def __init__(self, device, chk, obs=None):
+        self._lib = load()
+        mats = (chk,) if obs is None else (chk, obs)
+        self._cp = tuple(np.ascontiguousarray(a, dtype=np.int32) for M in mats for a in (M.indptr, M.indices))
+        ptrs = [a.ctypes.data_as(_i32p) for a in self._cp] + [None, None] * (obs is None)
+        h = C.c_void_p()
+        check(self._lib.swd_window_create(int(device), chk.shape[0], chk.shape[1], ptrs[0], ptrs[1],
+                                          0 if obs is None else obs.shape[0], ptrs[2], ptrs[3], C.byref(h)), "swd_window_create")
+        self._as_parameter_ = h
+
+    def __del__(self):
+        h = getattr(self, "_as_parameter_", None)
+        if h is not None and h.value:
+            self._lib.swd_window_destroy(h)
+            h.value = None
 
 
 def check(status, what=""):

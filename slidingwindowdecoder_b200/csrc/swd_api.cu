@@ -1210,22 +1210,40 @@ extern "C" void swd_window_destroy(swd_window *w) {
     clear_circuit_readout(w);
     delete w;
 }
+static u32 prob_threshold(double p) {          // the samplers' rule: floor(p * 2^32), clamped to 0xffffffff
+    const double x = p * 4294967296.0;
+    return x >= 4294967295.0 ? 0xffffffffu : (u32)x;
+}
+// Launches a sampler kernel with one warp per shot and warp_bytes of dynamic shared memory per warp (parity words, and the
+// circuit sampler's column words and class bytes): up to 8 warps per block within 200 KB.  A shot's draws depend only on
+// (seed, shot index), so the warps per block do not change the results.
+template <typename... P, typename... A>
+static int launch_sampler(void (*kernel)(P...), const swd_window *w, size_t warp_bytes, int64_t B, void *stream, const char *who,
+                          A... args) {
+    CK(cudaSetDevice(w->device));
+    const size_t limit = 200 * 1024;
+    if (warp_bytes > limit) { set_err(std::string(who) + ": one warp's parity and column words exceed the shared-memory limit"); return SWD_ERR_UNSUPPORTED; }
+    const int wpb = (int)std::min<size_t>(8, limit / warp_bytes);
+    const size_t smem = (size_t)wpb * warp_bytes;
+    if (smem > 48 * 1024) CK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kernel<<<(unsigned)std::min<long long>((B + wpb - 1) / wpb, 148 * 16), wpb * 32, smem, (cudaStream_t)stream>>>(args...);
+    CK(cudaGetLastError());
+    return SWD_OK;
+}
+// bytes of one shot's det and obs parity words
+static size_t parity_bytes(const swd_window *w) { return (size_t)(((w->num_det + 31) >> 5) + ((w->num_obs + 31) >> 5)) * sizeof(u32); }
+
 extern "C" int swd_window_set_priors(swd_window *w, const double *priors) {
     if (!w || !priors) { set_err("swd_window_set_priors: bad argument"); return SWD_ERR_INVALID; }
     std::vector<u32> t(w->num_col);
     for (int c = 0; c < w->num_col; c++) {
         const double p = priors[c];
         if (!(p >= 0.0 && p <= 1.0)) { set_err("swd_window_set_priors: prior outside [0, 1]"); return SWD_ERR_INVALID; }
-        const double x = p * 4294967296.0;
-        t[c] = x >= 4294967295.0 ? 0xffffffffu : (u32)x;
+        t[c] = prob_threshold(p);
     }
     CK(cudaSetDevice(w->device));
     if (w->thr) { cudaFree(w->thr); w->thr = nullptr; }
     return upload(t, (void **)&w->thr);
-}
-static u32 prob_threshold(double p) {          // the rule of swd_window_set_priors: floor(p * 2^32), clamped to 0xffffffff
-    const double x = p * 4294967296.0;
-    return x >= 4294967295.0 ? 0xffffffffu : (u32)x;
 }
 extern "C" int swd_window_set_pauli_priors(swd_window *w, int n, const double *px, const double *py, const double *pz,
                                            double erasure_rate, const double *llr5) {
@@ -1255,16 +1273,9 @@ extern "C" int swd_window_sample_pauli(swd_window *w, uint64_t seed, int64_t sho
     if (!w->pauli_n) { set_err("swd_window_sample_pauli: call swd_window_set_pauli_priors first"); return SWD_ERR_INVALID; }
     if (d_channel_llr && !w->pauli_llr5) { set_err("swd_window_sample_pauli: channel_llr needs the llr5 rows of swd_window_set_pauli_priors"); return SWD_ERR_INVALID; }
     if (B == 0) return SWD_OK;
-    CK(cudaSetDevice(w->device));
-    const int wpb = 8;
-    const size_t smem = (size_t)wpb * (((w->num_det + 31) >> 5) + ((w->num_obs + 31) >> 5)) * sizeof(u32);
-    if (smem > 200 * 1024) { set_err("swd_window_sample_pauli: too many detectors for the shared-memory parity words"); return SWD_ERR_UNSUPPORTED; }
-    if (smem > 48 * 1024) CK(cudaFuncSetAttribute(window_sample_pauli_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    window_sample_pauli_kernel<<<(unsigned)std::min<long long>((B + wpb - 1) / wpb, 148 * 16), wpb * 32, smem, (cudaStream_t)stream>>>(
+    return launch_sampler(window_sample_pauli_kernel, w, parity_bytes(w), B, stream, "swd_window_sample_pauli",
         w->pauli_thr, w->pauli_t_erase, w->pauli_n, w->pauli_llr5, w->chk_cp, w->chk_ri, w->num_det, w->obs_cp, w->obs_ri,
         w->num_obs, (unsigned long long)seed, (long long)shot_offset, (long long)B, d_det, d_obs, d_err, d_erased, d_channel_llr);
-    CK(cudaGetLastError());
-    return SWD_OK;
 }
 extern "C" int swd_window_set_circuit_noise(swd_window *w, int num_loc, const int32_t *mech_ptr, const int32_t *mech_col,
                                             const double *mech_prob, const double *erasure_rate, const double *col_llr) {
@@ -1352,25 +1363,17 @@ extern "C" int swd_window_set_circuit_readout(swd_window *w, int num_readout, co
     w->ro_K = K;
     return SWD_OK;
 }
-// one warp per shot, up to 8 warps per block; the per-warp words (and readout class bytes) live in dynamic shared memory
+// the per-warp words are the parity words, the optional err and LLR column words, and the readout class bytes
 template <bool READOUT>
 static int launch_sample_circuit(swd_window *w, const uint4 *work, const CircuitReadout &ro, uint64_t seed, int64_t shot_offset,
                                  int64_t B, uint8_t *d_det, uint8_t *d_obs, uint8_t *d_err, uint8_t *d_erased, double *d_channel_llr,
                                  void *stream, const char *who) {
-    CK(cudaSetDevice(w->device));
     const int wc = (w->num_col + 31) >> 5;
-    const size_t warp_bytes = (size_t)(((w->num_det + 31) >> 5) + ((w->num_obs + 31) >> 5) + (d_err ? wc : 0) + (d_channel_llr ? wc : 0) +
-                                       (READOUT && d_channel_llr ? (ro.num_readout + 3) >> 2 : 0)) * sizeof(u32);
-    const size_t limit = 200 * 1024;
-    if (warp_bytes > limit) { set_err(std::string(who) + ": one warp's parity and column words exceed the shared-memory limit"); return SWD_ERR_UNSUPPORTED; }
-    const int wpb = (int)std::min<size_t>(8, limit / warp_bytes);
-    const size_t smem = (size_t)wpb * warp_bytes;
-    if (smem > 48 * 1024) CK(cudaFuncSetAttribute(window_sample_circuit_kernel<READOUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    window_sample_circuit_kernel<READOUT><<<(unsigned)std::min<long long>((B + wpb - 1) / wpb, 148 * 16), wpb * 32, smem, (cudaStream_t)stream>>>(
+    const size_t warp_bytes = parity_bytes(w) + (size_t)((d_err ? wc : 0) + (d_channel_llr ? wc : 0) +
+                                                         (READOUT && d_channel_llr ? (ro.num_readout + 3) >> 2 : 0)) * sizeof(u32);
+    return launch_sampler(window_sample_circuit_kernel<READOUT>, w, warp_bytes, B, stream, who,
         work, w->circ_num_loc, w->circ_mech, w->circ_llr, w->num_col, w->chk_cp, w->chk_ri, w->num_det, w->obs_cp, w->obs_ri,
         w->num_obs, (unsigned long long)seed, (long long)shot_offset, (long long)B, d_det, d_obs, d_err, d_erased, d_channel_llr, ro);
-    CK(cudaGetLastError());
-    return SWD_OK;
 }
 extern "C" int swd_window_sample_circuit(swd_window *w, uint64_t seed, int64_t shot_offset, int64_t B, uint8_t *d_det, uint8_t *d_obs,
                                          uint8_t *d_err, uint8_t *d_erased, double *d_channel_llr, void *stream) {
@@ -1399,16 +1402,9 @@ extern "C" int swd_window_sample(swd_window *w, uint64_t seed, int64_t shot_offs
     if (!w || !d_det || B < 0 || shot_offset < 0 || (w->num_obs > 0 && !d_obs)) { set_err("swd_window_sample: bad argument"); return SWD_ERR_INVALID; }
     if (!w->thr) { set_err("swd_window_sample: call swd_window_set_priors first"); return SWD_ERR_INVALID; }
     if (B == 0) return SWD_OK;
-    CK(cudaSetDevice(w->device));
-    const int wpb = 8;
-    const size_t smem = (size_t)wpb * (((w->num_det + 31) >> 5) + ((w->num_obs + 31) >> 5)) * sizeof(u32);
-    if (smem > 200 * 1024) { set_err("swd_window_sample: too many detectors for the shared-memory parity words"); return SWD_ERR_UNSUPPORTED; }
-    if (smem > 48 * 1024) CK(cudaFuncSetAttribute(window_sample_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    window_sample_kernel<<<(unsigned)std::min<long long>((B + wpb - 1) / wpb, 148 * 16), wpb * 32, smem, (cudaStream_t)stream>>>(
+    return launch_sampler(window_sample_kernel, w, parity_bytes(w), B, stream, "swd_window_sample",
         w->thr, w->num_col, w->chk_cp, w->chk_ri, w->num_det, w->obs_cp, w->obs_ri, w->num_obs, (unsigned long long)seed,
         (long long)shot_offset, (long long)B, d_det, d_obs, d_err);
-    CK(cudaGetLastError());
-    return SWD_OK;
 }
 extern "C" int swd_window_extract(swd_window *w, const uint8_t *d_det, int64_t B, int row0, int m, uint8_t *d_synd, void *stream) {
     if (!w || !d_det || !d_synd || B < 0 || row0 < 0 || m <= 0 || row0 + m > w->num_det) { set_err("swd_window_extract: bad argument"); return SWD_ERR_INVALID; }
@@ -1616,74 +1612,81 @@ static int bp4_run(swd_bp4 *b, const u8 *d_sx, const u8 *d_sz, int64_t B, cudaSt
     return SWD_OK;
 }
 
-// host syndromes / outputs; llr5: host per-shot priors [5][B][n] or nullptr (static priors)
-static int bp4_decode_host_impl(swd_bp4 *b, const uint8_t *synd_x, const uint8_t *synd_z, int64_t B, uint8_t *dec, uint8_t *conv,
-                                uint8_t *bp_dec, uint8_t *osd0, double *lpr, int32_t *bp_iteration, const double *llr5) {
+// The argument check of the bp4 batch entry points: a decoder, B >= 0, the per-shot priors of an _llr entry point, and the
+// syndromes and the two required outputs when B > 0.
+static bool bp4_args_ok(const char *who, const swd_bp4 *b, int64_t B, const void *sx, const void *sz, const void *dec, const void *conv,
+                        bool llr_ok = true) {
+    if (b && B >= 0 && llr_ok && (B == 0 || (sx && sz && dec && conv))) return true;
+    set_err(std::string(who) + ": null argument");
+    return false;
+}
+
+// A host call stages its syndromes (into buf_x / buf_z) and its per-shot priors (into b->d_llr5) on the decoder's own stream
+// and points sx, sz and llr5 at the device copies.
+static int bp4_stage_inputs(swd_bp4 *b, u8 *buf_x, u8 *buf_z, const u8 *&sx, const u8 *&sz, const double *&llr5, int64_t B,
+                            cudaStream_t s) {
+    CK(cudaMemcpyAsync(buf_x, sx, (size_t)B * b->mx, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(buf_z, sz, (size_t)B * b->mz, cudaMemcpyHostToDevice, s));
+    sx = buf_x; sz = buf_z;
+    if (llr5) {
+        int st = bp4_stage_llr(b, llr5, B, s);
+        if (st) return st;
+        llr5 = b->d_llr5;
+    }
+    return SWD_OK;
+}
+
+// Copies the results out of the decoder's buffers into the caller's (a NULL destination is skipped): device-to-host followed
+// by a synchronise for a host call, device-to-device on the caller's stream otherwise.
+struct Bp4Out { void *dst; const void *src; size_t bytes; };
+static int bp4_copy_out(bool host, cudaStream_t s, std::initializer_list<Bp4Out> outs) {
+    for (const Bp4Out &o : outs)
+        if (o.dst) CK(cudaMemcpyAsync(o.dst, o.src, o.bytes, host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, s));
+    if (host) CK(cudaStreamSynchronize(s));
+    return SWD_OK;
+}
+
+// host: syndromes, outputs and llr5 in host memory, on the decoder's own stream, synchronised before returning; otherwise device
+// pointers on `stream` with no host synchronisation.  llr5: per-shot priors [5][B][n] or nullptr (static priors).
+static int bp4_decode_impl(swd_bp4 *b, bool host, const uint8_t *synd_x, const uint8_t *synd_z, int64_t B, uint8_t *dec, uint8_t *conv,
+                           uint8_t *bp_dec, uint8_t *osd0, double *lpr, int32_t *bp_iteration, const double *llr5, void *stream) {
     if (B == 0) return SWD_OK;
     CK(cudaSetDevice(b->device));
     const size_t n = b->n;
     int st;
     if ((st = bp4_reserve(b, B))) return st;
-    cudaStream_t s = b->stream;
-    CK(cudaMemcpyAsync(b->synd_x, synd_x, (size_t)B * b->mx, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(b->synd_z, synd_z, (size_t)B * b->mz, cudaMemcpyHostToDevice, s));
-    if (llr5 && (st = bp4_stage_llr(b, llr5, B, s))) return st;
-    if ((st = bp4_run(b, b->synd_x, b->synd_z, B, s, llr5 ? b->d_llr5 : nullptr))) return st;
-    CK(cudaMemcpyAsync(dec, b->dec, (size_t)B * 2 * n, cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(conv, b->conv, (size_t)B, cudaMemcpyDeviceToHost, s));
-    if (bp_dec) CK(cudaMemcpyAsync(bp_dec, b->bp_dec, (size_t)B * 2 * n, cudaMemcpyDeviceToHost, s));
-    if (osd0) CK(cudaMemcpyAsync(osd0, b->osd0, (size_t)B * 2 * n, cudaMemcpyDeviceToHost, s));
-    if (lpr) CK(cudaMemcpyAsync(lpr, b->lpr, (size_t)B * n * 24, cudaMemcpyDeviceToHost, s));
-    if (bp_iteration) CK(cudaMemcpyAsync(bp_iteration, b->iters, (size_t)B * 4, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    return SWD_OK;
+    cudaStream_t s = host ? b->stream : (cudaStream_t)stream;
+    if (host && (st = bp4_stage_inputs(b, b->synd_x, b->synd_z, synd_x, synd_z, llr5, B, s))) return st;
+    if ((st = bp4_run(b, synd_x, synd_z, B, s, llr5))) return st;
+    return bp4_copy_out(host, s, {{dec, b->dec, (size_t)B * 2 * n}, {conv, b->conv, (size_t)B}, {bp_dec, b->bp_dec, (size_t)B * 2 * n},
+                                  {osd0, b->osd0, (size_t)B * 2 * n}, {lpr, b->lpr, (size_t)B * n * 24}, {bp_iteration, b->iters, (size_t)B * 4}});
 }
 
 extern "C" int swd_bp4_decode_batch_host(swd_bp4 *b, const uint8_t *synd_x, const uint8_t *synd_z, int64_t B, uint8_t *dec, uint8_t *conv,
                                          uint8_t *bp_dec, uint8_t *osd0, double *lpr, int32_t *bp_iteration) {
-    if (!b || B < 0 || (B > 0 && (!synd_x || !synd_z || !dec || !conv))) { set_err("swd_bp4_decode_batch_host: null argument"); return SWD_ERR_INVALID; }
-    return bp4_decode_host_impl(b, synd_x, synd_z, B, dec, conv, bp_dec, osd0, lpr, bp_iteration, nullptr);
+    if (!bp4_args_ok(__func__, b, B, synd_x, synd_z, dec, conv)) return SWD_ERR_INVALID;
+    return bp4_decode_impl(b, true, synd_x, synd_z, B, dec, conv, bp_dec, osd0, lpr, bp_iteration, nullptr, nullptr);
 }
 
 extern "C" int swd_bp4_decode_batch_host_llr(swd_bp4 *b, const uint8_t *synd_x, const uint8_t *synd_z, int64_t B, uint8_t *dec, uint8_t *conv,
                                              uint8_t *bp_dec, uint8_t *osd0, double *lpr, int32_t *bp_iteration, const double *channel_llr) {
-    if (!b || B < 0 || !channel_llr || (B > 0 && (!synd_x || !synd_z || !dec || !conv))) { set_err("swd_bp4_decode_batch_host_llr: null argument"); return SWD_ERR_INVALID; }
-    return bp4_decode_host_impl(b, synd_x, synd_z, B, dec, conv, bp_dec, osd0, lpr, bp_iteration, channel_llr);
-}
-
-// device syndromes / outputs on the caller's stream, no host synchronisation; d_llr5: device per-shot priors [5][B][n] or nullptr
-static int bp4_decode_device_impl(swd_bp4 *b, const uint8_t *d_synd_x, const uint8_t *d_synd_z, int64_t B, uint8_t *d_dec,
-                                  uint8_t *d_conv, uint8_t *d_bp_dec, uint8_t *d_osd0, double *d_lpr, int32_t *d_bp_iteration,
-                                  void *stream, const double *d_llr5) {
-    if (B == 0) return SWD_OK;
-    CK(cudaSetDevice(b->device));
-    const size_t n = b->n;
-    int st;
-    if ((st = bp4_reserve(b, B))) return st;
-    cudaStream_t s = (cudaStream_t)stream;
-    if ((st = bp4_run(b, d_synd_x, d_synd_z, B, s, d_llr5))) return st;
-    CK(cudaMemcpyAsync(d_dec, b->dec, (size_t)B * 2 * n, cudaMemcpyDeviceToDevice, s));
-    CK(cudaMemcpyAsync(d_conv, b->conv, (size_t)B, cudaMemcpyDeviceToDevice, s));
-    if (d_bp_dec) CK(cudaMemcpyAsync(d_bp_dec, b->bp_dec, (size_t)B * 2 * n, cudaMemcpyDeviceToDevice, s));
-    if (d_osd0) CK(cudaMemcpyAsync(d_osd0, b->osd0, (size_t)B * 2 * n, cudaMemcpyDeviceToDevice, s));
-    if (d_lpr) CK(cudaMemcpyAsync(d_lpr, b->lpr, (size_t)B * n * 24, cudaMemcpyDeviceToDevice, s));
-    if (d_bp_iteration) CK(cudaMemcpyAsync(d_bp_iteration, b->iters, (size_t)B * 4, cudaMemcpyDeviceToDevice, s));
-    return SWD_OK;
+    if (!bp4_args_ok(__func__, b, B, synd_x, synd_z, dec, conv, channel_llr != nullptr)) return SWD_ERR_INVALID;
+    return bp4_decode_impl(b, true, synd_x, synd_z, B, dec, conv, bp_dec, osd0, lpr, bp_iteration, channel_llr, nullptr);
 }
 
 // the same with device pointers (e.g. torch tensors) on the caller's stream, no host synchronisation
 extern "C" int swd_bp4_decode_batch_device(swd_bp4 *b, const uint8_t *d_synd_x, const uint8_t *d_synd_z, int64_t B, uint8_t *d_dec,
                                            uint8_t *d_conv, uint8_t *d_bp_dec, uint8_t *d_osd0, double *d_lpr, int32_t *d_bp_iteration,
                                            void *stream) {
-    if (!b || B < 0 || (B > 0 && (!d_synd_x || !d_synd_z || !d_dec || !d_conv))) { set_err("swd_bp4_decode_batch_device: null argument"); return SWD_ERR_INVALID; }
-    return bp4_decode_device_impl(b, d_synd_x, d_synd_z, B, d_dec, d_conv, d_bp_dec, d_osd0, d_lpr, d_bp_iteration, stream, nullptr);
+    if (!bp4_args_ok(__func__, b, B, d_synd_x, d_synd_z, d_dec, d_conv)) return SWD_ERR_INVALID;
+    return bp4_decode_impl(b, false, d_synd_x, d_synd_z, B, d_dec, d_conv, d_bp_dec, d_osd0, d_lpr, d_bp_iteration, nullptr, stream);
 }
 
 extern "C" int swd_bp4_decode_batch_device_llr(swd_bp4 *b, const uint8_t *d_synd_x, const uint8_t *d_synd_z, int64_t B, uint8_t *d_dec,
                                                uint8_t *d_conv, uint8_t *d_bp_dec, uint8_t *d_osd0, double *d_lpr, int32_t *d_bp_iteration,
                                                const double *d_channel_llr, void *stream) {
-    if (!b || B < 0 || !d_channel_llr || (B > 0 && (!d_synd_x || !d_synd_z || !d_dec || !d_conv))) { set_err("swd_bp4_decode_batch_device_llr: null argument"); return SWD_ERR_INVALID; }
-    return bp4_decode_device_impl(b, d_synd_x, d_synd_z, B, d_dec, d_conv, d_bp_dec, d_osd0, d_lpr, d_bp_iteration, stream, d_channel_llr);
+    if (!bp4_args_ok(__func__, b, B, d_synd_x, d_synd_z, d_dec, d_conv, d_channel_llr != nullptr)) return SWD_ERR_INVALID;
+    return bp4_decode_impl(b, false, d_synd_x, d_synd_z, B, d_dec, d_conv, d_bp_dec, d_osd0, d_lpr, d_bp_iteration, d_channel_llr, stream);
 }
 
 // bp4_osd.camel_decode (src/bp4_osd.pyx:223-248) for a batch: four BP runs per shot with the last qubit pinned to I / X / Z / Y,
@@ -1719,65 +1722,42 @@ static int bp4_camel_run(swd_bp4 *b, const u8 *d_sx, const u8 *d_sz, int64_t B, 
     return SWD_OK;
 }
 
-static int bp4_camel_host_impl(swd_bp4 *b, const uint8_t *synd_x, const uint8_t *synd_z, int64_t B, uint8_t *dec, uint8_t *conv,
-                               double *min_pm, double *lpr, int32_t *bp_iteration, const double *llr5) {
+// host / device and llr5 as bp4_decode_impl
+static int bp4_camel_impl(swd_bp4 *b, bool host, const uint8_t *synd_x, const uint8_t *synd_z, int64_t B, uint8_t *dec, uint8_t *conv,
+                          double *min_pm, double *lpr, int32_t *bp_iteration, const double *llr5, void *stream) {
     if (B == 0) return SWD_OK;
     CK(cudaSetDevice(b->device));
     const size_t n = b->n;
     int st;
     if ((st = bp4_camel_reserve(b, B))) return st;
-    cudaStream_t s = b->stream;
-    CK(cudaMemcpyAsync(b->c_synd_x, synd_x, (size_t)B * b->mx, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(b->c_synd_z, synd_z, (size_t)B * b->mz, cudaMemcpyHostToDevice, s));
-    if (llr5 && (st = bp4_stage_llr(b, llr5, B, s))) return st;
-    if ((st = bp4_camel_run(b, b->c_synd_x, b->c_synd_z, B, s, llr5 ? b->d_llr5 : nullptr))) return st;
-    CK(cudaMemcpyAsync(dec, b->c_dec, (size_t)B * 2 * n, cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(conv, b->c_conv, (size_t)B, cudaMemcpyDeviceToHost, s));
-    if (min_pm) CK(cudaMemcpyAsync(min_pm, b->c_pm, (size_t)B * 8, cudaMemcpyDeviceToHost, s));
-    if (lpr) CK(cudaMemcpyAsync(lpr, b->c_lpr, (size_t)B * n * 24, cudaMemcpyDeviceToHost, s));
-    if (bp_iteration) CK(cudaMemcpyAsync(bp_iteration, b->c_it, (size_t)B * 4, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    return SWD_OK;
+    cudaStream_t s = host ? b->stream : (cudaStream_t)stream;
+    if (host && (st = bp4_stage_inputs(b, b->c_synd_x, b->c_synd_z, synd_x, synd_z, llr5, B, s))) return st;
+    if ((st = bp4_camel_run(b, synd_x, synd_z, B, s, llr5))) return st;
+    return bp4_copy_out(host, s, {{dec, b->c_dec, (size_t)B * 2 * n}, {conv, b->c_conv, (size_t)B}, {min_pm, b->c_pm, (size_t)B * 8},
+                                  {lpr, b->c_lpr, (size_t)B * n * 24}, {bp_iteration, b->c_it, (size_t)B * 4}});
 }
 
 extern "C" int swd_bp4_camel_decode_batch_host(swd_bp4 *b, const uint8_t *synd_x, const uint8_t *synd_z, int64_t B, uint8_t *dec, uint8_t *conv,
                                                double *min_pm, double *lpr, int32_t *bp_iteration) {
-    if (!b || B < 0 || (B > 0 && (!synd_x || !synd_z || !dec || !conv))) { set_err("swd_bp4_camel_decode_batch_host: null argument"); return SWD_ERR_INVALID; }
-    return bp4_camel_host_impl(b, synd_x, synd_z, B, dec, conv, min_pm, lpr, bp_iteration, nullptr);
+    if (!bp4_args_ok(__func__, b, B, synd_x, synd_z, dec, conv)) return SWD_ERR_INVALID;
+    return bp4_camel_impl(b, true, synd_x, synd_z, B, dec, conv, min_pm, lpr, bp_iteration, nullptr, nullptr);
 }
 
 extern "C" int swd_bp4_camel_decode_batch_host_llr(swd_bp4 *b, const uint8_t *synd_x, const uint8_t *synd_z, int64_t B, uint8_t *dec, uint8_t *conv,
                                                    double *min_pm, double *lpr, int32_t *bp_iteration, const double *channel_llr) {
-    if (!b || B < 0 || !channel_llr || (B > 0 && (!synd_x || !synd_z || !dec || !conv))) { set_err("swd_bp4_camel_decode_batch_host_llr: null argument"); return SWD_ERR_INVALID; }
-    return bp4_camel_host_impl(b, synd_x, synd_z, B, dec, conv, min_pm, lpr, bp_iteration, channel_llr);
-}
-
-static int bp4_camel_device_impl(swd_bp4 *b, const uint8_t *d_synd_x, const uint8_t *d_synd_z, int64_t B, uint8_t *d_dec,
-                                 uint8_t *d_conv, double *d_min_pm, double *d_lpr, int32_t *d_bp_iteration, void *stream, const double *d_llr5) {
-    if (B == 0) return SWD_OK;
-    CK(cudaSetDevice(b->device));
-    const size_t n = b->n;
-    int st;
-    if ((st = bp4_camel_reserve(b, B))) return st;
-    cudaStream_t s = (cudaStream_t)stream;
-    if ((st = bp4_camel_run(b, d_synd_x, d_synd_z, B, s, d_llr5))) return st;
-    CK(cudaMemcpyAsync(d_dec, b->c_dec, (size_t)B * 2 * n, cudaMemcpyDeviceToDevice, s));
-    CK(cudaMemcpyAsync(d_conv, b->c_conv, (size_t)B, cudaMemcpyDeviceToDevice, s));
-    if (d_min_pm) CK(cudaMemcpyAsync(d_min_pm, b->c_pm, (size_t)B * 8, cudaMemcpyDeviceToDevice, s));
-    if (d_lpr) CK(cudaMemcpyAsync(d_lpr, b->c_lpr, (size_t)B * n * 24, cudaMemcpyDeviceToDevice, s));
-    if (d_bp_iteration) CK(cudaMemcpyAsync(d_bp_iteration, b->c_it, (size_t)B * 4, cudaMemcpyDeviceToDevice, s));
-    return SWD_OK;
+    if (!bp4_args_ok(__func__, b, B, synd_x, synd_z, dec, conv, channel_llr != nullptr)) return SWD_ERR_INVALID;
+    return bp4_camel_impl(b, true, synd_x, synd_z, B, dec, conv, min_pm, lpr, bp_iteration, channel_llr, nullptr);
 }
 
 extern "C" int swd_bp4_camel_decode_batch_device(swd_bp4 *b, const uint8_t *d_synd_x, const uint8_t *d_synd_z, int64_t B, uint8_t *d_dec,
                                                  uint8_t *d_conv, double *d_min_pm, double *d_lpr, int32_t *d_bp_iteration, void *stream) {
-    if (!b || B < 0 || (B > 0 && (!d_synd_x || !d_synd_z || !d_dec || !d_conv))) { set_err("swd_bp4_camel_decode_batch_device: null argument"); return SWD_ERR_INVALID; }
-    return bp4_camel_device_impl(b, d_synd_x, d_synd_z, B, d_dec, d_conv, d_min_pm, d_lpr, d_bp_iteration, stream, nullptr);
+    if (!bp4_args_ok(__func__, b, B, d_synd_x, d_synd_z, d_dec, d_conv)) return SWD_ERR_INVALID;
+    return bp4_camel_impl(b, false, d_synd_x, d_synd_z, B, d_dec, d_conv, d_min_pm, d_lpr, d_bp_iteration, nullptr, stream);
 }
 
 extern "C" int swd_bp4_camel_decode_batch_device_llr(swd_bp4 *b, const uint8_t *d_synd_x, const uint8_t *d_synd_z, int64_t B, uint8_t *d_dec,
                                                      uint8_t *d_conv, double *d_min_pm, double *d_lpr, int32_t *d_bp_iteration,
                                                      const double *d_channel_llr, void *stream) {
-    if (!b || B < 0 || !d_channel_llr || (B > 0 && (!d_synd_x || !d_synd_z || !d_dec || !d_conv))) { set_err("swd_bp4_camel_decode_batch_device_llr: null argument"); return SWD_ERR_INVALID; }
-    return bp4_camel_device_impl(b, d_synd_x, d_synd_z, B, d_dec, d_conv, d_min_pm, d_lpr, d_bp_iteration, stream, d_channel_llr);
+    if (!bp4_args_ok(__func__, b, B, d_synd_x, d_synd_z, d_dec, d_conv, d_channel_llr != nullptr)) return SWD_ERR_INVALID;
+    return bp4_camel_impl(b, false, d_synd_x, d_synd_z, B, d_dec, d_conv, d_min_pm, d_lpr, d_bp_iteration, d_channel_llr, stream);
 }

@@ -65,6 +65,37 @@ def _is_torch_cuda(x):
     return type(x).__module__.startswith("torch") and hasattr(x, "is_cuda") and x.is_cuda
 
 
+def _check_llr(channel_llr, shape, device=None, allow_inf=True):
+    """Per-shot priors of a batched call, checked and contiguous.  device None: a host call, which takes a numpy float64 array
+    and rejects NaN (and +-inf unless allow_inf).  Otherwise a device call, which takes a torch CUDA float64 tensor on `device`;
+    it is not scanned for NaN or inf, as that would synchronise the stream (such values are undefined behaviour, as at the
+    C-ABI)."""
+    if device is None:
+        if _is_torch_cuda(channel_llr) or not isinstance(channel_llr, np.ndarray):
+            raise ValueError("channel_llr must be a numpy float64 array when the syndromes are host arrays "
+                             f"(got {type(channel_llr).__name__})")
+        if channel_llr.dtype != np.float64:
+            raise ValueError(f"channel_llr must be float64, got {channel_llr.dtype}")
+    else:
+        if not _is_torch_cuda(channel_llr):
+            raise ValueError("channel_llr must be a torch CUDA float64 tensor when the syndromes are torch CUDA tensors "
+                             f"(got {type(channel_llr).__name__})")
+        import torch
+        if channel_llr.dtype != torch.float64:
+            raise ValueError(f"channel_llr must be float64, got {channel_llr.dtype}")
+    if tuple(channel_llr.shape) != shape:
+        raise ValueError(f"channel_llr must have shape {list(shape)}, got {list(channel_llr.shape)}")
+    if device is not None:
+        if channel_llr.device != device:
+            raise ValueError(f"channel_llr lives on {channel_llr.device}, syndromes on {device}")
+        return channel_llr.contiguous()
+    if allow_inf and np.isnan(channel_llr).any():
+        raise ValueError("channel_llr contains NaN (allowed: finite values, +-inf; 0.0 marks an erasure)")
+    if not allow_inf and not np.isfinite(channel_llr).all():
+        raise ValueError("channel_llr contains inf or NaN (allowed: finite values)")
+    return np.ascontiguousarray(channel_llr)
+
+
 class _window_decoder_base:
     """Shared constructor checks (bp_guessing_decoder.pyx:6-46, osd_window.pyx:8-34) and batch plumbing."""
 
@@ -112,34 +143,6 @@ class _window_decoder_base:
         return self._converge
 
     # ------------------------------------------------------------------ batched entry points
-    def _host_llr(self, channel_llr, B):
-        """numpy float64 [B, n] per-shot priors for a host call (checked, C-contiguous)."""
-        if _is_torch_cuda(channel_llr) or not isinstance(channel_llr, np.ndarray):
-            raise ValueError("channel_llr must be a numpy float64 array when the syndromes are numpy arrays "
-                             f"(got {type(channel_llr).__name__})")
-        if channel_llr.dtype != np.float64:
-            raise ValueError(f"channel_llr must be float64, got {channel_llr.dtype}")
-        if channel_llr.shape != (B, self.n):
-            raise ValueError(f"channel_llr must have shape [B, n] = [{B}, {self.n}], got {channel_llr.shape}")
-        if np.isnan(channel_llr).any():
-            raise ValueError("channel_llr contains NaN (allowed: finite values, +-inf; 0.0 marks an erasure)")
-        return np.ascontiguousarray(channel_llr)
-
-    def _device_llr(self, channel_llr, B, device):
-        """torch CUDA float64 [B, n] per-shot priors for a device call (checked, contiguous).  NaN is not checked here
-        (that would synchronise the stream): it is undefined behaviour, as at the C-ABI."""
-        if not _is_torch_cuda(channel_llr):
-            raise ValueError("channel_llr must be a torch CUDA float64 tensor when the syndromes are torch CUDA tensors "
-                             f"(got {type(channel_llr).__name__})")
-        import torch
-        if channel_llr.dtype != torch.float64:
-            raise ValueError(f"channel_llr must be float64, got {channel_llr.dtype}")
-        if tuple(channel_llr.shape) != (B, self.n):
-            raise ValueError(f"channel_llr must have shape [B, n] = [{B}, {self.n}], got {tuple(channel_llr.shape)}")
-        if channel_llr.device != device:
-            raise ValueError(f"channel_llr lives on {channel_llr.device}, syndromes on {device}")
-        return channel_llr.contiguous()
-
     def decode_batch(self, syndromes, return_pm=False, channel_llr=None):
         """syndromes: [B, m] of 0/1.  numpy in -> numpy out (host copies inside the call);
         torch CUDA uint8 tensor in -> torch CUDA tensors out (asynchronous on the current stream).
@@ -148,107 +151,59 @@ class _window_decoder_base:
         0.0 marks an erasure (p = 1/2); +inf and negative values are allowed, NaN is not.
         Returns (corrections [B, n] uint8, converge [B] uint8[, min_pm [B] float64])."""
         if _is_torch_cuda(syndromes):
-            return self._decode_batch_torch(syndromes, return_pm, channel_llr)
-        s = np.ascontiguousarray(np.asarray(syndromes), dtype=np.uint8)
-        if s.ndim != 2 or s.shape[1] != self.m:
-            raise ValueError(f"decode_batch expects syndromes of shape [B, {self.m}], got {s.shape}")
-        B = s.shape[0]
-        llr = None if channel_llr is None else self._host_llr(channel_llr, B)
-        corr = np.empty((B, self.n), dtype=np.uint8)
-        conv = np.empty(B, dtype=np.uint8)
-        pm = np.empty(B, dtype=np.float64)
-        if llr is None:
-            st = self._lib.swd_decode_batch_host(self._handle, s.ctypes.data, B, corr.ctypes.data, conv.ctypes.data, pm.ctypes.data)
-            _lib.check(st, "swd_decode_batch_host")
+            import torch
+            s = (syndromes if syndromes.dtype == torch.uint8 else syndromes.to(torch.uint8)).contiguous()
         else:
-            st = self._lib.swd_decode_batch_host_llr(self._handle, s.ctypes.data, B, corr.ctypes.data, conv.ctypes.data, pm.ctypes.data,
-                                                     llr.ctypes.data)
-            _lib.check(st, "swd_decode_batch_host_llr")
-        self._last_B = B
-        return (corr, conv, pm) if return_pm else (corr, conv)
+            s = np.ascontiguousarray(np.asarray(syndromes), dtype=np.uint8)
+        if s.ndim != 2 or s.shape[1] != self.m:
+            raise ValueError(f"decode_batch expects syndromes of shape [B, {self.m}], got {tuple(s.shape)}")
+        return self._batch(s, False, return_pm, channel_llr)
 
     def decode_batch_packed(self, synd_packed, return_pm=False, channel_llr=None):
         """Bit-packed twin of decode_batch (swd_decode_batch_host_packed / _device_packed): synd_packed [B, ceil(m/64)] uint64
         (see pack_bits) -> (corrections [B, ceil(n/64)] uint64, converge [B] uint8[, min_pm]).  numpy in -> numpy out with the
         copies inside the call; torch CUDA int64/uint64 tensor in -> torch CUDA tensors out on the current stream.
         channel_llr: optional per-shot priors [B, n] float64, as for decode_batch."""
-        wm, wn = (self.m + 63) // 64, (self.n + 63) // 64
+        wm = (self.m + 63) // 64
         if _is_torch_cuda(synd_packed):
-            import torch
             s = synd_packed.contiguous()
-            if s.dim() != 2 or s.shape[1] != wm or s.element_size() != 8:
-                raise ValueError(f"decode_batch_packed expects 64-bit words of shape [B, {wm}], got {tuple(s.shape)}")
-            if s.device.index != self._device:
-                raise ValueError(f"syndromes live on cuda:{s.device.index}, decoder on cuda:{self._device}")
-            B = s.shape[0]
-            llr = None if channel_llr is None else self._device_llr(channel_llr, B, s.device)
-            corr = torch.empty((B, wn), dtype=torch.int64, device=s.device)
-            conv = torch.empty(B, dtype=torch.uint8, device=s.device)
-            pm = torch.empty(B, dtype=torch.float64, device=s.device)
-            stream = torch.cuda.current_stream(s.device).cuda_stream
-            if llr is None:
-                st = self._lib.swd_decode_batch_device_packed(self._handle, s.data_ptr(), B, corr.data_ptr(), conv.data_ptr(), pm.data_ptr(),
-                                                              C.c_void_p(stream))
-                _lib.check(st, "swd_decode_batch_device_packed")
-                self._keepalive = s
-            else:
-                st = self._lib.swd_decode_batch_device_packed_llr(self._handle, s.data_ptr(), B, corr.data_ptr(), conv.data_ptr(),
-                                                                  pm.data_ptr(), llr.data_ptr(), C.c_void_p(stream))
-                _lib.check(st, "swd_decode_batch_device_packed_llr")
-                self._keepalive = (s, llr)
-            self._last_B = B
-            return (corr, conv, pm) if return_pm else (corr, conv)
-        s = np.ascontiguousarray(synd_packed, dtype=np.uint64)
-        if s.ndim != 2 or s.shape[1] != wm:
-            raise ValueError(f"decode_batch_packed expects uint64 words of shape [B, {wm}], got {s.shape}")
-        B = s.shape[0]
-        llr = None if channel_llr is None else self._host_llr(channel_llr, B)
-        corr = np.empty((B, wn), dtype=np.uint64)
-        conv = np.empty(B, dtype=np.uint8)
-        pm = np.empty(B, dtype=np.float64)
-        if llr is None:
-            st = self._lib.swd_decode_batch_host_packed(self._handle, s.ctypes.data, B, corr.ctypes.data, conv.ctypes.data, pm.ctypes.data)
-            _lib.check(st, "swd_decode_batch_host_packed")
+            ok = s.element_size() == 8
         else:
-            st = self._lib.swd_decode_batch_host_packed_llr(self._handle, s.ctypes.data, B, corr.ctypes.data, conv.ctypes.data,
-                                                            pm.ctypes.data, llr.ctypes.data)
-            _lib.check(st, "swd_decode_batch_host_packed_llr")
+            s, ok = np.ascontiguousarray(synd_packed, dtype=np.uint64), True
+        if s.ndim != 2 or s.shape[1] != wm or not ok:
+            raise ValueError(f"decode_batch_packed expects 64-bit words of shape [B, {wm}], got {tuple(s.shape)}")
+        return self._batch(s, True, return_pm, channel_llr)
+
+    def _batch(self, s, packed, return_pm, channel_llr):
+        """Decodes the shape-checked syndromes s ([B, m] bytes, or [B, ceil(m/64)] words if packed): numpy in -> numpy out
+        through the host entry point, torch CUDA in -> torch CUDA out on the current stream through the device entry point."""
+        B, n_out = s.shape[0], (self.n + 63) // 64 if packed else self.n
+        device = _is_torch_cuda(s)
+        if device:
+            import torch
+            dev = s.device
+            if dev.index != self._device:
+                raise ValueError(f"syndromes live on cuda:{dev.index}, decoder on cuda:{self._device}")
+            llr = None if channel_llr is None else _check_llr(channel_llr, (B, self.n), dev)
+            out = (torch.empty((B, n_out), dtype=torch.int64 if packed else torch.uint8, device=dev),
+                   torch.empty(B, dtype=torch.uint8, device=dev), torch.empty(B, dtype=torch.float64, device=dev))
+            kind, ptr, stream = "device", torch.Tensor.data_ptr, _lib.current_stream(dev)
+        else:
+            llr = None if channel_llr is None else _check_llr(channel_llr, (B, self.n))
+            out = (np.empty((B, n_out), dtype=np.uint64 if packed else np.uint8), np.empty(B, dtype=np.uint8),
+                   np.empty(B, dtype=np.float64))
+            kind, ptr, stream = "host", (lambda a: a.ctypes.data), None
+        _lib.call("swd_decode_batch_" + kind + "_packed" * packed, (self._handle, ptr(s), B, *map(ptr, out)),
+                  None if llr is None else ptr(llr), stream)
+        if device:
+            self._keepalive = s if llr is None else (s, llr)
         self._last_B = B
-        return (corr, conv, pm) if return_pm else (corr, conv)
+        return out if return_pm else out[:2]
 
     @property
     def streamed_bp(self):
         """True if the full-window BP streams its messages from HBM (the window graph exceeds one SM's shared memory)."""
         return bool(self._lib.swd_is_streamed(self._handle) == 1)
-
-    def _decode_batch_torch(self, syndromes, return_pm, channel_llr=None):
-        import torch
-        s = syndromes
-        if s.dtype != torch.uint8:
-            s = s.to(torch.uint8)
-        s = s.contiguous()
-        if s.dim() != 2 or s.shape[1] != self.m:
-            raise ValueError(f"decode_batch expects syndromes of shape [B, {self.m}], got {tuple(s.shape)}")
-        if s.device.index != self._device:
-            raise ValueError(f"syndromes live on cuda:{s.device.index}, decoder on cuda:{self._device}")
-        B = s.shape[0]
-        llr = None if channel_llr is None else self._device_llr(channel_llr, B, s.device)
-        corr = torch.empty((B, self.n), dtype=torch.uint8, device=s.device)
-        conv = torch.empty(B, dtype=torch.uint8, device=s.device)
-        pm = torch.empty(B, dtype=torch.float64, device=s.device)
-        stream = torch.cuda.current_stream(s.device).cuda_stream
-        if llr is None:
-            st = self._lib.swd_decode_batch_device(self._handle, s.data_ptr(), B, corr.data_ptr(), conv.data_ptr(), pm.data_ptr(),
-                                                   C.c_void_p(stream))
-            _lib.check(st, "swd_decode_batch_device")
-            self._keepalive = s
-        else:
-            st = self._lib.swd_decode_batch_device_llr(self._handle, s.data_ptr(), B, corr.data_ptr(), conv.data_ptr(), pm.data_ptr(),
-                                                       llr.data_ptr(), C.c_void_p(stream))
-            _lib.check(st, "swd_decode_batch_device_llr")
-            self._keepalive = (s, llr)
-        self._last_B = B
-        return (corr, conv, pm) if return_pm else (corr, conv)
 
     def _decode_one(self, input_vector):
         input_length = input_vector.shape[0]
@@ -488,58 +443,12 @@ class bp4_osd:
             self._lib.swd_bp4_destroy(h)
             self._handle = C.c_void_p()
 
-    def _host_llr(self, channel_llr, B):
-        """numpy float64 [5, B, n] per-shot priors for a host call (checked, C-contiguous)."""
-        if _is_torch_cuda(channel_llr) or not isinstance(channel_llr, np.ndarray):
-            raise ValueError("channel_llr must be a numpy float64 array when the syndromes are numpy arrays "
-                             f"(got {type(channel_llr).__name__})")
-        if channel_llr.dtype != np.float64:
-            raise ValueError(f"channel_llr must be float64, got {channel_llr.dtype}")
-        if channel_llr.shape != (5, B, self.n):
-            raise ValueError(f"channel_llr must have shape [5, B, n] = [5, {B}, {self.n}], got {channel_llr.shape}")
-        if not np.isfinite(channel_llr).all():
-            raise ValueError("channel_llr contains inf or NaN (allowed: finite values; 0.0 in all five planes marks an erasure)")
-        return np.ascontiguousarray(channel_llr)
-
-    def _device_llr(self, channel_llr, B, device):
-        """torch CUDA float64 [5, B, n] per-shot priors for a device call (checked, contiguous).  inf and NaN are not checked
-        here (that would synchronise the stream): they are undefined behaviour, as at the C-ABI."""
-        if not _is_torch_cuda(channel_llr):
-            raise ValueError("channel_llr must be a torch CUDA float64 tensor when the syndromes are torch CUDA tensors "
-                             f"(got {type(channel_llr).__name__})")
-        import torch
-        if channel_llr.dtype != torch.float64:
-            raise ValueError(f"channel_llr must be float64, got {channel_llr.dtype}")
-        if tuple(channel_llr.shape) != (5, B, self.n):
-            raise ValueError(f"channel_llr must have shape [5, B, n] = [5, {B}, {self.n}], got {tuple(channel_llr.shape)}")
-        if channel_llr.device != device:
-            raise ValueError(f"channel_llr lives on {channel_llr.device}, syndromes on {device}")
-        return channel_llr.contiguous()
-
     def decode_batch(self, synd_x, synd_z, channel_llr=None):
         """-> dict(dec [B, 2, n] uint8, converge [B], bp_decoding [B, 2, n], osd0 [B, 2, n], log_prob_ratios [B, n, 3],
         bp_iteration [B]).  channel_llr: optional per-shot priors [5, B, n] float64 (numpy with numpy syndromes, a torch CUDA
         tensor on the decoder's device with torch syndromes): row b of the five planes decodes shot b as a bp4_osd built
         with those priors would.  Finite values only; 0.0 in all five planes marks an erased qubit."""
-        if _is_torch_cuda(synd_x) and _is_torch_cuda(synd_z):
-            return self._batch_torch(synd_x, synd_z, camel=False, channel_llr=channel_llr)
-        sx = np.ascontiguousarray(np.asarray(synd_x), dtype=np.uint8); sz = np.ascontiguousarray(np.asarray(synd_z), dtype=np.uint8)
-        if sx.ndim != 2 or sz.ndim != 2 or sx.shape[1] != self.mx or sz.shape[1] != self.mz or sx.shape[0] != sz.shape[0]:
-            raise ValueError(f"decode_batch expects syndromes of shape [B, {self.mx}] and [B, {self.mz}]")
-        B, n = sx.shape[0], self.n
-        llr = None if channel_llr is None else self._host_llr(channel_llr, B)
-        dec = np.empty((B, 2, n), dtype=np.uint8); bp = np.empty_like(dec); o0 = np.empty_like(dec)
-        conv = np.empty(B, dtype=np.uint8); lpr = np.empty((B, n, 3)); it = np.empty(B, dtype=np.int32)
-        if llr is None:
-            st = self._lib.swd_bp4_decode_batch_host(self._handle, sx.ctypes.data, sz.ctypes.data, B, dec.ctypes.data, conv.ctypes.data,
-                                                     bp.ctypes.data, o0.ctypes.data, lpr.ctypes.data, it.ctypes.data)
-            _lib.check(st, "swd_bp4_decode_batch_host")
-        else:
-            st = self._lib.swd_bp4_decode_batch_host_llr(self._handle, sx.ctypes.data, sz.ctypes.data, B, dec.ctypes.data,
-                                                         conv.ctypes.data, bp.ctypes.data, o0.ctypes.data, lpr.ctypes.data,
-                                                         it.ctypes.data, llr.ctypes.data)
-            _lib.check(st, "swd_bp4_decode_batch_host_llr")
-        return dict(dec=dec, converge=conv, bp_decoding=bp, osd0=o0, log_prob_ratios=lpr, bp_iteration=it)
+        return self._batch(synd_x, synd_z, channel_llr, camel=False)
 
     def decode(self, input_vector_x, input_vector_z):
         if input_vector_x.shape[0] != self.mx or input_vector_z.shape[0] != self.mz:
@@ -549,70 +458,43 @@ class bp4_osd:
         self.converge = int(self._last["converge"]); self.bp_iteration = int(self._last["bp_iteration"])
         return self._last["dec"].astype(np.int64)
 
-    def _batch_torch(self, synd_x, synd_z, camel, channel_llr=None):
-        """torch CUDA uint8 tensors in -> dict of torch CUDA tensors out, asynchronous on the current stream (device-pointer
-        entry points of the C-ABI; calls on one decoder must be stream-ordered)."""
-        import torch
-        sx = synd_x.to(torch.uint8).contiguous(); sz = synd_z.to(torch.uint8).contiguous()
-        if sx.dim() != 2 or sz.dim() != 2 or sx.shape[1] != self.mx or sz.shape[1] != self.mz or sx.shape[0] != sz.shape[0]:
-            raise ValueError(f"expected syndromes of shape [B, {self.mx}] and [B, {self.mz}]")
-        dev_index = getattr(self, "_device", 0)
-        if sx.device.index != dev_index or sz.device.index != dev_index:
-            raise ValueError(f"syndromes live on cuda:{sx.device.index} / cuda:{sz.device.index}, decoder on cuda:{dev_index}")
-        B, n, dev = sx.shape[0], self.n, sx.device
-        llr = None if channel_llr is None else self._device_llr(channel_llr, B, dev)
-        dec = torch.empty((B, 2, n), dtype=torch.uint8, device=dev); conv = torch.empty(B, dtype=torch.uint8, device=dev)
-        lpr = torch.empty((B, n, 3), dtype=torch.float64, device=dev); it = torch.empty(B, dtype=torch.int32, device=dev)
-        stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-        if camel:
-            pm = torch.empty(B, dtype=torch.float64, device=dev)
-            if llr is None:
-                st = self._lib.swd_bp4_camel_decode_batch_device(self._handle, sx.data_ptr(), sz.data_ptr(), B, dec.data_ptr(), conv.data_ptr(),
-                                                                 pm.data_ptr(), lpr.data_ptr(), it.data_ptr(), stream)
-                _lib.check(st, "swd_bp4_camel_decode_batch_device")
-            else:
-                st = self._lib.swd_bp4_camel_decode_batch_device_llr(self._handle, sx.data_ptr(), sz.data_ptr(), B, dec.data_ptr(),
-                                                                     conv.data_ptr(), pm.data_ptr(), lpr.data_ptr(), it.data_ptr(),
-                                                                     llr.data_ptr(), stream)
-                _lib.check(st, "swd_bp4_camel_decode_batch_device_llr")
-            out = dict(dec=dec, converge=conv, min_pm=pm, log_prob_ratios=lpr, bp_iteration=it)
-        else:
-            bp = torch.empty_like(dec); o0 = torch.empty_like(dec)
-            if llr is None:
-                st = self._lib.swd_bp4_decode_batch_device(self._handle, sx.data_ptr(), sz.data_ptr(), B, dec.data_ptr(), conv.data_ptr(),
-                                                           bp.data_ptr(), o0.data_ptr(), lpr.data_ptr(), it.data_ptr(), stream)
-                _lib.check(st, "swd_bp4_decode_batch_device")
-            else:
-                st = self._lib.swd_bp4_decode_batch_device_llr(self._handle, sx.data_ptr(), sz.data_ptr(), B, dec.data_ptr(),
-                                                               conv.data_ptr(), bp.data_ptr(), o0.data_ptr(), lpr.data_ptr(),
-                                                               it.data_ptr(), llr.data_ptr(), stream)
-                _lib.check(st, "swd_bp4_decode_batch_device_llr")
-            out = dict(dec=dec, converge=conv, bp_decoding=bp, osd0=o0, log_prob_ratios=lpr, bp_iteration=it)
-        self._keepalive = (sx, sz) if llr is None else (sx, sz, llr)
-        return out
-
     def camel_decode_batch(self, synd_x, synd_z, channel_llr=None):
         """-> dict(dec [B, 2, n] uint8, converge [B], min_pm [B], log_prob_ratios [B, n, 3] and bp_iteration [B] of the last run).
         channel_llr: optional per-shot priors [5, B, n], as for decode_batch (planes 0-2 are used)."""
-        if _is_torch_cuda(synd_x) and _is_torch_cuda(synd_z):
-            return self._batch_torch(synd_x, synd_z, camel=True, channel_llr=channel_llr)
-        sx = np.ascontiguousarray(np.asarray(synd_x), dtype=np.uint8); sz = np.ascontiguousarray(np.asarray(synd_z), dtype=np.uint8)
-        if sx.ndim != 2 or sz.ndim != 2 or sx.shape[1] != self.mx or sz.shape[1] != self.mz or sx.shape[0] != sz.shape[0]:
-            raise ValueError(f"camel_decode_batch expects syndromes of shape [B, {self.mx}] and [B, {self.mz}]")
-        B, n = sx.shape[0], self.n
-        llr = None if channel_llr is None else self._host_llr(channel_llr, B)
-        dec = np.empty((B, 2, n), dtype=np.uint8); conv = np.empty(B, dtype=np.uint8); pm = np.empty(B)
-        lpr = np.empty((B, n, 3)); it = np.empty(B, dtype=np.int32)
-        if llr is None:
-            st = self._lib.swd_bp4_camel_decode_batch_host(self._handle, sx.ctypes.data, sz.ctypes.data, B, dec.ctypes.data, conv.ctypes.data,
-                                                           pm.ctypes.data_as(C.POINTER(C.c_double)), lpr.ctypes.data_as(C.POINTER(C.c_double)), it.ctypes.data)
-            _lib.check(st, "swd_bp4_camel_decode_batch_host")
+        return self._batch(synd_x, synd_z, channel_llr, camel=True)
+
+    def _batch(self, synd_x, synd_z, channel_llr, camel):
+        """numpy syndromes in -> dict of numpy arrays out (host entry points, copies inside the call); torch CUDA tensors in ->
+        dict of torch CUDA tensors out, asynchronous on the current stream (device entry points; calls on one decoder must be
+        stream-ordered)."""
+        device = _is_torch_cuda(synd_x) and _is_torch_cuda(synd_z)
+        if device:
+            import torch
+            sx, sz = synd_x.to(torch.uint8).contiguous(), synd_z.to(torch.uint8).contiguous()
         else:
-            st = self._lib.swd_bp4_camel_decode_batch_host_llr(self._handle, sx.ctypes.data, sz.ctypes.data, B, dec.ctypes.data,
-                                                               conv.ctypes.data, pm.ctypes.data, lpr.ctypes.data, it.ctypes.data,
-                                                               llr.ctypes.data)
-            _lib.check(st, "swd_bp4_camel_decode_batch_host_llr")
-        return dict(dec=dec, converge=conv, min_pm=pm, log_prob_ratios=lpr, bp_iteration=it)
+            sx, sz = (np.ascontiguousarray(np.asarray(a), dtype=np.uint8) for a in (synd_x, synd_z))
+        if sx.ndim != 2 or sz.ndim != 2 or sx.shape[1] != self.mx or sz.shape[1] != self.mz or sx.shape[0] != sz.shape[0]:
+            raise ValueError(f"{'camel_decode_batch' if camel else 'decode_batch'} expects syndromes of shape [B, {self.mx}] "
+                             f"and [B, {self.mz}]")
+        B, n = sx.shape[0], self.n
+        spec = [("dec", (B, 2, n), "uint8"), ("converge", B, "uint8")]
+        spec += [("min_pm", B, "float64")] if camel else [("bp_decoding", (B, 2, n), "uint8"), ("osd0", (B, 2, n), "uint8")]
+        spec += [("log_prob_ratios", (B, n, 3), "float64"), ("bp_iteration", B, "int32")]
+        if device:
+            if sx.device.index != self._device or sz.device.index != self._device:
+                raise ValueError(f"syndromes live on cuda:{sx.device.index} / cuda:{sz.device.index}, decoder on cuda:{self._device}")
+            llr = None if channel_llr is None else _check_llr(channel_llr, (5, B, n), sx.device, allow_inf=False)
+            out = {k: torch.empty(shape, dtype=getattr(torch, dt), device=sx.device) for k, shape, dt in spec}
+            kind, ptr, stream = "device", (lambda t: t.data_ptr()), _lib.current_stream(sx.device)
+        else:
+            llr = None if channel_llr is None else _check_llr(channel_llr, (5, B, n), allow_inf=False)
+            out = {k: np.empty(shape, dtype=dt) for k, shape, dt in spec}
+            kind, ptr, stream = "host", (lambda a: a.ctypes.data), None
+        _lib.call("swd_bp4_" + "camel_" * camel + "decode_batch_" + kind, (self._handle, ptr(sx), ptr(sz), B, *map(ptr, out.values())),
+                  None if llr is None else ptr(llr), stream)
+        if device:
+            self._keepalive = (sx, sz) if llr is None else (sx, sz, llr)
+        return out
 
     def camel_decode(self, input_vector_x, input_vector_z):
         if input_vector_x.shape[0] != self.mx or input_vector_z.shape[0] != self.mz:

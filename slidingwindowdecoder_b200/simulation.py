@@ -49,6 +49,14 @@ def data_qubit_noise_decoding(code, p, num_shots=1000, max_step=40, max_tree_ste
     return results
 
 
+def _sample_args(B, seed, shot_offset):
+    """The checked (B, seed, shot_offset) of a sampler call, as ints."""
+    B, seed, shot_offset = int(B), int(seed), int(shot_offset)
+    if B < 0 or shot_offset < 0 or not 0 <= seed < 1 << 64:
+        raise ValueError(f"need B >= 0, shot_offset >= 0 and 0 <= seed < 2**64 (got {B}, {shot_offset}, {seed})")
+    return B, seed, shot_offset
+
+
 class CodeCapacitySampler:
     """Depolarizing noise with heralded erasures on the data qubits of a CSS code, sampled on the device
     (`swd_window_sample_pauli`).  The experiment is a window plan over 2n columns: column v is the X part of qubit v, column
@@ -88,36 +96,21 @@ class CodeCapacitySampler:
         chk.sort_indices(); obs.sort_indices()
         self.num_det, self.num_obs = chk.shape[0], obs.shape[0]
         self.chk, self.obs = chk, obs
-        self._cp = (np.ascontiguousarray(chk.indptr, dtype=np.int32), np.ascontiguousarray(chk.indices, dtype=np.int32),
-                    np.ascontiguousarray(obs.indptr, dtype=np.int32), np.ascontiguousarray(obs.indices, dtype=np.int32))
         self.lib = _lib.load()
-        i32p, dp = C.POINTER(C.c_int32), C.POINTER(C.c_double)
-        self._win = C.c_void_p()
-        _lib.check(self.lib.swd_window_create(self.device, self.num_det, 2 * n, *(a.ctypes.data_as(i32p) for a in self._cp[:2]),
-                                              self.num_obs, *(a.ctypes.data_as(i32p) for a in self._cp[2:]), C.byref(self._win)),
-                   "swd_window_create")
+        dp = C.POINTER(C.c_double)
+        self._win = _lib.Window(self.device, chk, obs)
+        self._cp = self._win._cp               # int32 CSC arrays of chk and obs: (chk indptr, chk indices, obs indptr, obs indices)
         self.has_llr = llr5 is not None
         _lib.check(self.lib.swd_window_set_pauli_priors(self._win, n, px.ctypes.data_as(dp), py.ctypes.data_as(dp), pz.ctypes.data_as(dp),
                                                         erasure_rate, llr5.ctypes.data_as(dp) if self.has_llr else None),
                    "swd_window_set_pauli_priors")
         self.erasure_rate = erasure_rate
 
-    def __del__(self):
-        w = getattr(self, "_win", None)
-        if w is not None and w.value:
-            self.lib.swd_window_destroy(w)
-            self._win = C.c_void_p()
-
-    def _stream(self):
-        return C.c_void_p(self.torch.cuda.current_stream(self.torch.device("cuda", self.device)).cuda_stream)
-
     def sample(self, B, seed=0, shot_offset=0, return_errors=False, return_erasures=False, return_llr=False):
         """-> dict of torch CUDA tensors on the current stream: synd_x [B, mx], synd_z [B, mz] (contiguous copies of det's two
         halves), det [B, mx + mz], obs [B, num_obs] (uint8), and on request err [B, 2, n], erased [B, n] (uint8),
         channel_llr [5, B, n] (float64)."""
-        B, seed, shot_offset = int(B), int(seed), int(shot_offset)
-        if B < 0 or shot_offset < 0 or not 0 <= seed < 1 << 64:
-            raise ValueError(f"need B >= 0, shot_offset >= 0 and 0 <= seed < 2**64 (got {B}, {shot_offset}, {seed})")
+        B, seed, shot_offset = _sample_args(B, seed, shot_offset)
         if return_llr and not self.has_llr:
             raise ValueError("return_llr needs the static rows: pass channel_llr to CodeCapacitySampler")
         torch, n = self.torch, self.n
@@ -133,7 +126,7 @@ class CodeCapacitySampler:
         if B:
             ptr = lambda k: out[k].data_ptr() if k in out and out[k].numel() else None    # noqa: E731
             _lib.check(self.lib.swd_window_sample_pauli(self._win, seed, shot_offset, B, ptr("det"), ptr("obs"), ptr("err"),
-                                                        ptr("erased"), ptr("channel_llr"), self._stream()),
+                                                        ptr("erased"), ptr("channel_llr"), _lib.current_stream(dev)),
                        "swd_window_sample_pauli")
         out["synd_x"] = out["det"][:, :self.mx].contiguous()
         out["synd_z"] = out["det"][:, self.mx:].contiguous()
@@ -152,7 +145,7 @@ class CodeCapacitySampler:
         if B == 0:
             return counts
         dec = dec.to(torch.uint8).contiguous()
-        stream = self._stream()
+        stream = _lib.current_stream(self.device)
         obs_ptr = obs.data_ptr() if self.num_obs else None
         _lib.check(self.lib.swd_window_commit(self._win, dec.data_ptr(), B, 2 * self.n, 0, 2 * self.n, det.data_ptr(), obs_ptr,
                                               stream), "swd_window_commit")
@@ -285,14 +278,10 @@ class CircuitNoiseSampler:
         self.locations, self.num_locations = locs, L
         self.erasure_rate = rate
         self.channel_llr = _libm_llr(priors, self.num_col)
-        self._cp = (np.ascontiguousarray(chk.indptr, dtype=np.int32), np.ascontiguousarray(chk.indices, dtype=np.int32),
-                    np.ascontiguousarray(obs.indptr, dtype=np.int32), np.ascontiguousarray(obs.indices, dtype=np.int32))
         self.lib = _lib.load()
         i32p, dp = C.POINTER(C.c_int32), C.POINTER(C.c_double)
-        self._win = C.c_void_p()
-        _lib.check(self.lib.swd_window_create(self.device, self.num_det, self.num_col, *(a.ctypes.data_as(i32p) for a in self._cp[:2]),
-                                              self.num_obs, *(a.ctypes.data_as(i32p) for a in self._cp[2:]), C.byref(self._win)),
-                   "swd_window_create")
+        self._win = _lib.Window(self.device, chk, obs)
+        self._cp = self._win._cp               # int32 CSC arrays of chk and obs: (chk indptr, chk indices, obs indptr, obs indices)
         _lib.check(self.lib.swd_window_set_circuit_noise(self._win, L, locs.mech_ptr.ctypes.data_as(i32p), locs.mech_col.ctypes.data_as(i32p),
                                                          locs.mech_prob.ctypes.data_as(dp), rate.ctypes.data_as(dp),
                                                          self.channel_llr.ctypes.data_as(dp)),
@@ -304,21 +293,13 @@ class CircuitNoiseSampler:
                                                                self.class_llr.ctypes.data_as(dp)),
                        "swd_window_set_circuit_readout")
 
-    def __del__(self):
-        w = getattr(self, "_win", None)
-        if w is not None and w.value:
-            self.lib.swd_window_destroy(w)
-            self._win = C.c_void_p()
-
     def sample(self, B, seed=0, shot_offset=0, return_errors=False, return_erasures=False, return_llr=False, return_readout=False):
         """-> (det [B, num_det], obs [B, num_obs][, err [B, num_col]][, erased [B, num_locations]][, readout [B, num_readout]]
         uint8 [, channel_llr [B, num_col] float64]) as torch CUDA tensors written on the current stream.  Columns are in the
         DEM's order (what build_windows and decode_device(channel_llr=...) take); err is the parity of the fired mechanisms
         per column, so det = chk . err and obs = obs . err; readout holds the classes in readout_locations order (needs a
         readout model)."""
-        B, seed, shot_offset = int(B), int(seed), int(shot_offset)
-        if B < 0 or shot_offset < 0 or not 0 <= seed < 1 << 64:
-            raise ValueError(f"need B >= 0, shot_offset >= 0 and 0 <= seed < 2**64 (got {B}, {shot_offset}, {seed})")
+        B, seed, shot_offset = _sample_args(B, seed, shot_offset)
         if return_readout and self.readout is None:
             raise ValueError("return_readout needs a sampler built with a readout model")
         torch = self.torch
@@ -335,7 +316,7 @@ class CircuitNoiseSampler:
             out["channel_llr"] = torch.empty((B, self.num_col), dtype=torch.float64, device=dev)
         if B:
             ptr = lambda k: out[k].data_ptr() if k in out and out[k].numel() else None    # noqa: E731
-            stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+            stream = _lib.current_stream(dev)
             if self.readout is None:
                 _lib.check(self.lib.swd_window_sample_circuit(self._win, seed, shot_offset, B, ptr("det"), ptr("obs"), ptr("err"),
                                                               ptr("erased"), ptr("channel_llr"), stream),

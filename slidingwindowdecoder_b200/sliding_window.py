@@ -11,7 +11,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from .decoders import bpgdg_decoder, osd_window
+from .decoders import _check_llr, bpgdg_decoder, osd_window
 from .windows import WindowPlan
 
 
@@ -43,16 +43,7 @@ class SlidingWindowDecoder:
         obs = plan.obs.tocsc(); obs.sort_indices()
         self.num_det, self.num_col = chk.shape
         self.num_obs = obs.shape[0]
-        self._chk_cp = np.ascontiguousarray(chk.indptr, dtype=np.int32)
-        self._chk_ri = np.ascontiguousarray(chk.indices, dtype=np.int32)
-        self._obs_cp = np.ascontiguousarray(obs.indptr, dtype=np.int32)
-        self._obs_ri = np.ascontiguousarray(obs.indices, dtype=np.int32)
-        i32p = C.POINTER(C.c_int32)
-        self._win = C.c_void_p()
-        st = self.lib.swd_window_create(self.device, self.num_det, self.num_col, self._chk_cp.ctypes.data_as(i32p),
-                                        self._chk_ri.ctypes.data_as(i32p), self.num_obs, self._obs_cp.ctypes.data_as(i32p),
-                                        self._obs_ri.ctypes.data_as(i32p), C.byref(self._win))
-        _lib.check(st, "swd_window_create")
+        self._win = _lib.Window(self.device, chk, obs)
         cls = {"gdg": bpgdg_decoder, "osd": osd_window}.get(decoder, decoder)
         self.nstreams = max(1, int(streams))
         self.decoder_sets = []                 # [stream][window] -> decoder (windows with equal matrices share one)
@@ -74,6 +65,7 @@ class SlidingWindowDecoder:
             self.decoder_sets.append(decs)
         self.decoders = self.decoder_sets[0]
         self._side_streams = None
+        self._res_win = {}                     # residual windows: decoder id -> _lib.Window over its window matrix
         self._llr_cache = {}                   # per-shot priors: plan column order, static noisy-column LLRs per window decoder
         # guessing.py:149-158,229-236: the GDG driver decodes the LAST window a second time with BP + OSD-CS
         # (ldpc.BpOsdDecoder there, this repository's BpOsdDecoder facade here) and reports a second set of counts.
@@ -86,16 +78,6 @@ class SlidingWindowDecoder:
                 kw.update(last_window_osd)
             w = plan.windows[-1]
             self.last_osd = [BpOsdDecoder(w.mat, channel_probs=list(w.prior), device=self.device, **kw) for _ in range(self.nstreams)]
-
-    def __del__(self):
-        w = getattr(self, "_win", None)
-        if w is not None and w.value:
-            self.lib.swd_window_destroy(w)
-            self._win = C.c_void_p()
-        for h, _, _ in getattr(self, "_res_win", {}).values():
-            if h.value:
-                self.lib.swd_window_destroy(h)
-        self.__dict__["_res_win"] = {}
 
     def sample_device(self, shots, seed=0, shot_offset=0, return_errors=False):
         """Draw `shots` DEM samples on the device (Philox, one Bernoulli per DEM column; the stand-in for
@@ -111,7 +93,7 @@ class SlidingWindowDecoder:
         det = torch.empty((shots, self.num_det), dtype=torch.uint8, device=dev)
         obs = torch.empty((shots, self.num_obs), dtype=torch.uint8, device=dev)
         err = torch.empty((shots, self.num_col), dtype=torch.uint8, device=dev) if return_errors else None
-        stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        stream = _lib.current_stream(dev)
         _lib.check(self.lib.swd_window_sample(self._win, int(seed), int(shot_offset), int(shots), det.data_ptr(),
                                               obs.data_ptr() if self.num_obs else None, err.data_ptr() if return_errors else None,
                                               stream), "sample")
@@ -126,34 +108,21 @@ class SlidingWindowDecoder:
         return out
 
     def _residual_window(self, w, dec):
-        """swd_window handle over one window matrix (cached per decoder): lets the commit / count kernels evaluate
+        """swd_window over one window matrix (cached per decoder): lets the commit / count kernels evaluate
         `(mat @ e_hat + detector_win) % 2` of osd.py:168."""
-        cache = self.__dict__.setdefault("_res_win", {})
-        if id(dec) not in cache:
+        if id(dec) not in self._res_win:
             A = w.mat.tocsc(); A.sort_indices()
-            cp = np.ascontiguousarray(A.indptr, dtype=np.int32); ri = np.ascontiguousarray(A.indices, dtype=np.int32)
-            h = C.c_void_p()
-            i32p = C.POINTER(C.c_int32)
-            _lib.check(self.lib.swd_window_create(self.device, A.shape[0], A.shape[1], cp.ctypes.data_as(i32p), ri.ctypes.data_as(i32p),
-                                                  0, None, None, C.byref(h)), "swd_window_create")
-            cache[id(dec)] = (h, cp, ri)
-        return cache[id(dec)][0]
+            self._res_win[id(dec)] = _lib.Window(self.device, A)
+        return self._res_win[id(dec)]
 
     def _plan_llr(self, channel_llr, det):
         """Per-shot priors [B, num_col] in the column order of the DEM given to build_windows (torch CUDA float64 on det's
         device) -> the same rows in the plan's column order."""
         torch = self.torch
-        if not (torch.is_tensor(channel_llr) and channel_llr.is_cuda):
-            raise ValueError(f"channel_llr must be a torch CUDA float64 tensor here, got {type(channel_llr).__name__}")
-        if channel_llr.dtype != torch.float64:
-            raise ValueError(f"channel_llr must be float64, got {channel_llr.dtype}")
-        if tuple(channel_llr.shape) != (det.shape[0], self.num_col):
-            raise ValueError(f"channel_llr must have shape [B, num_col] = [{det.shape[0]}, {self.num_col}], got {tuple(channel_llr.shape)}")
-        if channel_llr.device != det.device:
-            raise ValueError(f"channel_llr lives on {channel_llr.device}, shot data on {det.device}")
+        channel_llr = _check_llr(channel_llr, (det.shape[0], self.num_col), det.device)
         order = self.plan.col_order
         if order is None:
-            return channel_llr.contiguous()
+            return channel_llr
         key = ("order", det.device)
         if key not in self._llr_cache:
             self._llr_cache[key] = torch.as_tensor(np.asarray(order, dtype=np.int64), device=det.device)
@@ -177,7 +146,7 @@ class SlidingWindowDecoder:
         [B, num_col] in the plan's column order, or None."""
         torch = self.torch
         B = det.shape[0]
-        stream = C.c_void_p(torch.cuda.current_stream(det.device).cuda_stream)
+        stream = _lib.current_stream(det.device)
         unconv = []
         flagged = []
         counts_osd = None
@@ -272,17 +241,9 @@ class SlidingWindowDecoder:
     def _host_llr_to_device(self, channel_llr, B, dev):
         """numpy (or torch CPU) float64 [B, num_col] per-shot priors -> torch CUDA tensor; NaN is rejected here."""
         torch = self.torch
-        if torch.is_tensor(channel_llr):
-            if channel_llr.is_cuda:
-                raise ValueError("channel_llr is a CUDA tensor but the shot data are host arrays (use decode_device)")
+        if torch.is_tensor(channel_llr) and not channel_llr.is_cuda:
             channel_llr = channel_llr.numpy()
-        if not isinstance(channel_llr, np.ndarray) or channel_llr.dtype != np.float64:
-            raise ValueError(f"channel_llr must be a float64 array, got {getattr(channel_llr, 'dtype', type(channel_llr).__name__)}")
-        if channel_llr.shape != (B, self.num_col):
-            raise ValueError(f"channel_llr must have shape [B, num_col] = [{B}, {self.num_col}], got {channel_llr.shape}")
-        if np.isnan(channel_llr).any():
-            raise ValueError("channel_llr contains NaN (allowed: finite values, +-inf; 0.0 marks an erasure)")
-        return torch.from_numpy(np.ascontiguousarray(channel_llr)).to(dev)
+        return torch.from_numpy(_check_llr(channel_llr, (B, self.num_col))).to(dev)
 
     def decode_packed(self, det_packed, obs_packed, return_corrections=True, pinned_out=None, channel_llr=None):
         """Host entry point with bit-packed shot data (decoders.pack_bits layout): det_packed [B, ceil(num_det/64)] and
@@ -299,7 +260,7 @@ class SlidingWindowDecoder:
             return t.to(dev, non_blocking=True)
         dp, op = to_dev(det_packed), to_dev(obs_packed)
         B = dp.shape[0]
-        stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        stream = _lib.current_stream(dev)
         det = torch.empty((B, self.num_det), dtype=torch.uint8, device=dev)
         obs = torch.empty((B, self.num_obs), dtype=torch.uint8, device=dev)
         llr = None if channel_llr is None else self._host_llr_to_device(channel_llr, B, dev)
