@@ -27,6 +27,44 @@ static void set_err(const std::string &s) { g_last_error = s; }
         }                                                                                                 \
     } while (0)
 
+// Owns one device allocation of T[cap], freed on destruction (on the current device: the destroy entry points select the
+// handle's).  reserve() only grows it and discards the old contents; the raw-pointer views that kernels take by value
+// (GraphDev, Workspace, StreamWs, OsdWork) are re-pointed after it.
+template <typename T>
+struct DevBuf {
+    T *p = nullptr;
+    size_t cap = 0;
+    DevBuf() = default;
+    DevBuf(DevBuf &&o) noexcept : p(o.p), cap(o.cap) { o.p = nullptr; o.cap = 0; }
+    DevBuf &operator=(DevBuf &&o) noexcept { std::swap(p, o.p); std::swap(cap, o.cap); return *this; }
+    ~DevBuf() { release(); }
+    void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
+    // A refused allocation leaves the buffer empty and clears the runtime's last error, which would otherwise fail the next
+    // cudaGetLastError check of this or any other handle.
+    int reserve(size_t count) {
+        if (count <= cap) return SWD_OK;
+        release();
+        const size_t bytes = std::max<size_t>(16, count * sizeof(T));
+        const cudaError_t e = cudaMalloc((void **)&p, bytes);
+        if (e != cudaSuccess) {
+            p = nullptr;
+            cudaGetLastError();
+            set_err("cudaMalloc(" + std::to_string(bytes) + " bytes): " + cudaGetErrorString(e));
+            return SWD_ERR_NOMEM;
+        }
+        cap = count;
+        return SWD_OK;
+    }
+    // a fresh allocation holding v; an empty v still gets one (a table pointer is never null)
+    int upload(const std::vector<T> &v) {
+        release();
+        const int st = reserve(std::max<size_t>(1, v.size()));
+        if (st) return st;
+        CK(cudaMemcpy(p, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice));
+        return SWD_OK;
+    }
+};
+
 static inline int r16(int x) { return (x + 15) & ~15; }
 static inline int r32up(int x) { return (x + 31) & ~31; }
 
@@ -58,8 +96,11 @@ struct swd_decoder {
     int m = 0, n = 0, nnz = 0, nn = 0, max_col_deg = 0, max_row_deg = 0, es_max = 0, rank = -1;
     bool osd_only = false;
     int device = 0, num_sm = 0;
-    GraphDev g{};
-    void *d_graph[13] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+    GraphDev g{};               // views of the graph arrays below
+    DevBuf<int> g_rp, g_cp;
+    DevBuf<u16> g_rc, g_cr, g_cpos, g_vord, g_rowof, g_cpj;
+    DevBuf<u32> g_vrec, g_prow;
+    DevBuf<double> g_llr, g_llr_s, g_c2b1;
     int nphys = 0;              // message slots of the pre-BP kernel's physical layout (>= nnz)
     SubLayout L{}, LsA{}, LsB{};
     PathSmem PS{}, PSB{};
@@ -68,8 +109,8 @@ struct swd_decoder {
     path_fn_t path_fn_lat = nullptr; int T3lat = 0, grid3lat = 0;
     PreSmem PRE{};
     // graphs whose messages exceed one SM's shared memory: HBM-streamed full-window BP (swd_stream.cuh)
-    bool stream_mode = false; int Ts = 256; size_t stream_smem = 0; StreamWs sw{}; void *sw_block = nullptr; long long sw_G = 0;
-    double *sw_llrT = nullptr; long long sw_llr_G = 0;     // per-shot priors of a tile, [n][G] (allocated by the first per-shot call)
+    bool stream_mode = false; int Ts = 256; size_t stream_smem = 0; StreamWs sw{}; DevBuf<unsigned char> sw_block; long long sw_G = 0;
+    DevBuf<double> sw_llrT;     // per-shot priors of a tile, [n][G] (allocated by the first per-shot call)
     SortSmem SS{};
     OsdSmem OS{};
     GdgDev P{};
@@ -78,15 +119,16 @@ struct swd_decoder {
     int grid1 = 0, grid2 = 0, grid3 = 0, grid5 = 0;
     // workspace
     long long cap = 0;            // shots per chunk
-    Workspace ws{};
-    double *hscratch = nullptr;
-    OsdWork ow{};
-    void *ws_block = nullptr;
-    // staging for the host entry point
-    u8 *d_synd = nullptr, *d_corr = nullptr, *d_conv = nullptr; double *d_pm = nullptr; u64 *d_psynd = nullptr, *d_pcorr = nullptr;
-    u8 *h_pin = nullptr; size_t h_pin_bytes = 0;
-    long long stage_cap = 0;
-    double *d_llr = nullptr; long long llr_cap = 0;       // one chunk of host per-shot priors (swd_decode_batch_host*_llr)
+    Workspace ws{};             // views of ws_block
+    DevBuf<double> hscratch;
+    OsdWork ow{};               // views of the osd_* buffers and of ws_block
+    DevBuf<unsigned char> ws_block;
+    DevBuf<u8> osd_bp_dec, osd_osd0, osd_osdw, osd_scratch;
+    DevBuf<double> osd_lpr;
+    DevBuf<int> osd_bp_iter;
+    // staging for the host and packed entry points
+    DevBuf<u8> d_synd, d_corr, d_conv; DevBuf<double> d_pm; DevBuf<u64> d_psynd, d_pcorr;
+    DevBuf<double> d_llr;       // one chunk of host per-shot priors (swd_decode_batch_host*_llr)
     cudaStream_t stream = nullptr;
     // accumulated counters
     swd_counters ctr{};
@@ -99,6 +141,11 @@ struct swd_decoder {
     cudaEvent_t ev_get() {
         if (!ev_free.empty()) { cudaEvent_t e = ev_free.back(); ev_free.pop_back(); return e; }
         cudaEvent_t e; cudaEventCreate(&e); return e;
+    }
+    ~swd_decoder() {
+        for (auto &e : ev_used) { cudaEventDestroy(e.a); cudaEventDestroy(e.b); }
+        for (auto &e : ev_free) cudaEventDestroy(e);
+        if (stream) cudaStreamDestroy(stream);
     }
 };
 
@@ -125,13 +172,6 @@ extern "C" const char *swd_strerror(int s) {
     return "unknown";
 }
 
-template <typename T>
-static int upload(const std::vector<T> &v, void **out) {
-    CK(cudaMalloc(out, std::max<size_t>(16, v.size() * sizeof(T))));
-    CK(cudaMemcpy(*out, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice));
-    return SWD_OK;
-}
-
 // GF(2) rank of the pcm (what mod2sparse_rank returns, mod2sparse_extra.cpp:32-76), dense bit-packed.
 static int host_rank(int m, int n, const std::vector<int> &cp, const std::vector<int> &cr) {
     const int W = (m + 63) / 64;
@@ -150,8 +190,39 @@ static int host_rank(int m, int n, const std::vector<int> &cp, const std::vector
     return (int)basis.size();
 }
 
+// The flat graph of a CSC parity-check matrix whose rows may come in any order inside a column: the CSC with ascending rows,
+// the CSR with ascending columns (mod2sparse.c:358-432), the CSR position of every CSC entry, and the columns in descending
+// degree order (stable).
+struct FlatGraph {
+    std::vector<int> cp, cr, rp, rc, cpos;
+    std::vector<u16> vord;
+    int max_col_deg = 0, max_row_deg = 0;
+};
+// Returns nullptr, or what is malformed.  The caller has checked colptr[0] == 0 and 0 <= colptr[n] <= 65535.
+static const char *flat_graph(int m, int n, const int32_t *colptr, const int32_t *rowidx, FlatGraph &G) {
+    const int nnz = colptr[n];
+    G.cp.assign(colptr, colptr + n + 1); G.cr.assign(nnz, 0); G.rp.assign(m + 1, 0); G.rc.assign(nnz, 0); G.cpos.assign(nnz, 0);
+    for (int c = 0; c < n; c++) {
+        if (G.cp[c + 1] < G.cp[c]) return "colptr not monotone";
+        std::vector<int> rows(rowidx + G.cp[c], rowidx + G.cp[c + 1]);
+        std::sort(rows.begin(), rows.end());
+        for (size_t k = 0; k < rows.size(); k++) {
+            if (rows[k] < 0 || rows[k] >= m || (k && rows[k] == rows[k - 1])) return "bad row index";
+            G.cr[G.cp[c] + k] = rows[k]; G.rp[rows[k] + 1]++;
+        }
+        G.max_col_deg = std::max(G.max_col_deg, (int)rows.size());
+    }
+    for (int r = 0; r < m; r++) { G.max_row_deg = std::max(G.max_row_deg, G.rp[r + 1]); G.rp[r + 1] += G.rp[r]; }
+    std::vector<int> fill(G.rp.begin(), G.rp.end() - 1);
+    for (int c = 0; c < n; c++) for (int e = G.cp[c]; e < G.cp[c + 1]; e++) { const int p = fill[G.cr[e]]++; G.rc[p] = c; G.cpos[e] = p; }
+    std::vector<int> idx(n);
+    for (int c = 0; c < n; c++) idx[c] = c;
+    std::stable_sort(idx.begin(), idx.end(), [&](int a, int b) { return G.cp[a + 1] - G.cp[a] > G.cp[b + 1] - G.cp[b]; });
+    G.vord.assign(idx.begin(), idx.end());
+    return nullptr;
+}
+
 static int setup_kernels(swd_decoder *d);
-static int ensure_stage(swd_decoder *d, long long B);
 static int alloc_workspace(swd_decoder *d, long long want_cap, cudaStream_t s);
 
 static int create_impl(const swd_config *cfg, int m, int n, const int32_t *colptr, const int32_t *rowidx,
@@ -256,25 +327,13 @@ static int create_impl(const swd_config *cfg, int m, int n, const int32_t *colpt
     const int nnz = colptr[n];
     if (colptr[0] != 0 || nnz < 0) { set_err("swd_create: bad colptr"); return SWD_ERR_INVALID; }
     if (n > 65534 || m > 65534 || nnz > 65535) { set_err("swd_create: graph too large for 16-bit indices"); return SWD_ERR_UNSUPPORTED; }
+    FlatGraph G;
+    if (const char *why = flat_graph(m, n, colptr, rowidx, G)) { set_err(std::string("swd_create: ") + why); return SWD_ERR_INVALID; }
+    const std::vector<int> &cp = G.cp, &cr = G.cr, &rp = G.rp, &rc = G.rc, &cpos = G.cpos;
+    const std::vector<u16> &vord = G.vord;
     swd_decoder *d = new swd_decoder();
     d->cfg = *cfg; d->m = m; d->n = n; d->nnz = nnz; d->device = cfg->device; d->osd_only = osd_only;
-    // ---- flat graph: CSC with ascending rows, CSR with ascending columns (mod2sparse.c:358-432)
-    std::vector<int> cp(colptr, colptr + n + 1), cr(nnz), rp(m + 1, 0), rc(nnz), cpos(nnz);
-    for (int c = 0; c < n; c++) {
-        if (cp[c + 1] < cp[c]) { delete d; set_err("swd_create: colptr not monotone"); return SWD_ERR_INVALID; }
-        std::vector<int> rows(rowidx + cp[c], rowidx + cp[c + 1]);
-        std::sort(rows.begin(), rows.end());
-        for (size_t k = 0; k < rows.size(); k++) {
-            if (rows[k] < 0 || rows[k] >= m || (k && rows[k] == rows[k - 1])) { delete d; set_err("swd_create: bad row index"); return SWD_ERR_INVALID; }
-            cr[cp[c] + k] = rows[k]; rp[rows[k] + 1]++;
-        }
-        d->max_col_deg = std::max(d->max_col_deg, (int)rows.size());
-    }
-    for (int r = 0; r < m; r++) { d->max_row_deg = std::max(d->max_row_deg, rp[r + 1]); rp[r + 1] += rp[r]; }
-    {
-        std::vector<int> fill(rp.begin(), rp.end() - 1);
-        for (int c = 0; c < n; c++) for (int e = cp[c]; e < cp[c + 1]; e++) { int p = fill[cr[e]]++; rc[p] = c; cpos[e] = p; }
-    }
+    d->max_col_deg = G.max_col_deg; d->max_row_deg = G.max_row_deg;
     if (osd_only && cfg->kind != SWD_KIND_OSD_WINDOW) { delete d; set_err("swd_create: bad kind"); return SWD_ERR_INVALID; }
     if (!osd_only && d->max_col_deg > 16) { delete d; set_err("swd_create: column weight > 16 unsupported"); return SWD_ERR_UNSUPPORTED; }
     if (!osd_only && d->max_row_deg > 255) { delete d; set_err("swd_create: row weight > 255 unsupported"); return SWD_ERR_UNSUPPORTED; }
@@ -304,13 +363,6 @@ static int create_impl(const swd_config *cfg, int m, int n, const int32_t *colpt
     d->num_sm = prop.multiProcessorCount;
     std::vector<u16> cr16(cr.begin(), cr.end()), rc16(rc.begin(), rc.end()), cpos16(cpos.begin(), cpos.end());
     std::vector<double> llr(channel_llr, channel_llr + n);
-    std::vector<u16> vord(n);
-    {
-        std::vector<int> idx(n);
-        for (int c = 0; c < n; c++) idx[c] = c;
-        std::stable_sort(idx.begin(), idx.end(), [&](int a, int b) { return cp[a + 1] - cp[a] > cp[b + 1] - cp[b]; });
-        for (int c = 0; c < n; c++) vord[c] = (u16)idx[c];
-    }
     std::vector<u32> vrec(n);          // per ownership slot of the pre-BP kernel: first CSC entry | degree << 16
     std::vector<double> llr_s(n);
     for (int sl = 0; sl < n; sl++) {
@@ -327,13 +379,12 @@ static int create_impl(const swd_config *cfg, int m, int n, const int32_t *colpt
     } else { PL.nphys = nnz; PL.cpj.assign(std::max(nnz, 1), 0); for (int k = 0; k < 17; k++) PL.jb[k] = 0; }
     d->nphys = PL.nphys;
     int st;
-    if ((st = upload(prow, &d->d_graph[11])) || (st = upload(PL.cpj, &d->d_graph[12]))) { swd_destroy(d); return st; }
-    if ((st = upload(rp, &d->d_graph[0])) || (st = upload(rc16, &d->d_graph[1])) || (st = upload(cp, &d->d_graph[2])) ||
-        (st = upload(cr16, &d->d_graph[3])) || (st = upload(cpos16, &d->d_graph[4])) || (st = upload(llr, &d->d_graph[5])) ||
-        (st = upload(vord, &d->d_graph[6])) || (st = upload(vrec, &d->d_graph[7])) || (st = upload(llr_s, &d->d_graph[8]))) {
+    if ((st = d->g_prow.upload(prow)) || (st = d->g_cpj.upload(PL.cpj))) { swd_destroy(d); return st; }
+    if ((st = d->g_rp.upload(rp)) || (st = d->g_rc.upload(rc16)) || (st = d->g_cp.upload(cp)) ||
+        (st = d->g_cr.upload(cr16)) || (st = d->g_cpos.upload(cpos16)) || (st = d->g_llr.upload(llr)) ||
+        (st = d->g_vord.upload(vord)) || (st = d->g_vrec.upload(vrec)) || (st = d->g_llr_s.upload(llr_s))) {
         swd_destroy(d); return st;
     }
-    d->g.c2b1 = nullptr; d->g.rowof = nullptr;
     if (!osd_only && cfg->bp_method == SWD_BP_MIN_SUM && !getenv("SWD_NO_FIRST_PASS_TABLE")) {
         // the check pass of iteration 1 for syndrome 0, with the kernel's own arithmetic (osd / bpgd pyx:62-96)
         std::vector<double> t(std::max(PL.nphys, 1), 0.0); std::vector<u16> ro(std::max(PL.nphys, 1), 0);     // physical slot order
@@ -357,15 +408,14 @@ static int create_impl(const swd_config *cfg, int m, int n, const int32_t *colpt
                 ro[physof[p]] = (u16)r;
             }
         }
-        if ((st = upload(t, &d->d_graph[9])) || (st = upload(ro, &d->d_graph[10]))) { swd_destroy(d); return st; }
-        d->g.c2b1 = (const double *)d->d_graph[9]; d->g.rowof = (const u16 *)d->d_graph[10];
+        if ((st = d->g_c2b1.upload(t)) || (st = d->g_rowof.upload(ro))) { swd_destroy(d); return st; }
     }
+    d->g.c2b1 = d->g_c2b1.p; d->g.rowof = d->g_rowof.p;     // nullptr without the first-pass table
     d->g.m = m; d->g.n = n; d->g.nnz = nnz;
-    d->g.nphys = PL.nphys; d->g.prow = (const u32 *)d->d_graph[11]; d->g.cpj = (const u16 *)d->d_graph[12];
+    d->g.nphys = PL.nphys; d->g.prow = d->g_prow.p; d->g.cpj = d->g_cpj.p;
     for (int k = 0; k < 17; k++) d->g.jb[k] = PL.jb[k];
-    d->g.rp = (const int *)d->d_graph[0]; d->g.rc = (const u16 *)d->d_graph[1]; d->g.cp = (const int *)d->d_graph[2];
-    d->g.cr = (const u16 *)d->d_graph[3]; d->g.cpos = (const u16 *)d->d_graph[4]; d->g.llr = (const double *)d->d_graph[5];
-    d->g.vord = (const u16 *)d->d_graph[6]; d->g.vrec = (const u32 *)d->d_graph[7]; d->g.llr_s = (const double *)d->d_graph[8];
+    d->g.rp = d->g_rp.p; d->g.rc = d->g_rc.p; d->g.cp = d->g_cp.p; d->g.cr = d->g_cr.p; d->g.cpos = d->g_cpos.p; d->g.llr = d->g_llr.p;
+    d->g.vord = d->g_vord.p; d->g.vrec = d->g_vrec.p; d->g.llr_s = d->g_llr_s.p;
     if (cudaStreamCreateWithFlags(&d->stream, cudaStreamNonBlocking) != cudaSuccess) { swd_destroy(d); set_err("stream create failed"); return SWD_ERR_CUDA; }
     if ((st = setup_kernels(d)) != SWD_OK) { swd_destroy(d); return st; }
     *out = d;
@@ -375,23 +425,6 @@ static int create_impl(const swd_config *cfg, int m, int n, const int32_t *colpt
 extern "C" void swd_destroy(swd_decoder *d) {
     if (!d) return;
     cudaSetDevice(d->device);
-    for (auto &p : d->d_graph) if (p) cudaFree(p);
-    if (d->ws_block) cudaFree(d->ws_block);
-    if (d->hscratch) cudaFree(d->hscratch);
-    if (d->sw_block) cudaFree(d->sw_block);
-    if (d->sw_llrT) cudaFree(d->sw_llrT);
-    if (d->d_llr) cudaFree(d->d_llr);
-    if (d->d_synd) cudaFree(d->d_synd);
-    if (d->d_corr) cudaFree(d->d_corr);
-    if (d->d_conv) cudaFree(d->d_conv);
-    if (d->d_pm) cudaFree(d->d_pm);
-    if (d->d_psynd) cudaFree(d->d_psynd);
-    if (d->d_pcorr) cudaFree(d->d_pcorr);
-    if (d->h_pin) cudaFreeHost(d->h_pin);
-    for (auto &e : d->ev_used) { cudaEventDestroy(e.a); cudaEventDestroy(e.b); }
-    for (auto &e : d->ev_free) cudaEventDestroy(e);
-    osd_free_outputs(&d->ow);
-    if (d->stream) cudaStreamDestroy(d->stream);
     delete d;
 }
 
@@ -700,12 +733,13 @@ static int alloc_workspace(swd_decoder *d, long long want, cudaStream_t s) {
     long long cap = std::max<long long>(1, std::min<long long>(want, (long long)(budget / per)));
     if (cap <= d->cap) return SWD_OK;
     // growing the workspace: the accumulated work counters (ws.stats) survive the re-allocation
-    u64 keep_stats[16]; bool have_stats = false;
-    if (d->ws_block) {
+    u64 keep_stats[16];
+    const bool have_stats = d->ws_block.p != nullptr;
+    if (have_stats) {
         CK(cudaDeviceSynchronize());
-        CK(cudaMemcpy(keep_stats, d->ws.stats, sizeof(keep_stats), cudaMemcpyDeviceToHost)); have_stats = true;
-        cudaFree(d->ws_block); d->ws_block = nullptr; d->cap = 0;
+        CK(cudaMemcpy(keep_stats, d->ws.stats, sizeof(keep_stats), cudaMemcpyDeviceToHost));
     }
+    d->cap = 0;
     auto a256 = [](size_t x) { return (x + 255) & ~(size_t)255; };
     size_t o = 0;
     size_t o_cnt = o; o += a256(64 * sizeof(int));
@@ -722,11 +756,11 @@ static int alloc_workspace(swd_decoder *d, long long want, cudaStream_t s) {
     const long long wl_stride = cap * std::max(1, std::max(d->P.n_tree + 1, d->P.n_side));
     size_t o_bak = o; o += a256((size_t)cap * std::max(1, d->P.n_tree) * d->P.bak_stride);
     size_t o_wl = o; o += a256((size_t)wl_stride * SWD_WL_MAX * sizeof(u64));
-    cudaError_t e = cudaMalloc(&d->ws_block, o);
-    if (e != cudaSuccess) { set_err("workspace cudaMalloc failed"); return SWD_ERR_NOMEM; }
+    int st = d->ws_block.reserve(o);
+    if (st) { d->ws = Workspace{}; return st; }
     // counters / stats / work list zeroed on the caller's stream (the kernels that use them are launched there)
-    CK(cudaMemsetAsync(d->ws_block, 0, o_list, s));
-    unsigned char *b = (unsigned char *)d->ws_block;
+    CK(cudaMemsetAsync(d->ws_block.p, 0, o_list, s));
+    unsigned char *b = d->ws_block.p;
     d->ws.counters = (int *)(b + o_cnt); d->ws.stats = (u64 *)(b + o_stats); d->ws.gdg_list = (int *)(b + o_list);
     d->ws.sum = (double *)(b + o_sum); d->ws.hist = osd ? (double *)(b + o_hist) : nullptr;
     d->ws.blob = b + o_blob; d->ws.rec = b + o_rec; d->ws.side = b + o_side; d->ws.node = b + o_node;
@@ -734,11 +768,12 @@ static int alloc_workspace(swd_decoder *d, long long want, cudaStream_t s) {
     if (have_stats) CK(cudaMemcpyAsync(d->ws.stats, keep_stats, sizeof(keep_stats), cudaMemcpyHostToDevice, s));
     if (have_stats) CK(cudaStreamSynchronize(s));          // keep_stats is a stack buffer
     if (osd) osd_bind(&d->ow, b + o_osd, cap, d->m, n);
-    if (osd && d->OS.big && !d->ow.big_scratch) {
-        if (cudaMalloc(&d->ow.big_scratch, (size_t)d->grid5 * d->OS.big_stride) != cudaSuccess) { set_err("OSD scratch cudaMalloc failed"); return SWD_ERR_NOMEM; }
+    if (osd && d->OS.big) {
+        if ((st = d->osd_scratch.reserve((size_t)d->grid5 * d->OS.big_stride))) return st;
+        d->ow.big_scratch = d->osd_scratch.p;
     }
     // four posterior rows per CTA, and a fifth for the per-shot twin's slot-ordered priors
-    if (!d->hscratch && !d->stream_mode) CK(cudaMalloc(&d->hscratch, (size_t)d->grid1 * 5 * n * sizeof(double)));
+    if (!d->stream_mode && (st = d->hscratch.reserve((size_t)d->grid1 * 5 * n))) return st;
     d->cap = cap;
     return SWD_OK;
 }
@@ -772,7 +807,7 @@ static int stream_pre_bp(swd_decoder *d, const GraphDev &g, const u8 *d_synd, lo
     const long long want = std::min<long long>(Gmax, (B + Ts - 1) / Ts * Ts);
     if (want > d->sw_G) {
         CK(cudaStreamSynchronize(s));
-        if (d->sw_block) { cudaFree(d->sw_block); d->sw_block = nullptr; d->sw_G = 0; }
+        d->sw_G = 0;
         auto a256 = [](size_t x) { return (x + 255) & ~(size_t)255; };
         size_t o = 0;
         const size_t o_msg = o; o += a256((size_t)8 * d->nnz * want);
@@ -781,24 +816,22 @@ static int stream_pre_bp(swd_decoder *d, const GraphDev &g, const u8 *d_synd, lo
         const size_t o_sy = o; o += a256((size_t)4 * ((d->m + 31) / 32) * want);
         const size_t o_it = o; o += a256((size_t)4 * want);
         const size_t o_cv = o; o += a256((size_t)want);
-        if (cudaMalloc(&d->sw_block, o) != cudaSuccess) { set_err("streamed-BP message buffer cudaMalloc failed"); return SWD_ERR_NOMEM; }
-        unsigned char *b = (unsigned char *)d->sw_block;
+        if (int st = d->sw_block.reserve(o)) return st;
+        unsigned char *b = d->sw_block.p;
         d->sw.msg = (double *)(b + o_msg); d->sw.hs = (double *)(b + o_hs); d->sw.decw = (u32 *)(b + o_dec);
         d->sw.itdone = (int *)(b + o_it); d->sw.conv = b + o_cv; d->sw.syndw = (u32 *)(b + o_sy);
         d->sw_G = want;
     }
-    if (shot_llr && d->sw_llr_G < d->sw_G) {
+    if (shot_llr && d->sw_llrT.cap < (size_t)n * d->sw_G) {
         CK(cudaStreamSynchronize(s));
-        if (d->sw_llrT) { cudaFree(d->sw_llrT); d->sw_llrT = nullptr; d->sw_llr_G = 0; }
-        if (cudaMalloc(&d->sw_llrT, (size_t)8 * n * d->sw_G) != cudaSuccess) { set_err("streamed-BP prior buffer cudaMalloc failed"); return SWD_ERR_NOMEM; }
-        d->sw_llr_G = d->sw_G;
+        if (int st = d->sw_llrT.reserve((size_t)n * d->sw_G)) return st;
     }
     for (long long t0 = 0; t0 < B; t0 += d->sw_G) {
         const long long nb = std::min<long long>(d->sw_G, B - t0);
         StreamWs sw = d->sw; sw.G = (nb + Ts - 1) / Ts * Ts;
         if (shot_llr) {
-            sw.llrT = d->sw_llrT;
-            llr_transpose_kernel<<<dim3((unsigned)((n + 31) / 32), (unsigned)((nb + 31) / 32)), 256, 0, s>>>(g.llr_shot, B, t0, n, sw.G, d->sw_llrT);
+            sw.llrT = d->sw_llrT.p;
+            llr_transpose_kernel<<<dim3((unsigned)((n + 31) / 32), (unsigned)((nb + 31) / 32)), 256, 0, s>>>(g.llr_shot, B, t0, n, sw.G, d->sw_llrT.p);
             d->ctr.kernel_launches++;
         }
         fn<<<(unsigned)(sw.G / Ts), Ts, d->stream_smem, s>>>(g, d_synd, B, t0, d->cfg.max_iter, d->cfg.ms_scaling_factor, sw, full_hist, d->ws.stats);
@@ -828,7 +861,7 @@ static int launch_chunk(swd_decoder *d, const u8 *d_synd, long long B, u8 *d_cor
     } else {
     KTimer kt(d, s, SWD_K_PRE_BP);
     (d_llr ? d->pre_fn_llr : d->pre_fn)<<<g1, d->T1, d->PRE.total, s>>>(g, d_synd, B, c.max_iter, c.ms_scaling_factor, d_corr, d_conv, d->ws,
-                                                                     d->hscratch, full_hist, d->PRE, iter_out, lpr_out);
+                                                                     d->hscratch.p, full_hist, d->PRE, iter_out, lpr_out);
     d->ctr.kernel_launches++;
     }
     if (d_pm) {
@@ -891,24 +924,41 @@ static int launch_chunk(swd_decoder *d, const u8 *d_synd, long long B, u8 *d_cor
     return SWD_OK;
 }
 
+// The outputs of the last batch of an osd_window-kind decoder (swd_osd_last_outputs), grown with B.  The zero fill runs on the
+// caller's stream: the kernels that write these buffers run there (a legacy-stream memset would not be ordered against a
+// non-blocking stream).
+static int reserve_osd_outputs(swd_decoder *d, long long B, cudaStream_t s) {
+    if (B <= d->ow.out_cap) return SWD_OK;
+    const size_t n = d->n;
+    OsdWork &ow = d->ow;
+    ow.out_cap = 0;
+    int st;
+    if ((st = d->osd_bp_dec.reserve(B * n)) || (st = d->osd_osd0.reserve(B * n)) || (st = d->osd_osdw.reserve(B * n)) ||
+        (st = d->osd_lpr.reserve(B * n * 4)) || (st = d->osd_bp_iter.reserve(B)))
+        d->last_B = 0;          // the last batch's outputs may be gone
+    ow.bp_dec = d->osd_bp_dec.p; ow.osd0 = d->osd_osd0.p; ow.osdw = d->osd_osdw.p; ow.lpr = d->osd_lpr.p; ow.bp_iter = d->osd_bp_iter.p;
+    if (st) return st;
+    CK(cudaMemsetAsync(ow.osd0, 0, B * n, s)); CK(cudaMemsetAsync(ow.osdw, 0, B * n, s)); CK(cudaMemsetAsync(ow.bp_dec, 0, B * n, s));
+    ow.out_cap = B;
+    return SWD_OK;
+}
+
 // llr: per-shot priors [B][n] or nullptr; llr_host: llr is a host array, copied one workspace chunk at a time into d->d_llr
 static int decode_device_impl(swd_decoder *d, const uint8_t *d_synd, int64_t B, uint8_t *d_corr, uint8_t *d_conv, double *d_pm,
                               cudaStream_t s, const double *llr, bool llr_host) {
     int st = alloc_workspace(d, B, s);
     if (st) return st;
-    if (d->cfg.kind == SWD_KIND_OSD_WINDOW) { st = osd_reserve_outputs(&d->ow, B, d->n, s); if (st) { set_err("osd output alloc failed"); return st; } }
-    if (llr_host && d->llr_cap < d->cap) {
+    if (d->cfg.kind == SWD_KIND_OSD_WINDOW && (st = reserve_osd_outputs(d, B, s))) return st;
+    if (llr_host && d->d_llr.cap < (size_t)d->n * d->cap) {
         CK(cudaStreamSynchronize(s));
-        if (d->d_llr) { cudaFree(d->d_llr); d->d_llr = nullptr; d->llr_cap = 0; }
-        if (cudaMalloc(&d->d_llr, (size_t)8 * d->n * d->cap) != cudaSuccess) { set_err("prior staging cudaMalloc failed"); return SWD_ERR_NOMEM; }
-        d->llr_cap = d->cap;
+        if ((st = d->d_llr.reserve((size_t)d->n * d->cap))) return st;
     }
     for (long long b0 = 0; b0 < B; b0 += d->cap) {
         const long long nb = std::min<long long>(d->cap, B - b0);
         const double *cl = llr ? llr + (size_t)b0 * d->n : nullptr;
         if (llr_host) {     // the buffer is reused chunk after chunk: stream order puts each copy after the previous chunk's kernels
-            CK(cudaMemcpyAsync(d->d_llr, cl, (size_t)8 * nb * d->n, cudaMemcpyHostToDevice, s));
-            cl = d->d_llr;
+            CK(cudaMemcpyAsync(d->d_llr.p, cl, (size_t)8 * nb * d->n, cudaMemcpyHostToDevice, s));
+            cl = d->d_llr.p;
         }
         st = launch_chunk(d, d_synd + b0 * d->m, nb, d_corr + b0 * d->n, d_conv + b0, d_pm ? d_pm + b0 : nullptr, s, b0, cl);
         if (st) return st;
@@ -919,51 +969,6 @@ static int decode_device_impl(swd_decoder *d, const uint8_t *d_synd, int64_t B, 
     d->ctr.shots += (uint64_t)B;
     d->last_B = B;
     return SWD_OK;
-}
-
-extern "C" int swd_decode_batch_device(swd_decoder *d, const uint8_t *d_synd, int64_t B, uint8_t *d_corr, uint8_t *d_conv,
-                                       double *d_pm, void *stream) {
-    if (!d || B < 0 || (B > 0 && (!d_synd || !d_corr || !d_conv))) { set_err("decode: null argument"); return SWD_ERR_INVALID; }
-    if (B == 0) return SWD_OK;
-    CK(cudaSetDevice(d->device));
-    return decode_device_impl(d, d_synd, B, d_corr, d_conv, d_pm, (cudaStream_t)stream, nullptr, false);
-}
-
-extern "C" int swd_decode_batch_device_llr(swd_decoder *d, const uint8_t *d_synd, int64_t B, uint8_t *d_corr, uint8_t *d_conv,
-                                           double *d_pm, const double *d_channel_llr, void *stream) {
-    if (!d || B < 0 || !d_channel_llr || (B > 0 && (!d_synd || !d_corr || !d_conv))) { set_err("decode: null argument"); return SWD_ERR_INVALID; }
-    if (d->osd_only) { set_err("decode: not a window decoder"); return SWD_ERR_INVALID; }
-    if (B == 0) return SWD_OK;
-    CK(cudaSetDevice(d->device));
-    return decode_device_impl(d, d_synd, B, d_corr, d_conv, d_pm, (cudaStream_t)stream, d_channel_llr, false);
-}
-
-static int decode_host_impl(swd_decoder *d, const uint8_t *synd, int64_t B, uint8_t *corr, uint8_t *conv, double *pm, const double *llr) {
-    CK(cudaSetDevice(d->device));
-    { int st0 = ensure_stage(d, B); if (st0) return st0; }
-    cudaStream_t s = d->stream;
-    CK(cudaMemcpyAsync(d->d_synd, synd, (size_t)B * d->m, cudaMemcpyHostToDevice, s));
-    int st = decode_device_impl(d, d->d_synd, B, d->d_corr, d->d_conv, d->d_pm, s, llr, llr != nullptr);
-    if (st) return st;
-    CK(cudaMemcpyAsync(corr, d->d_corr, (size_t)B * d->n, cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(conv, d->d_conv, (size_t)B, cudaMemcpyDeviceToHost, s));
-    if (pm) CK(cudaMemcpyAsync(pm, d->d_pm, (size_t)B * 8, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    return SWD_OK;
-}
-
-extern "C" int swd_decode_batch_host(swd_decoder *d, const uint8_t *synd, int64_t B, uint8_t *corr, uint8_t *conv, double *pm) {
-    if (!d || B < 0 || (B > 0 && (!synd || !corr || !conv))) { set_err("decode: null argument"); return SWD_ERR_INVALID; }
-    if (B == 0) return SWD_OK;
-    return decode_host_impl(d, synd, B, corr, conv, pm, nullptr);
-}
-
-extern "C" int swd_decode_batch_host_llr(swd_decoder *d, const uint8_t *synd, int64_t B, uint8_t *corr, uint8_t *conv, double *pm,
-                                         const double *channel_llr) {
-    if (!d || B < 0 || !channel_llr || (B > 0 && (!synd || !corr || !conv))) { set_err("decode: null argument"); return SWD_ERR_INVALID; }
-    if (d->osd_only) { set_err("decode: not a window decoder"); return SWD_ERR_INVALID; }
-    if (B == 0) return SWD_OK;
-    return decode_host_impl(d, synd, B, corr, conv, pm, channel_llr);
 }
 
 // ---- bit-packed shot I/O ------------------------------------------------------------------------------------------
@@ -990,73 +995,87 @@ extern "C" int swd_unpack_bits(int device, const uint64_t *d_packed, int64_t B, 
     return launch_unpack((const u64 *)d_packed, B, nbits, d_bytes, (cudaStream_t)stream);
 }
 
+// the staging buffers of the host and packed entry points: byte and packed images of B shots' syndromes and corrections
 static int ensure_stage(swd_decoder *d, long long B) {
-    if (B > d->stage_cap) {
-        if (d->d_synd) { cudaFree(d->d_synd); cudaFree(d->d_corr); cudaFree(d->d_conv); cudaFree(d->d_pm); cudaFree(d->d_psynd); cudaFree(d->d_pcorr); d->d_synd = nullptr; }
-        CK(cudaMalloc(&d->d_synd, (size_t)B * d->m));
-        CK(cudaMalloc(&d->d_corr, (size_t)B * d->n));
-        CK(cudaMalloc(&d->d_conv, (size_t)B));
-        CK(cudaMalloc(&d->d_pm, (size_t)B * 8));
-        CK(cudaMalloc(&d->d_psynd, (size_t)B * ((d->m + 63) / 64) * 8));
-        CK(cudaMalloc(&d->d_pcorr, (size_t)B * ((d->n + 63) / 64) * 8));
-        d->stage_cap = B;
+    const size_t ws = (d->m + 63) / 64, wc = (d->n + 63) / 64;
+    int st;
+    if ((st = d->d_synd.reserve((size_t)B * d->m)) || (st = d->d_corr.reserve((size_t)B * d->n)) || (st = d->d_conv.reserve(B)) ||
+        (st = d->d_pm.reserve(B)) || (st = d->d_psynd.reserve((size_t)B * ws)) || (st = d->d_pcorr.reserve((size_t)B * wc))) return st;
+    return SWD_OK;
+}
+
+// The eight swd_decode_batch_* entry points.  host: syndromes, outputs and per-shot priors in host memory, on the decoder's
+// own stream, synchronised before returning; otherwise device pointers on `stream`.  packed: syndromes and corrections
+// bit-packed (8x fewer bytes over PCIe for a host call), unpacked and packed through the staging buffers, so calls on one
+// decoder must be stream-ordered.  llr: per-shot priors [B][n] or nullptr; llr_ok is false when an _llr entry point got none.
+static int decode_impl(swd_decoder *d, bool host, bool packed, const void *synd, int64_t B, void *corr, uint8_t *conv, double *pm,
+                       const double *llr, bool llr_ok, void *stream) {
+    if (!d || B < 0 || !llr_ok || (B > 0 && (!synd || !corr || !conv))) { set_err("decode: null argument"); return SWD_ERR_INVALID; }
+    if (d->osd_only) { set_err("decode: not a window decoder"); return SWD_ERR_INVALID; }
+    if (B == 0) return SWD_OK;
+    CK(cudaSetDevice(d->device));
+    int st;
+    if ((host || packed) && (st = ensure_stage(d, B))) return st;
+    cudaStream_t s = host ? d->stream : (cudaStream_t)stream;
+    // the device images of the syndromes and corrections in the call's format, and of conv and pm: the caller's, or staging
+    // buffers for a host call
+    const void *d_in = synd;
+    void *d_out = corr;
+    u8 *d_conv = conv;
+    double *d_pm = pm;
+    if (host) {
+        void *stage_in = packed ? (void *)d->d_psynd.p : d->d_synd.p;
+        CK(cudaMemcpyAsync(stage_in, synd, packed ? (size_t)B * ((d->m + 63) / 64) * 8 : (size_t)B * d->m, cudaMemcpyHostToDevice, s));
+        d_in = stage_in; d_out = packed ? (void *)d->d_pcorr.p : d->d_corr.p;
+        d_conv = d->d_conv.p; d_pm = d->d_pm.p;
+    }
+    if (packed && (st = launch_unpack((const u64 *)d_in, B, d->m, d->d_synd.p, s))) return st;
+    const u8 *d_synd = packed ? d->d_synd.p : (const u8 *)d_in;
+    u8 *d_corr = packed ? d->d_corr.p : (u8 *)d_out;
+    if ((st = decode_device_impl(d, d_synd, B, d_corr, d_conv, d_pm, s, llr, host && llr))) return st;
+    if (packed) {
+        d->ctr.kernel_launches += 2;
+        if ((st = launch_pack(d_corr, B, d->n, (u64 *)d_out, s))) return st;
+    }
+    if (host) {
+        CK(cudaMemcpyAsync(corr, d_out, packed ? (size_t)B * ((d->n + 63) / 64) * 8 : (size_t)B * d->n, cudaMemcpyDeviceToHost, s));
+        CK(cudaMemcpyAsync(conv, d_conv, (size_t)B, cudaMemcpyDeviceToHost, s));
+        if (pm) CK(cudaMemcpyAsync(pm, d_pm, (size_t)B * 8, cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
     }
     return SWD_OK;
 }
 
-// packed device pointers; the byte images live in the decoder's staging buffers (calls on one decoder must be stream-ordered)
-static int decode_device_packed_impl(swd_decoder *d, const uint64_t *d_synd_packed, int64_t B, uint64_t *d_corr_packed, uint8_t *d_conv,
-                                     double *d_pm, cudaStream_t s, const double *llr, bool llr_host) {
-    CK(cudaSetDevice(d->device));
-    int st = ensure_stage(d, B);
-    if (st) return st;
-    if ((st = launch_unpack((const u64 *)d_synd_packed, B, d->m, d->d_synd, s))) return st;
-    if ((st = decode_device_impl(d, d->d_synd, B, d->d_corr, d_conv, d_pm, s, llr, llr_host))) return st;
-    d->ctr.kernel_launches += 2;
-    return launch_pack(d->d_corr, B, d->n, (u64 *)d_corr_packed, s);
+extern "C" int swd_decode_batch_host(swd_decoder *d, const uint8_t *synd, int64_t B, uint8_t *corr, uint8_t *conv, double *pm) {
+    return decode_impl(d, true, false, synd, B, corr, conv, pm, nullptr, true, nullptr);
 }
-extern "C" int swd_decode_batch_device_packed(swd_decoder *d, const uint64_t *d_synd_packed, int64_t B, uint64_t *d_corr_packed,
-                                              uint8_t *d_conv, double *d_pm, void *stream) {
-    if (!d || B < 0 || (B > 0 && (!d_synd_packed || !d_corr_packed || !d_conv))) { set_err("decode: null argument"); return SWD_ERR_INVALID; }
-    if (B == 0) return SWD_OK;
-    return decode_device_packed_impl(d, d_synd_packed, B, d_corr_packed, d_conv, d_pm, (cudaStream_t)stream, nullptr, false);
+extern "C" int swd_decode_batch_host_llr(swd_decoder *d, const uint8_t *synd, int64_t B, uint8_t *corr, uint8_t *conv, double *pm,
+                                         const double *channel_llr) {
+    return decode_impl(d, true, false, synd, B, corr, conv, pm, channel_llr, channel_llr != nullptr, nullptr);
 }
-extern "C" int swd_decode_batch_device_packed_llr(swd_decoder *d, const uint64_t *d_synd_packed, int64_t B, uint64_t *d_corr_packed,
-                                                  uint8_t *d_conv, double *d_pm, const double *d_channel_llr, void *stream) {
-    if (!d || B < 0 || !d_channel_llr || (B > 0 && (!d_synd_packed || !d_corr_packed || !d_conv))) { set_err("decode: null argument"); return SWD_ERR_INVALID; }
-    if (d->osd_only) { set_err("decode: not a window decoder"); return SWD_ERR_INVALID; }
-    if (B == 0) return SWD_OK;
-    return decode_device_packed_impl(d, d_synd_packed, B, d_corr_packed, d_conv, d_pm, (cudaStream_t)stream, d_channel_llr, false);
+extern "C" int swd_decode_batch_device(swd_decoder *d, const uint8_t *d_synd, int64_t B, uint8_t *d_corr, uint8_t *d_conv,
+                                       double *d_pm, void *stream) {
+    return decode_impl(d, false, false, d_synd, B, d_corr, d_conv, d_pm, nullptr, true, stream);
 }
-
-// packed host pointers: 8x fewer bytes over PCIe in both directions
-static int decode_host_packed_impl(swd_decoder *d, const uint64_t *synd_packed, int64_t B, uint64_t *corr_packed, uint8_t *conv,
-                                   double *pm, const double *llr) {
-    CK(cudaSetDevice(d->device));
-    int st = ensure_stage(d, B);
-    if (st) return st;
-    cudaStream_t s = d->stream;
-    const size_t ws = (size_t)((d->m + 63) / 64) * 8, wc = (size_t)((d->n + 63) / 64) * 8;
-    CK(cudaMemcpyAsync(d->d_psynd, synd_packed, (size_t)B * ws, cudaMemcpyHostToDevice, s));
-    if ((st = decode_device_packed_impl(d, (const uint64_t *)d->d_psynd, B, (uint64_t *)d->d_pcorr, d->d_conv, d->d_pm, s, llr, llr != nullptr))) return st;
-    CK(cudaMemcpyAsync(corr_packed, d->d_pcorr, (size_t)B * wc, cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(conv, d->d_conv, (size_t)B, cudaMemcpyDeviceToHost, s));
-    if (pm) CK(cudaMemcpyAsync(pm, d->d_pm, (size_t)B * 8, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    return SWD_OK;
+extern "C" int swd_decode_batch_device_llr(swd_decoder *d, const uint8_t *d_synd, int64_t B, uint8_t *d_corr, uint8_t *d_conv,
+                                           double *d_pm, const double *d_channel_llr, void *stream) {
+    return decode_impl(d, false, false, d_synd, B, d_corr, d_conv, d_pm, d_channel_llr, d_channel_llr != nullptr, stream);
 }
 extern "C" int swd_decode_batch_host_packed(swd_decoder *d, const uint64_t *synd_packed, int64_t B, uint64_t *corr_packed, uint8_t *conv,
                                             double *pm) {
-    if (!d || B < 0 || (B > 0 && (!synd_packed || !corr_packed || !conv))) { set_err("decode: null argument"); return SWD_ERR_INVALID; }
-    if (B == 0) return SWD_OK;
-    return decode_host_packed_impl(d, synd_packed, B, corr_packed, conv, pm, nullptr);
+    return decode_impl(d, true, true, synd_packed, B, corr_packed, conv, pm, nullptr, true, nullptr);
 }
 extern "C" int swd_decode_batch_host_packed_llr(swd_decoder *d, const uint64_t *synd_packed, int64_t B, uint64_t *corr_packed, uint8_t *conv,
                                                 double *pm, const double *channel_llr) {
-    if (!d || B < 0 || !channel_llr || (B > 0 && (!synd_packed || !corr_packed || !conv))) { set_err("decode: null argument"); return SWD_ERR_INVALID; }
-    if (d->osd_only) { set_err("decode: not a window decoder"); return SWD_ERR_INVALID; }
-    if (B == 0) return SWD_OK;
-    return decode_host_packed_impl(d, synd_packed, B, corr_packed, conv, pm, channel_llr);
+    return decode_impl(d, true, true, synd_packed, B, corr_packed, conv, pm, channel_llr, channel_llr != nullptr, nullptr);
+}
+extern "C" int swd_decode_batch_device_packed(swd_decoder *d, const uint64_t *d_synd_packed, int64_t B, uint64_t *d_corr_packed,
+                                              uint8_t *d_conv, double *d_pm, void *stream) {
+    return decode_impl(d, false, true, d_synd_packed, B, d_corr_packed, d_conv, d_pm, nullptr, true, stream);
+}
+extern "C" int swd_decode_batch_device_packed_llr(swd_decoder *d, const uint64_t *d_synd_packed, int64_t B, uint64_t *d_corr_packed,
+                                                  uint8_t *d_conv, double *d_pm, const double *d_channel_llr, void *stream) {
+    return decode_impl(d, false, true, d_synd_packed, B, d_corr_packed, d_conv, d_pm, d_channel_llr, d_channel_llr != nullptr, stream);
 }
 
 extern "C" int swd_is_streamed(swd_decoder *d) { return d ? (d->stream_mode ? 1 : 0) : -1; }
@@ -1067,24 +1086,10 @@ extern "C" int swd_pre_bp_layout(int m, int n, const int32_t *colptr, const int3
     if (!colptr || !rowidx || m <= 0 || n <= 0 || colptr[0] != 0) { set_err("swd_pre_bp_layout: bad argument"); return SWD_ERR_INVALID; }
     const int nnz = colptr[n];
     if (n > 65534 || m > 65534 || nnz > 65535 || nnz < 0) { set_err("swd_pre_bp_layout: graph too large for 16-bit indices"); return SWD_ERR_UNSUPPORTED; }
-    std::vector<int> cp(colptr, colptr + n + 1), cr(std::max(nnz, 1)), rp(m + 1, 0), cpos(std::max(nnz, 1));
-    for (int c = 0; c < n; c++) {
-        if (cp[c + 1] < cp[c]) { set_err("swd_pre_bp_layout: colptr not monotone"); return SWD_ERR_INVALID; }
-        std::vector<int> rows(rowidx + cp[c], rowidx + cp[c + 1]);
-        std::sort(rows.begin(), rows.end());
-        for (size_t k = 0; k < rows.size(); k++) {
-            if (rows[k] < 0 || rows[k] >= m || (k && rows[k] == rows[k - 1])) { set_err("swd_pre_bp_layout: bad row index"); return SWD_ERR_INVALID; }
-            cr[cp[c] + k] = rows[k]; rp[rows[k] + 1]++;
-        }
-    }
-    for (int r = 0; r < m; r++) rp[r + 1] += rp[r];
-    { std::vector<int> fill(rp.begin(), rp.end() - 1); for (int c = 0; c < n; c++) for (int e = cp[c]; e < cp[c + 1]; e++) cpos[e] = fill[cr[e]]++; }
-    std::vector<u16> vord(n);
-    { std::vector<int> idx(n); for (int c = 0; c < n; c++) idx[c] = c;
-      std::stable_sort(idx.begin(), idx.end(), [&](int a, int b) { return cp[a + 1] - cp[a] > cp[b + 1] - cp[b]; });
-      for (int c = 0; c < n; c++) vord[c] = (u16)idx[c]; }
+    FlatGraph G;
+    if (const char *why = flat_graph(m, n, colptr, rowidx, G)) { set_err(std::string("swd_pre_bp_layout: ") + why); return SWD_ERR_INVALID; }
     PreLayout L;
-    pre_layout(m, n, nnz, cp, cr, rp, cpos, vord, optimize != 0, L);
+    pre_layout(m, n, nnz, G.cp, G.cr, G.rp, G.cpos, G.vord, optimize != 0, L);
     if (slot_of_entry) for (int e = 0; e < nnz; e++) slot_of_entry[e] = L.phys[e];     // CSC entry (rows ascending inside a column) -> slot
     if (row_start) for (int r = 0; r <= m; r++) row_start[r] = L.pstart[r];
     if (stats) { stats[0] = L.nphys; stats[1] = L.excess0; stats[2] = L.excess; }
@@ -1149,32 +1154,26 @@ extern "C" int swd_new_n(swd_decoder *d) { return d ? d->nn : -1; }
 // ------------------------------------------------------------------------------------------------
 struct swd_window {
     int device, num_det, num_col, num_obs;
-    int *chk_cp = nullptr, *chk_ri = nullptr, *obs_cp = nullptr, *obs_ri = nullptr;
-    u32 *thr = nullptr;          // floor(prior * 2^32) per DEM column (set by swd_window_set_priors)
-    u32 *pauli_thr = nullptr;    // code capacity (swd_window_set_pauli_priors): thr(px) | thr(px + py) | thr(px + py + pz), n each
+    DevBuf<int> chk_cp, chk_ri, obs_cp, obs_ri;
+    DevBuf<u32> thr;             // floor(prior * 2^32) per DEM column (set by swd_window_set_priors)
+    DevBuf<u32> pauli_thr;       // code capacity (swd_window_set_pauli_priors): thr(px) | thr(px + py) | thr(px + py + pz), n each
     u32 pauli_t_erase = 0;       // thr(erasure_rate)
     int pauli_n = 0;             // 0 until swd_window_set_pauli_priors
-    double *pauli_llr5 = nullptr; // static LLR rows [5][n] copied into the per-shot planes, or nullptr
-    uint4 *circ_work = nullptr;  // circuit noise (swd_window_set_circuit_noise): (l, m0, n_l, thr(e_l)) sorted by n_l
-    uint2 *circ_mech = nullptr;  // (DEM column or -1, thr(p)) per mechanism
-    double *circ_llr = nullptr;  // static LLR row [num_col], or nullptr
+    DevBuf<double> pauli_llr5;   // static LLR rows [5][n] copied into the per-shot planes, or empty
+    DevBuf<uint4> circ_work;     // circuit noise (swd_window_set_circuit_noise): (l, m0, n_l, thr(e_l)) sorted by n_l
+    DevBuf<uint2> circ_mech;     // (DEM column or -1, thr(p)) per mechanism
+    DevBuf<double> circ_llr;     // static LLR row [num_col], or empty
     int circ_num_loc = 0;        // 0 until swd_window_set_circuit_noise
     std::vector<uint4> circ_work_h;   // host copies of circ_work and of the mechanisms' columns (readout set-up reads them)
     std::vector<int> circ_col_h;
-    uint4 *ro_work = nullptr;    // soft readout (swd_window_set_circuit_readout): circ_work with z = 1 | (r + 1) << 4 at readout r
-    u32 *ro_thr = nullptr;       // thr(w_0 + .. + w_{k-1}) for k = 1 .. K-1, then thr(q_k) for k = 0 .. K-1
-    int *ro_col = nullptr;       // [num_col] readout location whose mechanism is in column c, or -1
-    double *ro_llr = nullptr;    // class_llr [num_readout][K], or nullptr
-    int ro_num = 0, ro_K = 0;    // 0 until swd_window_set_circuit_readout
+    struct Readout {             // soft readout (swd_window_set_circuit_readout); a new circuit-noise set-up clears it
+        DevBuf<uint4> work;      // circ_work with z = 1 | (r + 1) << 4 at readout r
+        DevBuf<u32> thr;         // thr(w_0 + .. + w_{k-1}) for k = 1 .. K-1, then thr(q_k) for k = 0 .. K-1
+        DevBuf<int> col;         // [num_col] readout location whose mechanism is in column c, or -1
+        DevBuf<double> llr;      // class_llr [num_readout][K], or empty
+        int num = 0, K = 0;      // 0 until swd_window_set_circuit_readout
+    } ro;
 };
-
-static void clear_circuit_readout(swd_window *w) {
-    if (w->ro_work) { cudaFree(w->ro_work); w->ro_work = nullptr; }
-    if (w->ro_thr) { cudaFree(w->ro_thr); w->ro_thr = nullptr; }
-    if (w->ro_col) { cudaFree(w->ro_col); w->ro_col = nullptr; }
-    if (w->ro_llr) { cudaFree(w->ro_llr); w->ro_llr = nullptr; }
-    w->ro_num = w->ro_K = 0;
-}
 
 extern "C" int swd_window_create(int device, int num_det, int num_col, const int32_t *chk_cp, const int32_t *chk_ri, int num_obs,
                                  const int32_t *obs_cp, const int32_t *obs_ri, swd_window **out) {
@@ -1186,10 +1185,10 @@ extern "C" int swd_window_create(int device, int num_det, int num_col, const int
     w->device = device; w->num_det = num_det; w->num_col = num_col; w->num_obs = num_obs;
     std::vector<int> a(chk_cp, chk_cp + num_col + 1), b(chk_ri, chk_ri + chk_cp[num_col]);
     int st;
-    if ((st = upload(a, (void **)&w->chk_cp)) || (st = upload(b, (void **)&w->chk_ri))) { swd_window_destroy(w); return st; }
+    if ((st = w->chk_cp.upload(a)) || (st = w->chk_ri.upload(b))) { swd_window_destroy(w); return st; }
     if (num_obs > 0) {
         std::vector<int> c(obs_cp, obs_cp + num_col + 1), e(obs_ri, obs_ri + obs_cp[num_col]);
-        if ((st = upload(c, (void **)&w->obs_cp)) || (st = upload(e, (void **)&w->obs_ri))) { swd_window_destroy(w); return st; }
+        if ((st = w->obs_cp.upload(c)) || (st = w->obs_ri.upload(e))) { swd_window_destroy(w); return st; }
     }
     *out = w;
     return SWD_OK;
@@ -1197,17 +1196,6 @@ extern "C" int swd_window_create(int device, int num_det, int num_col, const int
 extern "C" void swd_window_destroy(swd_window *w) {
     if (!w) return;
     cudaSetDevice(w->device);
-    if (w->chk_cp) cudaFree(w->chk_cp);
-    if (w->chk_ri) cudaFree(w->chk_ri);
-    if (w->obs_cp) cudaFree(w->obs_cp);
-    if (w->obs_ri) cudaFree(w->obs_ri);
-    if (w->thr) cudaFree(w->thr);
-    if (w->pauli_thr) cudaFree(w->pauli_thr);
-    if (w->pauli_llr5) cudaFree(w->pauli_llr5);
-    if (w->circ_work) cudaFree(w->circ_work);
-    if (w->circ_mech) cudaFree(w->circ_mech);
-    if (w->circ_llr) cudaFree(w->circ_llr);
-    clear_circuit_readout(w);
     delete w;
 }
 static u32 prob_threshold(double p) {          // the samplers' rule: floor(p * 2^32), clamped to 0xffffffff
@@ -1242,8 +1230,7 @@ extern "C" int swd_window_set_priors(swd_window *w, const double *priors) {
         t[c] = prob_threshold(p);
     }
     CK(cudaSetDevice(w->device));
-    if (w->thr) { cudaFree(w->thr); w->thr = nullptr; }
-    return upload(t, (void **)&w->thr);
+    return w->thr.upload(t);
 }
 extern "C" int swd_window_set_pauli_priors(swd_window *w, int n, const double *px, const double *py, const double *pz,
                                            double erasure_rate, const double *llr5) {
@@ -1257,12 +1244,11 @@ extern "C" int swd_window_set_pauli_priors(swd_window *w, int n, const double *p
         t[v] = prob_threshold(px[v]); t[n + v] = prob_threshold(xy); t[2 * n + v] = prob_threshold(xyz);
     }
     CK(cudaSetDevice(w->device));
-    if (w->pauli_thr) { cudaFree(w->pauli_thr); w->pauli_thr = nullptr; }
-    if (w->pauli_llr5) { cudaFree(w->pauli_llr5); w->pauli_llr5 = nullptr; }
+    w->pauli_llr5.release();
     w->pauli_n = 0;
     int st;
-    if ((st = upload(t, (void **)&w->pauli_thr))) return st;
-    if (llr5 && (st = upload(std::vector<double>(llr5, llr5 + 5 * (size_t)n), (void **)&w->pauli_llr5))) return st;
+    if ((st = w->pauli_thr.upload(t))) return st;
+    if (llr5 && (st = w->pauli_llr5.upload(std::vector<double>(llr5, llr5 + 5 * (size_t)n)))) return st;
     w->pauli_t_erase = prob_threshold(erasure_rate);
     w->pauli_n = n;
     return SWD_OK;
@@ -1271,10 +1257,10 @@ extern "C" int swd_window_sample_pauli(swd_window *w, uint64_t seed, int64_t sho
                                        uint8_t *d_err, uint8_t *d_erased, double *d_channel_llr, void *stream) {
     if (!w || !d_det || B < 0 || shot_offset < 0 || (w->num_obs > 0 && !d_obs)) { set_err("swd_window_sample_pauli: bad argument"); return SWD_ERR_INVALID; }
     if (!w->pauli_n) { set_err("swd_window_sample_pauli: call swd_window_set_pauli_priors first"); return SWD_ERR_INVALID; }
-    if (d_channel_llr && !w->pauli_llr5) { set_err("swd_window_sample_pauli: channel_llr needs the llr5 rows of swd_window_set_pauli_priors"); return SWD_ERR_INVALID; }
+    if (d_channel_llr && !w->pauli_llr5.p) { set_err("swd_window_sample_pauli: channel_llr needs the llr5 rows of swd_window_set_pauli_priors"); return SWD_ERR_INVALID; }
     if (B == 0) return SWD_OK;
     return launch_sampler(window_sample_pauli_kernel, w, parity_bytes(w), B, stream, "swd_window_sample_pauli",
-        w->pauli_thr, w->pauli_t_erase, w->pauli_n, w->pauli_llr5, w->chk_cp, w->chk_ri, w->num_det, w->obs_cp, w->obs_ri,
+        w->pauli_thr.p, w->pauli_t_erase, w->pauli_n, w->pauli_llr5.p, w->chk_cp.p, w->chk_ri.p, w->num_det, w->obs_cp.p, w->obs_ri.p,
         w->num_obs, (unsigned long long)seed, (long long)shot_offset, (long long)B, d_det, d_obs, d_err, d_erased, d_channel_llr);
 }
 extern "C" int swd_window_set_circuit_noise(swd_window *w, int num_loc, const int32_t *mech_ptr, const int32_t *mech_col,
@@ -1300,14 +1286,12 @@ extern "C" int swd_window_set_circuit_noise(swd_window *w, int num_loc, const in
     // lanes of a warp take consecutive work items: equal mechanism counts give them equal numbers of Philox calls
     std::stable_sort(work.begin(), work.end(), [](const uint4 &a, const uint4 &b) { return a.z > b.z; });
     CK(cudaSetDevice(w->device));
-    if (w->circ_work) { cudaFree(w->circ_work); w->circ_work = nullptr; }
-    if (w->circ_mech) { cudaFree(w->circ_mech); w->circ_mech = nullptr; }
-    if (w->circ_llr) { cudaFree(w->circ_llr); w->circ_llr = nullptr; }
-    clear_circuit_readout(w);
+    w->circ_llr.release();
+    w->ro = {};
     w->circ_num_loc = 0;
     int st;
-    if ((st = upload(work, (void **)&w->circ_work)) || (st = upload(mech, (void **)&w->circ_mech))) return st;
-    if (col_llr && (st = upload(std::vector<double>(col_llr, col_llr + w->num_col), (void **)&w->circ_llr))) return st;
+    if ((st = w->circ_work.upload(work)) || (st = w->circ_mech.upload(mech))) return st;
+    if (col_llr && (st = w->circ_llr.upload(std::vector<double>(col_llr, col_llr + w->num_col)))) return st;
     w->circ_work_h = work;
     w->circ_col_h.assign(mech_col, mech_col + M);
     w->circ_num_loc = num_loc;
@@ -1351,16 +1335,14 @@ extern "C" int swd_window_set_circuit_readout(swd_window *w, int num_readout, co
         return (a.z & 15u) != (b.z & 15u) ? (a.z & 15u) > (b.z & 15u) : (a.z >> 4 == 0) && (b.z >> 4 != 0);
     });
     CK(cudaSetDevice(w->device));
-    clear_circuit_readout(w);
+    w->ro = {};
     int st;
-    if ((st = upload(work, (void **)&w->ro_work)) || (st = upload(thr, (void **)&w->ro_thr)) || (st = upload(col_ro, (void **)&w->ro_col))) {
-        clear_circuit_readout(w); return st;
+    if ((st = w->ro.work.upload(work)) || (st = w->ro.thr.upload(thr)) || (st = w->ro.col.upload(col_ro)) ||
+        (class_llr && (st = w->ro.llr.upload(std::vector<double>(class_llr, class_llr + (size_t)num_readout * K))))) {
+        w->ro = {}; return st;
     }
-    if (class_llr && (st = upload(std::vector<double>(class_llr, class_llr + (size_t)num_readout * K), (void **)&w->ro_llr))) {
-        clear_circuit_readout(w); return st;
-    }
-    w->ro_num = num_readout;
-    w->ro_K = K;
+    w->ro.num = num_readout;
+    w->ro.K = K;
     return SWD_OK;
 }
 // the per-warp words are the parity words, the optional err and LLR column words, and the readout class bytes
@@ -1372,38 +1354,38 @@ static int launch_sample_circuit(swd_window *w, const uint4 *work, const Circuit
     const size_t warp_bytes = parity_bytes(w) + (size_t)((d_err ? wc : 0) + (d_channel_llr ? wc : 0) +
                                                          (READOUT && d_channel_llr ? (ro.num_readout + 3) >> 2 : 0)) * sizeof(u32);
     return launch_sampler(window_sample_circuit_kernel<READOUT>, w, warp_bytes, B, stream, who,
-        work, w->circ_num_loc, w->circ_mech, w->circ_llr, w->num_col, w->chk_cp, w->chk_ri, w->num_det, w->obs_cp, w->obs_ri,
+        work, w->circ_num_loc, w->circ_mech.p, w->circ_llr.p, w->num_col, w->chk_cp.p, w->chk_ri.p, w->num_det, w->obs_cp.p, w->obs_ri.p,
         w->num_obs, (unsigned long long)seed, (long long)shot_offset, (long long)B, d_det, d_obs, d_err, d_erased, d_channel_llr, ro);
 }
 extern "C" int swd_window_sample_circuit(swd_window *w, uint64_t seed, int64_t shot_offset, int64_t B, uint8_t *d_det, uint8_t *d_obs,
                                          uint8_t *d_err, uint8_t *d_erased, double *d_channel_llr, void *stream) {
     if (!w || !d_det || B < 0 || shot_offset < 0 || (w->num_obs > 0 && !d_obs)) { set_err("swd_window_sample_circuit: bad argument"); return SWD_ERR_INVALID; }
     if (!w->circ_num_loc) { set_err("swd_window_sample_circuit: call swd_window_set_circuit_noise first"); return SWD_ERR_INVALID; }
-    if (d_channel_llr && !w->circ_llr) { set_err("swd_window_sample_circuit: channel_llr needs the col_llr row of swd_window_set_circuit_noise"); return SWD_ERR_INVALID; }
+    if (d_channel_llr && !w->circ_llr.p) { set_err("swd_window_sample_circuit: channel_llr needs the col_llr row of swd_window_set_circuit_noise"); return SWD_ERR_INVALID; }
     if (B == 0) return SWD_OK;
-    return launch_sample_circuit<false>(w, w->circ_work, CircuitReadout{}, seed, shot_offset, B, d_det, d_obs, d_err, d_erased,
+    return launch_sample_circuit<false>(w, w->circ_work.p, CircuitReadout{}, seed, shot_offset, B, d_det, d_obs, d_err, d_erased,
                                         d_channel_llr, stream, "swd_window_sample_circuit");
 }
 extern "C" int swd_window_sample_circuit_readout(swd_window *w, uint64_t seed, int64_t shot_offset, int64_t B, uint8_t *d_det,
                                                  uint8_t *d_obs, uint8_t *d_err, uint8_t *d_erased, uint8_t *d_readout,
                                                  double *d_channel_llr, void *stream) {
     if (!w || !d_det || B < 0 || shot_offset < 0 || (w->num_obs > 0 && !d_obs)) { set_err("swd_window_sample_circuit_readout: bad argument"); return SWD_ERR_INVALID; }
-    if (!w->ro_num) { set_err("swd_window_sample_circuit_readout: call swd_window_set_circuit_readout first"); return SWD_ERR_INVALID; }
-    if (d_channel_llr && (!w->circ_llr || !w->ro_llr)) {
+    if (!w->ro.num) { set_err("swd_window_sample_circuit_readout: call swd_window_set_circuit_readout first"); return SWD_ERR_INVALID; }
+    if (d_channel_llr && (!w->circ_llr.p || !w->ro.llr.p)) {
         set_err("swd_window_sample_circuit_readout: channel_llr needs the col_llr row and the class_llr table"); return SWD_ERR_INVALID;
     }
     if (B == 0) return SWD_OK;
-    const CircuitReadout ro{w->ro_thr, w->ro_thr + (w->ro_K - 1), w->ro_col, w->ro_llr, d_readout, w->ro_K, w->ro_num};
-    return launch_sample_circuit<true>(w, w->ro_work, ro, seed, shot_offset, B, d_det, d_obs, d_err, d_erased, d_channel_llr, stream,
+    const CircuitReadout ro{w->ro.thr.p, w->ro.thr.p + (w->ro.K - 1), w->ro.col.p, w->ro.llr.p, d_readout, w->ro.K, w->ro.num};
+    return launch_sample_circuit<true>(w, w->ro.work.p, ro, seed, shot_offset, B, d_det, d_obs, d_err, d_erased, d_channel_llr, stream,
                                        "swd_window_sample_circuit_readout");
 }
 extern "C" int swd_window_sample(swd_window *w, uint64_t seed, int64_t shot_offset, int64_t B, uint8_t *d_det, uint8_t *d_obs,
                                  uint8_t *d_err, void *stream) {
     if (!w || !d_det || B < 0 || shot_offset < 0 || (w->num_obs > 0 && !d_obs)) { set_err("swd_window_sample: bad argument"); return SWD_ERR_INVALID; }
-    if (!w->thr) { set_err("swd_window_sample: call swd_window_set_priors first"); return SWD_ERR_INVALID; }
+    if (!w->thr.p) { set_err("swd_window_sample: call swd_window_set_priors first"); return SWD_ERR_INVALID; }
     if (B == 0) return SWD_OK;
     return launch_sampler(window_sample_kernel, w, parity_bytes(w), B, stream, "swd_window_sample",
-        w->thr, w->num_col, w->chk_cp, w->chk_ri, w->num_det, w->obs_cp, w->obs_ri, w->num_obs, (unsigned long long)seed,
+        w->thr.p, w->num_col, w->chk_cp.p, w->chk_ri.p, w->num_det, w->obs_cp.p, w->obs_ri.p, w->num_obs, (unsigned long long)seed,
         (long long)shot_offset, (long long)B, d_det, d_obs, d_err);
 }
 extern "C" int swd_window_extract(swd_window *w, const uint8_t *d_det, int64_t B, int row0, int m, uint8_t *d_synd, void *stream) {
@@ -1425,7 +1407,7 @@ extern "C" int swd_window_commit(swd_window *w, const uint8_t *d_corr, int64_t B
     CK(cudaSetDevice(w->device));
     const int wpb = 8;
     window_commit_kernel<<<(unsigned)std::min<long long>((B + wpb - 1) / wpb, 1 << 20), wpb * 32, 0, (cudaStream_t)stream>>>(
-        d_corr, B, n_win, col0, ncommit, w->chk_cp, w->chk_ri, w->num_det, d_det, w->obs_cp, w->obs_ri, w->num_obs, d_obs);
+        d_corr, B, n_win, col0, ncommit, w->chk_cp.p, w->chk_ri.p, w->num_det, d_det, w->obs_cp.p, w->obs_ri.p, w->num_obs, d_obs);
     CK(cudaGetLastError());
     return SWD_OK;
 }
@@ -1449,48 +1431,30 @@ struct swd_bp4 {
     int device = 0, n = 0, mx = 0, mz = 0, max_iter = 32, num_sm = 0;
     double alpha = 1.0;
     swd_decoder *dx = nullptr, *dz = nullptr;      // osd_window-kind decoders over Hx / Hz: graph upload, rank, OSD machinery
-    double *llr = nullptr;                         // device: llr_x | llr_y | llr_z, n each
+    DevBuf<double> llr;                            // llr_x | llr_y | llr_z, n each
     Bp4Smem S{};
     int grid = 0;
     int grid_llr[2] = {0, 0};                      // per-shot priors: bp4_kernel<false, true>, <true, true> (camel)
-    double *d_llr5 = nullptr; long long llr5_cap = 0;     // host per-shot priors staged on the device, [5][B][n]; first _llr call
+    DevBuf<double> d_llr5;                         // host per-shot priors staged on the device, [5][B][n]; first _llr call
     // per-batch device buffers
-    long long cap = 0;
-    u8 *synd_x = nullptr, *synd_z = nullptr, *bp_dec = nullptr, *conv = nullptr, *dec = nullptr, *osd0 = nullptr, *tmp = nullptr;
-    int *iters = nullptr;
-    double *lpr = nullptr, *key_x = nullptr, *key_z = nullptr;
+    DevBuf<u8> synd_x, synd_z, bp_dec, conv, dec, osd0, tmp;
+    DevBuf<int> iters;
+    DevBuf<double> lpr, key_x, key_z;
     // camel_decode: four runs per shot
-    long long cap4 = 0;
-    u8 *c_synd_x = nullptr, *c_synd_z = nullptr, *c_bp_dec = nullptr, *c_conv4 = nullptr, *c_dec = nullptr, *c_conv = nullptr;
-    int *c_it4 = nullptr, *c_it = nullptr;
-    double *c_pm4 = nullptr, *c_pm = nullptr, *c_lpr = nullptr;
+    DevBuf<u8> c_synd_x, c_synd_z, c_bp_dec, c_conv4, c_dec, c_conv;
+    DevBuf<int> c_it4, c_it;
+    DevBuf<double> c_pm4, c_pm, c_lpr;
     cudaStream_t stream = nullptr;
+    ~swd_bp4() {
+        swd_destroy(dx);
+        swd_destroy(dz);
+        if (stream) cudaStreamDestroy(stream);
+    }
 };
-
-static void bp4_free_camel(swd_bp4 *b) {
-    void *ptrs[] = {b->c_synd_x, b->c_synd_z, b->c_bp_dec, b->c_conv4, b->c_dec, b->c_conv, b->c_it4, b->c_it, b->c_pm4, b->c_pm, b->c_lpr};
-    for (void *p : ptrs) if (p) cudaFree(p);
-    b->c_synd_x = b->c_synd_z = b->c_bp_dec = b->c_conv4 = b->c_dec = b->c_conv = nullptr; b->c_it4 = b->c_it = nullptr;
-    b->c_pm4 = b->c_pm = b->c_lpr = nullptr; b->cap4 = 0;
-}
-
-static void bp4_free_buffers(swd_bp4 *b) {
-    void *ptrs[] = {b->synd_x, b->synd_z, b->bp_dec, b->conv, b->dec, b->osd0, b->tmp, b->iters, b->lpr, b->key_x, b->key_z};
-    for (void *p : ptrs) if (p) cudaFree(p);
-    b->synd_x = b->synd_z = b->bp_dec = b->conv = b->dec = b->osd0 = b->tmp = nullptr; b->iters = nullptr;
-    b->lpr = b->key_x = b->key_z = nullptr; b->cap = 0;
-}
 
 extern "C" void swd_bp4_destroy(swd_bp4 *b) {
     if (!b) return;
     cudaSetDevice(b->device);
-    bp4_free_buffers(b);
-    bp4_free_camel(b);
-    if (b->llr) cudaFree(b->llr);
-    if (b->d_llr5) cudaFree(b->d_llr5);
-    if (b->dx) swd_destroy(b->dx);
-    if (b->dz) swd_destroy(b->dz);
-    if (b->stream) cudaStreamDestroy(b->stream);
     delete b;
 }
 
@@ -1511,7 +1475,7 @@ extern "C" int swd_bp4_create(int device, int mx, int mz, int n, const int32_t *
     b->num_sm = b->dx->num_sm;
     std::vector<double> l(3 * (size_t)n);
     for (int v = 0; v < n; v++) { l[v] = llr_x[v]; l[n + v] = llr_y[v]; l[2 * (size_t)n + v] = llr_z[v]; }
-    if ((st = upload(l, (void **)&b->llr)) != SWD_OK) { swd_bp4_destroy(b); return st; }
+    if ((st = b->llr.upload(l)) != SWD_OK) { swd_bp4_destroy(b); return st; }
     int o = 0;
     b->S.off_mx = o; o += 8 * std::max(1, b->dx->nnz); o = r16(o);
     b->S.off_mz = o; o += 8 * std::max(1, b->dz->nnz); o = r16(o);
@@ -1548,7 +1512,7 @@ static int bp4_osd_pass(swd_decoder *d, const u8 *d_synd, const double *d_keys, 
                         const double *d_prior) {
     int st = alloc_workspace(d, B, s);
     if (st) return st;
-    if ((st = osd_reserve_outputs(&d->ow, B, d->n, s))) { set_err("osd output alloc failed"); return SWD_ERR_NOMEM; }
+    if ((st = reserve_osd_outputs(d, B, s))) return st;
     for (long long b0 = 0; b0 < B; b0 += d->cap) {
         const long long nb = std::min<long long>(d->cap, B - b0);
         CK(cudaMemsetAsync(d->ws.counters, 0, 64 * sizeof(int), s));
@@ -1569,25 +1533,18 @@ static int bp4_osd_pass(swd_decoder *d, const u8 *d_synd, const double *d_keys, 
 
 static int bp4_reserve(swd_bp4 *b, int64_t B) {
     const size_t n = b->n;
-    if (B > b->cap) {
-        bp4_free_buffers(b);
-        CK(cudaMalloc(&b->synd_x, (size_t)B * b->mx)); CK(cudaMalloc(&b->synd_z, (size_t)B * b->mz));
-        CK(cudaMalloc(&b->bp_dec, (size_t)B * 2 * n)); CK(cudaMalloc(&b->conv, (size_t)B)); CK(cudaMalloc(&b->dec, (size_t)B * 2 * n));
-        CK(cudaMalloc(&b->osd0, (size_t)B * 2 * n)); CK(cudaMalloc(&b->tmp, (size_t)B * n)); CK(cudaMalloc(&b->iters, (size_t)B * 4));
-        CK(cudaMalloc(&b->lpr, (size_t)B * n * 24)); CK(cudaMalloc(&b->key_x, (size_t)B * n * 8)); CK(cudaMalloc(&b->key_z, (size_t)B * n * 8));
-        b->cap = B;
-    }
+    int st;
+    if ((st = b->synd_x.reserve((size_t)B * b->mx)) || (st = b->synd_z.reserve((size_t)B * b->mz)) ||
+        (st = b->bp_dec.reserve((size_t)B * 2 * n)) || (st = b->conv.reserve(B)) || (st = b->dec.reserve((size_t)B * 2 * n)) ||
+        (st = b->osd0.reserve((size_t)B * 2 * n)) || (st = b->tmp.reserve((size_t)B * n)) || (st = b->iters.reserve(B)) ||
+        (st = b->lpr.reserve((size_t)B * n * 3)) || (st = b->key_x.reserve((size_t)B * n)) || (st = b->key_z.reserve((size_t)B * n))) return st;
     return SWD_OK;
 }
 
 // host per-shot priors [5][B][n] -> b->d_llr5 on `s` (allocated on the first call that needs it, grown with B)
 static int bp4_stage_llr(swd_bp4 *b, const double *llr5, int64_t B, cudaStream_t s) {
-    if (B > b->llr5_cap) {
-        if (b->d_llr5) { cudaFree(b->d_llr5); b->d_llr5 = nullptr; b->llr5_cap = 0; }
-        if (cudaMalloc(&b->d_llr5, (size_t)40 * B * b->n) != cudaSuccess) { set_err("bp4 prior staging cudaMalloc failed"); return SWD_ERR_NOMEM; }
-        b->llr5_cap = B;
-    }
-    CK(cudaMemcpyAsync(b->d_llr5, llr5, (size_t)40 * B * b->n, cudaMemcpyHostToDevice, s));
+    if (int st = b->d_llr5.reserve((size_t)5 * B * b->n)) return st;
+    CK(cudaMemcpyAsync(b->d_llr5.p, llr5, (size_t)40 * B * b->n, cudaMemcpyHostToDevice, s));
     return SWD_OK;
 }
 
@@ -1598,16 +1555,16 @@ static int bp4_run(swd_bp4 *b, const u8 *d_sx, const u8 *d_sz, int64_t B, cudaSt
     const size_t P = (size_t)B * n;                                            // plane stride
     if (d_llr5)
         bp4_kernel<false, true><<<(int)std::min<long long>(B, b->grid_llr[0]), 256, b->S.total, s>>>(b->dx->g, b->dz->g, d_llr5, d_llr5 + P, d_llr5 + 2 * P,
-            d_sx, d_sz, B, b->max_iter, b->alpha, b->bp_dec, b->conv, b->iters, b->lpr, b->key_x, b->key_z, b->S, nullptr);
+            d_sx, d_sz, B, b->max_iter, b->alpha, b->bp_dec.p, b->conv.p, b->iters.p, b->lpr.p, b->key_x.p, b->key_z.p, b->S, nullptr);
     else
-        bp4_kernel<false><<<(int)std::min<long long>(B, b->grid), 256, b->S.total, s>>>(b->dx->g, b->dz->g, b->llr, b->llr + n, b->llr + 2 * n, d_sx, d_sz, B,
-                                                                                        b->max_iter, b->alpha, b->bp_dec, b->conv, b->iters, b->lpr, b->key_x, b->key_z, b->S, nullptr);
+        bp4_kernel<false><<<(int)std::min<long long>(B, b->grid), 256, b->S.total, s>>>(b->dx->g, b->dz->g, b->llr.p, b->llr.p + n, b->llr.p + 2 * n, d_sx, d_sz, B,
+                                                                                        b->max_iter, b->alpha, b->bp_dec.p, b->conv.p, b->iters.p, b->lpr.p, b->key_x.p, b->key_z.p, b->S, nullptr);
     CK(cudaGetLastError());
     int st;
-    if ((st = bp4_osd_pass(b->dx, d_sx, b->key_x, b->conv, B, b->tmp, s, d_llr5 ? d_llr5 + 3 * P : nullptr))) return st;      // osd('x') -> z part
-    if ((st = bp4_osd_pass(b->dz, d_sz, b->key_z, b->conv, B, b->tmp, s, d_llr5 ? d_llr5 + 4 * P : nullptr))) return st;      // osd('z') -> x part
+    if ((st = bp4_osd_pass(b->dx, d_sx, b->key_x.p, b->conv.p, B, b->tmp.p, s, d_llr5 ? d_llr5 + 3 * P : nullptr))) return st;      // osd('x') -> z part
+    if ((st = bp4_osd_pass(b->dz, d_sz, b->key_z.p, b->conv.p, B, b->tmp.p, s, d_llr5 ? d_llr5 + 4 * P : nullptr))) return st;      // osd('z') -> x part
     bp4_finish_kernel<<<(unsigned)std::min<long long>((B * 2 * (long long)n + 255) / 256, 8192), 256, 0, s>>>(
-        b->bp_dec, b->conv, b->dx->ow.osdw, b->dx->ow.osd0, b->dz->ow.osdw, b->dz->ow.osd0, B, (int)n, b->dec, b->osd0);
+        b->bp_dec.p, b->conv.p, b->dx->ow.osdw, b->dx->ow.osd0, b->dz->ow.osdw, b->dz->ow.osd0, B, (int)n, b->dec.p, b->osd0.p);
     CK(cudaGetLastError());
     return SWD_OK;
 }
@@ -1631,7 +1588,7 @@ static int bp4_stage_inputs(swd_bp4 *b, u8 *buf_x, u8 *buf_z, const u8 *&sx, con
     if (llr5) {
         int st = bp4_stage_llr(b, llr5, B, s);
         if (st) return st;
-        llr5 = b->d_llr5;
+        llr5 = b->d_llr5.p;
     }
     return SWD_OK;
 }
@@ -1656,10 +1613,10 @@ static int bp4_decode_impl(swd_bp4 *b, bool host, const uint8_t *synd_x, const u
     int st;
     if ((st = bp4_reserve(b, B))) return st;
     cudaStream_t s = host ? b->stream : (cudaStream_t)stream;
-    if (host && (st = bp4_stage_inputs(b, b->synd_x, b->synd_z, synd_x, synd_z, llr5, B, s))) return st;
+    if (host && (st = bp4_stage_inputs(b, b->synd_x.p, b->synd_z.p, synd_x, synd_z, llr5, B, s))) return st;
     if ((st = bp4_run(b, synd_x, synd_z, B, s, llr5))) return st;
-    return bp4_copy_out(host, s, {{dec, b->dec, (size_t)B * 2 * n}, {conv, b->conv, (size_t)B}, {bp_dec, b->bp_dec, (size_t)B * 2 * n},
-                                  {osd0, b->osd0, (size_t)B * 2 * n}, {lpr, b->lpr, (size_t)B * n * 24}, {bp_iteration, b->iters, (size_t)B * 4}});
+    return bp4_copy_out(host, s, {{dec, b->dec.p, (size_t)B * 2 * n}, {conv, b->conv.p, (size_t)B}, {bp_dec, b->bp_dec.p, (size_t)B * 2 * n},
+                                  {osd0, b->osd0.p, (size_t)B * 2 * n}, {lpr, b->lpr.p, (size_t)B * n * 24}, {bp_iteration, b->iters.p, (size_t)B * 4}});
 }
 
 extern "C" int swd_bp4_decode_batch_host(swd_bp4 *b, const uint8_t *synd_x, const uint8_t *synd_z, int64_t B, uint8_t *dec, uint8_t *conv,
@@ -1694,14 +1651,11 @@ extern "C" int swd_bp4_decode_batch_device_llr(swd_bp4 *b, const uint8_t *d_synd
 // lpr / bp_iteration: those of the last run (Y), as the reference's properties show after the call.
 static int bp4_camel_reserve(swd_bp4 *b, int64_t B) {
     const size_t n = b->n;
-    if (B > b->cap4) {
-        bp4_free_camel(b);
-        CK(cudaMalloc(&b->c_synd_x, (size_t)B * b->mx)); CK(cudaMalloc(&b->c_synd_z, (size_t)B * b->mz));
-        CK(cudaMalloc(&b->c_bp_dec, (size_t)B * 8 * n)); CK(cudaMalloc(&b->c_conv4, (size_t)B * 4)); CK(cudaMalloc(&b->c_dec, (size_t)B * 2 * n));
-        CK(cudaMalloc(&b->c_conv, (size_t)B)); CK(cudaMalloc(&b->c_it4, (size_t)B * 16)); CK(cudaMalloc(&b->c_it, (size_t)B * 4));
-        CK(cudaMalloc(&b->c_pm4, (size_t)B * 32)); CK(cudaMalloc(&b->c_pm, (size_t)B * 8)); CK(cudaMalloc(&b->c_lpr, (size_t)B * n * 24));
-        b->cap4 = B;
-    }
+    int st;
+    if ((st = b->c_synd_x.reserve((size_t)B * b->mx)) || (st = b->c_synd_z.reserve((size_t)B * b->mz)) ||
+        (st = b->c_bp_dec.reserve((size_t)B * 8 * n)) || (st = b->c_conv4.reserve((size_t)B * 4)) || (st = b->c_dec.reserve((size_t)B * 2 * n)) ||
+        (st = b->c_conv.reserve(B)) || (st = b->c_it4.reserve((size_t)B * 4)) || (st = b->c_it.reserve(B)) ||
+        (st = b->c_pm4.reserve((size_t)B * 4)) || (st = b->c_pm.reserve(B)) || (st = b->c_lpr.reserve((size_t)B * n * 3))) return st;
     return SWD_OK;
 }
 
@@ -1711,13 +1665,13 @@ static int bp4_camel_run(swd_bp4 *b, const u8 *d_sx, const u8 *d_sz, int64_t B, 
     const size_t P = (size_t)B * n;
     if (d_llr5)
         bp4_kernel<true, true><<<(int)std::min<long long>(4 * B, b->grid_llr[1]), 256, b->S.total, s>>>(b->dx->g, b->dz->g, d_llr5, d_llr5 + P, d_llr5 + 2 * P,
-            d_sx, d_sz, B, b->max_iter, b->alpha, b->c_bp_dec, b->c_conv4, b->c_it4, b->c_lpr, nullptr, nullptr, b->S, b->c_pm4);
+            d_sx, d_sz, B, b->max_iter, b->alpha, b->c_bp_dec.p, b->c_conv4.p, b->c_it4.p, b->c_lpr.p, nullptr, nullptr, b->S, b->c_pm4.p);
     else
-        bp4_kernel<true><<<(int)std::min<long long>(4 * B, b->grid), 256, b->S.total, s>>>(b->dx->g, b->dz->g, b->llr, b->llr + n, b->llr + 2 * n, d_sx, d_sz, B,
-                                                                                           b->max_iter, b->alpha, b->c_bp_dec, b->c_conv4, b->c_it4, b->c_lpr, nullptr, nullptr, b->S, b->c_pm4);
+        bp4_kernel<true><<<(int)std::min<long long>(4 * B, b->grid), 256, b->S.total, s>>>(b->dx->g, b->dz->g, b->llr.p, b->llr.p + n, b->llr.p + 2 * n, d_sx, d_sz, B,
+                                                                                           b->max_iter, b->alpha, b->c_bp_dec.p, b->c_conv4.p, b->c_it4.p, b->c_lpr.p, nullptr, nullptr, b->S, b->c_pm4.p);
     CK(cudaGetLastError());
-    bp4_camel_finish_kernel<<<(unsigned)std::min<long long>((B + 7) / 8, 4096), 256, 0, s>>>(b->c_bp_dec, b->c_conv4, b->c_pm4, b->c_it4, B, (int)n,
-                                                                                             b->c_dec, b->c_conv, b->c_pm, b->c_it);
+    bp4_camel_finish_kernel<<<(unsigned)std::min<long long>((B + 7) / 8, 4096), 256, 0, s>>>(b->c_bp_dec.p, b->c_conv4.p, b->c_pm4.p, b->c_it4.p, B, (int)n,
+                                                                                             b->c_dec.p, b->c_conv.p, b->c_pm.p, b->c_it.p);
     CK(cudaGetLastError());
     return SWD_OK;
 }
@@ -1731,10 +1685,10 @@ static int bp4_camel_impl(swd_bp4 *b, bool host, const uint8_t *synd_x, const ui
     int st;
     if ((st = bp4_camel_reserve(b, B))) return st;
     cudaStream_t s = host ? b->stream : (cudaStream_t)stream;
-    if (host && (st = bp4_stage_inputs(b, b->c_synd_x, b->c_synd_z, synd_x, synd_z, llr5, B, s))) return st;
+    if (host && (st = bp4_stage_inputs(b, b->c_synd_x.p, b->c_synd_z.p, synd_x, synd_z, llr5, B, s))) return st;
     if ((st = bp4_camel_run(b, synd_x, synd_z, B, s, llr5))) return st;
-    return bp4_copy_out(host, s, {{dec, b->c_dec, (size_t)B * 2 * n}, {conv, b->c_conv, (size_t)B}, {min_pm, b->c_pm, (size_t)B * 8},
-                                  {lpr, b->c_lpr, (size_t)B * n * 24}, {bp_iteration, b->c_it, (size_t)B * 4}});
+    return bp4_copy_out(host, s, {{dec, b->c_dec.p, (size_t)B * 2 * n}, {conv, b->c_conv.p, (size_t)B}, {min_pm, b->c_pm.p, (size_t)B * 8},
+                                  {lpr, b->c_lpr.p, (size_t)B * n * 24}, {bp_iteration, b->c_it.p, (size_t)B * 4}});
 }
 
 extern "C" int swd_bp4_camel_decode_batch_host(swd_bp4 *b, const uint8_t *synd_x, const uint8_t *synd_z, int64_t B, uint8_t *dec, uint8_t *conv,

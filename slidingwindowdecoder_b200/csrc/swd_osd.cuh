@@ -37,25 +37,6 @@ struct OsdWork {
 static inline size_t osd_bytes_per_shot(int m, int n) { return 2; }   // need_osd[cap] + in_list[cap]
 static inline void osd_bind(OsdWork *ow, unsigned char *base, long long cap, int m, int n) { ow->need_osd = base; }
 
-static inline int osd_reserve_outputs(OsdWork *ow, long long B, int n, cudaStream_t s) {
-    if (B <= ow->out_cap) return 0;
-    if (ow->bp_dec) { cudaFree(ow->bp_dec); cudaFree(ow->osd0); cudaFree(ow->osdw); cudaFree(ow->lpr); cudaFree(ow->bp_iter); ow->bp_dec = nullptr; }
-    if (cudaMalloc(&ow->bp_dec, (size_t)B * n) != cudaSuccess) return -4;
-    if (cudaMalloc(&ow->osd0, (size_t)B * n) != cudaSuccess) return -4;
-    if (cudaMalloc(&ow->osdw, (size_t)B * n) != cudaSuccess) return -4;
-    if (cudaMalloc(&ow->lpr, (size_t)B * n * 32) != cudaSuccess) return -4;
-    if (cudaMalloc(&ow->bp_iter, (size_t)B * 4) != cudaSuccess) return -4;
-    // zero-fill on the caller's stream: the kernels that write these buffers run there (a legacy-stream memset would not be
-    // ordered against a non-blocking stream)
-    cudaMemsetAsync(ow->osd0, 0, (size_t)B * n, s); cudaMemsetAsync(ow->osdw, 0, (size_t)B * n, s); cudaMemsetAsync(ow->bp_dec, 0, (size_t)B * n, s);
-    ow->out_cap = B;
-    return 0;
-}
-static inline void osd_free_outputs(OsdWork *ow) {
-    if (ow->big_scratch) { cudaFree(ow->big_scratch); ow->big_scratch = nullptr; }
-    if (ow->bp_dec) { cudaFree(ow->bp_dec); cudaFree(ow->osd0); cudaFree(ow->osdw); cudaFree(ow->lpr); cudaFree(ow->bp_iter); ow->bp_dec = nullptr; }
-}
-
 // ----------------------------------------------------------------------------------------------
 // post-BP on the shortened graph (osd_window.pyx:187-192): one CTA per non-converged shot
 // ----------------------------------------------------------------------------------------------
